@@ -15,6 +15,9 @@ on a synthetic 100 M-row x 8-column (4 f64 + 4 i64) table with 5 % nulls per col
                all host cores, on a bounded row sample (rank 0, N=1 only)
     --impl reference   times that CPU restatement alone (the reference itself is Rust + DataFusion and
                cannot be built in this image: no cargo/rustc; see DESIGN.md)
+    --dump-outputs DIR   after the timed steps, writes the suite's results of the last step (rank 0) as
+               DIR/metric.npy and DIR/status.npy (float64, one entry per constraint in suite order), so that two
+               builds run with the same arguments (hence the same seeded inputs) can be compared output for output
 """
 import argparse
 import json
@@ -401,6 +404,15 @@ def check_gpu_against_cpu(gpu_results, cpu):
     return "GPU results equal the CPU arm's on the same host table (size / min / predicate ratio exact, mean 1e-9, correlation 1e-6)"
 
 
+def dump_outputs(results, out_dir):
+    """the ConstraintResults a caller of the timed plan receives, as arrays: metric (NaN when a result has none) and
+    status (ConstraintStatus value: 0 Success, 1 Failure, 2 Skipped), in suite order"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "metric.npy"), np.array([np.nan if r.metric is None else r.metric for r in results], dtype=np.float64))
+    np.save(os.path.join(out_dir, "status.npy"), np.array([r.status.value for r in results], dtype=np.float64))
+
+
 # ------------------------------------------------------------------------------ GPU arm ----
 def main():
     ap = argparse.ArgumentParser()
@@ -412,7 +424,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--variants", action="store_true", help="(kept for old scripts: the full numeric set is one of the suites now)")
     ap.add_argument("--suites", default="all", help="'all', 'none' or a comma list of c1,c2full,c3,c4,c5,mixed")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/metric.npy and DIR/status.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path computed; it does not apply to --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
 
     if args.impl == "reference":
@@ -501,6 +518,8 @@ def main():
     value = n * world * args.steps / (total_ms / 1e3)
 
     results = [plan.result(s) for _, _, s in slots]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(results, args.dump_outputs)
     kernel_ms = sum(scan_ms) / len(scan_ms)
     alg_bytes = algorithmic_bytes(n)
     peak, peak_src = measured_peak_gbs()
