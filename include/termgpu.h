@@ -364,7 +364,15 @@ TG_API tg_status tg_table_shuffle_fingerprints(tg_engine* eng, const char* table
                                                const char* shard_table, int64_t* n_rows);
 
 /* Arrow C Data Interface ingestion: `schema`/`array` are struct ArrowSchema* / struct ArrowArray* of a
- * struct-typed array (a RecordBatch). The engine copies; the caller keeps ownership and releases. */
+ * struct-typed array (a RecordBatch). The engine copies; the caller keeps ownership and releases.
+ * String encodings: Utf8 ("u"), LargeUtf8 ("U"), Utf8View ("vu") and dictionaries with any integer index type ("c" .. "L")
+ * over Utf8 / LargeUtf8 values are all stored as one Utf8 column of the logical values (batches of a column may mix them,
+ * each with its own dictionary; array offsets on the column and on the dictionary are honoured). Views and dictionaries
+ * cross PCIe encoded and are decoded on the device. A row is NULL when its validity bit is clear or its index names a
+ * NULL dictionary value; indices and views under NULL rows are never read. Errors: TG_ERR_INVALID_ARG for a valid row whose
+ * index lies outside the dictionary (any valid row of an empty one) or whose view lies outside its data buffer;
+ * TG_ERR_UNSUPPORTED for a string of 16 MiB or more, for BinaryView ("vz") and for dictionaries of any other value type
+ * (Binary, Utf8View, numeric, temporal, Boolean). Columns before the failing one may already hold the batch's rows. */
 TG_API tg_status tg_table_append_arrow(tg_table* t, const void* arrow_schema, const void* arrow_array);
 
 /* ------------------------------------------------------------------ plan ---- */

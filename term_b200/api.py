@@ -336,8 +336,9 @@ class SessionContext:
                 F.check(F.lib().tg_table_append_host(t, col_name.encode(), F.TG_BOOL, n, vals, None, validity, off))
             else:
                 # Int8 .. UInt64, Date / Time / Timestamp / Duration, LargeUtf8: the Arrow C Data Interface entry point widens /
-                # narrows them on the host and records the delivered type (DataFusion types MIN / MAX / SUM after it);
-                # anything it does not know either (decimals, nested types, ..) raises TG_ERR_UNSUPPORTED
+                # narrows them on the host and records the delivered type (DataFusion types MIN / MAX / SUM after it); string
+                # dictionaries and string_view arrays (sliced ones too) are decoded to Utf8 on the device; anything it does not
+                # know either (decimals, nested types, binary views, non-string dictionaries, ..) raises TG_ERR_UNSUPPORTED
                 self._append_batch_c(t, pa.record_batch([arr], names=[col_name]))
 
     def _append_batch_c(self, t, batch):
@@ -1082,10 +1083,13 @@ def arrow_type_debug(t) -> str:
     """`{:?}` of the arrow-rs DataType a pyarrow type corresponds to (what DataTypeConstraint::specific_type compares with)"""
     simple = {"int8": "Int8", "int16": "Int16", "int32": "Int32", "int64": "Int64", "uint8": "UInt8", "uint16": "UInt16", "uint32": "UInt32",
               "uint64": "UInt64", "float": "Float32", "double": "Float64", "halffloat": "Float16", "bool": "Boolean", "string": "Utf8",
-              "large_string": "LargeUtf8", "binary": "Binary", "large_binary": "LargeBinary", "date32[day]": "Date32", "date64[ms]": "Date64", "null": "Null"}
+              "large_string": "LargeUtf8", "binary": "Binary", "large_binary": "LargeBinary", "date32[day]": "Date32", "date64[ms]": "Date64", "null": "Null",
+              "string_view": "Utf8View", "binary_view": "BinaryView"}
     k = str(t)
     if k in simple:
         return simple[k]
+    if pa.types.is_dictionary(t):
+        return f"Dictionary({arrow_type_debug(t.index_type)}, {arrow_type_debug(t.value_type)})"
     units = {"s": "Second", "ms": "Millisecond", "us": "Microsecond", "ns": "Nanosecond"}
     if pa.types.is_timestamp(t):
         return f"Timestamp({units[t.unit]}, " + ("None" if t.tz is None else f'Some("{t.tz}")') + ")"

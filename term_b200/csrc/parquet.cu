@@ -29,6 +29,7 @@
 #include <thread>
 
 #include "engine.hpp"
+#include "str_entries.cuh"
 
 namespace tg {
 
@@ -493,16 +494,6 @@ size_t page_decompress(int32_t codec, const uint8_t* src, size_t n, uint8_t* dst
     }
     throw Error(TG_ERR_UNSUPPORTED, "Parquet: codec " + std::to_string(codec));
 }
-
-struct PqBlock {
-    uint64_t src_off;     // PLAIN: byte offset in the staging buffer of the block's first non-NULL value
-    uint32_t first_row;   // chunk-relative
-    uint32_t n_rows;      // <= PQ_BLOCK_ROWS
-    uint32_t first_dense; // dictionary: dense index (inside the block's section) of the block's first non-NULL value
-    uint32_t run_lo, run_hi;  // dictionary: the section's runs [run_lo, run_hi) in the run table; run_hi == 0: a PLAIN block
-    uint32_t pad;
-};
-constexpr int PQ_BLOCK_ROWS = 1024, PQ_THREADS = 256;
 
 }  // namespace
 
@@ -1046,10 +1037,7 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
 // pages (one entry {staging offset, length} per value); the dictionary page's own entries likewise (it is small).
 // ---------------------------------------------------------------------------------------------------------------------
 namespace {
-// {byte offset in the staging buffer : 40 bits | length : 24 bits}; strings of 16 MiB or more are refused
-inline uint64_t pq_str_ent(uint64_t off, uint32_t len) { return off | ((uint64_t)len << 40); }
-constexpr uint32_t PQ_STR_MAX_LEN = (1u << 24) - 1u;
-
+// entries: pq_str_ent / PQ_STR_MAX_LEN (str_entries.cuh)
 // walks `count` PLAIN BYTE_ARRAY values at p (length prefixes interleaved) into entries; stage_off = where p sits in staging
 void walk_plain_strings(const uint8_t* p, int64_t n_bytes, int64_t count, uint64_t stage_off, std::vector<uint64_t>& ents) {
     int64_t pos = 0;
@@ -1199,7 +1187,7 @@ static void append_parquet_utf8(Table& t, const std::string& name, int32_t max_d
     const size_t dict_off = stage_bytes;
     stage_bytes += ((size_t)pc.dict_bytes + 15) & ~(size_t)15;
     stage_bytes += 64;
-    if (stage_bytes >= ((size_t)1 << 40)) throw Error(TG_ERR_UNSUPPORTED, "Parquet: column chunk of 1 TiB or more");
+    if (stage_bytes >= PQ_STAGE_MAX) throw Error(TG_ERR_UNSUPPORTED, "Parquet: column chunk of 1 TiB or more");
     std::vector<uint8_t> bits;
     std::vector<PqBlock> blocks;
     std::vector<PqRun> runs;
@@ -1288,25 +1276,45 @@ static void append_parquet_utf8(Table& t, const std::string& name, int32_t max_d
     unsigned long long* d_tot = (unsigned long long*)q;
     q += bb_b;
     unsigned long long* d_base = (unsigned long long*)q;
-    const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((nb + PQ_THREADS / 32 - 1) / (PQ_THREADS / 32), (int64_t)e.sm_count * 8));
+    const int grid = pq_str_grid(e, nb);
     pq_str_locate_kernel<<<grid, PQ_THREADS, 0, e.copy_stream>>>(stage, d_bits, d_blocks, nb, d_runs, d_pe, d_de, (uint32_t)pc.dict_count, d_row, d_tot);
-    pq_block_scan_kernel<<<1, 1024, 0, e.copy_stream>>>(d_tot, nb, d_base);
     TG_CUDA(cudaGetLastError());
+    e.launches += 1;
+    Utf8Entries x;
+    x.stage = stage;
+    x.blocks = d_blocks;
+    x.n_blocks = nb;
+    x.row_ent = d_row;
+    x.block_bytes = d_tot;
+    x.block_base = d_base;
+    append_utf8_from_entries(e, t, c, x, num_values);
+}
+
+uint32_t append_utf8_from_entries(Engine& e, Table& t, Column& c, const Utf8Entries& x, int64_t num_values) {
+    const int64_t have = c.n_rows, nb = x.n_blocks;
+    const int grid = pq_str_grid(e, nb);
+    pq_block_scan_kernel<<<1, 1024, 0, e.copy_stream>>>(x.block_bytes, nb, x.block_base);
+    TG_CUDA(cudaGetLastError());
+    e.launches += 1;
     unsigned long long total = 0;
-    TG_CUDA(cudaMemcpyAsync(&total, d_base + nb, 8, cudaMemcpyDeviceToHost, e.copy_stream));
+    uint32_t err = 0;
+    TG_CUDA(cudaMemcpyAsync(&total, x.block_base + nb, 8, cudaMemcpyDeviceToHost, e.copy_stream));
+    if (x.err) TG_CUDA(cudaMemcpyAsync(&err, x.err, 4, cudaMemcpyDeviceToHost, e.copy_stream));
     TG_CUDA(cudaStreamSynchronize(e.copy_stream));  // the byte total decides the value buffer's size
+    if (err) return err;
     if ((unsigned long long)c.value_bytes + total > (unsigned long long)INT32_MAX)
         throw Error(TG_ERR_UNSUPPORTED, "Utf8 column exceeds 2 GiB of value bytes (32-bit offsets)");
     e.dev_reserve(c.values, (size_t)(c.value_bytes + (int64_t)total), (size_t)c.value_bytes);
     e.dev_reserve(c.offsets, (size_t)(have + num_values + 1) * 4, have ? (size_t)(have + 1) * 4 : 0);
-    pq_str_write_kernel<<<grid, PQ_THREADS, 0, e.copy_stream>>>(stage, d_blocks, nb, d_row, d_base, reinterpret_cast<int32_t*>(c.offsets.p) + have, c.values.p,
-                                                               c.value_bytes, num_values);
+    pq_str_write_kernel<<<grid, PQ_THREADS, 0, e.copy_stream>>>(x.stage, x.blocks, nb, x.row_ent, x.block_base,
+                                                               reinterpret_cast<int32_t*>(c.offsets.p) + have, c.values.p, c.value_bytes, num_values);
     TG_CUDA(cudaGetLastError());
-    e.launches += 3;
+    e.launches += 1;
     c.value_bytes += (int64_t)total;
     c.last_offset = (int32_t)c.value_bytes;
     c.n_rows = have + num_values;
     t.n_rows = std::max(t.n_rows, c.n_rows);
+    return 0;
 }
 
 // host-only (tests): one page's value section of a DELTA_* / BYTE_STREAM_SPLIT encoding rewritten to the PLAIN layout

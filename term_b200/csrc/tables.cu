@@ -5,6 +5,7 @@
 #include <cstring>
 
 #include "engine.hpp"
+#include "str_entries.cuh"
 
 namespace tg {
 
@@ -310,6 +311,311 @@ void table_set_column_arrow_type(Table& t, const std::string& name, const std::s
     c->temporal_unit = f.temporal_unit;
 }
 
+// ---- string dictionaries and Utf8View -> Utf8, decoded on the device ----
+// A column delivered as dictionary<int*, utf8 | large_utf8> or as utf8_view is stored as the plain Utf8 column of its
+// LOGICAL values (what DataFusion's string functions, comparisons, COUNT(DISTINCT) and GROUP BY see). What crosses PCIe is
+// the encoded form: the dictionary's bytes and the rows' indices, or the views and their data buffers. A locate kernel
+// turns every row into an entry {staging offset, length} (str_entries.cuh) and the Parquet BYTE_ARRAY tail writes the
+// offsets and bytes. A row is NULL when its validity bit is clear or its index names a NULL dictionary value (Arrow's
+// logical NULL); the index or view under a NULL row is never read. Malformed input (an index outside the dictionary, a
+// view outside its data buffer) raises a flag and is clamped before any load: an error, never an out-of-bounds access.
+
+__device__ __forceinline__ bool arrow_row_valid(const uint8_t* __restrict__ bits, uint64_t bit) {
+    return !bits || ((__ldg(bits + (bit >> 3)) >> (bit & 7)) & 1);
+}
+
+// one warp per block: each valid row's index -> the dictionary value's entry; NULL rows get length 0
+template <typename IndexT>
+__global__ void __launch_bounds__(PQ_THREADS) arrow_dict_locate_kernel(const IndexT* __restrict__ idx, const uint8_t* __restrict__ bits, uint32_t bit_shift,
+                                                                      const PqBlock* __restrict__ blocks, int64_t n_blocks,
+                                                                      const uint64_t* __restrict__ dict_ents, uint64_t dict_count,
+                                                                      uint64_t* __restrict__ row_ent, unsigned long long* __restrict__ block_bytes,
+                                                                      uint32_t* __restrict__ err) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warps = (int64_t)gridDim.x * (PQ_THREADS / 32);
+    for (int64_t b = (int64_t)blockIdx.x * (PQ_THREADS / 32) + (threadIdx.x >> 5); b < n_blocks; b += warps) {
+        const PqBlock blk = blocks[b];
+        unsigned long long total = 0;
+        bool bad = false;
+        for (uint32_t i = lane; i < blk.n_rows; i += 32) {
+            const uint64_t r = (uint64_t)blk.first_row + i;
+            uint64_t ent = 0;
+            if (arrow_row_valid(bits, r + bit_shift)) {
+                const int64_t v = (int64_t)__ldg(idx + r);  // (a UInt64 index of 2^63 or more reads as negative: out of range too)
+                if (v < 0 || (uint64_t)v >= dict_count) bad = true;
+                else ent = __ldg(dict_ents + v);
+            }
+            row_ent[r] = ent;
+            total += ent >> 40;
+        }
+#pragma unroll
+        for (int m = 16; m > 0; m >>= 1) total += __shfl_xor_sync(0xffffffffu, total, m);
+        if (lane == 0) block_bytes[b] = total;
+        if (bad) atomicOr(err, STR_ERR_RANGE);
+    }
+}
+
+// one warp per block: each valid row's 16-byte view -> the entry of its bytes: inline (length <= 12, the bytes sit in the
+// staged view itself at +4) or in data buffer `buf` at `offset` (the buffer's staging offset from buf_base, bounds from
+// buf_size); NULL rows get length 0
+__global__ void __launch_bounds__(PQ_THREADS) arrow_view_locate_kernel(const uint4* __restrict__ views /* at staging offset 0 */, const uint8_t* __restrict__ bits,
+                                                                      uint32_t bit_shift, const PqBlock* __restrict__ blocks, int64_t n_blocks,
+                                                                      const uint64_t* __restrict__ buf_base, const uint64_t* __restrict__ buf_size,
+                                                                      uint32_t n_bufs, uint64_t* __restrict__ row_ent,
+                                                                      unsigned long long* __restrict__ block_bytes, uint32_t* __restrict__ err) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warps = (int64_t)gridDim.x * (PQ_THREADS / 32);
+    for (int64_t b = (int64_t)blockIdx.x * (PQ_THREADS / 32) + (threadIdx.x >> 5); b < n_blocks; b += warps) {
+        const PqBlock blk = blocks[b];
+        unsigned long long total = 0;
+        uint32_t flags = 0;
+        for (uint32_t i = lane; i < blk.n_rows; i += 32) {
+            const uint64_t r = (uint64_t)blk.first_row + i;
+            uint64_t ent = 0;
+            if (arrow_row_valid(bits, r + bit_shift)) {
+                const uint4 v = __ldg(views + r);
+                const int32_t len = (int32_t)v.x;
+                if (len < 0) {
+                    flags |= STR_ERR_RANGE;
+                } else if ((uint32_t)len > PQ_STR_MAX_LEN) {
+                    flags |= STR_ERR_LONG;
+                } else if (len <= 12) {
+                    ent = pq_str_ent(r * 16 + 4, (uint32_t)len);
+                } else if (v.z >= n_bufs || (uint64_t)v.w + (uint32_t)len > __ldg(buf_size + v.z)) {
+                    flags |= STR_ERR_RANGE;  // (buffer index and offset are unsigned here: a negative Int32 is out of range too)
+                } else {
+                    ent = pq_str_ent(__ldg(buf_base + v.z) + v.w, (uint32_t)len);
+                }
+            }
+            row_ent[r] = ent;
+            total += ent >> 40;
+        }
+#pragma unroll
+        for (int m = 16; m > 0; m >>= 1) total += __shfl_xor_sync(0xffffffffu, total, m);
+        if (lane == 0) block_bytes[b] = total;
+        if (flags) atomicOr(err, flags);
+    }
+}
+
+namespace {
+
+// One staging block per append: [payload | validity bits | blocks | tables | row entries | block totals | bases | flag].
+// The caller fills payload and tables; the rest is laid out and uploaded here.
+struct ArrowStage {
+    uint8_t* p = nullptr;              // the block; the payload starts at p
+    const uint8_t* bits = nullptr;     // staged validity (nullptr: no NULLs)
+    uint8_t* tables = nullptr;         // the caller's lookup tables
+    Utf8Entries x;
+};
+
+size_t r16(size_t x) { return (x + 15) & ~(size_t)15; }
+
+// validity: `bits` read from bit `bit_off` (nullptr: no NULLs); staged from its byte bit_off / 8 on
+ArrowStage arrow_stage(Engine& e, size_t payload_b, size_t tables_b, int64_t n, const uint8_t* bits, int64_t bit_off, uint32_t* bit_shift) {
+    ArrowStage s;
+    const int64_t nb = (n + PQ_BLOCK_ROWS - 1) / PQ_BLOCK_ROWS;
+    const size_t bits_n = bits ? (size_t)((bit_off & 7) + n + 7) / 8 : 0;
+    const size_t pay_b = r16(payload_b), bits_b = r16(bits_n), blk_b = r16((size_t)nb * sizeof(PqBlock)), tab_b = r16(tables_b);
+    const size_t re_b = r16((size_t)n * 8), bb_b = r16((size_t)(nb + 1) * 8);
+    const size_t total = pay_b + bits_b + blk_b + tab_b + re_b + 2 * bb_b + 16 + 64;
+    if (pay_b >= PQ_STAGE_MAX) throw Error(TG_ERR_UNSUPPORTED, "Arrow string batch of 1 TiB or more");
+    s.p = e.dev_alloc(total);
+    e.deferred_free.emplace_back(s.p, total);
+    uint8_t* q = s.p + pay_b;
+    if (bits) {
+        e.h2d(q, bits + bit_off / 8, bits_n);
+        s.bits = q;
+    }
+    *bit_shift = (uint32_t)(bits ? bit_off & 7 : 0);
+    q += bits_b;
+    std::vector<PqBlock> blocks((size_t)nb);
+    for (int64_t b = 0; b < nb; ++b)
+        blocks[(size_t)b] = PqBlock{0, (uint32_t)(b * PQ_BLOCK_ROWS), (uint32_t)std::min<int64_t>(PQ_BLOCK_ROWS, n - b * PQ_BLOCK_ROWS), 0u, 0u, 0u, 0u};
+    e.h2d(q, blocks.data(), blocks.size() * sizeof(PqBlock));
+    s.x.blocks = (const PqBlock*)q;
+    s.x.n_blocks = nb;
+    q += blk_b;
+    s.tables = q;
+    q += tab_b;
+    s.x.row_ent = (const uint64_t*)q;
+    q += re_b;
+    s.x.block_bytes = (unsigned long long*)q;
+    q += bb_b;
+    s.x.block_base = (unsigned long long*)q;
+    q += bb_b;
+    s.x.err = (const uint32_t*)q;
+    TG_CUDA(cudaMemsetAsync(q, 0, 4, e.copy_stream));
+    s.x.stage = s.p;
+    return s;
+}
+
+Column& arrow_utf8_column(Table& t, const char* name) {
+    Column& c = *table_get_or_add(t, name, TG_UTF8);
+    if (c.adopted) throw Error(TG_ERR_INVALID_ARG, "cannot append to an adopted device column");
+    return c;
+}
+
+// the shared tail; a flag raised by the locate kernel becomes the error (and nothing was appended)
+void arrow_utf8_finish(Engine& e, Table& t, Column& c, const ArrowStage& s, int64_t n, const std::string& range_msg, const char* name) {
+    const uint32_t err = append_utf8_from_entries(e, t, c, s.x, n);
+    if (err & STR_ERR_RANGE) throw Error(TG_ERR_INVALID_ARG, std::string("column '") + name + "': " + range_msg);
+    if (err & STR_ERR_LONG) throw Error(TG_ERR_UNSUPPORTED, std::string("column '") + name + "': string value of 16 MiB or more");
+}
+
+}  // namespace
+
+// dictionary<index fmt, utf8 | large_utf8>: `dict` is the dictionary child (its own offset and validity)
+static void append_arrow_dict_utf8(Table& t, const char* name, char index_fmt, bool large_values, const ArrowArray* ca, const ArrowArray* dict) {
+    Engine& e = *t.eng;
+    std::lock_guard<std::mutex> g(e.mu);
+    TG_CUDA(cudaSetDevice(e.device));
+    Column& c = arrow_utf8_column(t, name);
+    const int64_t n = ca->length, off = ca->offset;
+    if (n == 0) {
+        t.n_rows = std::max(t.n_rows, c.n_rows);
+        return;
+    }
+    if (n >= ((int64_t)1 << 31)) throw Error(TG_ERR_UNSUPPORTED, std::string("column '") + name + "': a batch of 2^31 rows or more");
+    const int iw = index_fmt == 'c' || index_fmt == 'C' ? 1 : index_fmt == 's' || index_fmt == 'S' ? 2 : index_fmt == 'i' || index_fmt == 'I' ? 4 : 8;
+    const bool idx_signed = index_fmt == 'c' || index_fmt == 's' || index_fmt == 'i' || index_fmt == 'l';
+    const uint8_t* validity = ca->null_count == 0 ? nullptr : (const uint8_t*)ca->buffers[0];
+    const uint8_t* idx = (const uint8_t*)ca->buffers[1] + off * iw;
+    // ---- the dictionary's entries (host: it is small next to the rows), relative to the dictionary bytes' first byte
+    const int64_t dn = dict->length, doff = dict->offset;
+    std::vector<uint64_t> ents((size_t)dn);
+    std::vector<uint8_t> dict_valid;
+    int64_t d0 = 0, d1 = 0;
+    if (dn > 0) {
+        auto o = [&](int64_t k) -> int64_t {
+            return large_values ? ((const int64_t*)dict->buffers[1])[doff + k] : (int64_t)((const int32_t*)dict->buffers[1])[doff + k];
+        };
+        d0 = o(0);
+        d1 = o(dn);
+        if (d1 < d0) throw Error(TG_ERR_INVALID_ARG, std::string("dictionary of column '") + name + "': offsets are not monotonic");
+        const uint8_t* dbits = dict->null_count == 0 ? nullptr : (const uint8_t*)dict->buffers[0];
+        dict_valid.assign((size_t)dn, 1);
+        bool dict_nulls = false;
+        for (int64_t k = 0; k < dn; ++k) {
+            const int64_t a = o(k), b = o(k + 1);
+            if (a < d0 || b < a || b > d1) throw Error(TG_ERR_INVALID_ARG, std::string("dictionary of column '") + name + "': offsets are not monotonic");
+            if (b - a > (int64_t)PQ_STR_MAX_LEN) throw Error(TG_ERR_UNSUPPORTED, std::string("dictionary of column '") + name + "': string value of 16 MiB or more");
+            const bool ok = !dbits || ((dbits[(doff + k) >> 3] >> ((doff + k) & 7)) & 1);
+            dict_valid[(size_t)k] = ok;
+            dict_nulls |= !ok;
+            ents[(size_t)k] = ok ? pq_str_ent((uint64_t)(a - d0), (uint32_t)(b - a)) : 0;
+        }
+        if (!dict_nulls) dict_valid.clear();
+    }
+    // ---- a NULL dictionary value makes the rows naming it NULL: the rows' bitmap AND "index -> value valid", on the host
+    std::vector<uint8_t> combined;
+    int64_t bit_off = off;
+    if (!dict_valid.empty()) {
+        combined.assign((size_t)(n + 7) / 8, 0);
+        for (int64_t r = 0; r < n; ++r) {
+            if (validity && !((validity[(off + r) >> 3] >> ((off + r) & 7)) & 1)) continue;
+            int64_t v;
+            switch (iw) {
+                case 1: v = idx_signed ? (int64_t)((const int8_t*)idx)[r] : (int64_t)idx[r]; break;
+                case 2: v = idx_signed ? (int64_t)((const int16_t*)idx)[r] : (int64_t)((const uint16_t*)idx)[r]; break;
+                case 4: v = idx_signed ? (int64_t)((const int32_t*)idx)[r] : (int64_t)((const uint32_t*)idx)[r]; break;
+                default: v = ((const int64_t*)idx)[r]; break;
+            }
+            if (v < 0 || v >= dn) throw Error(TG_ERR_INVALID_ARG, std::string("dictionary column '") + name + "': an index lies outside the dictionary");
+            if (dict_valid[(size_t)v]) combined[(size_t)(r >> 3)] |= (uint8_t)(1u << (r & 7));
+        }
+        validity = combined.data();
+        bit_off = 0;
+    }
+    // ---- staging: dictionary bytes | indices | (validity, blocks, entries, ..)
+    const size_t dict_b = r16((size_t)(d1 - d0)), idx_b = (size_t)n * iw;
+    uint32_t bit_shift = 0;
+    ArrowStage s = arrow_stage(e, dict_b + idx_b, (size_t)dn * 8, n, validity, bit_off, &bit_shift);
+    if (d1 > d0) e.h2d(s.p, (const uint8_t*)dict->buffers[2] + d0, (size_t)(d1 - d0));
+    e.h2d(s.p + dict_b, idx, idx_b);
+    if (dn > 0) e.h2d(s.tables, ents.data(), (size_t)dn * 8);
+    const uint64_t* d_ents = (const uint64_t*)s.tables;
+    uint64_t* row = const_cast<uint64_t*>(s.x.row_ent);
+    uint32_t* err = const_cast<uint32_t*>(s.x.err);
+    const int grid = pq_str_grid(e, s.x.n_blocks);
+    const uint8_t* d_idx = s.p + dict_b;
+#define TG_DICT_LOCATE(T)                                                                                                           \
+    arrow_dict_locate_kernel<T><<<grid, PQ_THREADS, 0, e.copy_stream>>>((const T*)d_idx, s.bits, bit_shift, s.x.blocks, s.x.n_blocks, d_ents, \
+                                                                         (uint64_t)dn, row, s.x.block_bytes, err)
+    switch (index_fmt) {
+        case 'c': TG_DICT_LOCATE(int8_t); break;
+        case 'C': TG_DICT_LOCATE(uint8_t); break;
+        case 's': TG_DICT_LOCATE(int16_t); break;
+        case 'S': TG_DICT_LOCATE(uint16_t); break;
+        case 'i': TG_DICT_LOCATE(int32_t); break;
+        case 'I': TG_DICT_LOCATE(uint32_t); break;
+        case 'l': TG_DICT_LOCATE(int64_t); break;
+        default: TG_DICT_LOCATE(uint64_t); break;
+    }
+#undef TG_DICT_LOCATE
+    TG_CUDA(cudaGetLastError());
+    e.launches += 1;
+    const int64_t have = c.n_rows;
+    arrow_utf8_finish(e, t, c, s, n, "a dictionary index lies outside the dictionary", name);
+    append_validity(e, c, have, validity, bit_off, n);
+}
+
+// utf8_view: buffers = validity, views, data buffers.., variadic buffer sizes (int64 per data buffer)
+static void append_arrow_view_utf8(Table& t, const char* name, const ArrowArray* ca) {
+    Engine& e = *t.eng;
+    std::lock_guard<std::mutex> g(e.mu);
+    TG_CUDA(cudaSetDevice(e.device));
+    Column& c = arrow_utf8_column(t, name);
+    const int64_t n = ca->length, off = ca->offset;
+    if (n == 0) {
+        t.n_rows = std::max(t.n_rows, c.n_rows);
+        return;
+    }
+    if (n >= ((int64_t)1 << 31)) throw Error(TG_ERR_UNSUPPORTED, std::string("column '") + name + "': a batch of 2^31 rows or more");
+    if (ca->n_buffers < 3) throw Error(TG_ERR_INVALID_ARG, std::string("Utf8View column '") + name + "': expected a variadic buffer-sizes buffer");
+    const int64_t n_data = ca->n_buffers - 3;
+    if (n_data >= ((int64_t)1 << 32)) throw Error(TG_ERR_INVALID_ARG, std::string("Utf8View column '") + name + "': too many data buffers");
+    const int64_t* sizes = (const int64_t*)ca->buffers[ca->n_buffers - 1];
+    const uint8_t* validity = ca->null_count == 0 ? nullptr : (const uint8_t*)ca->buffers[0];
+    // ---- staging: views | data buffers (16-byte aligned) | (validity, blocks, buffer bases + sizes, ..)
+    const size_t views_b = r16((size_t)n * 16);
+    std::vector<uint64_t> tab((size_t)n_data * 2);  // [base.. | size..]
+    size_t pos = views_b;
+    for (int64_t k = 0; k < n_data; ++k) {
+        const int64_t sz = sizes ? sizes[k] : 0;
+        if (sz < 0) throw Error(TG_ERR_INVALID_ARG, std::string("Utf8View column '") + name + "': negative data buffer size");
+        tab[(size_t)k] = pos;
+        tab[(size_t)(n_data + k)] = (uint64_t)sz;
+        pos += r16((size_t)sz);
+    }
+    uint32_t bit_shift = 0;
+    ArrowStage s = arrow_stage(e, pos, tab.size() * 8, n, validity, off, &bit_shift);
+    e.h2d(s.p, (const uint8_t*)ca->buffers[1] + off * 16, (size_t)n * 16);
+    for (int64_t k = 0; k < n_data; ++k)
+        if (tab[(size_t)(n_data + k)]) e.h2d(s.p + tab[(size_t)k], ca->buffers[2 + k], (size_t)tab[(size_t)(n_data + k)]);
+    if (!tab.empty()) e.h2d(s.tables, tab.data(), tab.size() * 8);
+    const uint64_t* d_tab = (const uint64_t*)s.tables;
+    arrow_view_locate_kernel<<<pq_str_grid(e, s.x.n_blocks), PQ_THREADS, 0, e.copy_stream>>>(
+        (const uint4*)s.p, s.bits, bit_shift, s.x.blocks, s.x.n_blocks, d_tab, d_tab + n_data, (uint32_t)n_data,
+        const_cast<uint64_t*>(s.x.row_ent), s.x.block_bytes, const_cast<uint32_t*>(s.x.err));
+    TG_CUDA(cudaGetLastError());
+    e.launches += 1;
+    const int64_t have = c.n_rows;
+    arrow_utf8_finish(e, t, c, s, n, "a Utf8View view lies outside its data buffer", name);
+    append_validity(e, c, have, validity, off, n);
+}
+
+// the Arrow type of a dictionary's values as arrow-rs names it (for the refusal message)
+static std::string arrow_type_name(const char* fmt) {
+    static const char* const names[][2] = {{"z", "Binary"}, {"Z", "LargeBinary"}, {"vz", "BinaryView"}, {"vu", "Utf8View"}, {"b", "Boolean"},
+                                           {"c", "Int8"}, {"C", "UInt8"}, {"s", "Int16"}, {"S", "UInt16"}, {"i", "Int32"}, {"I", "UInt32"},
+                                           {"l", "Int64"}, {"L", "UInt64"}, {"e", "Float16"}, {"f", "Float32"}, {"g", "Float64"},
+                                           {"u", "Utf8"}, {"U", "LargeUtf8"}, {"tdD", "Date32"}, {"tdm", "Date64"}};
+    const std::string f = fmt ? fmt : "";
+    for (const auto& n : names)
+        if (f == n[0]) return n[1];
+    return "Arrow format '" + f + "'";
+}
+
 void table_append_arrow(Table& t, const void* schema_p, const void* array_p) {
     const ArrowSchema* sc = (const ArrowSchema*)schema_p;
     const ArrowArray* ar = (const ArrowArray*)array_p;
@@ -320,6 +626,23 @@ void table_append_arrow(Table& t, const void* schema_p, const void* array_p) {
         const ArrowSchema* cs = sc->children[i];
         const ArrowArray* ca = ar->children[i];
         const std::string fmt = cs->format;
+        if (cs->dictionary) {
+            // dictionary<integer, utf8 | large_utf8>: decoded to the Utf8 column of the logical values; other value types are
+            // refused (DataFusion's typing of MIN / MAX / SUM over numeric / temporal / Boolean dictionaries is not pinned)
+            const char* vf = cs->dictionary->format;
+            const bool int_index = fmt.size() == 1 && strchr("cCsSiIlL", fmt[0]) != nullptr;
+            const bool utf8_values = vf && (strcmp(vf, "u") == 0 || strcmp(vf, "U") == 0);
+            if (!int_index || !utf8_values || !ca->dictionary)
+                throw Error(TG_ERR_UNSUPPORTED, std::string("column '") + cs->name + "': dictionary of " + arrow_type_name(vf) +
+                                                    " values (index type " + arrow_type_name(fmt.c_str()) + ") is not supported; string dictionaries only");
+            append_arrow_dict_utf8(t, cs->name, fmt[0], vf[0] == 'U', ca, ca->dictionary);
+            continue;
+        }
+        if (fmt == "vu") {
+            append_arrow_view_utf8(t, cs->name, ca);
+            continue;
+        }
+        if (fmt == "vz") throw Error(TG_ERR_UNSUPPORTED, std::string("column '") + cs->name + "': BinaryView is not supported");
         const ArrowFormat F = arrow_format(fmt, cs->name);
         const int32_t dtype = F.dtype;
         const int src_w = F.src_w;
