@@ -57,8 +57,10 @@ typedef enum {
     TG_INT32 = 4,
     TG_FLOAT32 = 5,
     TG_BOOL = 6,   /* Arrow Boolean: bit-packed values */
-    TG_FP128 = 7   /* internal: 24-byte records {h1, h2, null flag} of a hash-shuffled Utf8 / composite key
+    TG_FP128 = 7,  /* internal: 24-byte records {h1, h2, null flag} of a hash-shuffled Utf8 / composite key
                       (tg_table_partition_fingerprints); only COUNT(DISTINCT ..)-type aggregates read it */
+    TG_PQ_INT96 = 8 /* tg_table_append_parquet_chunk only: a Parquet INT96 (legacy timestamp) chunk, stored as a TG_INT64
+                       column of nanoseconds since the epoch, delivered as Timestamp(Nanosecond, None); no other entry point accepts it */
 } tg_dtype;
 
 /* ConstraintStatus (core/constraint.rs:11-20) */
@@ -251,11 +253,16 @@ TG_API tg_status tg_table_column_buffers(tg_engine* eng, const char* table, cons
  * hybrid, only its run headers are walked on the host) and the chunk's dictionary.
  * BYTE_ARRAY strings (dtype TG_UTF8) become int32 offsets + concatenated bytes: the device locates every row's bytes
  * (dictionary entry or PLAIN value), scans the lengths and copies; the host walks the PLAIN pages' length prefixes.
- * Supported: INT64 / DOUBLE / INT32 / FLOAT / BYTE_ARRAY (Utf8), codec UNCOMPRESSED (0) / SNAPPY (1) / GZIP (2) / BROTLI (4) / ZSTD (6) /
+ * BOOLEAN (dtype TG_BOOL) becomes the bit-packed Arrow Boolean values; its PLAIN and RLE values are decoded on the device.
+ * INT96 (dtype TG_PQ_INT96, the legacy Impala / Hive / Spark timestamp: int64 nanoseconds of the day, int32 Julian day)
+ * becomes an Int64 column of nanoseconds since the epoch (wrapping outside 1677 .. 2262), declared Timestamp(Nanosecond,
+ * None) by this call; appending it to a column of another delivered type is TG_ERR_TYPE_MISMATCH.
+ * Supported: INT64 / DOUBLE / INT32 / FLOAT / INT96 / BOOLEAN / BYTE_ARRAY (Utf8), codec UNCOMPRESSED (0) / SNAPPY (1) / GZIP (2) / BROTLI (4) / ZSTD (6) /
  * LZ4_RAW (7) (parquet.thrift CompressionCodec numbers; LZO and the deprecated hadoop-framed LZ4 are refused), data
- * pages V1 / V2, PLAIN / PLAIN_DICTIONARY / RLE_DICTIONARY values (on the device) and DELTA_BINARY_PACKED / DELTA_LENGTH_BYTE_ARRAY /
- * DELTA_BYTE_ARRAY / BYTE_STREAM_SPLIT values (serial streams: rewritten to PLAIN on the host), RLE levels, flat columns; anything else ->
- * TG_ERR_UNSUPPORTED (there is no host decode path). Appends num_values rows; `chunk`
+ * pages V1 / V2, PLAIN / PLAIN_DICTIONARY / RLE_DICTIONARY values (on the device; BOOLEAN: PLAIN / RLE) and DELTA_BINARY_PACKED /
+ * DELTA_LENGTH_BYTE_ARRAY / DELTA_BYTE_ARRAY / BYTE_STREAM_SPLIT values of INT64 / DOUBLE / INT32 / FLOAT / BYTE_ARRAY (serial streams:
+ * rewritten to PLAIN on the host), RLE levels, flat columns; anything else -> TG_ERR_UNSUPPORTED (there is no host decode path).
+ * Appends num_values rows; `chunk`
  * must stay readable until the next tg_plan_execute* / tg_table_column_buffers on this engine when it is pinned memory.
  */
 TG_API tg_status tg_table_append_parquet_chunk(tg_table* t, const char* name, int32_t dtype, int32_t max_definition_level,

@@ -28,6 +28,7 @@ TG_ERR_SECURITY, TG_ERR_UNSUPPORTED, TG_ERR_CUDA, TG_ERR_VALIDATION, TG_ERR_CONF
 
 # tg_dtype
 TG_INT64, TG_FLOAT64, TG_UTF8, TG_INT32, TG_FLOAT32, TG_BOOL, TG_FP128 = 1, 2, 3, 4, 5, 6, 7
+TG_PQ_INT96 = 8  # tg_table_append_parquet_chunk only: a Parquet INT96 timestamp chunk
 # tg_constraint_status
 TG_SUCCESS, TG_FAILURE, TG_SKIPPED = 0, 1, 2
 

@@ -358,7 +358,9 @@ class SessionContext:
                 C.CFUNCTYPE(None, C.c_void_p)(rel_s)(C.addressof(schema_buf))
 
     # Parquet physical type -> tg_dtype, decoded on the device (tg_table_append_parquet_chunk)
-    _PARQUET_TYPES = {"INT64": F.TG_INT64, "DOUBLE": F.TG_FLOAT64, "INT32": F.TG_INT32, "FLOAT": F.TG_FLOAT32, "BYTE_ARRAY": F.TG_UTF8}
+    # (INT96: the legacy timestamp, stored as Int64 nanoseconds and declared Timestamp(Nanosecond, None) by the engine itself)
+    _PARQUET_TYPES = {"INT64": F.TG_INT64, "DOUBLE": F.TG_FLOAT64, "INT32": F.TG_INT32, "FLOAT": F.TG_FLOAT32, "BYTE_ARRAY": F.TG_UTF8,
+                      "BOOLEAN": F.TG_BOOL, "INT96": F.TG_PQ_INT96}
 
     # parquet.thrift CompressionCodec numbers by pyarrow's names: its "LZ4" is the raw block format (thrift LZ4_RAW = 7; the
     # deprecated hadoop-framed thrift LZ4 = 5 reads back as "LZ4_HADOOP")
@@ -382,7 +384,8 @@ class SessionContext:
     def _check_parquet_logical_type(col, leaf):
         """The device path delivers the PHYSICAL values. Returns the Arrow C-Data format string to declare on the column
         (tg_table_set_column_arrow_type) when the annotation names a type whose Arrow values ARE the physical values — DATE,
-        TIME, TIMESTAMP, INT(8|16) — or None for plain columns. Annotations that would need converted values (DECIMAL,
+        TIME, TIMESTAMP, INT(8|16) — or None for plain columns (unannotated BOOLEAN and INT96 too: the engine declares an INT96
+        column Timestamp(Nanosecond, None) itself). Annotations that would need converted values (DECIMAL,
         UINT_32 / UINT_64, raw BYTE_ARRAY) are refused: the reference's ParquetSource yields their logical Arrow types
         (sources/parquet.rs:150-230) and the physical values would be silently wrong."""
         lt = str(getattr(leaf, "logical_type", "NONE") or "NONE").upper()
@@ -393,7 +396,7 @@ class SessionContext:
             if lt == "STRING" or ct == "UTF8":
                 return None
             raise F.TermGpuError(F.TG_ERR_UNSUPPORTED, f"Parquet column '{col}': BYTE_ARRAY with logical type {lt} / {ct} (only STRING columns)")
-        if phys in ("FLOAT", "DOUBLE"):
+        if phys in ("FLOAT", "DOUBLE", "BOOLEAN", "INT96"):
             if lt in ("NONE", "NULL") and ct == "NONE":
                 return None
         elif lt in ("NONE", "NULL") and ct in ("NONE", "INT_64", "INT_32"):
@@ -420,7 +423,7 @@ class SessionContext:
             if phys == "INT64" and "NANOSECONDS" in lt:
                 return "ttn"
         raise F.TermGpuError(F.TG_ERR_UNSUPPORTED, f"Parquet column '{col}': logical type {lt} / {ct} is not decoded on the device "
-                                                    "(plain and DATE / TIME / TIMESTAMP / INT(8|16) annotated INT32 / INT64, FLOAT / DOUBLE, STRING)")
+                                                    "(plain and DATE / TIME / TIMESTAMP / INT(8|16) annotated INT32 / INT64, FLOAT / DOUBLE, BOOLEAN, INT96, STRING)")
 
     def _register_parquet(self, t, paths, columns):
         import pyarrow.parquet as pq

@@ -15,9 +15,14 @@
 // Snappy-compressed pages are decompressed on the host into the staging source (the raw format's tag stream is serial
 // by construction); the levels of V2 pages are never compressed.
 //
+// BOOLEAN chunks become the bit-packed Arrow Boolean values: PLAIN sections (bit-packed, LSB first) and RLE sections
+// (4-byte length, then an RLE / bit-packed hybrid stream at bit width 1) are staged as they are; pq_expand_bool_kernel
+// writes 32 rows per ballot into the column's value bitmap. INT96 chunks (12-byte legacy Impala / Hive timestamps) become
+// Int64 nanoseconds since the epoch, converted by pq_expand_kernel as it loads each value.
+//
 // Supported (everything else is TG_ERR_UNSUPPORTED, there is no host decode path): physical INT64 / DOUBLE /
-// INT32 / FLOAT and BYTE_ARRAY strings (below), codecs UNCOMPRESSED and SNAPPY, data pages V1 and V2, PLAIN / PLAIN_DICTIONARY / RLE_DICTIONARY values
-// (a chunk may mix them: writers fall back to PLAIN when the dictionary grows too large), RLE definition levels, flat
+// INT32 / FLOAT / INT96 / BOOLEAN and BYTE_ARRAY strings (below), codecs UNCOMPRESSED and SNAPPY, data pages V1 and V2, PLAIN / PLAIN_DICTIONARY / RLE_DICTIONARY values
+// (a chunk may mix them: writers fall back to PLAIN when the dictionary grows too large; BOOLEAN: PLAIN and RLE), RLE definition levels, flat
 // columns (max definition level 0 or 1, no repetition levels).
 #include <dlfcn.h>
 
@@ -114,6 +119,13 @@ enum { PQ_DATA_PAGE = 0, PQ_INDEX_PAGE = 1, PQ_DICTIONARY_PAGE = 2, PQ_DATA_PAGE
 enum { PQ_ENC_PLAIN = 0, PQ_ENC_PLAIN_DICTIONARY = 2, PQ_ENC_RLE = 3, PQ_ENC_DELTA_BINARY_PACKED = 5, PQ_ENC_DELTA_LENGTH_BYTE_ARRAY = 6,
        PQ_ENC_DELTA_BYTE_ARRAY = 7, PQ_ENC_RLE_DICTIONARY = 8, PQ_ENC_BYTE_STREAM_SPLIT = 9 };
 enum { PQ_CODEC_UNCOMPRESSED = 0, PQ_CODEC_SNAPPY = 1, PQ_CODEC_GZIP = 2, PQ_CODEC_BROTLI = 4, PQ_CODEC_ZSTD = 6, PQ_CODEC_LZ4_RAW = 7 };
+
+std::string encoding_name(int32_t enc) {
+    static const char* const names[] = {"PLAIN", "GROUP_VAR_INT", "PLAIN_DICTIONARY", "RLE", "BIT_PACKED", "DELTA_BINARY_PACKED",
+                                        "DELTA_LENGTH_BYTE_ARRAY", "DELTA_BYTE_ARRAY", "RLE_DICTIONARY", "BYTE_STREAM_SPLIT"};
+    const std::string num = std::to_string(enc);
+    return enc >= 0 && enc < 10 ? std::string(names[enc]) + " (" + num + ")" : "encoding " + num;
+}
 
 // parquet.thrift: PageHeader {1 type, 2 uncompressed_page_size, 3 compressed_page_size, 4 crc, 5 data_page_header,
 // 6 index_page_header, 7 dictionary_page_header, 8 data_page_header_v2}; DataPageHeader {1 num_values, 2 encoding,
@@ -321,14 +333,10 @@ struct PqRun {
     uint32_t bw;      // bit width of the page (0..32)
     uint32_t packed;  // 1: bit-packed, 0: RLE
 };
-// Walks the run headers of an index stream: p[0] = bit width, then <varint header> (header & 1 ? bit-packed groups of 8
-// : RLE run) until `n_values` are covered. `stage_off` = where p[0] sits in the staging buffer.
-void parse_index_runs(const uint8_t* p, const uint8_t* end, int64_t n_values, uint64_t stage_off, std::vector<PqRun>& runs) {
-    if (n_values == 0) return;
-    if (p >= end) throw Error(TG_ERR_INVALID_ARG, "Parquet: empty dictionary-index section");
-    const uint32_t bw = p[0];
-    if (bw > 32) throw Error(TG_ERR_INVALID_ARG, "Parquet: dictionary index bit width > 32");
-    Thrift t{p + 1, end};
+// Walks the run headers of an RLE / bit-packed hybrid stream at bit width `bw`: <varint header> (header & 1 ? bit-packed
+// groups of 8 : RLE run) until `n_values` are covered. `stage_off` = where p[0] sits in the staging buffer.
+void parse_hybrid_runs(const uint8_t* p, const uint8_t* end, uint32_t bw, int64_t n_values, uint64_t stage_off, std::vector<PqRun>& runs) {
+    Thrift t{p, end};
     int64_t done = 0;
     while (done < n_values) {
         const uint64_t h = t.varint();
@@ -354,6 +362,39 @@ void parse_index_runs(const uint8_t* p, const uint8_t* end, int64_t n_values, ui
             done += take;
         }
     }
+}
+// A dictionary-index stream: p[0] = bit width, then the hybrid runs
+void parse_index_runs(const uint8_t* p, const uint8_t* end, int64_t n_values, uint64_t stage_off, std::vector<PqRun>& runs) {
+    if (n_values == 0) return;
+    if (p >= end) throw Error(TG_ERR_INVALID_ARG, "Parquet: empty dictionary-index section");
+    const uint32_t bw = p[0];
+    if (bw > 32) throw Error(TG_ERR_INVALID_ARG, "Parquet: dictionary index bit width > 32");
+    parse_hybrid_runs(p + 1, end, bw, n_values, stage_off + 1, runs);
+}
+// An RLE-encoded BOOLEAN value section: a 4-byte little-endian length, then the hybrid runs at bit width 1 (no width byte)
+void parse_bool_runs(const uint8_t* p, int64_t n_bytes, int64_t n_values, uint64_t stage_off, std::vector<PqRun>& runs) {
+    if (n_values == 0) return;
+    if (n_bytes < 4) throw Error(TG_ERR_INVALID_ARG, "Parquet: RLE BOOLEAN section shorter than its 4-byte length");
+    uint32_t len;
+    memcpy(&len, p, 4);
+    if ((int64_t)len > n_bytes - 4) throw Error(TG_ERR_INVALID_ARG, "Parquet: RLE BOOLEAN length runs past the page");
+    const size_t first = runs.size();
+    parse_hybrid_runs(p + 4, p + 4 + len, 1, n_values, stage_off + 4, runs);
+    for (size_t k = first; k < runs.size(); ++k)
+        if (!runs[k].packed && runs[k].data > 1) throw Error(TG_ERR_INVALID_ARG, "Parquet: RLE BOOLEAN run of a value other than 0 / 1");
+}
+
+// INT96 (Impala / Hive / Spark timestamps): int64 nanoseconds of the day, then the int32 Julian day; nanoseconds since the
+// epoch in wrapping int64 arithmetic (instants outside 1677 .. 2262 wrap, as in arrow-rs)
+__host__ __device__ inline uint64_t pq_int96_ns(uint64_t nanos, int32_t julian_day) {
+    return ((uint64_t)(int64_t)julian_day - 2440588ull) * 86400000000000ull + nanos;
+}
+uint64_t pq_int96_ns_host(const uint8_t* p) {
+    uint64_t nanos;
+    int32_t day;
+    memcpy(&nanos, p, 8);
+    memcpy(&day, p + 8, 4);
+    return pq_int96_ns(nanos, day);
 }
 
 // the first `want` indices of an index stream, decoded on the host (the column's pivot is chosen from its first values)
@@ -497,19 +538,55 @@ size_t page_decompress(int32_t codec, const uint8_t* src, size_t n, uint8_t* dst
 
 }  // namespace
 
+// The value of dense index d of a hybrid stream: the last of runs [lo, hi) with start <= d, then its RLE value or the d-th
+// packed value (two 32-bit loads; the staging buffer keeps slack behind every section)
+__device__ __forceinline__ uint64_t pq_run_value(const uint8_t* __restrict__ stage, const PqRun* __restrict__ runs, uint32_t lo, uint32_t hi,
+                                                 uint32_t d) {
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (__ldg(&runs[mid].start) <= d) lo = mid;
+        else hi = mid;
+    }
+    const PqRun run = runs[lo];
+    uint64_t idx = run.data;
+    if (run.packed) {
+        const uint64_t bit = (uint64_t)(d - run.start) * run.bw;
+        const uint64_t byte = run.data + (bit >> 3);
+        const uint32_t* wp = reinterpret_cast<const uint32_t*>(stage + (byte & ~(uint64_t)3));
+        const uint64_t w = (uint64_t)__ldg(wp) | ((uint64_t)__ldg(wp + 1) << 32);
+        const uint32_t sh = (uint32_t)((byte & 3) * 8 + (bit & 7));
+        idx = run.bw ? ((w >> sh) & (((uint64_t)1 << run.bw) - 1ull)) : 0ull;
+    }
+    return idx;
+}
+
+// How pq_expand_kernel reads value i of a PLAIN section or a dictionary: the stored type as it is ...
+template <typename V>
+struct PqLoadNative {
+    static __device__ __forceinline__ V at(const uint8_t* __restrict__ base, uint64_t i) { return __ldg(reinterpret_cast<const V*>(base) + i); }
+};
+// ... or a 12-byte INT96 converted to Int64 nanoseconds. Sections and the dictionary start 16-byte aligned, so every value
+// is 4-byte aligned: three 32-bit loads
+struct PqLoadInt96 {
+    static __device__ __forceinline__ uint64_t at(const uint8_t* __restrict__ base, uint64_t i) {
+        const uint32_t* p = reinterpret_cast<const uint32_t*>(base + i * 12);
+        return pq_int96_ns((uint64_t)__ldg(p) | ((uint64_t)__ldg(p + 1) << 32), (int32_t)__ldg(p + 2));
+    }
+};
+
 // One warp per block. Row r of the block is non-NULL iff its bit is set (bits == nullptr: a required column, every row
 // is); its value is the (number of set bits before r in the block)-th of the block's dense source values — read directly
 // (PLAIN) or through the section's index stream and the chunk's dictionary. NULL rows are written as 0 so the column is
 // deterministic. Indices past the dictionary (a corrupt file) read its last entry: memory-safe, never out of bounds.
-template <typename V>
+template <typename V, typename Load = PqLoadNative<V>>
 __global__ void __launch_bounds__(PQ_THREADS) pq_expand_kernel(const uint8_t* __restrict__ stage, const uint8_t* __restrict__ bits,
                                                               const PqBlock* __restrict__ blocks, int64_t n_blocks, V* __restrict__ dst,
-                                                              const PqRun* __restrict__ runs, const V* __restrict__ dict, uint32_t dict_count) {
+                                                              const PqRun* __restrict__ runs, const uint8_t* __restrict__ dict, uint32_t dict_count) {
     const int lane = threadIdx.x & 31;
     const int64_t warps = (int64_t)gridDim.x * (PQ_THREADS / 32);
     for (int64_t b = (int64_t)blockIdx.x * (PQ_THREADS / 32) + (threadIdx.x >> 5); b < n_blocks; b += warps) {
         const PqBlock blk = blocks[b];
-        const V* src = reinterpret_cast<const V*>(stage + blk.src_off);
+        const uint8_t* src = stage + blk.src_off;
         uint32_t running = 0;
         for (uint32_t i = 0; i < blk.n_rows; i += 32) {
             const bool in = i + lane < blk.n_rows;
@@ -520,30 +597,53 @@ __global__ void __launch_bounds__(PQ_THREADS) pq_expand_kernel(const uint8_t* __
             V v = 0;
             if (valid) {
                 if (blk.run_hi == 0) {
-                    v = __ldg(src + rank);
+                    v = Load::at(src, rank);
                 } else {
-                    const uint32_t d = blk.first_dense + rank;
-                    uint32_t lo = blk.run_lo, hi = blk.run_hi;  // the last run with start <= d
-                    while (hi - lo > 1) {
-                        const uint32_t mid = (lo + hi) >> 1;
-                        if (__ldg(&runs[mid].start) <= d) lo = mid;
-                        else hi = mid;
-                    }
-                    const PqRun run = runs[lo];
-                    uint64_t idx = run.data;
-                    if (run.packed) {
-                        const uint64_t bit = (uint64_t)(d - run.start) * run.bw;
-                        const uint64_t byte = run.data + (bit >> 3);
-                        const uint32_t* wp = reinterpret_cast<const uint32_t*>(stage + (byte & ~(uint64_t)3));
-                        const uint64_t w = (uint64_t)__ldg(wp) | ((uint64_t)__ldg(wp + 1) << 32);
-                        const uint32_t sh = (uint32_t)((byte & 3) * 8 + (bit & 7));
-                        idx = run.bw ? ((w >> sh) & (((uint64_t)1 << run.bw) - 1ull)) : 0ull;
-                    }
+                    uint64_t idx = pq_run_value(stage, runs, blk.run_lo, blk.run_hi, blk.first_dense + rank);
                     if (idx >= dict_count) idx = dict_count - 1;
-                    v = __ldg(dict + idx);
+                    v = Load::at(dict, idx);
                 }
             }
             if (in) dst[r] = v;
+            running += __popc(mask);
+        }
+    }
+}
+
+// BOOLEAN values, one warp per block as above. A valid row's value is bit (block src_off + rank) of the staged PLAIN
+// section (src_off is a BIT offset here) or the value of its run in the section's RLE stream; NULL rows read 0. One
+// ballot gives the bits of 32 consecutive rows, OR-ed into the column's value bitmap at bit dst_bit0 + row: pages and
+// appends start at any row, so a word may straddle two blocks (the host zeroed the new bytes first; OR order does not matter).
+__global__ void __launch_bounds__(PQ_THREADS) pq_expand_bool_kernel(const uint8_t* __restrict__ stage, const uint8_t* __restrict__ bits,
+                                                                   const PqBlock* __restrict__ blocks, int64_t n_blocks, uint32_t* __restrict__ dst,
+                                                                   uint64_t dst_bit0, const PqRun* __restrict__ runs) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warps = (int64_t)gridDim.x * (PQ_THREADS / 32);
+    for (int64_t b = (int64_t)blockIdx.x * (PQ_THREADS / 32) + (threadIdx.x >> 5); b < n_blocks; b += warps) {
+        const PqBlock blk = blocks[b];
+        uint32_t running = 0;
+        for (uint32_t i = 0; i < blk.n_rows; i += 32) {
+            const bool in = i + lane < blk.n_rows;
+            const uint64_t r = (uint64_t)blk.first_row + i + lane;
+            const bool valid = in && (!bits || ((__ldg(bits + (r >> 3)) >> (r & 7)) & 1));
+            const unsigned mask = __ballot_sync(0xffffffffu, valid);
+            const uint32_t rank = running + __popc(mask & ((1u << lane) - 1u));
+            uint32_t v = 0;
+            if (valid) {
+                if (blk.run_hi == 0) {
+                    const uint64_t sb = blk.src_off + rank;
+                    v = (__ldg(stage + (sb >> 3)) >> (sb & 7)) & 1u;
+                } else {
+                    v = (uint32_t)pq_run_value(stage, runs, blk.run_lo, blk.run_hi, blk.first_dense + rank) & 1u;
+                }
+            }
+            const unsigned out = __ballot_sync(0xffffffffu, v != 0);
+            if (lane == 0 && out) {
+                const uint64_t pos = dst_bit0 + blk.first_row + i;
+                const uint32_t sh = (uint32_t)(pos & 31);
+                atomicOr(dst + (pos >> 5), out << sh);
+                if (sh && (out >> (32 - sh))) atomicOr(dst + (pos >> 5) + 1, out >> (32 - sh));
+            }
             running += __popc(mask);
         }
     }
@@ -742,6 +842,7 @@ struct PqSection {
     const uint8_t* levels;
     int64_t levels_bytes;
     bool dict;
+    bool rle;  // BOOLEAN values in the RLE encoding
 };
 struct PqChunk {
     std::vector<PqSection> secs;
@@ -751,9 +852,15 @@ struct PqChunk {
     int64_t dict_bytes = 0, dict_count = 0;
     bool any_dict = false;
 };
+// width in the file of one fixed-width value of a chunk handed over as `dtype` (0: BYTE_ARRAY, and BOOLEAN's bits)
+size_t source_width(int32_t dtype) {
+    return dtype == TG_PQ_INT96 ? 12 : (dtype == TG_INT64 || dtype == TG_FLOAT64) ? 8 : (dtype == TG_INT32 || dtype == TG_FLOAT32) ? 4 : 0;
+}
+
 // Every page body as UNCOMPRESSED bytes (a view of the chunk, or of `inflated` for Snappy pages), cut into its level and
-// value sections. elem_w: width of a fixed-width value (0: BYTE_ARRAY).
-void collect_sections(const uint8_t* chunk, int64_t n_bytes, int32_t codec, int32_t max_def_level, int64_t num_values, size_t elem_w, PqChunk& out) {
+// value sections. dtype: the chunk's type as tg_table_append_parquet_chunk received it.
+void collect_sections(const uint8_t* chunk, int64_t n_bytes, int32_t codec, int32_t max_def_level, int64_t num_values, int32_t dtype, PqChunk& out) {
+    const size_t elem_w = source_width(dtype);
     const std::vector<tg_parquet_page> pages = walk_pages(chunk, n_bytes);
     {
         size_t need = 0;
@@ -786,6 +893,7 @@ void collect_sections(const uint8_t* chunk, int64_t n_bytes, int32_t codec, int3
             inflated_used += (size_t)pg.uncompressed_bytes + 16;
         }
         if (pg.page_type == PQ_DICTIONARY_PAGE) {
+            if (dtype == TG_BOOL) throw Error(TG_ERR_UNSUPPORTED, "Parquet: dictionary-encoded BOOLEAN chunk (PLAIN and RLE values only)");
             if (pg.encoding != PQ_ENC_PLAIN && pg.encoding != PQ_ENC_PLAIN_DICTIONARY)
                 throw Error(TG_ERR_UNSUPPORTED, "Parquet: dictionary page encoding " + std::to_string(pg.encoding));
             if (out.dict_values) throw Error(TG_ERR_INVALID_ARG, "Parquet: more than one dictionary page in a column chunk");
@@ -797,10 +905,15 @@ void collect_sections(const uint8_t* chunk, int64_t n_bytes, int32_t codec, int3
             continue;
         }
         const bool is_dict = pg.encoding == PQ_ENC_RLE_DICTIONARY || pg.encoding == PQ_ENC_PLAIN_DICTIONARY;
-        if (!is_dict && pg.encoding != PQ_ENC_PLAIN && !encoding_rewritten_on_host(pg.encoding))
+        const bool is_rle = dtype == TG_BOOL && pg.encoding == PQ_ENC_RLE;
+        if (dtype == TG_BOOL && pg.encoding != PQ_ENC_PLAIN && !is_rle)
+            throw Error(TG_ERR_UNSUPPORTED, "Parquet: BOOLEAN values encoded " + encoding_name(pg.encoding) + " (PLAIN and RLE only)");
+        if (dtype == TG_PQ_INT96 && pg.encoding != PQ_ENC_PLAIN && !is_dict)
+            throw Error(TG_ERR_UNSUPPORTED, "Parquet: INT96 values encoded " + encoding_name(pg.encoding) + " (PLAIN and dictionary only)");
+        if (!is_dict && !is_rle && pg.encoding != PQ_ENC_PLAIN && !encoding_rewritten_on_host(pg.encoding))
             throw Error(TG_ERR_UNSUPPORTED, "Parquet: value encoding " + std::to_string(pg.encoding) +
                                                 " (PLAIN, dictionary, DELTA_* and BYTE_STREAM_SPLIT encodings only)");
-        PqSection s{rows, pg.num_values, body, body_bytes, nullptr, 0, is_dict};
+        PqSection s{rows, pg.num_values, body, body_bytes, nullptr, 0, is_dict, is_rle};
         if (max_def_level > 0) {
             if (pg.definition_level_encoding != PQ_ENC_RLE) throw Error(TG_ERR_UNSUPPORTED, "Parquet: definition levels not RLE-encoded");
             if (pg.version == 1) {
@@ -861,15 +974,28 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
         append_parquet_utf8(t, name, max_def_level, codec, chunk, n_bytes, num_values);
         return;
     }
-    if (dtype != TG_INT64 && dtype != TG_FLOAT64 && dtype != TG_INT32 && dtype != TG_FLOAT32)
-        throw Error(TG_ERR_UNSUPPORTED, "Parquet: only INT64 / DOUBLE / INT32 / FLOAT / BYTE_ARRAY (Utf8) columns are decoded on the device");
-    Column& c = *table_get_or_add(t, name, dtype);
+    const bool is_bool = dtype == TG_BOOL, int96 = dtype == TG_PQ_INT96;
+    if (dtype != TG_INT64 && dtype != TG_FLOAT64 && dtype != TG_INT32 && dtype != TG_FLOAT32 && !is_bool && !int96)
+        throw Error(TG_ERR_UNSUPPORTED, "Parquet: only INT64 / DOUBLE / INT32 / FLOAT / INT96 / BOOLEAN / BYTE_ARRAY (Utf8) columns are decoded on the device");
+    const int32_t stored = int96 ? TG_INT64 : dtype;
+    if (int96) {  // an INT96 column is Timestamp(Nanosecond, None) and nothing else
+        const Column* have_c = t.find(name);
+        if (have_c && !(have_c->src_type && strcmp(have_c->src_type, "Timestamp") == 0 && have_c->temporal_unit == 'n'))
+            throw Error(TG_ERR_TYPE_MISMATCH, "column '" + name + "' was registered with a different type than INT96 (Timestamp(Nanosecond, None))");
+    }
+    Column& c = *table_get_or_add(t, name, stored);
     if (c.adopted) throw Error(TG_ERR_INVALID_ARG, "cannot append to an adopted device column");
+    if (int96) {  // what tg_table_set_column_arrow_type(.., "tsn:") declares
+        c.src_type = "Timestamp";
+        c.src_unsigned = false;
+        c.temporal = true;
+        c.temporal_unit = 'n';
+    }
     const int64_t have = c.n_rows;
-    const size_t w = (size_t)c.elem_bytes();
+    const size_t w = (size_t)c.elem_bytes(), sw = source_width(dtype);  // stored / file width of a value (Boolean: bits, 0)
 
     PqChunk pc;
-    collect_sections(chunk, n_bytes, codec, max_def_level, num_values, w, pc);
+    collect_sections(chunk, n_bytes, codec, max_def_level, num_values, dtype, pc);
     using Section = PqSection;
     std::vector<PqSection>& secs = pc.secs;
     const uint8_t* dict_values = pc.dict_values;
@@ -884,7 +1010,8 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
     // a host memcpy into the pinned ring per piece, so the two halves of the host work run side by side. Every page's
     // value section goes to a 16-byte aligned place in a staging block (PLAIN pages of required columns: straight into
     // place); the dictionary's values sit in the same block ----
-    e.dev_reserve(c.values, (size_t)(have + num_values) * w, (size_t)have * w);
+    if (is_bool) e.dev_reserve(c.values, (size_t)(have + num_values + 7) / 8, (size_t)(have + 7) / 8);
+    else e.dev_reserve(c.values, (size_t)(have + num_values) * w, (size_t)have * w);
     uint8_t* dst = c.values.p + (size_t)have * w;
     std::vector<int64_t> stage_off(secs.size(), -1);
     size_t stage_bytes = 0;
@@ -892,7 +1019,8 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
     std::vector<uint8_t> bits;
     std::vector<PqBlock> blocks;
     std::vector<PqRun> runs;
-    const bool direct = max_def_level == 0 && !any_dict;
+    std::vector<std::pair<uint32_t, uint32_t>> sec_runs(secs.size());  // each section's runs [lo, hi) in `runs`
+    const bool direct = max_def_level == 0 && !any_dict && sw == w && !is_bool;
     if (direct) {
         for (auto& s : secs) {
             if (s.values_bytes != s.n_rows * (int64_t)w) throw Error(TG_ERR_INVALID_ARG, "Parquet: PLAIN page size does not match its value count");
@@ -904,9 +1032,9 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
             stage_bytes += ((size_t)secs[i].values_bytes + 15) & ~(size_t)15;
         }
         const size_t dict_off = stage_bytes;
-        stage_bytes += (((size_t)dict_count * w) + 15) & ~(size_t)15;
+        stage_bytes += (((size_t)dict_count * sw) + 15) & ~(size_t)15;
         stage_bytes += 64;
-        // definition levels -> chunk-relative validity bits + blocks (+ the run tables of dictionary-index sections)
+        // definition levels -> chunk-relative validity bits + blocks (+ the run tables of dictionary-index / RLE sections)
         std::exception_ptr decode_err;
         auto decode = [&]() {
             try {
@@ -920,18 +1048,25 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
                     int64_t prefix = 0;
                     for (int64_t r = 0; r < s.n_rows; r += PQ_BLOCK_ROWS) {
                         const int64_t nr = std::min<int64_t>(PQ_BLOCK_ROWS, s.n_rows - r);
-                        blocks.push_back(PqBlock{(uint64_t)stage_off[i] + (uint64_t)prefix * w, (uint32_t)(s.first_row + r), (uint32_t)nr, (uint32_t)prefix, 0u, 0u, 0u});
+                        // (Boolean PLAIN: the BIT offset of the block's first value)
+                        const uint64_t src = is_bool ? (uint64_t)stage_off[i] * 8 + (uint64_t)prefix : (uint64_t)stage_off[i] + (uint64_t)prefix * sw;
+                        blocks.push_back(PqBlock{src, (uint32_t)(s.first_row + r), (uint32_t)nr, (uint32_t)prefix, 0u, 0u, 0u});
                         prefix += max_def_level > 0 ? count_ones(bits.data(), s.first_row + r, s.first_row + r + nr) : nr;
                     }
-                    if (s.dict) {
-                        if (prefix > 0 && dict_count <= 0) throw Error(TG_ERR_INVALID_ARG, "Parquet: dictionary-encoded page without a dictionary page");
-                        parse_index_runs(s.values, s.values + s.values_bytes, prefix, (uint64_t)stage_off[i], runs);
+                    if (s.dict || s.rle) {
+                        if (s.dict) {
+                            if (prefix > 0 && dict_count <= 0) throw Error(TG_ERR_INVALID_ARG, "Parquet: dictionary-encoded page without a dictionary page");
+                            parse_index_runs(s.values, s.values + s.values_bytes, prefix, (uint64_t)stage_off[i], runs);
+                        } else {
+                            parse_bool_runs(s.values, s.values_bytes, prefix, (uint64_t)stage_off[i], runs);
+                        }
                         const uint32_t run_hi = (uint32_t)runs.size();
+                        sec_runs[i] = {run_lo, run_hi};
                         for (size_t k = blk_lo; k < blocks.size(); ++k) {
                             blocks[k].run_lo = run_lo;
                             blocks[k].run_hi = run_hi > run_lo ? run_hi : run_lo + 1;  // (an all-NULL section has no runs: never looked up)
                         }
-                    } else if (prefix * (int64_t)w != s.values_bytes) {
+                    } else if (is_bool ? s.values_bytes < (prefix + 7) / 8 : prefix * (int64_t)sw != s.values_bytes) {
                         throw Error(TG_ERR_INVALID_ARG, "Parquet: PLAIN page holds " + std::to_string(s.values_bytes) + " value bytes for " +
                                                             std::to_string(prefix) + " non-null rows");
                     }
@@ -951,34 +1086,36 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
         e.deferred_free.emplace_back(stage, stage_bytes);  // released by the next sync_copies(), also on the error paths
         for (size_t i = 0; i < secs.size(); ++i)
             if (secs[i].values_bytes) e.h2d(stage + stage_off[i], secs[i].values, (size_t)secs[i].values_bytes);
-        if (dict_count > 0) e.h2d(stage + dict_off, dict_values, (size_t)dict_count * w);
+        if (dict_count > 0) e.h2d(stage + dict_off, dict_values, (size_t)dict_count * sw);
         helper.join();
         if (decode_err) std::rethrow_exception(decode_err);
 
         // ---- pivot of the shifted sums: from the column's FIRST values, like the Arrow path (same K, bit-identical sums):
-        // the first PLAIN page's dense values, or the dictionary entries the first page's first indices name ----
-        if (!c.pivot_set && (dtype == TG_INT64 || dtype == TG_FLOAT64)) {
+        // the first PLAIN page's dense values, or the dictionary entries the first page's first indices name (INT96:
+        // converted, so the pivot is the one of the same instants delivered as timestamp[ns]) ----
+        auto head_value = [&](const uint8_t* p) {
+            uint64_t v;
+            if (int96) v = pq_int96_ns_host(p);
+            else memcpy(&v, p, 8);
+            return v;
+        };
+        if (!c.pivot_set && (stored == TG_INT64 || stored == TG_FLOAT64)) {
             for (auto& s0 : secs) {
                 if (s0.n_rows == 0) continue;
                 std::vector<uint64_t> head;
                 if (!s0.dict) {
-                    const int64_t nv = std::min<int64_t>(s0.values_bytes / (int64_t)w, 4096);
-                    head.resize((size_t)nv);
-                    memcpy(head.data(), s0.values, (size_t)nv * 8);
+                    const int64_t nv = std::min<int64_t>(s0.values_bytes / (int64_t)sw, 4096);
+                    for (int64_t k = 0; k < nv; ++k) head.push_back(head_value(s0.values + (size_t)k * sw));
                 } else if (dict_count > 0) {
                     std::vector<uint32_t> idx;
                     try {
                         decode_first_indices(s0.values, s0.values + s0.values_bytes, s0.n_rows, 256, idx);
                     } catch (Error&) {  // (a malformed stream is reported by the run walk below, with its own message)
                     }
-                    for (uint32_t k : idx) {
-                        uint64_t v;
-                        memcpy(&v, dict_values + (size_t)std::min<int64_t>(k, dict_count - 1) * 8, 8);
-                        head.push_back(v);
-                    }
+                    for (uint32_t k : idx) head.push_back(head_value(dict_values + (size_t)std::min<int64_t>(k, dict_count - 1) * sw));
                 }
                 if (!head.empty()) {
-                    set_pivot_host(c, dtype, (int64_t)head.size(), head.data(), nullptr, 0);
+                    set_pivot_host(c, stored, (int64_t)head.size(), head.data(), nullptr, 0);
                     break;
                 }
             }
@@ -999,12 +1136,22 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
         const uint8_t* d_bits = bits_b ? aux : nullptr;
         const PqBlock* d_blocks = reinterpret_cast<const PqBlock*>(aux + bits_b);
         const PqRun* d_runs = reinterpret_cast<const PqRun*>(aux + bits_b + blk_b);
-        if (w == 8)
+        if (is_bool) {
+            // the kernel ORs whole words: the new bytes start at zero (the partial byte before them keeps its earlier rows)
+            const size_t z0 = (size_t)(have + 7) / 8, z1 = (size_t)(have + num_values + 7) / 8;
+            if (z1 > z0) TG_CUDA(cudaMemsetAsync(c.values.p + z0, 0, z1 - z0, e.copy_stream));
+            pq_expand_bool_kernel<<<grid, PQ_THREADS, 0, e.copy_stream>>>(stage, d_bits, d_blocks, nb, reinterpret_cast<uint32_t*>(c.values.p),
+                                                                          (uint64_t)have, d_runs);
+        } else if (int96) {
+            pq_expand_kernel<uint64_t, PqLoadInt96><<<grid, PQ_THREADS, 0, e.copy_stream>>>(stage, d_bits, d_blocks, nb, reinterpret_cast<uint64_t*>(dst),
+                                                                                           d_runs, stage + dict_off, (uint32_t)dict_count);
+        } else if (w == 8) {
             pq_expand_kernel<uint64_t><<<grid, PQ_THREADS, 0, e.copy_stream>>>(stage, d_bits, d_blocks, nb, reinterpret_cast<uint64_t*>(dst), d_runs,
-                                                                               reinterpret_cast<const uint64_t*>(stage + dict_off), (uint32_t)dict_count);
-        else
+                                                                               stage + dict_off, (uint32_t)dict_count);
+        } else {
             pq_expand_kernel<uint32_t><<<grid, PQ_THREADS, 0, e.copy_stream>>>(stage, d_bits, d_blocks, nb, reinterpret_cast<uint32_t*>(dst), d_runs,
-                                                                               reinterpret_cast<const uint32_t*>(stage + dict_off), (uint32_t)dict_count);
+                                                                               stage + dict_off, (uint32_t)dict_count);
+        }
         TG_CUDA(cudaGetLastError());
         e.launches += 1;
         e.deferred_free.emplace_back(aux, bits_b + blk_b + run_b + 64);
@@ -1020,7 +1167,35 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
         }
         append_validity(e, c, have, nullptr, 0, num_values);
     }
-    c.value_bytes = (have + num_values) * (int64_t)w;
+    if (is_bool) {
+        // host mirror of the value bitmap's last partial byte (table_append_host continues from it): its rows before this
+        // chunk from the old mirror, the chunk's own (at most 7) rows decoded here from the staged sources
+        const int64_t total = have + num_values, lo = total & ~(int64_t)7;
+        uint8_t tail = lo < have ? (uint8_t)(c.tail_vbyte & ((1u << (have - lo)) - 1u)) : 0;
+        for (int64_t row = std::max(lo, have); row < total; ++row) {
+            const int64_t r = row - have;
+            if (max_def_level > 0 && !((bits[(size_t)(r >> 3)] >> (r & 7)) & 1)) continue;
+            size_t i = secs.size() - 1;
+            while (secs[i].first_row > r) --i;
+            const Section& s = secs[i];
+            const int64_t d = max_def_level > 0 ? count_ones(bits.data(), s.first_row, r) : r - s.first_row;
+            uint32_t v;
+            if (!s.rle) {
+                v = (s.values[d >> 3] >> (d & 7)) & 1u;
+            } else {
+                uint32_t k = sec_runs[i].second - 1;
+                while (runs[k].start > (uint64_t)d) --k;
+                const PqRun& run = runs[k];
+                const int64_t bit = d - (int64_t)run.start;
+                v = run.packed ? (s.values[run.data - (uint64_t)stage_off[i] + (uint64_t)(bit >> 3)] >> (bit & 7)) & 1u : (uint32_t)run.data;
+            }
+            tail |= (uint8_t)(v << (row - lo));
+        }
+        c.tail_vbyte = tail;
+        c.value_bytes = (total + 7) / 8;
+    } else {
+        c.value_bytes = (have + num_values) * (int64_t)w;
+    }
     c.n_rows = have + num_values;
     t.n_rows = std::max(t.n_rows, c.n_rows);
 }
@@ -1058,23 +1233,7 @@ __device__ __forceinline__ uint64_t pq_row_entry(const PqBlock& blk, uint32_t ra
                                                  const PqRun* __restrict__ runs, const uint64_t* __restrict__ plain_ents,
                                                  const uint64_t* __restrict__ dict_ents, uint32_t dict_count) {
     if (blk.run_hi == 0) return __ldg(plain_ents + blk.src_off + rank);  // PLAIN: src_off = the block's first entry
-    const uint32_t d = blk.first_dense + rank;
-    uint32_t lo = blk.run_lo, hi = blk.run_hi;
-    while (hi - lo > 1) {
-        const uint32_t mid = (lo + hi) >> 1;
-        if (__ldg(&runs[mid].start) <= d) lo = mid;
-        else hi = mid;
-    }
-    const PqRun run = runs[lo];
-    uint64_t idx = run.data;
-    if (run.packed) {
-        const uint64_t bit = (uint64_t)(d - run.start) * run.bw;
-        const uint64_t byte = run.data + (bit >> 3);
-        const uint32_t* wp = reinterpret_cast<const uint32_t*>(stage + (byte & ~(uint64_t)3));
-        const uint64_t w = (uint64_t)__ldg(wp) | ((uint64_t)__ldg(wp + 1) << 32);
-        const uint32_t sh = (uint32_t)((byte & 3) * 8 + (bit & 7));
-        idx = run.bw ? ((w >> sh) & (((uint64_t)1 << run.bw) - 1ull)) : 0ull;
-    }
+    uint64_t idx = pq_run_value(stage, runs, blk.run_lo, blk.run_hi, blk.first_dense + rank);
     if (idx >= dict_count) idx = dict_count - 1;
     return __ldg(dict_ents + idx);
 }
@@ -1171,7 +1330,7 @@ static void append_parquet_utf8(Table& t, const std::string& name, int32_t max_d
     if (c.adopted) throw Error(TG_ERR_INVALID_ARG, "cannot append to an adopted device column");
     const int64_t have = c.n_rows;
     PqChunk pc;
-    collect_sections(chunk, n_bytes, codec, max_def_level, num_values, 0, pc);
+    collect_sections(chunk, n_bytes, codec, max_def_level, num_values, TG_UTF8, pc);
     std::vector<PqSection>& secs = pc.secs;
     if (num_values == 0) {
         t.n_rows = std::max(t.n_rows, c.n_rows);

@@ -10,7 +10,7 @@
 namespace tg {
 
 struct PqBlock {
-    uint64_t src_off;     // PLAIN: byte offset in the staging buffer of the block's first non-NULL value
+    uint64_t src_off;     // PLAIN: byte offset in the staging buffer of the block's first non-NULL value (BOOLEAN: bit offset)
     uint32_t first_row;   // chunk-relative
     uint32_t n_rows;      // <= PQ_BLOCK_ROWS
     uint32_t first_dense; // dictionary: dense index (inside the block's section) of the block's first non-NULL value
