@@ -397,44 +397,6 @@ uint64_t pq_int96_ns_host(const uint8_t* p) {
     return pq_int96_ns(nanos, day);
 }
 
-// the first `want` indices of an index stream, decoded on the host (the column's pivot is chosen from its first values)
-void decode_first_indices(const uint8_t* p, const uint8_t* end, int64_t n_values, int64_t want, std::vector<uint32_t>& out) {
-    if (n_values <= 0 || p >= end) return;
-    const uint32_t bw = p[0];
-    if (bw > 32) return;
-    Thrift t{p + 1, end};
-    int64_t done = 0;
-    const int64_t target = std::min(n_values, want);  // (n_values may count NULL rows too: the stream simply ends earlier)
-    while (done < target && t.p < t.end) {
-        const uint64_t h = t.varint();
-        if (h & 1) {
-            const uint64_t groups = h >> 1;
-            if (groups * bw > (uint64_t)(t.end - t.p)) return;
-            const int64_t take = std::min<int64_t>((int64_t)groups * 8, target - done);
-            for (int64_t i = 0; i < take; ++i) {
-                const uint64_t bit = (uint64_t)i * bw;
-                uint64_t w = 0;
-                const size_t byte = (size_t)(bit >> 3), avail = (size_t)(t.end - t.p) - byte;
-                memcpy(&w, t.p + byte, std::min<size_t>(8, avail));
-                out.push_back(bw ? (uint32_t)((w >> (bit & 7)) & (((uint64_t)1 << bw) - 1ull)) : 0u);
-            }
-            t.p += groups * bw;
-            done += take;
-        } else {
-            const uint64_t run = h >> 1;
-            if (run == 0) return;
-            const int vb = (int)(bw + 7) / 8;
-            if (vb > t.end - t.p) return;
-            uint32_t v = 0;
-            for (int k = 0; k < vb; ++k) v |= (uint32_t)t.p[k] << (8 * k);
-            t.p += vb;
-            const int64_t take = std::min<int64_t>((int64_t)run, target - done);
-            for (int64_t i = 0; i < take; ++i) out.push_back(v);
-            done += take;
-        }
-    }
-}
-
 // ---- GZIP / ZSTD / LZ4_RAW / BROTLI pages: inflated on the host by the system's own codec libraries, bound at run time the first
 // time a chunk needs one (dlopen, like libnccl: libtermgpu.so keeps no link-time dependency); Snappy stays hand-written above.
 struct PqCodecLibs {
@@ -677,33 +639,6 @@ int32_t parquet_inspect_chunk(const uint8_t* chunk, int64_t n_bytes, tg_parquet_
     return (int32_t)v.size();
 }
 
-// Host-only: the validity bitmap (chunk-relative, LSB first, (num_values + 7) / 8 bytes) a flat optional column chunk
-// decodes to, and its non-NULL count. The device path builds exactly this before it scatters the values.
-int64_t parquet_chunk_validity(const uint8_t* chunk, int64_t n_bytes, int64_t num_values, uint8_t* out_bits) {
-    const std::vector<tg_parquet_page> pages = walk_pages(chunk, n_bytes);
-    std::vector<uint8_t> bits((size_t)(num_values + 7) / 8 + 16, 0);
-    int64_t rows = 0;
-    for (auto& pg : pages) {
-        if (pg.page_type != PQ_DATA_PAGE && pg.page_type != PQ_DATA_PAGE_V2) continue;
-        if (rows + pg.num_values > num_values) throw Error(TG_ERR_INVALID_ARG, "Parquet: more values than the chunk metadata says");
-        int64_t off = pg.body_offset, len = pg.definition_levels_bytes;
-        if (pg.version == 1) {
-            if (pg.body_bytes < 4) throw Error(TG_ERR_INVALID_ARG, "Parquet: data page too short");
-            uint32_t l;
-            memcpy(&l, chunk + off, 4);
-            off += 4;
-            len = l;
-            if ((int64_t)l > (int64_t)pg.body_bytes - 4) throw Error(TG_ERR_INVALID_ARG, "Parquet: definition levels run past the page");
-        } else if (pg.repetition_levels_bytes != 0) {
-            throw Error(TG_ERR_UNSUPPORTED, "Parquet: repeated column");
-        }
-        decode_levels(chunk + off, chunk + off + len, bits.data(), rows, pg.num_values);
-        rows += pg.num_values;
-    }
-    if (out_bits) memcpy(out_bits, bits.data(), (size_t)(num_values + 7) / 8);
-    return count_ones(bits.data(), 0, rows);
-}
-
 namespace {
 // the number of non-NULL rows among the `n` definition levels of one page
 int64_t count_levels_set(const uint8_t* p, const uint8_t* end, int64_t n) {
@@ -852,6 +787,27 @@ struct PqChunk {
     int64_t dict_bytes = 0, dict_count = 0;
     bool any_dict = false;
 };
+// Cuts a data page's uncompressed body into its definition levels and its values. V1: a 4-byte length and the levels (when
+// `levels`: an optional column), then the values; V2: the level sections the header sizes, then the values.
+void split_levels(const tg_parquet_page& pg, const uint8_t* body, int64_t body_bytes, bool levels, PqSection& s) {
+    int64_t lev_at = 0, lev_len = 0;
+    if (pg.version == 2) {
+        if (pg.repetition_levels_bytes != 0) throw Error(TG_ERR_UNSUPPORTED, "Parquet: repeated column");
+        lev_len = pg.definition_levels_bytes;
+    } else if (levels) {
+        if (body_bytes < 4) throw Error(TG_ERR_INVALID_ARG, "Parquet: data page too short");
+        uint32_t len;
+        memcpy(&len, body, 4);
+        if ((int64_t)len > body_bytes - 4) throw Error(TG_ERR_INVALID_ARG, "Parquet: definition levels run past the page");
+        lev_at = 4;
+        lev_len = len;
+    }
+    s.levels = levels ? body + lev_at : nullptr;
+    s.levels_bytes = levels ? lev_len : 0;
+    s.values = body + lev_at + lev_len;
+    s.values_bytes = body_bytes - lev_at - lev_len;
+    if (s.values_bytes < 0) throw Error(TG_ERR_INVALID_ARG, "Parquet: definition levels run past the page");
+}
 // width in the file of one fixed-width value of a chunk handed over as `dtype` (0: BYTE_ARRAY, and BOOLEAN's bits)
 size_t source_width(int32_t dtype) {
     return dtype == TG_PQ_INT96 ? 12 : (dtype == TG_INT64 || dtype == TG_FLOAT64) ? 8 : (dtype == TG_INT32 || dtype == TG_FLOAT32) ? 4 : 0;
@@ -874,7 +830,6 @@ void collect_sections(const uint8_t* chunk, int64_t n_bytes, int32_t codec, int3
         if (pg.page_type == PQ_INDEX_PAGE) continue;
         if (pg.page_type != PQ_DATA_PAGE && pg.page_type != PQ_DATA_PAGE_V2 && pg.page_type != PQ_DICTIONARY_PAGE)
             throw Error(TG_ERR_UNSUPPORTED, "Parquet: unknown page type");
-        if (pg.version == 2 && (pg.repetition_levels_bytes != 0)) throw Error(TG_ERR_UNSUPPORTED, "Parquet: repeated column");
         // the uncompressed body: V1 and dictionary pages are compressed as a whole, V2 keeps its level sections plain
         const uint8_t* body = chunk + pg.body_offset;
         int64_t body_bytes = pg.body_bytes;
@@ -913,29 +868,10 @@ void collect_sections(const uint8_t* chunk, int64_t n_bytes, int32_t codec, int3
         if (!is_dict && !is_rle && pg.encoding != PQ_ENC_PLAIN && !encoding_rewritten_on_host(pg.encoding))
             throw Error(TG_ERR_UNSUPPORTED, "Parquet: value encoding " + std::to_string(pg.encoding) +
                                                 " (PLAIN, dictionary, DELTA_* and BYTE_STREAM_SPLIT encodings only)");
-        PqSection s{rows, pg.num_values, body, body_bytes, nullptr, 0, is_dict, is_rle};
-        if (max_def_level > 0) {
-            if (pg.definition_level_encoding != PQ_ENC_RLE) throw Error(TG_ERR_UNSUPPORTED, "Parquet: definition levels not RLE-encoded");
-            if (pg.version == 1) {
-                if (body_bytes < 4) throw Error(TG_ERR_INVALID_ARG, "Parquet: data page too short");
-                uint32_t len;
-                memcpy(&len, body, 4);
-                if ((int64_t)len > body_bytes - 4) throw Error(TG_ERR_INVALID_ARG, "Parquet: definition levels run past the page");
-                s.levels = body + 4;
-                s.levels_bytes = len;
-                s.values = s.levels + len;
-                s.values_bytes = body_bytes - 4 - (int64_t)len;
-            } else {
-                s.levels = body;
-                s.levels_bytes = pg.definition_levels_bytes;
-                s.values = s.levels + s.levels_bytes;
-                s.values_bytes = body_bytes - s.levels_bytes;
-            }
-            if (s.values_bytes < 0) throw Error(TG_ERR_INVALID_ARG, "Parquet: definition levels run past the page");
-        } else if (pg.version == 2 && pg.definition_levels_bytes) {
-            s.values = body + pg.definition_levels_bytes;
-            s.values_bytes = body_bytes - pg.definition_levels_bytes;
-        }
+        if (max_def_level > 0 && pg.definition_level_encoding != PQ_ENC_RLE)
+            throw Error(TG_ERR_UNSUPPORTED, "Parquet: definition levels not RLE-encoded");
+        PqSection s{rows, pg.num_values, nullptr, 0, nullptr, 0, is_dict, is_rle};
+        split_levels(pg, body, body_bytes, max_def_level > 0, s);
         if (encoding_rewritten_on_host(pg.encoding)) {
             // the number of values present = the page's rows minus its NULLs (counted from the levels when the header has no count)
             int64_t present = pg.num_values;
@@ -955,7 +891,207 @@ void collect_sections(const uint8_t* chunk, int64_t n_bytes, int32_t codec, int3
     if (rows != num_values) throw Error(TG_ERR_INVALID_ARG, "Parquet: pages hold " + std::to_string(rows) + " values, the chunk metadata says " + std::to_string(num_values));
     if (!out.dict_values) out.dict_count = 0;  // (a dictionary-encoded page needs one unless all its rows are NULL: checked with the levels)
 }
+
+// entries: pq_str_ent / PQ_STR_MAX_LEN (str_entries.cuh)
+// walks `count` PLAIN BYTE_ARRAY values at p (length prefixes interleaved) into entries; stage_off = where p sits in staging
+void walk_plain_strings(const uint8_t* p, int64_t n_bytes, int64_t count, uint64_t stage_off, std::vector<uint64_t>& ents) {
+    int64_t pos = 0;
+    for (int64_t i = 0; i < count; ++i) {
+        if (pos + 4 > n_bytes) throw Error(TG_ERR_INVALID_ARG, "Parquet: BYTE_ARRAY page is truncated");
+        uint32_t len;
+        memcpy(&len, p + pos, 4);
+        pos += 4;
+        if ((int64_t)len > n_bytes - pos) throw Error(TG_ERR_INVALID_ARG, "Parquet: BYTE_ARRAY value runs past its page");
+        if (len > PQ_STR_MAX_LEN) throw Error(TG_ERR_UNSUPPORTED, "Parquet: string value of 16 MiB or more");
+        ents.push_back(pq_str_ent(stage_off + (uint64_t)pos, len));
+        pos += len;
+    }
+}
+
+// What a chunk's values are; decides a block's src_off and what a section without dictionary indices gets
+enum PqKind { PQ_KIND_FIXED, PQ_KIND_BOOL, PQ_KIND_STR };
+
+// A chunk's sections staged on the device and described for the expand / locate kernels
+struct PqStaged {
+    uint8_t* stage = nullptr;       // every section's value bytes, then the dictionary; freed through deferred_free
+    std::vector<int64_t> sec_off;   // each section's offset in `stage`
+    size_t dict_off = 0;
+    std::vector<uint8_t> bits;      // chunk-relative validity (16 bytes of slack); empty: a required column
+    std::vector<PqBlock> blocks;
+    std::vector<PqRun> runs;        // dictionary-index and RLE BOOLEAN streams
+    std::vector<std::pair<uint32_t, uint32_t>> sec_runs;  // each section's runs [lo, hi) in `runs`
+    std::vector<uint64_t> plain_ents;  // BYTE_ARRAY: one entry per value of the PLAIN sections
+};
+
+// Section i: its levels -> st.bits, its blocks of <= PQ_BLOCK_ROWS rows (non-NULL counts from popcounts of the bits), and
+// the run table of its dictionary indices / RLE BOOLEAN values, or the check / entries of its PLAIN values
+void cut_section(const PqChunk& pc, size_t i, PqKind kind, size_t sw, PqStaged& st) {
+    const PqSection& s = pc.secs[i];
+    const bool levels = !st.bits.empty();
+    const uint64_t off = (uint64_t)st.sec_off[i];
+    if (levels) decode_levels(s.levels, s.levels + s.levels_bytes, st.bits.data(), s.first_row, s.n_rows);
+    const uint32_t run_lo = (uint32_t)st.runs.size();
+    const size_t blk_lo = st.blocks.size();
+    const uint64_t ent_lo = (uint64_t)st.plain_ents.size();
+    int64_t prefix = 0;
+    for (int64_t r = 0; r < s.n_rows; r += PQ_BLOCK_ROWS) {
+        const int64_t nr = std::min<int64_t>(PQ_BLOCK_ROWS, s.n_rows - r);
+        // the block's first value: an index into plain_ents (BYTE_ARRAY), a bit offset (BOOLEAN) or a byte offset in `stage`
+        const uint64_t src = kind == PQ_KIND_STR ? ent_lo + (uint64_t)prefix
+                             : kind == PQ_KIND_BOOL ? off * 8 + (uint64_t)prefix
+                                                    : off + (uint64_t)prefix * sw;
+        st.blocks.push_back(PqBlock{src, (uint32_t)(s.first_row + r), (uint32_t)nr, (uint32_t)prefix, 0u, 0u, 0u});
+        prefix += levels ? count_ones(st.bits.data(), s.first_row + r, s.first_row + r + nr) : nr;
+    }
+    if (s.dict) {
+        if (prefix > 0 && pc.dict_count <= 0) throw Error(TG_ERR_INVALID_ARG, "Parquet: dictionary-encoded page without a dictionary page");
+        parse_index_runs(s.values, s.values + s.values_bytes, prefix, off, st.runs);
+    } else if (s.rle) {
+        parse_bool_runs(s.values, s.values_bytes, prefix, off, st.runs);
+    } else if (kind == PQ_KIND_STR) {
+        walk_plain_strings(s.values, s.values_bytes, prefix, off, st.plain_ents);
+    } else if (kind == PQ_KIND_BOOL ? s.values_bytes < (prefix + 7) / 8 : prefix * (int64_t)sw != s.values_bytes) {
+        throw Error(TG_ERR_INVALID_ARG, "Parquet: PLAIN page holds " + std::to_string(s.values_bytes) + " value bytes for " +
+                                            std::to_string(prefix) + " non-null rows");
+    }
+    const uint32_t run_hi = (uint32_t)st.runs.size();
+    st.sec_runs[i] = {run_lo, run_hi};
+    if (s.dict || s.rle)
+        for (size_t k = blk_lo; k < st.blocks.size(); ++k) {
+            st.blocks[k].run_lo = run_lo;
+            st.blocks[k].run_hi = run_hi > run_lo ? run_hi : run_lo + 1;  // (an all-NULL section has no runs: never looked up)
+        }
+}
+
+// Stages a chunk: every section's value bytes at a 16-byte aligned place of one device block, then the dictionary
+// (dict_count * sw bytes of fixed-width values, or the whole page body of a BYTE_ARRAY dictionary), then 64 bytes of
+// slack. Staging a pageable source is a host memcpy into the pinned ring per piece, so a helper thread cuts the sections
+// (cut_section) meanwhile. sw: the file width of a fixed-width value.
+PqStaged stage_chunk(Engine& e, const PqChunk& pc, PqKind kind, size_t sw, int32_t max_def_level, int64_t num_values) {
+    PqStaged st;
+    size_t stage_bytes = 0;
+    for (const PqSection& s : pc.secs) {
+        st.sec_off.push_back((int64_t)stage_bytes);
+        stage_bytes += r16((size_t)s.values_bytes);
+    }
+    st.dict_off = stage_bytes;
+    const size_t dict_b = kind == PQ_KIND_STR ? (size_t)pc.dict_bytes : (size_t)pc.dict_count * sw;
+    stage_bytes += r16(dict_b) + 64;
+    if (stage_bytes >= PQ_STAGE_MAX) throw Error(TG_ERR_UNSUPPORTED, "Parquet: column chunk of 1 TiB or more");
+    st.sec_runs.resize(pc.secs.size());
+    std::exception_ptr cut_err;
+    std::thread helper([&]() {
+        try {
+            if (max_def_level > 0) st.bits.assign((size_t)(num_values + 7) / 8 + 16, 0);
+            st.blocks.reserve((size_t)num_values / PQ_BLOCK_ROWS + pc.secs.size() + 1);
+            for (size_t i = 0; i < pc.secs.size(); ++i) cut_section(pc, i, kind, sw, st);
+        } catch (...) {
+            cut_err = std::current_exception();
+        }
+    });
+    struct Join {
+        std::thread& t;
+        ~Join() {
+            if (t.joinable()) t.join();
+        }
+    } join{helper};
+    st.stage = e.dev_alloc(stage_bytes);
+    e.deferred_free.emplace_back(st.stage, stage_bytes);  // released by the next sync_copies(), also on the error paths
+    for (size_t i = 0; i < pc.secs.size(); ++i)
+        if (pc.secs[i].values_bytes) e.h2d(st.stage + st.sec_off[i], pc.secs[i].values, (size_t)pc.secs[i].values_bytes);
+    if (dict_b) e.h2d(st.stage + st.dict_off, pc.dict_values, dict_b);
+    helper.join();
+    if (cut_err) std::rethrow_exception(cut_err);
+    return st;
+}
+
+// Host mirror of pq_run_value: the value of dense index d of section i, from its runs and its host bytes
+uint64_t pq_run_value_host(const PqChunk& pc, const PqStaged& st, size_t i, uint32_t d) {
+    uint32_t lo = st.sec_runs[i].first, hi = st.sec_runs[i].second;
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (st.runs[mid].start <= d) lo = mid;
+        else hi = mid;
+    }
+    const PqRun& run = st.runs[lo];
+    if (!run.packed) return run.data;
+    const PqSection& s = pc.secs[i];
+    const uint64_t bit = (uint64_t)(d - run.start) * run.bw;
+    const size_t byte = (size_t)(run.data - (uint64_t)st.sec_off[i] + (bit >> 3));
+    uint64_t w = 0;
+    memcpy(&w, s.values + byte, std::min<size_t>(8, (size_t)s.values_bytes - byte));
+    return run.bw ? (w >> (bit & 7)) & (((uint64_t)1 << run.bw) - 1ull) : 0ull;
+}
+
+// The column's first values (at most 4096; INT96 converted, so the pivot is the one of the same instants delivered as
+// timestamp[ns]), which the pivot of the shifted sums is chosen from like on the Arrow path (same K, bit-identical sums):
+// the first section with values, its PLAIN values or the dictionary entries its indices name
+std::vector<uint64_t> head_values(const PqChunk& pc, const PqStaged& st, size_t sw, bool int96) {
+    auto at = [&](const uint8_t* p) {
+        uint64_t v;
+        if (int96) v = pq_int96_ns_host(p);
+        else memcpy(&v, p, 8);
+        return v;
+    };
+    std::vector<uint64_t> head;
+    for (size_t i = 0; i < pc.secs.size() && head.empty(); ++i) {
+        const PqSection& s = pc.secs[i];
+        if (!s.dict) {
+            const int64_t n = std::min<int64_t>(s.values_bytes / (int64_t)sw, 4096);
+            for (int64_t k = 0; k < n; ++k) head.push_back(at(s.values + (size_t)k * sw));
+        } else if (st.sec_runs[i].second > st.sec_runs[i].first) {
+            const PqRun& last = st.runs[st.sec_runs[i].second - 1];
+            const uint32_t n = std::min<uint32_t>(last.start + last.count, 4096);
+            for (uint32_t d = 0; d < n; ++d) {
+                const uint64_t idx = std::min<uint64_t>(pq_run_value_host(pc, st, i, d), (uint64_t)pc.dict_count - 1);
+                head.push_back(at(pc.dict_values + (size_t)idx * sw));
+            }
+        }
+    }
+    return head;
+}
+
+// One device block of tables, on deferred_free from the start: bits | blocks | runs, then the caller's `extra` tables
+// ({host bytes or nullptr for device scratch, size}), each 16-byte aligned, 64 bytes of slack. Returns where each starts
+// (bits: nullptr for a required column).
+std::vector<uint8_t*> upload_tables(Engine& e, const PqStaged& st, int64_t num_values,
+                                    std::initializer_list<std::pair<const void*, size_t>> extra = {}) {
+    std::vector<std::pair<const void*, size_t>> parts = {{st.bits.data(), st.bits.empty() ? 0 : (size_t)(num_values + 7) / 8},
+                                                         {st.blocks.data(), st.blocks.size() * sizeof(PqBlock)},
+                                                         {st.runs.data(), st.runs.size() * sizeof(PqRun)}};
+    parts.insert(parts.end(), extra);
+    size_t total = 64;
+    for (auto& p : parts) total += r16(p.second);
+    uint8_t* q = e.dev_alloc(total);
+    e.deferred_free.emplace_back(q, total);
+    std::vector<uint8_t*> at;
+    for (auto& p : parts) {
+        at.push_back(q);
+        if (p.first && p.second) e.h2d(q, p.first, p.second);
+        q += r16(p.second);
+    }
+    if (st.bits.empty()) at[0] = nullptr;
+    return at;
+}
 }  // namespace
+
+// Host-only: the validity bitmap (chunk-relative, LSB first, (num_values + 7) / 8 bytes) a flat optional column chunk
+// decodes to, and its non-NULL count. The device path builds exactly this before it scatters the values.
+int64_t parquet_chunk_validity(const uint8_t* chunk, int64_t n_bytes, int64_t num_values, uint8_t* out_bits) {
+    const std::vector<tg_parquet_page> pages = walk_pages(chunk, n_bytes);
+    std::vector<uint8_t> bits((size_t)(num_values + 7) / 8 + 16, 0);
+    int64_t rows = 0;
+    for (auto& pg : pages) {
+        if (pg.page_type != PQ_DATA_PAGE && pg.page_type != PQ_DATA_PAGE_V2) continue;
+        if (rows + pg.num_values > num_values) throw Error(TG_ERR_INVALID_ARG, "Parquet: more values than the chunk metadata says");
+        PqSection s{};
+        split_levels(pg, chunk + pg.body_offset, pg.body_bytes, true, s);
+        decode_levels(s.levels, s.levels + s.levels_bytes, bits.data(), rows, pg.num_values);
+        rows += pg.num_values;
+    }
+    if (out_bits) memcpy(out_bits, bits.data(), (size_t)(num_values + 7) / 8);
+    return count_ones(bits.data(), 0, rows);
+}
 
 static void append_parquet_utf8(Table& t, const std::string& name, int32_t max_def_level, int32_t codec, const uint8_t* chunk, int64_t n_bytes,
                                 int64_t num_values);
@@ -996,200 +1132,73 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
 
     PqChunk pc;
     collect_sections(chunk, n_bytes, codec, max_def_level, num_values, dtype, pc);
-    using Section = PqSection;
-    std::vector<PqSection>& secs = pc.secs;
-    const uint8_t* dict_values = pc.dict_values;
-    int64_t dict_count = pc.dict_count;
     if (num_values == 0) {
         t.n_rows = std::max(t.n_rows, c.n_rows);
         return;
     }
-    const bool any_dict = pc.any_dict;
 
-    // ---- the value sections travel while a helper thread expands the definition levels: staging a pageable source is
-    // a host memcpy into the pinned ring per piece, so the two halves of the host work run side by side. Every page's
-    // value section goes to a 16-byte aligned place in a staging block (PLAIN pages of required columns: straight into
-    // place); the dictionary's values sit in the same block ----
+    // PLAIN pages of required columns go straight into place; everything else is staged and expanded by a kernel
     if (is_bool) e.dev_reserve(c.values, (size_t)(have + num_values + 7) / 8, (size_t)(have + 7) / 8);
     else e.dev_reserve(c.values, (size_t)(have + num_values) * w, (size_t)have * w);
     uint8_t* dst = c.values.p + (size_t)have * w;
-    std::vector<int64_t> stage_off(secs.size(), -1);
-    size_t stage_bytes = 0;
-    uint8_t* stage = nullptr;
-    std::vector<uint8_t> bits;
-    std::vector<PqBlock> blocks;
-    std::vector<PqRun> runs;
-    std::vector<std::pair<uint32_t, uint32_t>> sec_runs(secs.size());  // each section's runs [lo, hi) in `runs`
-    const bool direct = max_def_level == 0 && !any_dict && sw == w && !is_bool;
+    const bool direct = max_def_level == 0 && !pc.any_dict && sw == w && !is_bool;
+    PqStaged st;
     if (direct) {
-        for (auto& s : secs) {
+        for (auto& s : pc.secs) {
             if (s.values_bytes != s.n_rows * (int64_t)w) throw Error(TG_ERR_INVALID_ARG, "Parquet: PLAIN page size does not match its value count");
             e.h2d(dst + (size_t)s.first_row * w, s.values, (size_t)s.values_bytes);
         }
     } else {
-        for (size_t i = 0; i < secs.size(); ++i) {
-            stage_off[i] = (int64_t)stage_bytes;
-            stage_bytes += ((size_t)secs[i].values_bytes + 15) & ~(size_t)15;
-        }
-        const size_t dict_off = stage_bytes;
-        stage_bytes += (((size_t)dict_count * sw) + 15) & ~(size_t)15;
-        stage_bytes += 64;
-        // definition levels -> chunk-relative validity bits + blocks (+ the run tables of dictionary-index / RLE sections)
-        std::exception_ptr decode_err;
-        auto decode = [&]() {
-            try {
-                if (max_def_level > 0) bits.assign((size_t)(num_values + 7) / 8 + 16, 0);
-                blocks.reserve((size_t)num_values / PQ_BLOCK_ROWS + secs.size() + 1);
-                for (size_t i = 0; i < secs.size(); ++i) {
-                    const Section& s = secs[i];
-                    if (max_def_level > 0) decode_levels(s.levels, s.levels + s.levels_bytes, bits.data(), s.first_row, s.n_rows);
-                    const uint32_t run_lo = (uint32_t)runs.size();
-                    const size_t blk_lo = blocks.size();
-                    int64_t prefix = 0;
-                    for (int64_t r = 0; r < s.n_rows; r += PQ_BLOCK_ROWS) {
-                        const int64_t nr = std::min<int64_t>(PQ_BLOCK_ROWS, s.n_rows - r);
-                        // (Boolean PLAIN: the BIT offset of the block's first value)
-                        const uint64_t src = is_bool ? (uint64_t)stage_off[i] * 8 + (uint64_t)prefix : (uint64_t)stage_off[i] + (uint64_t)prefix * sw;
-                        blocks.push_back(PqBlock{src, (uint32_t)(s.first_row + r), (uint32_t)nr, (uint32_t)prefix, 0u, 0u, 0u});
-                        prefix += max_def_level > 0 ? count_ones(bits.data(), s.first_row + r, s.first_row + r + nr) : nr;
-                    }
-                    if (s.dict || s.rle) {
-                        if (s.dict) {
-                            if (prefix > 0 && dict_count <= 0) throw Error(TG_ERR_INVALID_ARG, "Parquet: dictionary-encoded page without a dictionary page");
-                            parse_index_runs(s.values, s.values + s.values_bytes, prefix, (uint64_t)stage_off[i], runs);
-                        } else {
-                            parse_bool_runs(s.values, s.values_bytes, prefix, (uint64_t)stage_off[i], runs);
-                        }
-                        const uint32_t run_hi = (uint32_t)runs.size();
-                        sec_runs[i] = {run_lo, run_hi};
-                        for (size_t k = blk_lo; k < blocks.size(); ++k) {
-                            blocks[k].run_lo = run_lo;
-                            blocks[k].run_hi = run_hi > run_lo ? run_hi : run_lo + 1;  // (an all-NULL section has no runs: never looked up)
-                        }
-                    } else if (is_bool ? s.values_bytes < (prefix + 7) / 8 : prefix * (int64_t)sw != s.values_bytes) {
-                        throw Error(TG_ERR_INVALID_ARG, "Parquet: PLAIN page holds " + std::to_string(s.values_bytes) + " value bytes for " +
-                                                            std::to_string(prefix) + " non-null rows");
-                    }
-                }
-            } catch (...) {
-                decode_err = std::current_exception();
-            }
-        };
-        std::thread helper(decode);
-        struct Join {
-            std::thread& t;
-            ~Join() {
-                if (t.joinable()) t.join();
-            }
-        } join{helper};
-        stage = e.dev_alloc(stage_bytes);
-        e.deferred_free.emplace_back(stage, stage_bytes);  // released by the next sync_copies(), also on the error paths
-        for (size_t i = 0; i < secs.size(); ++i)
-            if (secs[i].values_bytes) e.h2d(stage + stage_off[i], secs[i].values, (size_t)secs[i].values_bytes);
-        if (dict_count > 0) e.h2d(stage + dict_off, dict_values, (size_t)dict_count * sw);
-        helper.join();
-        if (decode_err) std::rethrow_exception(decode_err);
+        st = stage_chunk(e, pc, is_bool ? PQ_KIND_BOOL : PQ_KIND_FIXED, sw, max_def_level, num_values);
+    }
+    if (!c.pivot_set && (stored == TG_INT64 || stored == TG_FLOAT64)) {
+        const std::vector<uint64_t> head = head_values(pc, st, sw, int96);
+        if (!head.empty()) set_pivot_host(c, stored, (int64_t)head.size(), head.data(), nullptr, 0);
+    }
+    // validity through the common path (keeps the host mirror of a partial tail byte)
+    append_validity(e, c, have, st.bits.empty() ? nullptr : st.bits.data(), 0, num_values);
 
-        // ---- pivot of the shifted sums: from the column's FIRST values, like the Arrow path (same K, bit-identical sums):
-        // the first PLAIN page's dense values, or the dictionary entries the first page's first indices name (INT96:
-        // converted, so the pivot is the one of the same instants delivered as timestamp[ns]) ----
-        auto head_value = [&](const uint8_t* p) {
-            uint64_t v;
-            if (int96) v = pq_int96_ns_host(p);
-            else memcpy(&v, p, 8);
-            return v;
-        };
-        if (!c.pivot_set && (stored == TG_INT64 || stored == TG_FLOAT64)) {
-            for (auto& s0 : secs) {
-                if (s0.n_rows == 0) continue;
-                std::vector<uint64_t> head;
-                if (!s0.dict) {
-                    const int64_t nv = std::min<int64_t>(s0.values_bytes / (int64_t)sw, 4096);
-                    for (int64_t k = 0; k < nv; ++k) head.push_back(head_value(s0.values + (size_t)k * sw));
-                } else if (dict_count > 0) {
-                    std::vector<uint32_t> idx;
-                    try {
-                        decode_first_indices(s0.values, s0.values + s0.values_bytes, s0.n_rows, 256, idx);
-                    } catch (Error&) {  // (a malformed stream is reported by the run walk below, with its own message)
-                    }
-                    for (uint32_t k : idx) head.push_back(head_value(dict_values + (size_t)std::min<int64_t>(k, dict_count - 1) * sw));
-                }
-                if (!head.empty()) {
-                    set_pivot_host(c, stored, (int64_t)head.size(), head.data(), nullptr, 0);
-                    break;
-                }
-            }
-        }
-        // ---- validity through the common path (keeps the host mirror of a partial tail byte) ----
-        append_validity(e, c, have, max_def_level > 0 ? bits.data() : nullptr, 0, num_values);
-
-        // ---- expand ----
-        const size_t bits_b = max_def_level > 0 ? (((size_t)(num_values + 7) / 8 + 15) & ~(size_t)15) : 0;
-        const size_t blk_b = (blocks.size() * sizeof(PqBlock) + 15) & ~(size_t)15, run_b = runs.size() * sizeof(PqRun);
-        uint8_t* aux = e.dev_alloc(bits_b + blk_b + run_b + 64);
-        if (bits_b) e.h2d(aux, bits.data(), (size_t)(num_values + 7) / 8);
-        e.h2d(aux + bits_b, blocks.data(), blocks.size() * sizeof(PqBlock));
-        if (run_b) e.h2d(aux + bits_b + blk_b, runs.data(), run_b);
-        // h2d of pageable memory returns once the bytes sit in the pinned ring, so `bits` / `blocks` / `inflated` may go out of scope
-        const int64_t nb = (int64_t)blocks.size();
-        const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((nb + PQ_THREADS / 32 - 1) / (PQ_THREADS / 32), (int64_t)e.sm_count * 8));
-        const uint8_t* d_bits = bits_b ? aux : nullptr;
-        const PqBlock* d_blocks = reinterpret_cast<const PqBlock*>(aux + bits_b);
-        const PqRun* d_runs = reinterpret_cast<const PqRun*>(aux + bits_b + blk_b);
+    if (!direct) {
+        // h2d of pageable memory returns once the bytes sit in the pinned ring, so `st` / `pc` may go out of scope
+        const std::vector<uint8_t*> d = upload_tables(e, st, num_values);
+        const int64_t nb = (int64_t)st.blocks.size();
+        const int grid = pq_str_grid(e, nb);
+        const PqBlock* d_blocks = reinterpret_cast<const PqBlock*>(d[1]);
+        const PqRun* d_runs = reinterpret_cast<const PqRun*>(d[2]);
+        const uint8_t* dict = st.stage + st.dict_off;
         if (is_bool) {
             // the kernel ORs whole words: the new bytes start at zero (the partial byte before them keeps its earlier rows)
             const size_t z0 = (size_t)(have + 7) / 8, z1 = (size_t)(have + num_values + 7) / 8;
             if (z1 > z0) TG_CUDA(cudaMemsetAsync(c.values.p + z0, 0, z1 - z0, e.copy_stream));
-            pq_expand_bool_kernel<<<grid, PQ_THREADS, 0, e.copy_stream>>>(stage, d_bits, d_blocks, nb, reinterpret_cast<uint32_t*>(c.values.p),
+            pq_expand_bool_kernel<<<grid, PQ_THREADS, 0, e.copy_stream>>>(st.stage, d[0], d_blocks, nb, reinterpret_cast<uint32_t*>(c.values.p),
                                                                           (uint64_t)have, d_runs);
         } else if (int96) {
-            pq_expand_kernel<uint64_t, PqLoadInt96><<<grid, PQ_THREADS, 0, e.copy_stream>>>(stage, d_bits, d_blocks, nb, reinterpret_cast<uint64_t*>(dst),
-                                                                                           d_runs, stage + dict_off, (uint32_t)dict_count);
+            pq_expand_kernel<uint64_t, PqLoadInt96><<<grid, PQ_THREADS, 0, e.copy_stream>>>(st.stage, d[0], d_blocks, nb, reinterpret_cast<uint64_t*>(dst),
+                                                                                           d_runs, dict, (uint32_t)pc.dict_count);
         } else if (w == 8) {
-            pq_expand_kernel<uint64_t><<<grid, PQ_THREADS, 0, e.copy_stream>>>(stage, d_bits, d_blocks, nb, reinterpret_cast<uint64_t*>(dst), d_runs,
-                                                                               stage + dict_off, (uint32_t)dict_count);
+            pq_expand_kernel<uint64_t><<<grid, PQ_THREADS, 0, e.copy_stream>>>(st.stage, d[0], d_blocks, nb, reinterpret_cast<uint64_t*>(dst), d_runs,
+                                                                               dict, (uint32_t)pc.dict_count);
         } else {
-            pq_expand_kernel<uint32_t><<<grid, PQ_THREADS, 0, e.copy_stream>>>(stage, d_bits, d_blocks, nb, reinterpret_cast<uint32_t*>(dst), d_runs,
-                                                                               stage + dict_off, (uint32_t)dict_count);
+            pq_expand_kernel<uint32_t><<<grid, PQ_THREADS, 0, e.copy_stream>>>(st.stage, d[0], d_blocks, nb, reinterpret_cast<uint32_t*>(dst), d_runs,
+                                                                               dict, (uint32_t)pc.dict_count);
         }
         TG_CUDA(cudaGetLastError());
         e.launches += 1;
-        e.deferred_free.emplace_back(aux, bits_b + blk_b + run_b + 64);
-    }
-    if (direct) {
-        if (!c.pivot_set && !secs.empty() && (dtype == TG_INT64 || dtype == TG_FLOAT64)) {
-            const int64_t nv = std::min<int64_t>(secs[0].values_bytes / (int64_t)w, 4096);
-            if (nv > 0) {
-                std::vector<uint64_t> head((size_t)nv);
-                memcpy(head.data(), secs[0].values, (size_t)nv * 8);
-                set_pivot_host(c, dtype, nv, head.data(), nullptr, 0);
-            }
-        }
-        append_validity(e, c, have, nullptr, 0, num_values);
     }
     if (is_bool) {
         // host mirror of the value bitmap's last partial byte (table_append_host continues from it): its rows before this
-        // chunk from the old mirror, the chunk's own (at most 7) rows decoded here from the staged sources
+        // chunk from the old mirror, the chunk's own (at most 7) rows decoded here from the host copies of the sections
         const int64_t total = have + num_values, lo = total & ~(int64_t)7;
         uint8_t tail = lo < have ? (uint8_t)(c.tail_vbyte & ((1u << (have - lo)) - 1u)) : 0;
         for (int64_t row = std::max(lo, have); row < total; ++row) {
             const int64_t r = row - have;
-            if (max_def_level > 0 && !((bits[(size_t)(r >> 3)] >> (r & 7)) & 1)) continue;
-            size_t i = secs.size() - 1;
-            while (secs[i].first_row > r) --i;
-            const Section& s = secs[i];
-            const int64_t d = max_def_level > 0 ? count_ones(bits.data(), s.first_row, r) : r - s.first_row;
-            uint32_t v;
-            if (!s.rle) {
-                v = (s.values[d >> 3] >> (d & 7)) & 1u;
-            } else {
-                uint32_t k = sec_runs[i].second - 1;
-                while (runs[k].start > (uint64_t)d) --k;
-                const PqRun& run = runs[k];
-                const int64_t bit = d - (int64_t)run.start;
-                v = run.packed ? (s.values[run.data - (uint64_t)stage_off[i] + (uint64_t)(bit >> 3)] >> (bit & 7)) & 1u : (uint32_t)run.data;
-            }
-            tail |= (uint8_t)(v << (row - lo));
+            if (!st.bits.empty() && !((st.bits[(size_t)(r >> 3)] >> (r & 7)) & 1)) continue;
+            size_t i = pc.secs.size() - 1;
+            while (pc.secs[i].first_row > r) --i;
+            const PqSection& s = pc.secs[i];
+            const int64_t d = st.bits.empty() ? r - s.first_row : count_ones(st.bits.data(), s.first_row, r);
+            const uint64_t v = s.rle ? pq_run_value_host(pc, st, i, (uint32_t)d) : (uint64_t)(s.values[d >> 3] >> (d & 7));
+            tail |= (uint8_t)((v & 1u) << (row - lo));
         }
         c.tail_vbyte = tail;
         c.value_bytes = (total + 7) / 8;
@@ -1211,24 +1220,6 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
 // The host walks what is serial by construction: page headers, run headers, and the interleaved length prefixes of PLAIN
 // pages (one entry {staging offset, length} per value); the dictionary page's own entries likewise (it is small).
 // ---------------------------------------------------------------------------------------------------------------------
-namespace {
-// entries: pq_str_ent / PQ_STR_MAX_LEN (str_entries.cuh)
-// walks `count` PLAIN BYTE_ARRAY values at p (length prefixes interleaved) into entries; stage_off = where p sits in staging
-void walk_plain_strings(const uint8_t* p, int64_t n_bytes, int64_t count, uint64_t stage_off, std::vector<uint64_t>& ents) {
-    int64_t pos = 0;
-    for (int64_t i = 0; i < count; ++i) {
-        if (pos + 4 > n_bytes) throw Error(TG_ERR_INVALID_ARG, "Parquet: BYTE_ARRAY page is truncated");
-        uint32_t len;
-        memcpy(&len, p + pos, 4);
-        pos += 4;
-        if ((int64_t)len > n_bytes - pos) throw Error(TG_ERR_INVALID_ARG, "Parquet: BYTE_ARRAY value runs past its page");
-        if (len > PQ_STR_MAX_LEN) throw Error(TG_ERR_UNSUPPORTED, "Parquet: string value of 16 MiB or more");
-        ents.push_back(pq_str_ent(stage_off + (uint64_t)pos, len));
-        pos += len;
-    }
-}
-}  // namespace
-
 __device__ __forceinline__ uint64_t pq_row_entry(const PqBlock& blk, uint32_t rank, const uint8_t* __restrict__ stage,
                                                  const PqRun* __restrict__ runs, const uint64_t* __restrict__ plain_ents,
                                                  const uint64_t* __restrict__ dict_ents, uint32_t dict_count) {
@@ -1331,121 +1322,38 @@ static void append_parquet_utf8(Table& t, const std::string& name, int32_t max_d
     const int64_t have = c.n_rows;
     PqChunk pc;
     collect_sections(chunk, n_bytes, codec, max_def_level, num_values, TG_UTF8, pc);
-    std::vector<PqSection>& secs = pc.secs;
     if (num_values == 0) {
         t.n_rows = std::max(t.n_rows, c.n_rows);
         return;
     }
-    // ---- staging layout: every section's value bytes as they are, then the dictionary page's body
-    std::vector<int64_t> stage_off(secs.size(), 0);
-    size_t stage_bytes = 0;
-    for (size_t i = 0; i < secs.size(); ++i) {
-        stage_off[i] = (int64_t)stage_bytes;
-        stage_bytes += ((size_t)secs[i].values_bytes + 15) & ~(size_t)15;
-    }
-    const size_t dict_off = stage_bytes;
-    stage_bytes += ((size_t)pc.dict_bytes + 15) & ~(size_t)15;
-    stage_bytes += 64;
-    if (stage_bytes >= PQ_STAGE_MAX) throw Error(TG_ERR_UNSUPPORTED, "Parquet: column chunk of 1 TiB or more");
-    std::vector<uint8_t> bits;
-    std::vector<PqBlock> blocks;
-    std::vector<PqRun> runs;
-    std::vector<uint64_t> plain_ents, dict_ents;
+    const PqStaged st = stage_chunk(e, pc, PQ_KIND_STR, 0, max_def_level, num_values);
+    std::vector<uint64_t> dict_ents;
     if (pc.dict_count > 0) {
         dict_ents.reserve((size_t)pc.dict_count);
-        walk_plain_strings(pc.dict_values, pc.dict_bytes, pc.dict_count, (uint64_t)dict_off, dict_ents);
+        walk_plain_strings(pc.dict_values, pc.dict_bytes, pc.dict_count, (uint64_t)st.dict_off, dict_ents);
     }
-    std::exception_ptr decode_err;
-    auto decode = [&]() {
-        try {
-            if (max_def_level > 0) bits.assign((size_t)(num_values + 7) / 8 + 16, 0);
-            blocks.reserve((size_t)num_values / PQ_BLOCK_ROWS + secs.size() + 1);
-            for (size_t i = 0; i < secs.size(); ++i) {
-                const PqSection& s = secs[i];
-                if (max_def_level > 0) decode_levels(s.levels, s.levels + s.levels_bytes, bits.data(), s.first_row, s.n_rows);
-                const uint32_t run_lo = (uint32_t)runs.size();
-                const size_t blk_lo = blocks.size();
-                const uint64_t ent_lo = (uint64_t)plain_ents.size();
-                int64_t prefix = 0;
-                for (int64_t r = 0; r < s.n_rows; r += PQ_BLOCK_ROWS) {
-                    const int64_t nr = std::min<int64_t>(PQ_BLOCK_ROWS, s.n_rows - r);
-                    blocks.push_back(PqBlock{ent_lo + (uint64_t)prefix, (uint32_t)(s.first_row + r), (uint32_t)nr, (uint32_t)prefix, 0u, 0u, 0u});
-                    prefix += max_def_level > 0 ? count_ones(bits.data(), s.first_row + r, s.first_row + r + nr) : nr;
-                }
-                if (s.dict) {
-                    if (prefix > 0 && pc.dict_count <= 0) throw Error(TG_ERR_INVALID_ARG, "Parquet: dictionary-encoded page without a dictionary page");
-                    parse_index_runs(s.values, s.values + s.values_bytes, prefix, (uint64_t)stage_off[i], runs);
-                    const uint32_t run_hi = (uint32_t)runs.size();
-                    for (size_t k = blk_lo; k < blocks.size(); ++k) {
-                        blocks[k].run_lo = run_lo;
-                        blocks[k].run_hi = run_hi > run_lo ? run_hi : run_lo + 1;
-                    }
-                } else {
-                    walk_plain_strings(s.values, s.values_bytes, prefix, (uint64_t)stage_off[i], plain_ents);
-                }
-            }
-        } catch (...) {
-            decode_err = std::current_exception();
-        }
-    };
-    std::thread helper(decode);
-    struct Join {
-        std::thread& t;
-        ~Join() {
-            if (t.joinable()) t.join();
-        }
-    } join{helper};
-    uint8_t* stage = e.dev_alloc(stage_bytes);
-    e.deferred_free.emplace_back(stage, stage_bytes);
-    for (size_t i = 0; i < secs.size(); ++i)
-        if (secs[i].values_bytes) e.h2d(stage + stage_off[i], secs[i].values, (size_t)secs[i].values_bytes);
-    if (pc.dict_bytes > 0) e.h2d(stage + dict_off, pc.dict_values, (size_t)pc.dict_bytes);
-    helper.join();
-    if (decode_err) std::rethrow_exception(decode_err);
+    append_validity(e, c, have, st.bits.empty() ? nullptr : st.bits.data(), 0, num_values);
 
-    append_validity(e, c, have, max_def_level > 0 ? bits.data() : nullptr, 0, num_values);
-
-    // ---- device tables: bits | blocks | runs | plain entries | dictionary entries | per-row entries | block totals + bases
-    const int64_t nb = (int64_t)blocks.size();
-    auto r16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
-    const size_t bits_b = max_def_level > 0 ? r16((size_t)(num_values + 7) / 8) : 0, blk_b = r16(blocks.size() * sizeof(PqBlock));
-    const size_t run_b = r16(runs.size() * sizeof(PqRun)), pe_b = r16(plain_ents.size() * 8), de_b = r16(dict_ents.size() * 8);
-    const size_t re_b = r16((size_t)num_values * 8), bb_b = r16((size_t)(nb + 1) * 8);
-    const size_t aux_b = bits_b + blk_b + run_b + pe_b + de_b + re_b + 2 * bb_b + 64;
-    uint8_t* aux = e.dev_alloc(aux_b);
-    e.deferred_free.emplace_back(aux, aux_b);
-    uint8_t* q = aux;
-    const uint8_t* d_bits = bits_b ? q : nullptr;
-    if (bits_b) e.h2d(q, bits.data(), (size_t)(num_values + 7) / 8);
-    q += bits_b;
-    const PqBlock* d_blocks = (const PqBlock*)q;
-    e.h2d(q, blocks.data(), blocks.size() * sizeof(PqBlock));
-    q += blk_b;
-    const PqRun* d_runs = (const PqRun*)q;
-    if (!runs.empty()) e.h2d(q, runs.data(), runs.size() * sizeof(PqRun));
-    q += run_b;
-    const uint64_t* d_pe = (const uint64_t*)q;
-    if (!plain_ents.empty()) e.h2d(q, plain_ents.data(), plain_ents.size() * 8);
-    q += pe_b;
-    const uint64_t* d_de = (const uint64_t*)q;
-    if (!dict_ents.empty()) e.h2d(q, dict_ents.data(), dict_ents.size() * 8);
-    q += de_b;
-    uint64_t* d_row = (uint64_t*)q;
-    q += re_b;
-    unsigned long long* d_tot = (unsigned long long*)q;
-    q += bb_b;
-    unsigned long long* d_base = (unsigned long long*)q;
-    const int grid = pq_str_grid(e, nb);
-    pq_str_locate_kernel<<<grid, PQ_THREADS, 0, e.copy_stream>>>(stage, d_bits, d_blocks, nb, d_runs, d_pe, d_de, (uint32_t)pc.dict_count, d_row, d_tot);
+    // device tables: bits | blocks | runs | plain entries | dictionary entries | per-row entries | block totals | bases
+    const int64_t nb = (int64_t)st.blocks.size();
+    const std::vector<uint8_t*> d = upload_tables(e, st, num_values,
+                                                  {{st.plain_ents.data(), st.plain_ents.size() * 8},
+                                                   {dict_ents.data(), dict_ents.size() * 8},
+                                                   {nullptr, (size_t)num_values * 8},
+                                                   {nullptr, (size_t)(nb + 1) * 8},
+                                                   {nullptr, (size_t)(nb + 1) * 8}});
+    Utf8Entries x;
+    x.stage = st.stage;
+    x.blocks = reinterpret_cast<const PqBlock*>(d[1]);
+    x.n_blocks = nb;
+    x.row_ent = reinterpret_cast<const uint64_t*>(d[5]);
+    x.block_bytes = reinterpret_cast<unsigned long long*>(d[6]);
+    x.block_base = reinterpret_cast<unsigned long long*>(d[7]);
+    pq_str_locate_kernel<<<pq_str_grid(e, nb), PQ_THREADS, 0, e.copy_stream>>>(
+        st.stage, d[0], x.blocks, nb, reinterpret_cast<const PqRun*>(d[2]), reinterpret_cast<const uint64_t*>(d[3]),
+        reinterpret_cast<const uint64_t*>(d[4]), (uint32_t)pc.dict_count, reinterpret_cast<uint64_t*>(d[5]), x.block_bytes);
     TG_CUDA(cudaGetLastError());
     e.launches += 1;
-    Utf8Entries x;
-    x.stage = stage;
-    x.blocks = d_blocks;
-    x.n_blocks = nb;
-    x.row_ent = d_row;
-    x.block_bytes = d_tot;
-    x.block_base = d_base;
     append_utf8_from_entries(e, t, c, x, num_values);
 }
 

@@ -24,6 +24,9 @@ __host__ __device__ inline uint64_t pq_str_ent(uint64_t off, uint32_t len) { ret
 constexpr uint32_t PQ_STR_MAX_LEN = (1u << 24) - 1u;
 constexpr uint64_t PQ_STAGE_MAX = (uint64_t)1 << 40;
 
+// staged sections and device tables start 16-byte aligned
+inline size_t r16(size_t x) { return (x + 15) & ~(size_t)15; }
+
 // error flags a locate kernel raises (and clamps past); the host turns them into a status
 constexpr uint32_t STR_ERR_RANGE = 1u;  // an index / view outside the dictionary / its data buffer: TG_ERR_INVALID_ARG
 constexpr uint32_t STR_ERR_LONG = 2u;   // a string of 16 MiB or more: TG_ERR_UNSUPPORTED

@@ -408,8 +408,6 @@ struct ArrowStage {
     Utf8Entries x;
 };
 
-size_t r16(size_t x) { return (x + 15) & ~(size_t)15; }
-
 // validity: `bits` read from bit `bit_off` (nullptr: no NULLs); staged from its byte bit_off / 8 on
 ArrowStage arrow_stage(Engine& e, size_t payload_b, size_t tables_b, int64_t n, const uint8_t* bits, int64_t bit_off, uint32_t* bit_shift) {
     ArrowStage s;
