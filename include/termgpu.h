@@ -382,6 +382,31 @@ TG_API tg_status tg_table_shuffle_fingerprints(tg_engine* eng, const char* table
  * (Binary, Utf8View, numeric, temporal, Boolean). Columns before the failing one may already hold the batch's rows. */
 TG_API tg_status tg_table_append_arrow(tg_table* t, const void* arrow_schema, const void* arrow_array);
 
+/*
+ * CSV -> HBM: replaces the reference's CsvSource::register -> DataFusion CSV scan (arrow-csv) -> Arrow batches -> H2D for
+ * the GPU path. `bytes` = the file's bytes, or any run of whole records (the caller maps the file; the engine does no I/O).
+ * Columns are given by the caller's schema, in file order: name + Arrow C Data Interface format string — "l" Int64, "i"
+ * Int32, "g" Float64, "b" Boolean, "u" Utf8, "tdD" Date32, "tss:" / "tsm:" / "tsu:" / "tsn:" naive Timestamp (temporal columns
+ * are declared as tg_table_set_column_arrow_type declares them); any other format is TG_ERR_UNSUPPORTED, naming the type.
+ * Format: records end at LF, CRLF or a lone CR, blank lines are skipped, the last record needs no terminator; `delimiter` is
+ * one byte, the quote is '"' (RFC 4180: it opens quoting at a field's start only, "" inside quotes is a quote, bytes after
+ * the closing quote are kept); `has_header` skips the first record without checking its names. An empty field, quoted or
+ * not, is NULL for every type. Values: Int64 / Int32 [+-]?[0-9]+ in range; Float64 [+-]?(d+[.d*] | .d+)([eE][+-]?d+)? and
+ * nan / inf / infinity (case-insensitive, signed), correctly rounded; Boolean true / false (case-insensitive); Date32
+ * YYYY-MM-DD; Timestamp YYYY-MM-DD[T| ]HH:MM:SS[.f{1,9}] (fraction digits past the unit dropped); Utf8 valid UTF-8. No
+ * whitespace is trimmed. A wrong field count, an unterminated quote, a value outside its grammar or range and invalid UTF-8
+ * are TG_ERR_INVALID_ARG, the message naming the line the record starts on and the column. A failed call leaves every
+ * column of the table as it was; appending to a column of another type is TG_ERR_TYPE_MISMATCH. *rows_out (may be NULL):
+ * the rows appended. The bytes are staged in chunks of TG_CSV_CHUNK_BYTES (default 256 MiB); a longer record grows its chunk.
+ */
+TG_API tg_status tg_table_append_csv(tg_table* t, const char* const* columns, const char* const* arrow_formats, int32_t n_columns,
+                                     const void* bytes, int64_t n_bytes, int32_t delimiter, int32_t has_header, int64_t* rows_out);
+/* Host-only: the value parser the device runs, for one raw field (quoted or not) of the given format (tests / diagnostics).
+ * `out` (may be NULL) receives the stored value — 8 bytes for Int64 / Float64 / Timestamp, 4 for Int32 / Date32, 1 (0 / 1)
+ * for Boolean, and for Utf8 the unescaped length as an int64 — and *is_null (may be NULL) whether the field is NULL.
+ * Errors as tg_table_append_csv's, without the line and column. */
+TG_API tg_status tg_csv_parse_value(const char* arrow_format, const void* field, int64_t n_bytes, void* out, int32_t* is_null);
+
 /* ------------------------------------------------------------------ plan ---- */
 
 /* A plan is the fused form of a Check / ValidationSuite / AnalysisRunner: every add_* returns a slot

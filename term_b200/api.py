@@ -464,6 +464,40 @@ class SessionContext:
                 F.check(F.lib().tg_table_set_column_arrow_type(t, col.encode(), fmt.encode()))
         return t
 
+    def register_csv(self, name: str, path, schema, has_header: bool = True, delimiter: str = ","):
+        """CsvSource::register for the GPU path: the file is mapped and tokenized / parsed into the Arrow layout in HBM
+        (tg_table_append_csv), with `schema` (a pyarrow.Schema, in file order) giving every column's name and type. Schema
+        inference is not done here: DataFusion infers with arrow-csv's rules, which the Rust shim would call on the host.
+        Unsupported types and malformed records raise; no half-registered table stays behind."""
+        if pa is None or not isinstance(schema, pa.Schema):
+            raise TypeError("register_csv needs a pyarrow.Schema")
+        d = delimiter.encode() if isinstance(delimiter, str) else bytes(delimiter)
+        if len(d) != 1:
+            raise ValueError("the delimiter must be one byte")
+        names, fmts = _strs([f.name for f in schema]), _strs([_arrow_format(f.type) for f in schema])
+        t = self._create(name)
+        try:
+            with open(path, "rb") as f:
+                size = os.fstat(f.fileno()).st_size
+                rows = C.c_int64()
+                if size == 0:
+                    F.check(F.lib().tg_table_append_csv(t, names[0], fmts[0], len(schema), None, 0, d[0], int(has_header), C.byref(rows)))
+                else:
+                    with mmap.mmap(f.fileno(), 0, flags=mmap.MAP_SHARED | getattr(mmap, "MAP_POPULATE", 0), prot=mmap.PROT_READ) as mm:
+                        view = np.frombuffer(mm, dtype=np.uint8)
+                        try:
+                            F.check(F.lib().tg_table_append_csv(t, names[0], fmts[0], len(schema), view.ctypes.data, size, d[0],
+                                                                int(has_header), C.byref(rows)))
+                        finally:
+                            del view  # the mapping cannot close while a buffer export is alive
+        except Exception:
+            F.lib().tg_table_drop(self._h, name.encode())
+            raise
+        if not hasattr(self, "_schemas"):
+            self._schemas = {}
+        self._schemas[name] = schema
+        return t
+
     def register_device_table(self, name: str, columns: Dict[str, dict], keepalive=None):
         """Adopt HBM-resident Arrow buffers without copying. columns[name] = dict(dtype=TG_*, n_rows=,
         values=ptr, validity=ptr|None, offsets=ptr|None, n_value_bytes=int). Pointers are device addresses."""
@@ -641,6 +675,18 @@ class AnalyzerOutput:
         if self.error:
             return None
         return {0: self.metric_double, 1: self.metric_long, 2: self.map}.get(self.metric_kind)
+
+
+def _arrow_format(typ):
+    """the Arrow C Data Interface format string of a pyarrow type (what tg_table_append_csv takes)"""
+    schema_buf = (C.c_uint8 * 72)()
+    typ._export_to_c(C.addressof(schema_buf))
+    try:
+        return C.cast(C.cast(C.addressof(schema_buf), C.POINTER(C.c_void_p))[0], C.c_char_p).value.decode()
+    finally:
+        rel = C.cast(C.addressof(schema_buf) + 56, C.POINTER(C.c_void_p))[0]
+        if rel:
+            C.CFUNCTYPE(None, C.c_void_p)(rel)(C.addressof(schema_buf))
 
 
 def _strs(cols):

@@ -22,6 +22,9 @@ int64_t parquet_decode_to_plain(int32_t encoding, int32_t elem_width, const uint
 void table_adopt_device(Table& t, const std::string& name, int32_t dtype, int64_t n, const void* d_values,
                         const int32_t* d_offsets, const uint8_t* d_validity, int64_t n_value_bytes);
 void table_append_arrow(Table& t, const void* schema_p, const void* array_p);
+void table_append_csv(Table& t, const std::vector<std::string>& names, const std::vector<std::string>& fmts, const uint8_t* bytes, int64_t n_bytes,
+                      int32_t delimiter, bool has_header, int64_t* rows_out);
+void csv_parse_value(const std::string& fmt, const uint8_t* p, int64_t n, void* out, int32_t* is_null);
 }  // namespace tg
 
 using namespace tg;
@@ -317,6 +320,25 @@ tg_status tg_table_adopt_device(tg_table* t, const char* name, int32_t dtype, in
     });
 }
 
+tg_status tg_table_append_csv(tg_table* t, const char* const* columns, const char* const* arrow_formats, int32_t n_columns, const void* bytes,
+                              int64_t n_bytes, int32_t delimiter, int32_t has_header, int64_t* rows_out) {
+    return guard([&] {
+        if (!t || (n_columns > 0 && (!columns || !arrow_formats)) || n_columns < 0) throw Error(TG_ERR_INVALID_ARG, "NULL argument");
+        std::vector<std::string> names, fmts;
+        for (int32_t i = 0; i < n_columns; ++i) {
+            if (!columns[i] || !arrow_formats[i]) throw Error(TG_ERR_INVALID_ARG, "NULL column name or format");
+            names.emplace_back(columns[i]);
+            fmts.emplace_back(arrow_formats[i]);
+        }
+        table_append_csv(*reinterpret_cast<Table*>(t), names, fmts, (const uint8_t*)bytes, n_bytes, delimiter, has_header != 0, rows_out);
+    });
+}
+tg_status tg_csv_parse_value(const char* arrow_format, const void* field, int64_t n_bytes, void* out, int32_t* is_null) {
+    return guard([&] {
+        if (!arrow_format) throw Error(TG_ERR_INVALID_ARG, "NULL argument");
+        csv_parse_value(arrow_format, (const uint8_t*)field, n_bytes, out, is_null);
+    });
+}
 tg_status tg_table_append_arrow(tg_table* t, const void* schema, const void* array) {
     return guard([&] {
         if (!t) throw Error(TG_ERR_INVALID_ARG, "NULL argument");

@@ -110,14 +110,15 @@ void Engine::dev_reserve(DevBuf& b, size_t need, size_t keep_bytes) {
     TG_CUDA(cudaMemsetAsync(b.p + need, 0, padded - need, copy_stream));
 }
 
-void Engine::h2d(void* dst, const void* src, size_t bytes) {
+void Engine::h2d(void* dst, const void* src, size_t bytes, cudaStream_t s) {
     if (bytes == 0) return;
+    if (!s) s = copy_stream;
     cudaPointerAttributes attr{};
     bool pinned_src = false;
     if (cudaPointerGetAttributes(&attr, src) == cudaSuccess) pinned_src = attr.type == cudaMemoryTypeHost;
     else cudaGetLastError();
     if (pinned_src) {
-        TG_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, copy_stream));
+        TG_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, s));
         return;
     }
     // pageable source: stage through the pinned ring so the CPU memcpy of chunk i+1 overlaps the DMA of chunk i
@@ -128,8 +129,8 @@ void Engine::h2d(void* dst, const void* src, size_t bytes) {
         pinned_next ^= 1;
         TG_CUDA(cudaEventSynchronize(pinned_free[k]));
         memcpy(pinned[k], (const uint8_t*)src + off, n);
-        TG_CUDA(cudaMemcpyAsync((uint8_t*)dst + off, pinned[k], n, cudaMemcpyHostToDevice, copy_stream));
-        TG_CUDA(cudaEventRecord(pinned_free[k], copy_stream));
+        TG_CUDA(cudaMemcpyAsync((uint8_t*)dst + off, pinned[k], n, cudaMemcpyHostToDevice, s));
+        TG_CUDA(cudaEventRecord(pinned_free[k], s));
         off += n;
     }
 }

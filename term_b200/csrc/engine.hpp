@@ -176,7 +176,8 @@ struct Engine {
     uint8_t* scratch(size_t bytes);
     uint8_t* host_scratch(size_t bytes);
     void dev_reserve(DevBuf& b, size_t need, size_t keep_bytes);
-    void h2d(void* dst, const void* src, size_t bytes);  // staged through the pinned ring unless src is pinned
+    // staged through the pinned ring unless src is pinned; queued on `s` (nullptr: copy_stream)
+    void h2d(void* dst, const void* src, size_t bytes, cudaStream_t s = nullptr);
     void sync_copies();
     // device blocks still read by work queued on copy_stream (Parquet staging): released by the next sync_copies()
     std::vector<std::pair<uint8_t*, size_t>> deferred_free;
@@ -190,6 +191,12 @@ void column_free(Engine& e, Column& c);
 Column* table_get_or_add(Table& t, const std::string& name, int32_t dtype);
 void set_pivot_host(Column& c, int32_t dtype, int64_t n, const void* values, const uint8_t* validity, int64_t bit_offset);
 void append_validity(Engine& e, Column& c, int64_t have, const uint8_t* validity, int64_t bit_offset, int64_t n);
+// device-side counterparts for the CSV path (csv.cu): `words` = a chunk-relative device bitmap of n rows (bit r of word r / 32),
+// last64 = its bits of rows n - 64 .. n - 1 (bit k: row n - 64 + k) read back from the device, zeros = its clear bits
+void append_validity_device(Engine& e, Column& c, int64_t have, const uint32_t* words, int64_t n, int64_t zeros, uint64_t last64);
+void append_bits_device(Engine& e, DevBuf& buf, uint8_t& tail, int64_t have, const uint32_t* words, int64_t n, uint64_t last64);
+// table_set_column_arrow_type without the engine's lock (the caller holds it)
+void declare_arrow_type(Column& c, const std::string& fmt);
 
 // jobs (each fills the partial state of the aggregates it owns)
 void exec_scan_jobs(Engine& e, Table& t, Plan& p, const std::vector<int>& agg_ids);   // engine.cu + scan.cu

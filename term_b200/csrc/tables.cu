@@ -145,6 +145,52 @@ void append_validity(Engine& e, Column& c, int64_t have, const uint8_t* validity
     }
 }
 
+// ORs a chunk-relative bitmap (32-bit words) into a column bitmap at bit `have`; the destination bits from `have` on are 0
+__global__ void merge_bits_kernel(uint32_t* __restrict__ dst, uint64_t have, const uint32_t* __restrict__ words, uint64_t n_words) {
+    for (uint64_t w = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; w < n_words; w += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t v = words[w];
+        if (!v) continue;
+        const uint64_t pos = have + 32 * w;
+        const uint32_t sh = (uint32_t)(pos & 31);
+        atomicOr(dst + (pos >> 5), v << sh);
+        if (sh && (v >> (32 - sh))) atomicOr(dst + (pos >> 5) + 1, v >> (32 - sh));
+    }
+}
+
+// the device counterpart of append_bits: appends n bits of a chunk-relative device bitmap to `buf` (holding `have` bits);
+// `tail` (host mirror of the last partial byte) continues from the read-back of the chunk's last 64 bits
+void append_bits_device(Engine& e, DevBuf& buf, uint8_t& tail, int64_t have, const uint32_t* words, int64_t n, uint64_t last64) {
+    if (n <= 0) return;
+    const int64_t total = have + n;
+    e.dev_reserve(buf, (size_t)(total + 7) / 8, (size_t)(have + 7) / 8);
+    // the partial byte keeps only its earlier rows (a device byte may hold stale bits past them), the bytes after it start at 0
+    const uint8_t part = (have & 7) ? (uint8_t)(tail & ((1u << (have & 7)) - 1u)) : 0;
+    const size_t b0 = (size_t)have / 8, b1 = (size_t)(total + 7) / 8;
+    TG_CUDA(cudaMemsetAsync(buf.p + b0, 0, b1 - b0, e.copy_stream));
+    if (part) e.h2d(buf.p + b0, &part, 1);
+    const uint64_t n_words = (uint64_t)(n + 31) / 32;
+    const int grid = (int)std::max<uint64_t>(1, std::min<uint64_t>((n_words + 255) / 256, (uint64_t)e.sm_count * 8));
+    merge_bits_kernel<<<grid, 256, 0, e.copy_stream>>>(reinterpret_cast<uint32_t*>(buf.p), (uint64_t)have, words, n_words);
+    TG_CUDA(cudaGetLastError());
+    e.launches += 1;
+    uint8_t t = 0;
+    for (int64_t row = total & ~(int64_t)7; row < total; ++row) {
+        const int bit = row < have ? (tail >> (row & 7)) & 1 : (int)((last64 >> (row - have - n + 64)) & 1);
+        t |= (uint8_t)(bit << (row & 7));
+    }
+    tail = t;
+}
+
+// the device counterpart of append_validity: the bitmap is materialised (all-ones for the earlier rows) when the column
+// first sees a NULL, as there
+void append_validity_device(Engine& e, Column& c, int64_t have, const uint32_t* words, int64_t n, int64_t zeros, uint64_t last64) {
+    if (zeros > 0 && !c.validity.p && have > 0) append_bits(e, c.validity, c.tail_byte, 0, nullptr, 0, have, nullptr);
+    if (zeros > 0 || c.validity.p) {
+        append_bits_device(e, c.validity, c.tail_byte, have, words, n, last64);
+        c.null_count += zeros;
+    }
+}
+
 void table_append_host(Table& t, const std::string& name, int32_t dtype, int64_t n, const void* values,
                        const int32_t* offsets, const uint8_t* validity, int64_t bit_offset) {
     Engine& e = *t.eng;
@@ -296,19 +342,23 @@ static ArrowFormat arrow_format(const std::string& fmt, const char* column) {
 // Declares the Arrow type a stored Int32 / Int64 column stands for when its values arrived already in the stored
 // representation (Parquet chunks annotated DATE / TIME / TIMESTAMP / INT(8|16): the physical INT32 / INT64 values ARE the
 // Arrow values): the typing rules of table_append_arrow then apply to it.
+void declare_arrow_type(Column& c, const std::string& fmt) {
+    const ArrowFormat f = arrow_format(fmt, c.name.c_str());
+    if (f.dtype != c.dtype || f.large_offsets) throw Error(TG_ERR_TYPE_MISMATCH, "column '" + c.name + "' does not store Arrow format '" + fmt + "'");
+    if (f.src_w == 4 || f.src_w == 8)  // UInt32 / UInt64 need a conversion of the stored values, not a label
+        throw Error(TG_ERR_UNSUPPORTED, "column '" + c.name + "': Arrow format '" + fmt + "' cannot be declared on stored values");
+    c.src_type = f.src_type;
+    c.src_unsigned = f.src_unsigned;
+    c.temporal = f.temporal;
+    c.temporal_unit = f.temporal_unit;
+}
+
 void table_set_column_arrow_type(Table& t, const std::string& name, const std::string& fmt) {
     Engine& e = *t.eng;
     std::lock_guard<std::mutex> g(e.mu);
     Column* c = t.find(name);
     if (!c) throw Error(TG_ERR_COLUMN_NOT_FOUND, "Schema error: No field named " + name + ". Valid fields are " + t.valid_fields() + ".");
-    const ArrowFormat f = arrow_format(fmt, name.c_str());
-    if (f.dtype != c->dtype || f.large_offsets) throw Error(TG_ERR_TYPE_MISMATCH, "column '" + name + "' does not store Arrow format '" + fmt + "'");
-    if (f.src_w == 4 || f.src_w == 8)  // UInt32 / UInt64 need a conversion of the stored values, not a label
-        throw Error(TG_ERR_UNSUPPORTED, "column '" + name + "': Arrow format '" + fmt + "' cannot be declared on stored values");
-    c->src_type = f.src_type;
-    c->src_unsigned = f.src_unsigned;
-    c->temporal = f.temporal;
-    c->temporal_unit = f.temporal_unit;
+    declare_arrow_type(*c, fmt);
 }
 
 // ---- string dictionaries and Utf8View -> Utf8, decoded on the device ----
