@@ -489,7 +489,9 @@ TG_API int32_t tg_plan_add_analyzer(tg_plan* plan, int32_t analyzer_kind, const 
 TG_API int32_t tg_plan_add_kll(tg_plan* plan, const char* column, int32_t k, const double* quantiles,
                                int32_t n_quantiles);
 /* CompletenessAnalyzer::with_grouping (analyzers/basic/grouped_completeness.rs:99-239,
- * analyzers/grouped.rs:17-59) */
+ * analyzers/grouped.rs:17-59). At most 8 group columns, and at most 1048576 (2^20) groups per row shard, whatever
+ * max_groups says: above either the slot's result is an error (TG_ERR_UNSUPPORTED, "grouped completeness: more than
+ * 8 grouping columns" / "... more than 1048576 groups"). tg_plan_add_value_histogram has the same group limit. */
 TG_API int32_t tg_plan_add_grouped_completeness(tg_plan* plan, const char* column,
                                                 const char* const* group_columns, int32_t n_group_columns,
                                                 int32_t max_groups, int32_t include_overall);

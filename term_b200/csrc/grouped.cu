@@ -27,6 +27,7 @@ constexpr int GRP_SMEM_BYTES = 222 * 1024;  // dynamic shared memory of the fuse
 constexpr int GRP_MAX_PROBE = 24;   // after this many probes the row goes to the global table
 constexpr int GRP_MAX_COLS = 8;     // distinct group columns per batch
 constexpr int GRP_MAX_JOBS = 4;     // groupings per batch (one kernel launch)
+constexpr uint64_t GRP_MAX_GROUPS_DEV = 1u << 20;  // groups per grouping: more is reported as TG_ERR_UNSUPPORTED
 
 struct GrpCol {
     const uint8_t* values;
@@ -77,7 +78,11 @@ __device__ __forceinline__ void utf8_pair(const uint8_t* __restrict__ values, in
     y |= 0x8000000000000000ull;
 }
 
+// Once a grouping holds more than GRP_MAX_GROUPS_DEV groups (the most the host reports), it stops counting: the result
+// is the "more than 1048576 groups" error anyway, and the global table (up to 4 x GRP_MAX_GROUPS_DEV slots, at least
+// 2 x n) stays far from full, where upsert128 would probe without end. The overshoot is bounded by the threads in flight.
 __device__ __noinline__ void global_count(const GrpJob& J, Fp f, unsigned long long tot, unsigned long long nn, long long first) {
+    if (*reinterpret_cast<volatile unsigned long long*>(J.n_groups) > GRP_MAX_GROUPS_DEV) return;
     bool created;
     const uint64_t slot = upsert128(J.gt, f, created);
     if (created) atomicAdd(J.n_groups, 1ull);
@@ -88,25 +93,29 @@ __device__ __noinline__ void global_count(const GrpJob& J, Fp f, unsigned long l
 
 // find-or-insert (a, b) in a grouping's shared table; returns the slot or -1 when the probe limit is hit. Kept out of
 // line: it is called GRP_ILP x groupings times per iteration and inlining every copy overflows the instruction cache.
+// Only the thread that claimed the first word writes the second one; others wait for it (as upsert128 does). Two groups
+// may share the first word (Utf8 values that differ in trailing NUL bytes only, or a key whose bits equal NULL_TAG1 next
+// to a NULL): a second thread must not take the slot before the claimer has published which group it holds.
 __device__ __noinline__ int smem_upsert(unsigned long long* s_h1, unsigned long long* s_h2, uint32_t mask, unsigned long long a,
                                         unsigned long long b, bool& created) {
     created = false;
     uint32_t s = (uint32_t)(a ^ (b >> 32)) & mask;
     for (int probe = 0; probe < GRP_MAX_PROBE; ++probe, s = (s + 1) & mask) {
         unsigned long long v = s_h1[s];
-        bool claimed = false;
         if (v == EMPTY64) {
             v = atomicCAS(&s_h1[s], EMPTY64, a);
-            claimed = v == EMPTY64;
-        }
-        if (claimed || v == a) {
-            // the first arrival publishes the second word; a different second word = another group
-            unsigned long long w = s_h2[s];
-            if (w == EMPTY64) w = atomicCAS(&s_h2[s], EMPTY64, b);
-            if (w == EMPTY64 || w == b) {
-                created = claimed;
+            if (v == EMPTY64) {  // claimed: publish the second word (never EMPTY64: the caller maps it to 0)
+                atomicExch(&s_h2[s], b);
+                created = true;
                 return (int)s;
             }
+        }
+        if (v == a) {
+            unsigned long long w;
+            do {
+                w = *reinterpret_cast<volatile unsigned long long*>(&s_h2[s]);
+            } while (w == EMPTY64);
+            if (w == b) return (int)s;  // a different second word: another group
         }
     }
     return -1;
@@ -1049,7 +1058,6 @@ struct GrpBatch {
     std::vector<Column*> dcols;              // distinct group columns
     std::vector<std::vector<int>> job_cols;  // per job: indices into dcols, in the grouping's order
 };
-constexpr uint64_t GRP_MAX_GROUPS_DEV = 1u << 20;
 
 // global tables of the dictionary path: a column's dictionary holds at most 148 CTAs x 1024 entries (and at most n)
 static uint64_t gd_cap_dict(int64_t n) { return pow2_at_least(std::min<uint64_t>((uint64_t)n * 2, (uint64_t)1 << 18)); }
@@ -1544,7 +1552,7 @@ static void run_grouped_batch(Engine& e, Table& t, Plan& p, const GrpBatch& B) {
                         memcpy(&d, &x, 8);
                         key += fmt_f64(d);
                     } break;
-                    default:  // Boolean group values print as the empty string, as before; a value histogram casts them to VARCHAR
+                    default:  // Boolean group values print as the empty string, as before (unpinned, DESIGN §5); a value histogram casts them to VARCHAR
                         if (a.flags & 2) key += x ? "true" : "false";
                         break;
                 }
