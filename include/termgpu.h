@@ -401,6 +401,42 @@ TG_API tg_status tg_table_append_arrow(tg_table* t, const void* arrow_schema, co
  */
 TG_API tg_status tg_table_append_csv(tg_table* t, const char* const* columns, const char* const* arrow_formats, int32_t n_columns,
                                      const void* bytes, int64_t n_bytes, int32_t delimiter, int32_t has_header, int64_t* rows_out);
+
+/*
+ * A CSV dialect, as arrow-csv's Format (DataFusion's CsvReadOptions: delimiter, quote, escape, comment, terminator,
+ * null_regex) reads it through csv-core. Each byte field is 0..255 or -1: delimiter -1 = ','; quote -1 = '"'; escape and
+ * comment -1 = none; terminator -1 = LF, CRLF or a lone CR. The delimiter, quote, escape, comment and terminator bytes must
+ * be pairwise distinct (the default terminator counts as both CR and LF); a clash is TG_ERR_INVALID_ARG naming both.
+ *  - quote: opens quoting at a field's start only; inside quotes a doubled quote is one quote; bytes after the closing quote
+ *    are kept.
+ *  - escape: only inside quotes, the escape byte and the byte after it stand for that byte (whatever it is: a quote, the
+ *    escape byte, a terminator). Outside quotes it is an ordinary byte.
+ *  - comment: a record whose first byte is the comment byte is skipped up to and including its terminator. The byte counts
+ *    only at a record's start; comment lines before the header are skipped, the header is the first other record.
+ *  - terminator: when given, only that byte ends a record and CR and LF are ordinary bytes (a CRLF file read with LF keeps
+ *    the CR in its last field). Blank records are skipped with every terminator.
+ *  - null_regex (NULL = none): a field is NULL when the regex finds a match in its unescaped value (unanchored search with
+ *    the Rust regex crate's semantics, as arrow-csv's NullRegex::is_null). With a regex, an empty field is NULL only when
+ *    the regex matches ""; otherwise it is "" in a Utf8 column and a value error in any other. Without one, an empty field
+ *    is NULL. An invalid pattern is TG_ERR_INVALID_ARG; a construct the DFA compiler does not support TG_ERR_UNSUPPORTED.
+ * Error messages name the line a record starts on, where a line is what the terminator ends (comment and blank lines count).
+ */
+typedef struct {
+    int32_t delimiter, quote, escape, comment, terminator; /* -1 = none / default */
+    int32_t has_header;
+    const char* null_regex; /* NULL = none */
+} tg_csv_format;
+
+/* tg_table_append_csv with a CSV dialect; tg_table_append_csv is this call with {delimiter, -1, -1, -1, -1, has_header, NULL}. */
+TG_API tg_status tg_table_append_csv_format(tg_table* t, const char* const* columns, const char* const* arrow_formats, int32_t n_columns,
+                                            const void* bytes, int64_t n_bytes, const tg_csv_format* format, int64_t* rows_out);
+/* Host-only: the tokenizer's transition table and the field rules run on the CPU (tests / diagnostics), without a schema.
+ * For n_bytes of input: `values` (room for n_bytes) receives every field's unescaped bytes back to back, value_ends[i] the
+ * end of field i in `values` and is_null[i] whether it is NULL (room for n_bytes + 1 fields each); record_fields[r] the
+ * number of fields of record r and record_lines[r] the line it starts on (room for n_bytes + 1 records each); *n_fields and
+ * *n_records (may be NULL) the counts. An unterminated quote is TG_ERR_INVALID_ARG naming its record's line. */
+TG_API tg_status tg_csv_split_host(const tg_csv_format* format, const void* bytes, int64_t n_bytes, uint8_t* values, int64_t* value_ends,
+                                   uint8_t* is_null, int64_t* record_fields, int64_t* record_lines, int64_t* n_fields, int64_t* n_records);
 /* Host-only: the value parser the device runs, for one raw field (quoted or not) of the given format (tests / diagnostics).
  * `out` (may be NULL) receives the stored value — 8 bytes for Int64 / Float64 / Timestamp, 4 for Int32 / Date32, 1 (0 / 1)
  * for Boolean, and for Utf8 the unescaped length as an int64 — and *is_null (may be NULL) whether the field is NULL.

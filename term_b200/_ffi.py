@@ -65,6 +65,11 @@ class tg_parquet_page(C.Structure):
                 ("reserved", C.c_int32), ("header_offset", C.c_int64), ("body_offset", C.c_int64)]
 
 
+class tg_csv_format(C.Structure):
+    _fields_ = [("delimiter", C.c_int32), ("quote", C.c_int32), ("escape", C.c_int32), ("comment", C.c_int32), ("terminator", C.c_int32),
+                ("has_header", C.c_int32), ("null_regex", C.c_char_p)]
+
+
 class tg_exec_stats(C.Structure):
     _fields_ = [("gpu_ms", C.c_double), ("scan_ms", C.c_double), ("string_ms", C.c_double),
                 ("hash_ms", C.c_double), ("sketch_ms", C.c_double), ("bytes_scanned", C.c_uint64),
@@ -102,6 +107,9 @@ SIGNATURES = {
     "tg_table_append_arrow": (C.c_int, [P, P, P]),
     "tg_table_append_csv": (C.c_int, [P, STRS, STRS, C.c_int32, P, C.c_int64, C.c_int32, C.c_int32, C.POINTER(C.c_int64)]),
     "tg_csv_parse_value": (C.c_int, [C.c_char_p, P, C.c_int64, P, C.POINTER(C.c_int32)]),
+    "tg_table_append_csv_format": (C.c_int, [P, STRS, STRS, C.c_int32, P, C.c_int64, C.POINTER(tg_csv_format), C.POINTER(C.c_int64)]),
+    "tg_csv_split_host": (C.c_int, [C.POINTER(tg_csv_format), P, C.c_int64, P, C.POINTER(C.c_int64), P, C.POINTER(C.c_int64),
+                                    C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "tg_table_partition_fingerprints": (C.c_int, [P, C.c_char_p, STRS, C.c_int32, C.c_int32, PP, C.POINTER(C.c_int64)]),
     "tg_table_partition_keys": (C.c_int, [P, C.c_char_p, C.c_char_p, C.c_int32, PP, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "tg_plan_create": (C.c_int, [PP]),

@@ -464,16 +464,17 @@ class SessionContext:
                 F.check(F.lib().tg_table_set_column_arrow_type(t, col.encode(), fmt.encode()))
         return t
 
-    def register_csv(self, name: str, path, schema, has_header: bool = True, delimiter: str = ","):
+    def register_csv(self, name: str, path, schema, has_header: bool = True, delimiter: str = ",", quote: str = '"', escape: Optional[str] = None,
+                     comment: Optional[str] = None, terminator: Optional[str] = None, null_regex: Optional[str] = None):
         """CsvSource::register for the GPU path: the file is mapped and tokenized / parsed into the Arrow layout in HBM
-        (tg_table_append_csv), with `schema` (a pyarrow.Schema, in file order) giving every column's name and type. Schema
+        (tg_table_append_csv_format), with `schema` (a pyarrow.Schema, in file order) giving every column's name and type. Schema
         inference is not done here: DataFusion infers with arrow-csv's rules, which the Rust shim would call on the host.
+        quote / escape / comment / terminator (one byte each; None: no escape, no comment, records end at LF, CRLF or CR) and
+        null_regex (None: an empty field is NULL) are CsvReadOptions' fields of the same names (include/termgpu.h states the rules).
         Unsupported types and malformed records raise; no half-registered table stays behind."""
         if pa is None or not isinstance(schema, pa.Schema):
             raise TypeError("register_csv needs a pyarrow.Schema")
-        d = delimiter.encode() if isinstance(delimiter, str) else bytes(delimiter)
-        if len(d) != 1:
-            raise ValueError("the delimiter must be one byte")
+        fmt = csv_format(delimiter, quote, escape, comment, terminator, null_regex, has_header)
         names, fmts = _strs([f.name for f in schema]), _strs([_arrow_format(f.type) for f in schema])
         t = self._create(name)
         try:
@@ -481,13 +482,13 @@ class SessionContext:
                 size = os.fstat(f.fileno()).st_size
                 rows = C.c_int64()
                 if size == 0:
-                    F.check(F.lib().tg_table_append_csv(t, names[0], fmts[0], len(schema), None, 0, d[0], int(has_header), C.byref(rows)))
+                    F.check(F.lib().tg_table_append_csv_format(t, names[0], fmts[0], len(schema), None, 0, C.byref(fmt), C.byref(rows)))
                 else:
                     with mmap.mmap(f.fileno(), 0, flags=mmap.MAP_SHARED | getattr(mmap, "MAP_POPULATE", 0), prot=mmap.PROT_READ) as mm:
                         view = np.frombuffer(mm, dtype=np.uint8)
                         try:
-                            F.check(F.lib().tg_table_append_csv(t, names[0], fmts[0], len(schema), view.ctypes.data, size, d[0],
-                                                                int(has_header), C.byref(rows)))
+                            F.check(F.lib().tg_table_append_csv_format(t, names[0], fmts[0], len(schema), view.ctypes.data, size, C.byref(fmt),
+                                                                       C.byref(rows)))
                         finally:
                             del view  # the mapping cannot close while a buffer export is alive
         except Exception:
@@ -675,6 +676,22 @@ class AnalyzerOutput:
         if self.error:
             return None
         return {0: self.metric_double, 1: self.metric_long, 2: self.map}.get(self.metric_kind)
+
+
+def csv_format(delimiter=",", quote='"', escape=None, comment=None, terminator=None, null_regex=None, has_header=True):
+    """a tg_csv_format from register_csv's options (each byte option one byte, as str or bytes; None: the default)"""
+    def byte(what, v):
+        if v is None:
+            return -1
+        b = v.encode() if isinstance(v, str) else bytes(v)
+        if len(b) != 1:
+            raise ValueError(f"the {what} must be one byte")
+        return b[0]
+    if delimiter is None or quote is None:
+        raise ValueError("the delimiter and the quote must be one byte")
+    rx = null_regex.encode() if isinstance(null_regex, str) else null_regex
+    return F.tg_csv_format(byte("delimiter", delimiter), byte("quote", quote), byte("escape", escape), byte("comment", comment),
+                           byte("terminator", terminator), int(has_header), rx)
 
 
 def _arrow_format(typ):

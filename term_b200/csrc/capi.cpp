@@ -23,8 +23,10 @@ void table_adopt_device(Table& t, const std::string& name, int32_t dtype, int64_
                         const int32_t* d_offsets, const uint8_t* d_validity, int64_t n_value_bytes);
 void table_append_arrow(Table& t, const void* schema_p, const void* array_p);
 void table_append_csv(Table& t, const std::vector<std::string>& names, const std::vector<std::string>& fmts, const uint8_t* bytes, int64_t n_bytes,
-                      int32_t delimiter, bool has_header, int64_t* rows_out);
+                      const tg_csv_format* format, int64_t* rows_out);
 void csv_parse_value(const std::string& fmt, const uint8_t* p, int64_t n, void* out, int32_t* is_null);
+void csv_split_host(const tg_csv_format* format, const uint8_t* p, int64_t n, uint8_t* values, int64_t* value_ends, uint8_t* is_null,
+                    int64_t* record_fields, int64_t* record_lines, int64_t* n_fields, int64_t* n_records);
 }  // namespace tg
 
 using namespace tg;
@@ -322,6 +324,12 @@ tg_status tg_table_adopt_device(tg_table* t, const char* name, int32_t dtype, in
 
 tg_status tg_table_append_csv(tg_table* t, const char* const* columns, const char* const* arrow_formats, int32_t n_columns, const void* bytes,
                               int64_t n_bytes, int32_t delimiter, int32_t has_header, int64_t* rows_out) {
+    if (delimiter < 0 || delimiter > 255) return fail(TG_ERR_INVALID_ARG, "CSV: the delimiter must be a byte (0..255)");
+    const tg_csv_format f{delimiter, -1, -1, -1, -1, has_header, nullptr};
+    return tg_table_append_csv_format(t, columns, arrow_formats, n_columns, bytes, n_bytes, &f, rows_out);
+}
+tg_status tg_table_append_csv_format(tg_table* t, const char* const* columns, const char* const* arrow_formats, int32_t n_columns, const void* bytes,
+                                     int64_t n_bytes, const tg_csv_format* format, int64_t* rows_out) {
     return guard([&] {
         if (!t || (n_columns > 0 && (!columns || !arrow_formats)) || n_columns < 0) throw Error(TG_ERR_INVALID_ARG, "NULL argument");
         std::vector<std::string> names, fmts;
@@ -330,7 +338,13 @@ tg_status tg_table_append_csv(tg_table* t, const char* const* columns, const cha
             names.emplace_back(columns[i]);
             fmts.emplace_back(arrow_formats[i]);
         }
-        table_append_csv(*reinterpret_cast<Table*>(t), names, fmts, (const uint8_t*)bytes, n_bytes, delimiter, has_header != 0, rows_out);
+        table_append_csv(*reinterpret_cast<Table*>(t), names, fmts, (const uint8_t*)bytes, n_bytes, format, rows_out);
+    });
+}
+tg_status tg_csv_split_host(const tg_csv_format* format, const void* bytes, int64_t n_bytes, uint8_t* values, int64_t* value_ends, uint8_t* is_null,
+                            int64_t* record_fields, int64_t* record_lines, int64_t* n_fields, int64_t* n_records) {
+    return guard([&] {
+        csv_split_host(format, (const uint8_t*)bytes, n_bytes, values, value_ends, is_null, record_fields, record_lines, n_fields, n_records);
     });
 }
 tg_status tg_csv_parse_value(const char* arrow_format, const void* field, int64_t n_bytes, void* out, int32_t* is_null) {

@@ -15,6 +15,8 @@
 //                   field index. Float64 is exact (Clinger's fast path, then Eisel-Lemire over a 128-bit power-of-five
 //                   table); a field it cannot decide goes to a fallback list the host re-parses with strtod. Utf8 fields
 //                   are unescaped in place and validated, and the Parquet BYTE_ARRAY tail writes offsets and bytes.
+// Any other dialect (quote, escape, comment or terminator bytes, a NULL regex) runs the general 7-state machine from a
+// byte-indexed transition table built on the host, and parsers that unescape every field and test the NULL regex's DFA.
 // One read-back per chunk (records, bytes consumed, first error, NULL counts, fallback count, the pivot's head values);
 // Utf8 columns add the byte total read inside append_utf8_from_entries.
 #include <algorithm>
@@ -23,6 +25,7 @@
 #include <cstring>
 
 #include "engine.hpp"
+#include "regex_dfa.hpp"
 #include "str_entries.cuh"
 
 namespace tg {
@@ -352,23 +355,29 @@ HD bool csv_utf8_valid(const uint8_t* p, uint32_t n) {
     return true;
 }
 
-// unescapes a field in place (`dst` may equal `p`: the result is never longer) and returns its length
-HD uint32_t csv_unescape(const uint8_t* p, uint32_t n, uint8_t* dst) {
-    if (n == 0 || p[0] != '"') {
+// unescapes a field in place (`dst` may equal `p`: the result is never longer) and returns its length. Inside quotes a
+// doubled quote is one quote and the escape byte (esc >= 0) stands for the byte after it; bytes after the closing quote
+// and an unquoted field are kept as they are.
+HD uint32_t csv_unescape(const uint8_t* p, uint32_t n, uint8_t* dst, int32_t quote = '"', int32_t esc = -1) {
+    if (n == 0 || p[0] != quote) {
         if (dst != p)
             for (uint32_t i = 0; i < n; ++i) dst[i] = p[i];
         return n;
     }
     uint32_t o = 0;
-    int st = 2;  // 2 quoted, 3 quote seen, 1 after the closing quote
+    int st = 2;  // 2 quoted, 3 quote seen, 1 after the closing quote, 4 escape seen
     for (uint32_t i = 1; i < n; ++i) {
         const uint8_t c = p[i];
         if (st == 2) {
-            if (c == '"') st = 3;
+            if (c == quote) st = 3;
+            else if (c == esc) st = 4;
             else dst[o++] = c;
+        } else if (st == 4) {
+            dst[o++] = c;
+            st = 2;
         } else if (st == 3) {
             dst[o++] = c;
-            st = c == '"' ? 2 : 1;
+            st = c == quote ? 2 : 1;
         } else {
             dst[o++] = c;
         }
@@ -376,11 +385,8 @@ HD uint32_t csv_unescape(const uint8_t* p, uint32_t n, uint8_t* dst) {
     return o;
 }
 
-// one non-string field -> its stored value (8 bytes; Int32 / Date32 in the low 4, Boolean 0 / 1)
-HD int32_t csv_parse_fixed(int32_t kind, char unit, const uint8_t* p, uint32_t n, uint64_t* v) {
-    CsvText t;
-    if (!csv_text(p, n, t)) return CSV_BAD;
-    if (t.size() == 0) return CSV_NULL;
+// a non-string value's text -> its stored value (8 bytes; Int32 / Date32 in the low 4, Boolean 0 / 1)
+HD int32_t csv_parse_text(int32_t kind, char unit, const CsvText& t, uint64_t* v) {
     int64_t x = 0;
     int32_t st;
     switch (kind) {
@@ -399,6 +405,55 @@ HD int32_t csv_parse_fixed(int32_t kind, char unit, const uint8_t* p, uint32_t n
     return st;
 }
 
+// one raw non-string field of the default format: an empty field, quoted or not, is NULL
+HD int32_t csv_parse_fixed(int32_t kind, char unit, const uint8_t* p, uint32_t n, uint64_t* v) {
+    CsvText t;
+    if (!csv_text(p, n, t)) return CSV_BAD;
+    if (t.size() == 0) return CSV_NULL;
+    return csv_parse_text(kind, unit, t, v);
+}
+
+// ---- formats with other quote, escape, comment or terminator bytes, or a NULL regex
+struct CsvFieldFmt {
+    int32_t quote, esc, comment, term;  // esc / comment: -1 none; term: -1 LF, CRLF or a lone CR
+    const uint8_t* null_tab;            // the NULL regex (csv_null_table), or nullptr: an empty field is NULL
+};
+
+HD bool csv_is_term(uint8_t c, int32_t term) { return term < 0 ? (c == '\n' || c == '\r') : c == term; }
+
+// the first byte of a record's first field in [a, e): blank records and comment lines before it are skipped
+HD uint32_t csv_record_start(const uint8_t* p, uint32_t a, uint32_t e, int32_t comment, int32_t term) {
+    while (a < e) {
+        if (csv_is_term(p[a], term)) ++a;
+        else if (p[a] == comment)
+            while (a < e && !csv_is_term(p[a], term)) ++a;
+        else break;
+    }
+    return a;
+}
+
+// the NULL regex's DFA (regex_dfa.cpp) as one table: n_classes, start state (uint32 each, then 8 bytes of padding), the
+// 256-entry byte class map, then one row per state of n_classes next states and an END entry (1: a haystack ending in
+// this state matches), uint16 each, as strings.cu lays out its rows. Unanchored search, as Regex::is_match.
+HD bool csv_null_match(const uint8_t* tab, const uint8_t* p, uint32_t n) {
+    const uint32_t nc = reinterpret_cast<const uint32_t*>(tab)[0];
+    uint32_t st = reinterpret_cast<const uint32_t*>(tab)[1];
+    const uint8_t* cls = tab + 16;
+    const uint16_t* rows = reinterpret_cast<const uint16_t*>(tab + 16 + 256);
+    for (uint32_t i = 0; i < n && st > 1; ++i) st = rows[st * (nc + 1) + cls[p[i]]];
+    return st == 1 || (st != 0 && rows[st * (nc + 1) + nc] != 0);  // 1 = DFA_MATCH, 0 = DFA_DEAD
+}
+
+// one raw field of a general format, unescaped in place: NULL when the regex finds a match in the unescaped value (no
+// regex: when it is empty); otherwise the value (a non-NULL empty field is "" for Utf8 and a value error for the others)
+HD int32_t csv_parse_general(int32_t kind, char unit, uint8_t* p, uint32_t n, const CsvFieldFmt& f, uint64_t* v, uint32_t* len) {
+    const uint32_t m = csv_unescape(p, n, p, f.quote, f.esc);
+    *len = m;
+    if (f.null_tab ? csv_null_match(f.null_tab, p, m) : m == 0) return CSV_NULL;
+    if (kind == CSV_UTF8) return m > PQ_STR_MAX_LEN ? CSV_LONG : csv_utf8_valid(p, m) ? CSV_OK : CSV_BADUTF8;
+    return csv_parse_text(kind, unit, CsvText{p, m, p, 0}, v);
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // K8a tokenizer
 // ---------------------------------------------------------------------------------------------------------------------
@@ -410,29 +465,59 @@ constexpr uint32_t CSV_NEXT = (ST_UNQ | ST_UNQ << 2 | ST_QUO << 4 | ST_UNQ << 6)
                               (ST_FIELD | ST_FIELD << 2 | ST_QUO << 4 | ST_FIELD << 6) << 16 |  // delimiter
                               (ST_FIELD | ST_FIELD << 2 | ST_QUO << 4 | ST_FIELD << 6) << 24;   // terminator
 __device__ __forceinline__ uint32_t csv_next(uint32_t cls) { return (CSV_NEXT >> (8 * cls)) & 0xFFu; }
-constexpr uint32_t CSV_IDENTITY = 0 | 1 << 2 | 2 << 4 | 3 << 6;
 
-// what a run of bytes does from each of the four start states: the end state and the separators emitted
+// The general machine (any other format): 7 states, 3 bits each in a map. Every byte value has one transition word,
+// built on the host from the format (csv_machine): bits [3s, 3s + 3) the next state from state s, bit 21 + s set when the
+// byte ends a field from state s, bit 28 set when the byte is a record terminator. csv-core's reader: the comment byte
+// counts only at a record's start, the escape byte only inside quotes; a terminator at a record's start is a blank record.
+enum : uint32_t { G_REC = 0, G_FIELD = 1, G_UNQ = 2, G_QUO = 3, G_QSEEN = 4, G_ESC = 5, G_CMT = 6 };
+constexpr int G_EMIT = 21, G_TERM = 28;
+
+// bits per map entry and the number of start states of the 4-state (default format) and the general machine
+__host__ __device__ constexpr int csv_sb(int ns) { return ns == 4 ? 2 : 3; }
+template <int NS>
+__host__ __device__ constexpr uint32_t csv_identity() {
+    uint32_t m = 0;
+    for (int s = 0; s < NS; ++s) m |= (uint32_t)s << (csv_sb(NS) * s);
+    return m;
+}
+template <int NS>
+__device__ __forceinline__ uint32_t csv_at(uint32_t map, uint32_t s) {
+    return (map >> (csv_sb(NS) * s)) & ((1u << csv_sb(NS)) - 1);
+}
+
+// what a run of bytes does from each of the NS start states: the end state and the separators emitted
+template <int NS>
 struct CsvSeg {
     uint32_t map;
-    uint32_t c[4];
+    uint32_t c[NS];
 };
-__device__ __forceinline__ CsvSeg csv_combine(const CsvSeg& a, const CsvSeg& b) {  // a, then b
-    CsvSeg r;
+template <int NS>
+__device__ __forceinline__ CsvSeg<NS> csv_seg_identity() {
+    CsvSeg<NS> g;
+    g.map = csv_identity<NS>();
+#pragma unroll
+    for (int s = 0; s < NS; ++s) g.c[s] = 0;
+    return g;
+}
+template <int NS>
+__device__ __forceinline__ CsvSeg<NS> csv_combine(const CsvSeg<NS>& a, const CsvSeg<NS>& b) {  // a, then b
+    CsvSeg<NS> r;
     r.map = 0;
 #pragma unroll
-    for (int s = 0; s < 4; ++s) {
-        const uint32_t m = (a.map >> (2 * s)) & 3;
-        r.map |= ((b.map >> (2 * m)) & 3) << (2 * s);
+    for (int s = 0; s < NS; ++s) {
+        const uint32_t m = csv_at<NS>(a.map, s);
+        r.map |= csv_at<NS>(b.map, m) << (csv_sb(NS) * s);
         r.c[s] = a.c[s] + b.c[m];
     }
     return r;
 }
-__device__ __forceinline__ CsvSeg csv_shfl_up(const CsvSeg& x, int o) {
-    CsvSeg r;
+template <int NS>
+__device__ __forceinline__ CsvSeg<NS> csv_shfl_up(const CsvSeg<NS>& x, int o) {
+    CsvSeg<NS> r;
     r.map = __shfl_up_sync(0xffffffffu, x.map, o);
 #pragma unroll
-    for (int s = 0; s < 4; ++s) r.c[s] = __shfl_up_sync(0xffffffffu, x.c[s], o);
+    for (int s = 0; s < NS; ++s) r.c[s] = __shfl_up_sync(0xffffffffu, x.c[s], o);
     return r;
 }
 
@@ -458,10 +543,8 @@ __device__ __forceinline__ void csv_load_tile(const uint8_t* __restrict__ chunk,
     __syncthreads();
 }
 
-__device__ __forceinline__ CsvSeg csv_thread_seg(const uint8_t* s_bytes, uint8_t prev, int nb, uint8_t delim) {
-    CsvSeg g;
-    g.map = CSV_IDENTITY;
-    g.c[0] = g.c[1] = g.c[2] = g.c[3] = 0;
+__device__ __forceinline__ CsvSeg<4> csv_thread_seg(const uint8_t* s_bytes, uint8_t prev, int nb, uint8_t delim) {
+    CsvSeg<4> g = csv_seg_identity<4>();
     const int t0 = threadIdx.x * CSV_BPT;
     for (int k = 0; k < nb; ++k) {
         const uint8_t c = s_bytes[t0 + k];
@@ -480,6 +563,23 @@ __device__ __forceinline__ CsvSeg csv_thread_seg(const uint8_t* s_bytes, uint8_t
     return g;
 }
 
+__device__ __forceinline__ CsvSeg<7> csv_thread_seg7(const uint8_t* s_bytes, const uint32_t* s_lut, int nb) {
+    CsvSeg<7> g = csv_seg_identity<7>();
+    const int t0 = threadIdx.x * CSV_BPT;
+    for (int k = 0; k < nb; ++k) {
+        const uint32_t t = s_lut[s_bytes[t0 + k]];
+        uint32_t m = 0;
+#pragma unroll
+        for (int s = 0; s < 7; ++s) {
+            const uint32_t cur = csv_at<7>(g.map, s);
+            g.c[s] += (t >> (G_EMIT + cur)) & 1u;
+            m |= csv_at<7>(t, cur) << (3 * s);
+        }
+        g.map = m;
+    }
+    return g;
+}
+
 // the byte before the thread's first byte; the chunk's first byte counts as following a terminator
 __device__ __forceinline__ uint8_t csv_prev_byte(const uint8_t* __restrict__ chunk, uint64_t pos, const uint8_t* s_bytes, int k) {
     if (pos == 0) return '\n';
@@ -491,29 +591,49 @@ __device__ __forceinline__ int csv_thread_bytes(uint64_t pos, uint64_t n) {
 }
 
 // warp inclusive scan of the segments; x becomes the lane's inclusive prefix
-__device__ __forceinline__ CsvSeg csv_warp_scan(CsvSeg x) {
+template <int NS>
+__device__ __forceinline__ CsvSeg<NS> csv_warp_scan(CsvSeg<NS> x) {
     const int lane = threadIdx.x & 31;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
-        const CsvSeg y = csv_shfl_up(x, o);
+        const CsvSeg<NS> y = csv_shfl_up(x, o);
         if (lane >= o) x = csv_combine(y, x);
     }
     return x;
 }
 
-__global__ void __launch_bounds__(CSV_THREADS) csv_tok_pass1_kernel(const uint8_t* __restrict__ chunk, uint64_t n, uint8_t delim, CsvSeg* __restrict__ tiles) {
+// the general machine's transition words (`lut`, 256 entries) into shared memory; NS == 4 has none
+template <int NS>
+__device__ __forceinline__ void csv_load_lut(const uint32_t* __restrict__ lut, uint32_t* s_lut) {
+    static_assert(CSV_THREADS == 256, "one transition word per thread");
+    if (NS != 4) s_lut[threadIdx.x] = __ldg(lut + threadIdx.x);
+}
+
+// the thread's segment from its bytes: NS == 4 is the default format's machine, NS == 7 the general one
+template <int NS>
+__device__ __forceinline__ CsvSeg<NS> csv_thread_segment(const uint8_t* s_bytes, uint8_t prev, int nb, uint8_t delim, const uint32_t* s_lut) {
+    if constexpr (NS == 4) return csv_thread_seg(s_bytes, prev, nb, delim);
+    else return csv_thread_seg7(s_bytes, s_lut, nb);
+}
+
+template <int NS>
+__global__ void __launch_bounds__(CSV_THREADS) csv_tok_pass1_kernel(const uint8_t* __restrict__ chunk, uint64_t n, uint8_t delim,
+                                                                   const uint32_t* __restrict__ lut, CsvSeg<NS>* __restrict__ tiles) {
     __shared__ uint8_t s_bytes[CSV_TILE];
-    __shared__ CsvSeg s_warp[CSV_THREADS / 32];
+    __shared__ CsvSeg<NS> s_warp[CSV_THREADS / 32];
+    __shared__ uint32_t s_lut[NS == 4 ? 1 : 256];
     const uint64_t base = (uint64_t)blockIdx.x * CSV_TILE;
+    csv_load_lut<NS>(lut, s_lut);
     csv_load_tile(chunk, n, base, s_bytes);
     const int k0 = threadIdx.x * CSV_BPT;
     const uint64_t pos = base + k0;
-    const CsvSeg mine = csv_thread_seg(s_bytes, csv_prev_byte(chunk, pos, s_bytes, k0), csv_thread_bytes(pos, n), delim);
-    const CsvSeg inc = csv_warp_scan(mine);
+    const uint8_t prev = NS == 4 ? csv_prev_byte(chunk, pos, s_bytes, k0) : 0;  // the general machine has no previous-byte rule
+    const CsvSeg<NS> mine = csv_thread_segment<NS>(s_bytes, prev, csv_thread_bytes(pos, n), delim, s_lut);
+    const CsvSeg<NS> inc = csv_warp_scan(mine);
     if ((threadIdx.x & 31) == 31) s_warp[threadIdx.x >> 5] = inc;
     __syncthreads();
     if (threadIdx.x == 0) {
-        CsvSeg t = s_warp[0];
+        CsvSeg<NS> t = s_warp[0];
         for (int w = 1; w < CSV_THREADS / 32; ++w) t = csv_combine(t, s_warp[w]);
         tiles[blockIdx.x] = t;
     }
@@ -536,58 +656,62 @@ struct CsvFallback {
     uint32_t row, col, off, len;
 };
 
-// one CTA: the tiles' start states and separator bases (exclusive scan of the segments from the field-start state)
-__global__ void __launch_bounds__(1024) csv_tok_scan_kernel(const CsvSeg* __restrict__ tiles, int64_t n_tiles, uint32_t* __restrict__ tile_state,
+// one CTA: the tiles' start states and separator bases (exclusive scan of the segments from state 0, the state a chunk
+// starts in: field start after a terminator, or record start)
+template <int NS>
+__global__ void __launch_bounds__(1024) csv_tok_scan_kernel(const CsvSeg<NS>* __restrict__ tiles, int64_t n_tiles, uint32_t* __restrict__ tile_state,
                                                             uint32_t* __restrict__ tile_base, CsvInfo* __restrict__ info) {
-    __shared__ CsvSeg s[1024];
+    __shared__ CsvSeg<NS> s[1024];
     const int64_t per = (n_tiles + 1023) / 1024;
     const int64_t lo = (int64_t)threadIdx.x * per, hi = lo + per < n_tiles ? lo + per : n_tiles;
-    CsvSeg m;
-    m.map = CSV_IDENTITY;
-    m.c[0] = m.c[1] = m.c[2] = m.c[3] = 0;
+    CsvSeg<NS> m = csv_seg_identity<NS>();
     for (int64_t t = lo; t < hi; ++t) m = csv_combine(m, tiles[t]);
     s[threadIdx.x] = m;
     __syncthreads();
     for (int o = 1; o < 1024; o <<= 1) {
-        CsvSeg y;
+        CsvSeg<NS> y;
         const bool take = (int)threadIdx.x >= o;
         if (take) y = s[threadIdx.x - o];
         __syncthreads();
         if (take) s[threadIdx.x] = csv_combine(y, s[threadIdx.x]);
         __syncthreads();
     }
-    uint32_t st = ST_FIELD, base = 0;
+    uint32_t st = 0, base = 0;
     if (threadIdx.x) {
-        const CsvSeg& p = s[threadIdx.x - 1];
-        base = p.c[ST_FIELD];
-        st = p.map & 3;
+        const CsvSeg<NS>& p = s[threadIdx.x - 1];
+        base = p.c[0];
+        st = csv_at<NS>(p.map, 0);
     }
     for (int64_t t = lo; t < hi; ++t) {
         tile_state[t] = st;
         tile_base[t] = base;
-        const CsvSeg& g = tiles[t];
+        const CsvSeg<NS>& g = tiles[t];
         base += g.c[st];
-        st = (g.map >> (2 * st)) & 3;
+        st = csv_at<NS>(g.map, st);
     }
     if (threadIdx.x == 1023) {
-        info->n_seps = s[1023].c[ST_FIELD];
-        info->end_state = s[1023].map & 3;
+        info->n_seps = s[1023].c[0];
+        info->end_state = csv_at<NS>(s[1023].map, 0);
     }
 }
 
-__global__ void __launch_bounds__(CSV_THREADS) csv_tok_pass2_kernel(const uint8_t* __restrict__ chunk, uint64_t n, uint8_t delim, uint32_t K,
-                                                                   const uint32_t* __restrict__ tile_state, const uint32_t* __restrict__ tile_base,
-                                                                   uint32_t* __restrict__ sep, CsvInfo* __restrict__ info) {
+template <int NS>
+__global__ void __launch_bounds__(CSV_THREADS) csv_tok_pass2_kernel(const uint8_t* __restrict__ chunk, uint64_t n, uint8_t delim, const uint32_t* __restrict__ lut,
+                                                                   uint32_t K, const uint32_t* __restrict__ tile_state,
+                                                                   const uint32_t* __restrict__ tile_base, uint32_t* __restrict__ sep,
+                                                                   CsvInfo* __restrict__ info) {
     __shared__ uint8_t s_bytes[CSV_TILE];
-    __shared__ CsvSeg s_warp[CSV_THREADS / 32];
+    __shared__ CsvSeg<NS> s_warp[CSV_THREADS / 32];
+    __shared__ uint32_t s_lut[NS == 4 ? 1 : 256];
     const uint64_t base = (uint64_t)blockIdx.x * CSV_TILE;
+    csv_load_lut<NS>(lut, s_lut);
     csv_load_tile(chunk, n, base, s_bytes);
     const int k0 = threadIdx.x * CSV_BPT;
     const uint64_t pos = base + k0;
-    const uint8_t prev0 = csv_prev_byte(chunk, pos, s_bytes, k0);
+    const uint8_t prev0 = NS == 4 ? csv_prev_byte(chunk, pos, s_bytes, k0) : 0;
     const int nb = csv_thread_bytes(pos, n);
-    const CsvSeg mine = csv_thread_seg(s_bytes, prev0, nb, delim);
-    const CsvSeg inc = csv_warp_scan(mine);
+    const CsvSeg<NS> mine = csv_thread_segment<NS>(s_bytes, prev0, nb, delim, s_lut);
+    const CsvSeg<NS> inc = csv_warp_scan(mine);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (lane == 31) s_warp[warp] = inc;
     __syncthreads();
@@ -595,46 +719,63 @@ __global__ void __launch_bounds__(CSV_THREADS) csv_tok_pass2_kernel(const uint8_
     uint32_t st = tile_state[blockIdx.x], g = tile_base[blockIdx.x];
     for (int w = 0; w < warp; ++w) {
         g += s_warp[w].c[st];
-        st = (s_warp[w].map >> (2 * st)) & 3;
+        st = csv_at<NS>(s_warp[w].map, st);
     }
-    CsvSeg ex = csv_shfl_up(inc, 1);
+    CsvSeg<NS> ex = csv_shfl_up(inc, 1);
     if (lane > 0) {
         g += ex.c[st];
-        st = (ex.map >> (2 * st)) & 3;
+        st = csv_at<NS>(ex.map, st);
     }
     unsigned long long err = ~0ull, last = 0;
-    uint8_t prev = prev0;
-    for (int k = 0; k < nb; ++k) {
-        const uint8_t c = s_bytes[k0 + k];
-        const uint32_t cls = csv_class(c, delim);
-        if (csv_emits(st, cls, csv_is_crlf(prev))) {
-            sep[g] = (uint32_t)(pos + k);
-            const bool at_end = g % K == K - 1;
-            if (cls == 3) {
-                if (!at_end && err == ~0ull) err = 2ull * g;  // too few fields
-                last = g + 1;
-            } else if (at_end && err == ~0ull) {
-                err = 2ull * g;  // too many fields
-            }
-            ++g;
+    // a separator at byte `at`: its position, and the field count check (one test per separator)
+    auto emit = [&](bool is_term, uint32_t at) {
+        sep[g] = at;
+        const bool at_end = g % K == K - 1;
+        if (is_term) {
+            if (!at_end && err == ~0ull) err = 2ull * g;  // too few fields
+            last = g + 1;
+        } else if (at_end && err == ~0ull) {
+            err = 2ull * g;  // too many fields
         }
-        st = (csv_next(cls) >> (2 * st)) & 3;
-        prev = c;
+        ++g;
+    };
+    if constexpr (NS == 4) {
+        uint8_t prev = prev0;
+        for (int k = 0; k < nb; ++k) {
+            const uint8_t c = s_bytes[k0 + k];
+            const uint32_t cls = csv_class(c, delim);
+            if (csv_emits(st, cls, csv_is_crlf(prev))) emit(cls == 3, (uint32_t)(pos + k));
+            st = (csv_next(cls) >> (2 * st)) & 3;
+            prev = c;
+        }
+    } else {
+        for (int k = 0; k < nb; ++k) {
+            const uint32_t t = s_lut[s_bytes[k0 + k]];
+            if ((t >> (G_EMIT + st)) & 1u) emit((t >> G_TERM) & 1u, (uint32_t)(pos + k));
+            st = csv_at<7>(t, st);
+        }
     }
     if (err != ~0ull) atomicMin(&info->err_key, err);
     if (last) atomicMax(&info->last_term, last);
 }
 
+// the end states after which the input's last record is still open (it gets a virtual terminator) or inside quotes
+template <int NS>
+__device__ __forceinline__ bool csv_end_open(uint32_t s) { return NS == 4 ? s != ST_FIELD : (s == G_FIELD || s == G_UNQ || s == G_QSEEN); }
+template <int NS>
+__device__ __forceinline__ bool csv_end_quoted(uint32_t s) { return NS == 4 ? s == ST_QUO : (s == G_QUO || s == G_ESC); }
+
 // one thread: the input's last record without a terminator gets a virtual one at the chunk's end; the complete records
 // and the bytes they span. The chunk ends after the terminator of its last complete record (separator n_rec * K - 1), not
 // after its last terminator: a terminator past that one closes a record with too few fields, whose error lies beyond the
 // complete records, so the next chunk must start with that record and report it.
+template <int NS>
 __global__ void csv_tok_finish_kernel(uint32_t* __restrict__ sep, uint64_t n, uint32_t K, int is_last, CsvInfo* __restrict__ info) {
     unsigned long long total = info->n_seps, last = info->last_term;
     if (is_last) {
-        if (info->end_state == ST_QUO) {
+        if (csv_end_quoted<NS>(info->end_state)) {
             info->unterminated = 1;
-        } else if (info->end_state != ST_FIELD || total % K != 0) {
+        } else if (csv_end_open<NS>(info->end_state) || (NS == 4 && total % K != 0)) {
             if (total % K != K - 1) atomicMin(&info->err_key, 2ull * total);
             sep[total] = (uint32_t)n;
             last = ++total;
@@ -649,20 +790,26 @@ __global__ void csv_tok_finish_kernel(uint32_t* __restrict__ sep, uint64_t n, ui
 // ---------------------------------------------------------------------------------------------------------------------
 // K8b column parsers
 // ---------------------------------------------------------------------------------------------------------------------
-// field j of record r: [start, end) of the chunk; field 0 skips the CR / LF of blank lines or of a CRLF before it
+// field j of record r: [start, end) of the chunk; field 0 skips the CR / LF of blank lines or of a CRLF before it (the
+// general format: blank records and comment lines)
+template <bool GEN>
 __device__ __forceinline__ void csv_field(const uint8_t* __restrict__ chunk, const uint32_t* __restrict__ sep, uint64_t r, uint32_t K, uint32_t j,
-                                          uint32_t* s, uint32_t* e) {
+                                          const CsvFieldFmt& f, uint32_t* s, uint32_t* e) {
     const uint64_t g = r * K + j;
     *e = sep[g];
     uint32_t a = g ? sep[g - 1] + 1 : 0;
-    if (j == 0)
-        while (a < *e && csv_is_crlf(chunk[a])) ++a;
+    if (j == 0) {
+        if (GEN) a = csv_record_start(chunk, a, *e, f.comment, f.term);
+        else
+            while (a < *e && csv_is_crlf(chunk[a])) ++a;
+    }
     *s = a;
 }
 
 struct CsvColArgs {
     uint32_t K, j, first;   // first: records of the chunk to skip (the header)
     char unit;
+    CsvFieldFmt fmt;        // the general format (csv_parse_kernel<KIND, true>)
     void* values;           // fixed width: the column's values at its first new row; Boolean: chunk-relative value words
     uint32_t* valid;        // chunk-relative validity words
     CsvColInfo* col;
@@ -674,7 +821,8 @@ struct CsvColArgs {
     unsigned long long* block_bytes;
 };
 
-template <int32_t KIND>
+// GEN: the general format's fields, unescaped in place (non-string ones too) and tested against the NULL regex
+template <int32_t KIND, bool GEN>
 __global__ void __launch_bounds__(CSV_THREADS) csv_parse_kernel(uint8_t* __restrict__ chunk, const uint32_t* __restrict__ sep, CsvInfo* __restrict__ info,
                                                                CsvColArgs a) {
     const int lane = threadIdx.x & 31;
@@ -690,14 +838,18 @@ __global__ void __launch_bounds__(CSV_THREADS) csv_parse_kernel(uint8_t* __restr
         uint32_t len = 0;
         if (in) {
             uint32_t s, e;
-            csv_field(chunk, sep, r, a.K, a.j, &s, &e);
+            csv_field<GEN>(chunk, sep, r, a.K, a.j, a.fmt, &s, &e);
             if (KIND == CSV_UTF8) {
-                len = csv_unescape(chunk + s, e - s, chunk + s);
-                st = len == 0 ? CSV_NULL : len > PQ_STR_MAX_LEN ? CSV_LONG : csv_utf8_valid(chunk + s, len) ? CSV_OK : CSV_BADUTF8;
+                if (GEN) {
+                    st = csv_parse_general(KIND, a.unit, chunk + s, e - s, a.fmt, &v, &len);
+                } else {
+                    len = csv_unescape(chunk + s, e - s, chunk + s);
+                    st = len == 0 ? CSV_NULL : len > PQ_STR_MAX_LEN ? CSV_LONG : csv_utf8_valid(chunk + s, len) ? CSV_OK : CSV_BADUTF8;
+                }
                 if (st != CSV_OK) len = 0;
                 a.row_ent[o] = pq_str_ent(s, len);
             } else {
-                st = csv_parse_fixed(KIND, a.unit, chunk + s, e - s, &v);
+                st = GEN ? csv_parse_general(KIND, a.unit, chunk + s, e - s, a.fmt, &v, &len) : csv_parse_fixed(KIND, a.unit, chunk + s, e - s, &v);
                 if (st == CSV_SLOW) {
                     const unsigned long long k = atomicAdd(&info->n_fallback, 1ull);
                     if (k < a.fb_cap) a.fb[k] = CsvFallback{(uint32_t)o, a.j, s, e - s};
@@ -824,11 +976,103 @@ int64_t env_chunk_bytes() {
     return v > 0 ? (int64_t)v : (int64_t)256 << 20;
 }
 
-// 1-based line of byte `pos` (lines end at LF, CRLF or a lone CR)
-int64_t line_of(const uint8_t* p, int64_t pos) {
+// a tg_csv_format with its defaults filled in and checked
+struct CsvFormat {
+    int32_t delim = ',', quote = '"', esc = -1, comment = -1, term = -1;
+    bool header = true;
+    std::vector<uint8_t> null_tab;  // csv_null_match's table; empty: no NULL regex
+    // the default format runs the 4-state machine and the default field rules; any other the general ones
+    bool general() const { return quote != '"' || esc >= 0 || comment >= 0 || term >= 0 || !null_tab.empty(); }
+    CsvFieldFmt field(const uint8_t* tab) const { return CsvFieldFmt{quote, esc, comment, term, null_tab.empty() ? nullptr : tab}; }
+};
+
+std::string byte_name(int32_t b) {
+    char s[8];
+    if (b > 32 && b < 127) snprintf(s, sizeof s, "'%c'", (char)b);
+    else snprintf(s, sizeof s, "0x%02X", (unsigned)b);
+    return s;
+}
+
+CsvFormat csv_format(const tg_csv_format* f) {
+    if (!f) throw Error(TG_ERR_INVALID_ARG, "CSV: NULL format");
+    CsvFormat r;
+    const std::pair<const char*, int32_t> in[] = {{"delimiter", f->delimiter}, {"quote", f->quote}, {"escape", f->escape}, {"comment", f->comment},
+                                                  {"terminator", f->terminator}};
+    for (const auto& x : in)
+        if (x.second < -1 || x.second > 255) throw Error(TG_ERR_INVALID_ARG, std::string("CSV: the ") + x.first + " must be a byte (0..255) or -1");
+    if (f->delimiter >= 0) r.delim = f->delimiter;
+    if (f->quote >= 0) r.quote = f->quote;
+    r.esc = f->escape;
+    r.comment = f->comment;
+    r.term = f->terminator;
+    r.header = f->has_header != 0;
+    // the special bytes are pairwise distinct (the default terminator is both CR and LF)
+    std::vector<std::pair<std::string, int32_t>> sp = {{"delimiter", r.delim}, {"quote", r.quote}, {"escape", r.esc}, {"comment", r.comment}};
+    if (r.term >= 0) sp.push_back({"terminator", r.term});
+    else sp.insert(sp.end(), {{"terminator (LF)", '\n'}, {"terminator (CR)", '\r'}});
+    for (size_t i = 0; i < sp.size(); ++i)
+        for (size_t j = i + 1; j < sp.size(); ++j)
+            if (sp[i].second >= 0 && sp[i].second == sp[j].second)
+                throw Error(TG_ERR_INVALID_ARG, "CSV: the " + sp[i].first + " and the " + sp[j].first + " are the same byte " + byte_name(sp[i].second));
+    if (f->null_regex) {
+        Dfa d;
+        try {
+            d = compile_regex(f->null_regex, false);
+        } catch (Error& e) {  // a syntax error is the caller's argument; a construct the DFA compiler refuses stays unsupported
+            throw Error(e.code == TG_ERR_UNSUPPORTED ? TG_ERR_UNSUPPORTED : TG_ERR_INVALID_ARG, "CSV: NULL regex: " + e.msg);
+        }
+        const uint32_t nc = d.n_classes, row = nc + 1;
+        r.null_tab.assign(16 + 256 + (size_t)d.n_states * row * 2, 0);
+        const uint32_t hdr[2] = {nc, d.start};
+        memcpy(r.null_tab.data(), hdr, 8);
+        memcpy(r.null_tab.data() + 16, d.class_of, 256);
+        uint16_t* rows = reinterpret_cast<uint16_t*>(r.null_tab.data() + 16 + 256);
+        for (uint32_t s = 0; s < d.n_states; ++s) {
+            for (uint32_t c = 0; c < nc; ++c) rows[(size_t)s * row + c] = d.next[(size_t)s * nc + c];
+            rows[(size_t)s * row + nc] = d.accept_end[s];
+        }
+    }
+    return r;
+}
+
+// the general machine's transition word of every byte value (see G_REC)
+std::vector<uint32_t> csv_machine(const CsvFormat& f) {
+    std::vector<uint32_t> lut(256);
+    for (int b = 0; b < 256; ++b) {
+        const bool quote = b == f.quote, delim = b == f.delim, esc = b == f.esc, comment = b == f.comment;
+        const bool term = f.term >= 0 ? b == f.term : (b == '\n' || b == '\r');
+        uint32_t w = term ? 1u << G_TERM : 0u;
+        for (uint32_t s = 0; s < 7; ++s) {
+            uint32_t nx;
+            bool emit = false;
+            switch (s) {
+                case G_REC:
+                case G_FIELD:
+                    nx = quote ? G_QUO : delim ? G_FIELD : term ? G_REC : (comment && s == G_REC) ? G_CMT : G_UNQ;
+                    emit = delim || (term && s == G_FIELD);
+                    break;
+                case G_UNQ:
+                case G_QSEEN:
+                    nx = quote ? (s == G_QSEEN ? G_QUO : G_UNQ) : delim ? G_FIELD : term ? G_REC : G_UNQ;
+                    emit = delim || term;
+                    break;
+                case G_QUO: nx = quote ? G_QSEEN : esc ? G_ESC : G_QUO; break;
+                case G_ESC: nx = G_QUO; break;
+                default: nx = term ? G_REC : G_CMT; break;  // G_CMT
+            }
+            w |= nx << (3 * s);
+            if (emit) w |= 1u << (G_EMIT + s);
+        }
+        lut[b] = w;
+    }
+    return lut;
+}
+
+// 1-based line of byte `pos` of the n bytes: lines end at the terminator (the default: LF, CRLF or a lone CR)
+int64_t line_of(const uint8_t* p, int64_t n, int64_t pos, int32_t term) {
     int64_t line = 1;
     for (int64_t i = 0; i < pos; ++i)
-        if (p[i] == '\n' || (p[i] == '\r' && !(i + 1 < pos && p[i + 1] == '\n'))) ++line;
+        if (term >= 0 ? p[i] == term : (p[i] == '\n' || (p[i] == '\r' && !(i + 1 < n && p[i + 1] == '\n')))) ++line;
     return line;
 }
 
@@ -839,11 +1083,13 @@ std::string shown(const uint8_t* p, uint32_t n) {
 }
 
 // Float64 through strtod after the device's grammar check (or when it could not check: a too-long list)
-int32_t csv_f64_slow(const uint8_t* p, uint32_t n, uint64_t* bits) {
-    int32_t st = csv_parse_fixed(CSV_F64, 0, p, n, bits);
+// (gen: the general format's field rules, with the host copy of the NULL regex's table)
+int32_t csv_f64_slow(const uint8_t* p, uint32_t n, uint64_t* bits, const CsvFieldFmt* gen = nullptr) {
+    std::string s((const char*)p, n);
+    uint32_t m = 0;
+    const int32_t st = gen ? csv_parse_general(CSV_F64, 0, (uint8_t*)&s[0], n, *gen, bits, &m) : csv_parse_fixed(CSV_F64, 0, p, n, bits);
     if (st != CSV_SLOW) return st;
-    std::string s(n, '\0');
-    s.resize(csv_unescape(p, n, (uint8_t*)&s[0]));
+    s.resize(gen ? m : csv_unescape(p, n, (uint8_t*)&s[0]));
     const double d = strtod(s.c_str(), nullptr);
     memcpy(bits, &d, 8);
     return CSV_OK;
@@ -854,7 +1100,7 @@ struct CsvWork {
     uint8_t* p = nullptr;
     size_t bytes = 0;
     uint64_t cap = 0, bound = 0, words = 0, blocks = 0;
-    CsvSeg* tiles;
+    void* tiles;                         // CsvSeg<4> or CsvSeg<7> per tile
     uint32_t *tile_state, *tile_base, *sep, *vwords, *bwords;
     CsvInfo* info;
     CsvColInfo* cols;
@@ -871,7 +1117,7 @@ void work_alloc(Engine& e, CsvWork& w, uint64_t cap, uint32_t K, uint32_t n_utf8
     w.words = (w.bound + 31) / 32 + 2;
     w.blocks = (w.bound + PQ_BLOCK_ROWS - 1) / PQ_BLOCK_ROWS + 1;
     const uint64_t n_tiles = (cap + CSV_TILE - 1) / CSV_TILE + 1;
-    const size_t sz[] = {r16(n_tiles * sizeof(CsvSeg)), r16(n_tiles * 4), r16(n_tiles * 4), r16((cap + 2) * 4), r16(K * w.words * 4), r16(K * w.words * 4),
+    const size_t sz[] = {r16(n_tiles * sizeof(CsvSeg<7>)), r16(n_tiles * 4), r16(n_tiles * 4), r16((cap + 2) * 4), r16(K * w.words * 4), r16(K * w.words * 4),
                          r16(sizeof(CsvInfo)), r16(K * sizeof(CsvColInfo)), r16(CSV_FB_CAP * sizeof(CsvFallback)), r16(n_utf8 * w.bound * 8),
                          r16(n_utf8 * (w.blocks + 1) * 8), r16(n_utf8 * (w.blocks + 1) * 8), r16(w.blocks * sizeof(PqBlock))};
     size_t total = 0;
@@ -884,7 +1130,7 @@ void work_alloc(Engine& e, CsvWork& w, uint64_t cap, uint32_t K, uint32_t n_utf8
         q += sz[i];
         return r;
     };
-    w.tiles = (CsvSeg*)take(0);
+    w.tiles = take(0);
     w.tile_state = (uint32_t*)take(1);
     w.tile_base = (uint32_t*)take(2);
     w.sep = (uint32_t*)take(3);
@@ -951,16 +1197,65 @@ void csv_parse_value(const std::string& fmt, const uint8_t* p, int64_t n, void* 
     else memcpy(out, &v, 8);
 }
 
+// the general machine run on the host one byte at a time, with the device's field rules (tg_csv_split_host)
+void csv_split_host(const tg_csv_format* format, const uint8_t* p, int64_t n, uint8_t* values, int64_t* value_ends, uint8_t* is_null,
+                    int64_t* record_fields, int64_t* record_lines, int64_t* n_fields, int64_t* n_records) {
+    const CsvFormat f = csv_format(format);
+    if (n < 0 || (!p && n > 0)) throw Error(TG_ERR_INVALID_ARG, "CSV: NULL bytes");
+    if (n >= 0xFFFFFFF0ll) throw Error(TG_ERR_UNSUPPORTED, "CSV: 4 GiB or more");
+    if (n > 0 && (!values || !value_ends || !is_null || !record_fields || !record_lines)) throw Error(TG_ERR_INVALID_ARG, "NULL output");
+    const std::vector<uint32_t> lut = csv_machine(f);
+    const CsvFieldFmt ff = f.field(f.null_tab.data());
+    int64_t nf = 0, nr = 0, out = 0, rec_first = 0, rec_line = 1, line = 1, lp = 0;
+    auto line_at = [&](int64_t pos) {  // incremental line_of
+        for (; lp < pos; ++lp)
+            if (f.term >= 0 ? p[lp] == f.term : (p[lp] == '\n' || (p[lp] == '\r' && !(lp + 1 < n && p[lp + 1] == '\n')))) ++line;
+        return line;
+    };
+    auto field = [&](uint32_t a, uint32_t e, bool ends_record) {
+        if (nf == rec_first) {
+            a = csv_record_start(p, a, e, f.comment, f.term);
+            rec_line = line_at(a);
+        }
+        memcpy(values + out, p + a, e - a);
+        const uint32_t m = csv_unescape(values + out, e - a, values + out, f.quote, f.esc);
+        is_null[nf] = ff.null_tab ? csv_null_match(ff.null_tab, values + out, m) : m == 0;
+        out += m;
+        value_ends[nf++] = out;
+        if (ends_record) {
+            record_fields[nr] = nf - rec_first;
+            record_lines[nr++] = rec_line;
+            rec_first = nf;
+        }
+    };
+    uint32_t st = G_REC, fs = 0;
+    for (uint32_t i = 0; i < (uint32_t)n; ++i) {
+        const uint32_t t = lut[p[i]];
+        if ((t >> (G_EMIT + st)) & 1u) {
+            field(fs, i, (t >> G_TERM) & 1u);
+            fs = i + 1;
+        }
+        st = (t >> (3 * st)) & 7u;
+    }
+    if (st == G_QUO || st == G_ESC) {
+        const int64_t l = nf == rec_first ? line_at(csv_record_start(p, fs, (uint32_t)n, f.comment, f.term)) : rec_line;
+        throw Error(TG_ERR_INVALID_ARG, "CSV line " + std::to_string(l) + ": unterminated quote at the end of the input");
+    }
+    if (st == G_FIELD || st == G_UNQ || st == G_QSEEN) field(fs, (uint32_t)n, true);
+    if (n_fields) *n_fields = nf;
+    if (n_records) *n_records = nr;
+}
+
 void table_append_csv(Table& t, const std::vector<std::string>& names, const std::vector<std::string>& fmts, const uint8_t* bytes, int64_t n_bytes,
-                      int32_t delimiter, bool has_header, int64_t* rows_out) {
+                      const tg_csv_format* format, int64_t* rows_out) {
     Engine& e = *t.eng;
     std::lock_guard<std::mutex> g(e.mu);
     TG_CUDA(cudaSetDevice(e.device));
     const uint32_t K = (uint32_t)names.size();
     if (K == 0) throw Error(TG_ERR_INVALID_ARG, "CSV: no columns");
     if (n_bytes < 0 || (!bytes && n_bytes > 0)) throw Error(TG_ERR_INVALID_ARG, "CSV: NULL bytes");
-    if (delimiter < 0 || delimiter > 255 || delimiter == '"' || delimiter == '\n' || delimiter == '\r')
-        throw Error(TG_ERR_INVALID_ARG, "CSV: the delimiter must be one byte other than '\"', CR and LF");
+    const CsvFormat fmt = csv_format(format);
+    const bool gen = fmt.general();
     std::vector<CsvCol> cols;
     uint32_t n_utf8 = 0;
     for (uint32_t j = 0; j < K; ++j) {
@@ -993,6 +1288,8 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
     CsvWork w;
     uint8_t* buf[2] = {nullptr, nullptr};
     size_t buf_bytes = 0;
+    uint8_t* aux = nullptr;  // the general format: the machine's transition words, then the NULL regex's table
+    size_t aux_bytes = 0;
     try {
         std::vector<Column*> dcols;
         for (const CsvCol& c : cols) {
@@ -1014,6 +1311,15 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
             };
             alloc_bufs();
             work_alloc(e, w, C + L, K, n_utf8);
+            if (gen) {
+                const std::vector<uint32_t> lut = csv_machine(fmt);
+                aux_bytes = 1024 + r16(fmt.null_tab.size());
+                aux = e.dev_alloc(aux_bytes);
+                e.h2d(aux, lut.data(), 1024);
+                e.h2d(aux + 1024, fmt.null_tab.data(), fmt.null_tab.size());
+            }
+            const uint32_t* d_lut = reinterpret_cast<const uint32_t*>(aux);
+            const CsvFieldFmt dfmt = fmt.field(aux ? aux + 1024 : nullptr), hfmt = fmt.field(fmt.null_tab.data());
             const uint64_t n_windows = ((uint64_t)n_bytes + L - 1) / L;
             auto win_len = [&](uint64_t k) { return std::min<uint64_t>(L, (uint64_t)n_bytes - k * L); };
             auto upload = [&](uint64_t k) {
@@ -1027,7 +1333,7 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
             upload(0);
             uint64_t carry = 0;
             const uint8_t* carry_src = nullptr;
-            bool header = has_header;
+            bool header = fmt.header;
             for (uint64_t k = 0; k < n_windows; ++k) {
                 const int b = (int)(k & 1);
                 const bool is_last = k + 1 == n_windows;
@@ -1062,11 +1368,22 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
                 TG_CUDA(cudaMemsetAsync(&w.info->err_key, 0xFF, 8, e.copy_stream));
                 TG_CUDA(cudaMemsetAsync(w.cols, 0, K * sizeof(CsvColInfo), e.copy_stream));
                 const uint64_t n_tiles = (len + CSV_TILE - 1) / CSV_TILE;
-                csv_tok_pass1_kernel<<<(unsigned)n_tiles, CSV_THREADS, 0, e.copy_stream>>>(chunk, len, (uint8_t)delimiter, w.tiles);
-                csv_tok_scan_kernel<<<1, 1024, 0, e.copy_stream>>>(w.tiles, (int64_t)n_tiles, w.tile_state, w.tile_base, w.info);
-                csv_tok_pass2_kernel<<<(unsigned)n_tiles, CSV_THREADS, 0, e.copy_stream>>>(chunk, len, (uint8_t)delimiter, K, w.tile_state, w.tile_base,
-                                                                                          w.sep, w.info);
-                csv_tok_finish_kernel<<<1, 1, 0, e.copy_stream>>>(w.sep, len, K, is_last ? 1 : 0, w.info);
+                const uint8_t delim = (uint8_t)fmt.delim;
+                if (gen) {
+                    CsvSeg<7>* tiles = static_cast<CsvSeg<7>*>(w.tiles);
+                    csv_tok_pass1_kernel<7><<<(unsigned)n_tiles, CSV_THREADS, 0, e.copy_stream>>>(chunk, len, delim, d_lut, tiles);
+                    csv_tok_scan_kernel<7><<<1, 1024, 0, e.copy_stream>>>(tiles, (int64_t)n_tiles, w.tile_state, w.tile_base, w.info);
+                    csv_tok_pass2_kernel<7><<<(unsigned)n_tiles, CSV_THREADS, 0, e.copy_stream>>>(chunk, len, delim, d_lut, K, w.tile_state, w.tile_base,
+                                                                                                 w.sep, w.info);
+                    csv_tok_finish_kernel<7><<<1, 1, 0, e.copy_stream>>>(w.sep, len, K, is_last ? 1 : 0, w.info);
+                } else {
+                    CsvSeg<4>* tiles = static_cast<CsvSeg<4>*>(w.tiles);
+                    csv_tok_pass1_kernel<4><<<(unsigned)n_tiles, CSV_THREADS, 0, e.copy_stream>>>(chunk, len, delim, nullptr, tiles);
+                    csv_tok_scan_kernel<4><<<1, 1024, 0, e.copy_stream>>>(tiles, (int64_t)n_tiles, w.tile_state, w.tile_base, w.info);
+                    csv_tok_pass2_kernel<4><<<(unsigned)n_tiles, CSV_THREADS, 0, e.copy_stream>>>(chunk, len, delim, nullptr, K, w.tile_state, w.tile_base,
+                                                                                                 w.sep, w.info);
+                    csv_tok_finish_kernel<4><<<1, 1, 0, e.copy_stream>>>(w.sep, len, K, is_last ? 1 : 0, w.info);
+                }
                 TG_CUDA(cudaGetLastError());
                 e.launches += 4;
                 // ---- K8b: every column into its reserved tail
@@ -1082,6 +1399,7 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
                     a.first = first;
                     const int32_t kind = cols[j].kind;
                     a.unit = cols[j].unit;
+                    a.fmt = dfmt;
                     a.valid = w.vwords + j * w.words;
                     a.col = w.cols + j;
                     a.fb = w.fb;
@@ -1098,15 +1416,13 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
                         e.dev_reserve(c.values, (size_t)(have + (int64_t)bound) * wb, (size_t)have * wb);
                         a.values = c.values.p + (size_t)have * wb;
                     }
-                    switch (kind) {
-                        case CSV_I64: csv_parse_kernel<CSV_I64><<<grid, CSV_THREADS, 0, e.copy_stream>>>(chunk, w.sep, w.info, a); break;
-                        case CSV_I32: csv_parse_kernel<CSV_I32><<<grid, CSV_THREADS, 0, e.copy_stream>>>(chunk, w.sep, w.info, a); break;
-                        case CSV_F64: csv_parse_kernel<CSV_F64><<<grid, CSV_THREADS, 0, e.copy_stream>>>(chunk, w.sep, w.info, a); break;
-                        case CSV_BOOL: csv_parse_kernel<CSV_BOOL><<<grid, CSV_THREADS, 0, e.copy_stream>>>(chunk, w.sep, w.info, a); break;
-                        case CSV_UTF8: csv_parse_kernel<CSV_UTF8><<<grid, CSV_THREADS, 0, e.copy_stream>>>(chunk, w.sep, w.info, a); break;
-                        case CSV_DATE32: csv_parse_kernel<CSV_DATE32><<<grid, CSV_THREADS, 0, e.copy_stream>>>(chunk, w.sep, w.info, a); break;
-                        default: csv_parse_kernel<CSV_TS><<<grid, CSV_THREADS, 0, e.copy_stream>>>(chunk, w.sep, w.info, a); break;
-                    }
+                    using Kern = void (*)(uint8_t*, const uint32_t*, CsvInfo*, CsvColArgs);
+                    static const Kern kernels[2][7] = {
+                        {csv_parse_kernel<CSV_I64, false>, csv_parse_kernel<CSV_I32, false>, csv_parse_kernel<CSV_F64, false>, csv_parse_kernel<CSV_BOOL, false>,
+                         csv_parse_kernel<CSV_UTF8, false>, csv_parse_kernel<CSV_DATE32, false>, csv_parse_kernel<CSV_TS, false>},
+                        {csv_parse_kernel<CSV_I64, true>, csv_parse_kernel<CSV_I32, true>, csv_parse_kernel<CSV_F64, true>, csv_parse_kernel<CSV_BOOL, true>,
+                         csv_parse_kernel<CSV_UTF8, true>, csv_parse_kernel<CSV_DATE32, true>, csv_parse_kernel<CSV_TS, true>}};
+                    kernels[gen][kind]<<<grid, CSV_THREADS, 0, e.copy_stream>>>(chunk, w.sep, w.info, a);
                     TG_CUDA(cudaGetLastError());
                     e.launches += 1;
                 }
@@ -1148,7 +1464,7 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
                 if (info.n_fallback) {
                     // a patched value also replaces the read-back head value the pivot is taken from
                     auto slow = [&](uint64_t o, uint32_t j, uint32_t off, uint32_t flen, uint64_t* bits) {
-                        const int32_t st = csv_f64_slow(hchunk + off, flen, bits);
+                        const int32_t st = csv_f64_slow(hchunk + off, flen, bits, gen ? &hfmt : nullptr);
                         if (st != CSV_OK && st != CSV_NULL) {
                             err_key = std::min<unsigned long long>(err_key, 2ull * ((o + first) * (uint64_t)K + j) + 1);
                             return false;
@@ -1178,9 +1494,8 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
                                 const uint64_t gi = (o + first) * K + j;
                                 uint32_t fs = gi ? sep[gi - 1] + 1 : 0;
                                 const uint32_t fe = sep[gi];
-                                if (j == 0)
-                                    while (fs < fe && (hchunk[fs] == '\r' || hchunk[fs] == '\n')) ++fs;
-                                if (fe > fs) slow(o, j, fs, fe - fs, &patches[o]);
+                                if (j == 0) fs = csv_record_start(hchunk, fs, fe, fmt.comment, fmt.term);
+                                if (fe > fs || gen) slow(o, j, fs, fe - fs, &patches[o]);
                             }
                             e.h2d(dcols[j]->values.p + (size_t)dcols[j]->n_rows * 8, patches.data(), n_out * 8);
                         }
@@ -1201,13 +1516,13 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
                     if (!quote_err || r * K) TG_CUDA(cudaMemcpy(sp.data(), w.sep + lo, sp.size() * 4, cudaMemcpyDeviceToHost));
                     auto sep_at = [&](uint64_t x) -> uint64_t { return sp[x - lo]; };
                     uint64_t rs = r * K ? sep_at(r * K - 1) + 1 : 0;
-                    while (rs < len && (hchunk[rs] == '\r' || hchunk[rs] == '\n')) ++rs;
-                    const std::string where = "CSV line " + std::to_string(line_of(bytes, file_off + (int64_t)rs)) + ", column '" + cols[j].name + "': ";
+                    rs = csv_record_start(hchunk, (uint32_t)rs, (uint32_t)len, fmt.comment, fmt.term);
+                    const std::string where = "CSV line " + std::to_string(line_of(bytes, n_bytes, file_off + (int64_t)rs, fmt.term)) + ", column '" + cols[j].name + "': ";
                     if (quote_err) throw Error(TG_ERR_INVALID_ARG, where + "unterminated quote at the end of the input");
                     const uint64_t fe = sep_at(gi);
                     if (!is_value) {
-                        const bool term = fe >= len || hchunk[fe] == '\n' || hchunk[fe] == '\r';
-                        const std::string line = "CSV line " + std::to_string(line_of(bytes, file_off + (int64_t)rs));
+                        const bool term = fe >= len || csv_is_term(hchunk[fe], fmt.term);
+                        const std::string line = "CSV line " + std::to_string(line_of(bytes, n_bytes, file_off + (int64_t)rs, fmt.term));
                         if (term)  // the record ends after field j: column j + 1 is missing
                             throw Error(TG_ERR_INVALID_ARG, line + ", column '" + cols[j + 1].name + "': missing: the record has " + std::to_string(j + 1) +
                                                                 " fields, the schema " + std::to_string(K));
@@ -1217,12 +1532,15 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
                     const uint32_t fn = (uint32_t)(fe - fs);
                     if (cols[j].kind == CSV_UTF8) {
                         std::vector<uint8_t> tmp(fn + 1);
-                        const uint32_t ulen = csv_unescape(hchunk + fs, fn, tmp.data());
+                        const uint32_t ulen = csv_unescape(hchunk + fs, fn, tmp.data(), fmt.quote, fmt.esc);
                         if (ulen > PQ_STR_MAX_LEN) throw Error(TG_ERR_UNSUPPORTED, where + "string value of 16 MiB or more");
                         throw Error(TG_ERR_INVALID_ARG, where + "invalid UTF-8");
                     }
                     uint64_t v;
-                    const int32_t st = csv_parse_fixed(cols[j].kind, cols[j].unit, hchunk + fs, fn, &v);
+                    std::vector<uint8_t> tmp(hchunk + fs, hchunk + fs + fn);
+                    uint32_t ulen;
+                    const int32_t st = gen ? csv_parse_general(cols[j].kind, cols[j].unit, tmp.data(), fn, hfmt, &v, &ulen)
+                                           : csv_parse_fixed(cols[j].kind, cols[j].unit, hchunk + fs, fn, &v);
                     if (st == CSV_RANGE) throw Error(TG_ERR_INVALID_ARG, where + "'" + shown(hchunk + fs, fn) + "' is out of range for " + cols[j].type_name);
                     throw Error(TG_ERR_INVALID_ARG, where + "cannot parse '" + shown(hchunk + fs, fn) + "' as " + cols[j].type_name);
                 }
@@ -1276,8 +1594,10 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
             e.deferred_free.emplace_back(buf[0], buf_bytes);
             e.deferred_free.emplace_back(buf[1], buf_bytes);
             e.deferred_free.emplace_back(w.p, w.bytes);
+            if (aux) e.deferred_free.emplace_back(aux, aux_bytes);
             buf[0] = buf[1] = nullptr;
             w.p = nullptr;
+            aux = nullptr;
         }
         for (Column* c : dcols) t.n_rows = std::max(t.n_rows, c->n_rows);
         if (rows_out) *rows_out = rows;
@@ -1287,6 +1607,7 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
         if (buf[0]) e.dev_free(buf[0], buf_bytes);
         if (buf[1]) e.dev_free(buf[1], buf_bytes);
         if (w.p) e.dev_free(w.p, w.bytes);
+        if (aux) e.dev_free(aux, aux_bytes);
         for (const ColSnap& s : snaps) {
             Column& c = *s.c;
             c.n_rows = s.n_rows;

@@ -1,4 +1,4 @@
-"""Registration of a CSV file (csv.cu: the K8a tokenizer and the K8b column parsers).
+r"""Registration of a CSV file (csv.cu: the K8a tokenizer and the K8b column parsers).
 
 File, written into a temporary directory from a seeded generator: --rows records of Int64, Float64 (repr), Boolean, Utf8
 (C3-shaped emails, 10 % quoted with a comma inside, 2 % empty = NULL), Date32 and Timestamp(Microsecond) columns, several GB
@@ -12,7 +12,11 @@ line breaks), and in a separate profiled run (torch.profiler, CUDA activities: t
 kernel, no host clock) the device time of each CSV kernel. One JSON line on stdout
 (and in --out when given), with the card's name and power limit read in the same process.
 
-    python tools/bench_csv.py [--rows 40000000] [--steps 3] [--out FILE]
+    python tools/bench_csv.py [--rows 40000000] [--steps 3] [--out FILE] [--dialect dump] [--csv-only]
+
+--dialect dump writes the file as a database dump: the quoted emails carry a \" escape, NULL emails are \N and every block
+of 1 M records follows a # comment line; it is registered with escape '\', comment '#' and null_regex ^\\N$. pyarrow's
+reader has no comment lines, so that dialect times register_csv only, as --csv-only does for either.
 """
 import argparse
 import json
@@ -44,20 +48,25 @@ def card():
     return {"gpu": name, "power_limit": limit}
 
 
-def write_csv(path, n, seed):
+DUMP = dict(escape="\\", comment="#", null_regex=r"^\\N$")
+
+
+def write_csv(path, n, seed, dump=False):
     rng = np.random.default_rng(seed)
     step = 1_000_000
     with open(path, "w") as f:
         f.write(",".join(SCHEMA.names) + "\n")
         for lo in range(0, n, step):
+            if dump:
+                f.write(f'# block {lo},"x\n')
             idx = np.arange(lo, min(n, lo + step))
             m = len(idx)
             ids = rng.integers(-10**15, 10**15, m).astype(str)
             xs = np.array([repr(v) for v in rng.normal(100.0, 15.0, m).tolist()])
             flag = np.where(rng.random(m) < 0.5, "true", "false")
             em = np.char.add(np.char.add("user", idx.astype(str)), "@example.com")
-            em = np.where(idx % 10 == 0, np.char.add(np.char.add('"', np.char.replace(em, "@", ",x@")), '"'), em)
-            em = np.where(idx % 50 == 7, "", em)
+            em = np.where(idx % 10 == 0, np.char.add(np.char.add('"\\"' if dump else '"', np.char.replace(em, "@", ",x@")), '"'), em)
+            em = np.where(idx % 50 == 7, "\\N" if dump else "", em)
             days = rng.integers(-20000, 30000, m)
             day = np.datetime_as_string(days.astype("datetime64[D]"))
             ts = np.datetime_as_string((days * 86_400_000_000 + rng.integers(0, 86_400_000_000, m)).astype("datetime64[us]"))
@@ -88,6 +97,8 @@ def main():
     ap.add_argument("--rows", type=int, default=40_000_000)
     ap.add_argument("--steps", type=int, default=3)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--dialect", choices=["default", "dump"], default="default")
+    ap.add_argument("--csv-only", action="store_true")
     a = ap.parse_args()
     if a.steps < 1:
         ap.error("--steps must be at least 1")
@@ -98,14 +109,17 @@ def main():
     torch.cuda.set_device(0)
     tmp = tempfile.mkdtemp(prefix="tg_bench_csv_")
     path = os.path.join(tmp, "data.csv")
-    write_csv(path, a.rows, 1)
+    dump = a.dialect == "dump"
+    csv_only = a.csv_only or dump
+    opts = DUMP if dump else {}
+    write_csv(path, a.rows, 1, dump)
     ro = pacsv.ReadOptions(column_names=SCHEMA.names, skip_rows=1)
     po = pacsv.ParseOptions(newlines_in_values=True)
     co = pacsv.ConvertOptions(column_types=SCHEMA, strings_can_be_null=True, quoted_strings_can_be_null=True, null_values=[""],
                               true_values=["true"], false_values=["false"])
-    host = pacsv.read_csv(path, read_options=ro, parse_options=po, convert_options=co)
     pq_path = os.path.join(tmp, "data.parquet")
-    pq.write_table(host, pq_path, compression="SNAPPY")
+    if not csv_only:
+        pq.write_table(pacsv.read_csv(path, read_options=ro, parse_options=po, convert_options=co), pq_path, compression="SNAPPY")
     ctx = T.SessionContext(0)
 
     def timed(register):
@@ -120,12 +134,14 @@ def main():
             ctx.deregister_table("bench")
         return round(sum(ts[1:]) / a.steps, 3), [round(x, 3) for x in ts[1:]]
 
-    csv_ms, csv_runs = timed(lambda: ctx.register_csv("bench", path, SCHEMA))
-    arrow_ms, arrow_runs = timed(lambda: ctx.register_table("bench", pacsv.read_csv(path, read_options=ro, parse_options=po, convert_options=co)))
-    pq_ms, pq_runs = timed(lambda: ctx.register_parquet("bench", pq_path))
+    csv_ms, csv_runs = timed(lambda: ctx.register_csv("bench", path, SCHEMA, **opts))
+    arrow_ms = arrow_runs = pq_ms = pq_runs = None
+    if not csv_only:
+        arrow_ms, arrow_runs = timed(lambda: ctx.register_table("bench", pacsv.read_csv(path, read_options=ro, parse_options=po, convert_options=co)))
+        pq_ms, pq_runs = timed(lambda: ctx.register_parquet("bench", pq_path))
     from torch.profiler import ProfilerActivity, profile
     with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
-        ctx.register_csv("bench", path, SCHEMA)
+        ctx.register_csv("bench", path, SCHEMA, **opts)
         ctx.sync_copies()
         torch.cuda.synchronize()
     ctx.deregister_table("bench")
@@ -137,17 +153,19 @@ def main():
     size = os.path.getsize(path)
     window = int(os.environ.get("TG_CSV_CHUNK_BYTES") or 0) or 256 << 20  # as csv.cu reads it
     rec = {"workload": f"register one CSV file of {a.rows} records x 6 columns (Int64, Float64, Boolean, Utf8 with quoting, Date32, Timestamp(us))",
+           "dialect": a.dialect,
            "rows": a.rows, "file_bytes": size, "steps": a.steps,
            "timing": "host clock around the registration + device synchronise; mean of the timed runs after one warm-up",
            "kernel_timing": "torch.profiler CUDA activities, one registration in a separate run", **card(),
            "register_csv_ms": csv_ms, "register_csv_ms_runs": csv_runs, "h2d_bytes": size, "h2d_gbs": round(size / (csv_ms / 1e3) / 1e9, 2),
            "chunk_bytes": window, "d2d_carry_bytes": carry_bytes(path, window),
            "pyarrow_read_csv_plus_register_table_ms": arrow_ms, "pyarrow_runs": arrow_runs,
-           "register_parquet_ms": pq_ms, "register_parquet_runs": pq_runs, "parquet_bytes": os.path.getsize(pq_path),
+           "register_parquet_ms": pq_ms, "register_parquet_runs": pq_runs, "parquet_bytes": None if csv_only else os.path.getsize(pq_path),
            "kernel_ms": {k: round(v, 3) for k, v in kern.items()}, "kernel_ms_total": round(sum(kern.values()), 3)}
     ctx.close()
     os.remove(path)
-    os.remove(pq_path)
+    if not csv_only:
+        os.remove(pq_path)
     os.rmdir(tmp)
     out = json.dumps(rec)
     print(out, flush=True)
