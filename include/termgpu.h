@@ -264,6 +264,7 @@ TG_API tg_status tg_table_column_buffers(tg_engine* eng, const char* table, cons
  * rewritten to PLAIN on the host), RLE levels, flat columns; anything else -> TG_ERR_UNSUPPORTED (there is no host decode path).
  * Appends num_values rows; `chunk`
  * must stay readable until the next tg_plan_execute* / tg_table_column_buffers on this engine when it is pinned memory.
+ * A failed call leaves the table as it was (no column created, no type declared).
  */
 TG_API tg_status tg_table_append_parquet_chunk(tg_table* t, const char* name, int32_t dtype, int32_t max_definition_level,
                                                int32_t codec, const void* chunk, int64_t n_bytes, int64_t num_values);
@@ -308,7 +309,8 @@ TG_API int64_t tg_parquet_page_decompress(int32_t codec, const void* src, int64_
  * bitmap, LSB bit order, `bit_offset` = Arrow array offset). The call stages them through pinned
  * memory into HBM (async copies on the engine's copy stream) and returns after the copy is queued and
  * the caller's buffers are no longer needed. validity may be NULL (no nulls). For TG_UTF8 `values`
- * is the byte buffer and `offsets` has n_rows+1 entries. First call for a name defines its dtype.
+ * is the byte buffer and `offsets` has n_rows+1 entries. First call for a name defines its dtype. A failed call leaves the
+ * table as it was.
  */
 TG_API tg_status tg_table_append_host(tg_table* t, const char* name, int32_t dtype, int64_t n_rows,
                                       const void* values, const int32_t* offsets,
@@ -379,7 +381,8 @@ TG_API tg_status tg_table_shuffle_fingerprints(tg_engine* eng, const char* table
  * NULL dictionary value; indices and views under NULL rows are never read. Errors: TG_ERR_INVALID_ARG for a valid row whose
  * index lies outside the dictionary (any valid row of an empty one) or whose view lies outside its data buffer;
  * TG_ERR_UNSUPPORTED for a string of 16 MiB or more, for BinaryView ("vz") and for dictionaries of any other value type
- * (Binary, Utf8View, numeric, temporal, Boolean). Columns before the failing one may already hold the batch's rows. */
+ * (Binary, Utf8View, numeric, temporal, Boolean). A failed call leaves the table as it was: no column holds any of the
+ * batch's rows. */
 TG_API tg_status tg_table_append_arrow(tg_table* t, const void* arrow_schema, const void* arrow_array);
 
 /*

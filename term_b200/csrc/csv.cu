@@ -956,20 +956,6 @@ CsvCol csv_column(const std::string& name, const std::string& f) {
     return c;
 }
 
-// what a column held before the call (a failed call restores it)
-struct ColSnap {
-    Column* c;
-    int64_t n_rows, value_bytes, null_count;
-    int32_t last_offset;
-    uint8_t tail_byte, tail_vbyte;
-    bool pivot_set, had_validity;
-    double pivot;
-    int64_t ipivot;
-    const char* src_type;
-    bool src_unsigned, temporal;
-    char temporal_unit;
-};
-
 int64_t env_chunk_bytes() {
     const char* s = getenv("TG_CSV_CHUNK_BYTES");
     const long long v = s ? atoll(s) : 0;
@@ -1248,9 +1234,8 @@ void csv_split_host(const tg_csv_format* format, const uint8_t* p, int64_t n, ui
 
 void table_append_csv(Table& t, const std::vector<std::string>& names, const std::vector<std::string>& fmts, const uint8_t* bytes, int64_t n_bytes,
                       const tg_csv_format* format, int64_t* rows_out) {
-    Engine& e = *t.eng;
-    std::lock_guard<std::mutex> g(e.mu);
-    TG_CUDA(cudaSetDevice(e.device));
+    AppendTxn txn(t);
+    Engine& e = txn.e;
     const uint32_t K = (uint32_t)names.size();
     if (K == 0) throw Error(TG_ERR_INVALID_ARG, "CSV: no columns");
     if (n_bytes < 0 || (!bytes && n_bytes > 0)) throw Error(TG_ERR_INVALID_ARG, "CSV: NULL bytes");
@@ -1274,28 +1259,25 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
                                                                     have->temporal_unit == (c.kind == CSV_TS ? c.unit : 'D')
                                                               : have->src_type == nullptr);
         if (!same) throw Error(TG_ERR_TYPE_MISMATCH, "column '" + c.name + "' was registered with a different type than " + c.type_name);
-        if (have->adopted) throw Error(TG_ERR_INVALID_ARG, "cannot append to an adopted device column");
-    }
-    // ---- snapshot (a failed call leaves every column as it was)
-    std::vector<ColSnap> snaps;
-    const size_t n_cols_before = t.cols.size();
-    const int64_t table_rows_before = t.n_rows;
-    for (auto& up : t.cols) {
-        Column& c = *up;
-        snaps.push_back(ColSnap{&c, c.n_rows, c.value_bytes, c.null_count, c.last_offset, c.tail_byte, c.tail_vbyte, c.pivot_set, c.validity.p != nullptr,
-                                c.pivot, c.ipivot, c.src_type, c.src_unsigned, c.temporal, c.temporal_unit});
     }
     CsvWork w;
     uint8_t* buf[2] = {nullptr, nullptr};
     size_t buf_bytes = 0;
     uint8_t* aux = nullptr;  // the general format: the machine's transition words, then the NULL regex's table
     size_t aux_bytes = 0;
+    // the Utf8 tails read the staging buffers asynchronously: released at the next sync_copies, after a failed call too (the
+    // transaction has then waited for the streams)
+    auto release_staging = [&] {
+        const std::pair<uint8_t*, size_t> blocks[] = {{buf[0], buf_bytes}, {buf[1], buf_bytes}, {w.p, w.bytes}, {aux, aux_bytes}};
+        for (const auto& b : blocks)
+            if (b.first) e.deferred_free.push_back(b);
+    };
     try {
         std::vector<Column*> dcols;
         for (const CsvCol& c : cols) {
-            Column* col = table_get_or_add(t, c.name, c.dtype);
-            if (c.kind == CSV_DATE32 || c.kind == CSV_TS) declare_arrow_type(*col, c.fmt);
-            dcols.push_back(col);
+            Column& col = txn.column(c.name, c.dtype);
+            if (c.kind == CSV_DATE32 || c.kind == CSV_TS) declare_arrow_type(col, c.fmt);
+            dcols.push_back(&col);
         }
         int64_t rows = 0;
         if (n_bytes > 0) {
@@ -1571,7 +1553,7 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
                             x.block_bytes = w.block_bytes + (uint64_t)u * (w.blocks + 1);
                             x.block_base = w.block_base + (uint64_t)u * (w.blocks + 1);
                             ++u;
-                            append_utf8_from_entries(e, t, c, x, (int64_t)n_out);  // sets n_rows
+                            append_utf8_from_entries(e, c, x, (int64_t)n_out);  // sets n_rows
                             continue;
                         }
                         if (cols[j].kind == CSV_BOOL) {
@@ -1590,51 +1572,14 @@ void table_append_csv(Table& t, const std::vector<std::string>& names, const std
                     carry_src = chunk + info.consumed;
                 }
             }
-            // the Utf8 tails read the staging buffers asynchronously: released at the next sync_copies
-            e.deferred_free.emplace_back(buf[0], buf_bytes);
-            e.deferred_free.emplace_back(buf[1], buf_bytes);
-            e.deferred_free.emplace_back(w.p, w.bytes);
-            if (aux) e.deferred_free.emplace_back(aux, aux_bytes);
-            buf[0] = buf[1] = nullptr;
-            w.p = nullptr;
-            aux = nullptr;
         }
-        for (Column* c : dcols) t.n_rows = std::max(t.n_rows, c->n_rows);
         if (rows_out) *rows_out = rows;
     } catch (...) {
-        cudaStreamSynchronize(e.copy_stream);
-        if (e.side[0]) cudaStreamSynchronize(e.side[0]);
-        if (buf[0]) e.dev_free(buf[0], buf_bytes);
-        if (buf[1]) e.dev_free(buf[1], buf_bytes);
-        if (w.p) e.dev_free(w.p, w.bytes);
-        if (aux) e.dev_free(aux, aux_bytes);
-        for (const ColSnap& s : snaps) {
-            Column& c = *s.c;
-            c.n_rows = s.n_rows;
-            c.value_bytes = s.value_bytes;
-            c.null_count = s.null_count;
-            c.last_offset = s.last_offset;
-            c.tail_byte = s.tail_byte;
-            c.tail_vbyte = s.tail_vbyte;
-            c.pivot_set = s.pivot_set;
-            c.pivot = s.pivot;
-            c.ipivot = s.ipivot;
-            c.src_type = s.src_type;
-            c.src_unsigned = s.src_unsigned;
-            c.temporal = s.temporal;
-            c.temporal_unit = s.temporal_unit;
-            if (!s.had_validity && c.validity.p) {
-                if (c.validity.owned) e.dev_free(c.validity.p, c.validity.cap);
-                c.validity = DevBuf{};
-            }
-        }
-        while (t.cols.size() > n_cols_before) {
-            column_free(e, *t.cols.back());
-            t.cols.pop_back();
-        }
-        t.n_rows = table_rows_before;
+        release_staging();
         throw;
     }
+    release_staging();
+    txn.commit();
 }
 
 }  // namespace tg

@@ -187,6 +187,41 @@ struct Engine {
 Column* numeric_view(Engine& e, Column* c);
 void column_free(Engine& e, Column& c);
 
+// One append call (tg_table_append_*): holds the engine's lock and makes the call all or nothing. A call that throws
+// leaves the table as it was: every column it touched gets back its rows, byte count, NULL count, tail mirrors, pivot and
+// declared type, a validity bitmap the call created is freed, the columns it created are dropped. Capacity the call grew
+// is kept (it lies past the column's end). A successful call pays nothing for this but the record of the columns it touched.
+class AppendTxn {
+  public:
+    explicit AppendTxn(Table& t);
+    ~AppendTxn();
+    // the column to append to (created with `dtype` when missing); adopted device columns are refused
+    Column& column(const std::string& name, int32_t dtype);
+    // the call succeeded: the table's row count becomes the largest of its touched columns
+    void commit();
+    Engine& e;
+    Table& t;
+
+  private:
+    struct Saved {
+        Column* c;
+        int64_t n_rows, value_bytes, null_count;
+        int32_t last_offset;
+        uint8_t tail_byte, tail_vbyte;
+        bool pivot_set, had_validity;
+        double pivot;
+        int64_t ipivot;
+        const char* src_type;
+        bool src_unsigned, temporal;
+        char temporal_unit;
+    };
+    std::lock_guard<std::mutex> g;
+    size_t n_cols;
+    int64_t n_rows;
+    std::vector<Saved> saved;
+    bool committed = false;
+};
+
 // tables.cu helpers shared with the Parquet path (parquet.cu)
 Column* table_get_or_add(Table& t, const std::string& name, int32_t dtype);
 void set_pivot_host(Column& c, int32_t dtype, int64_t n, const void* values, const uint8_t* validity, int64_t bit_offset);

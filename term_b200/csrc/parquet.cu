@@ -1093,34 +1093,38 @@ int64_t parquet_chunk_validity(const uint8_t* chunk, int64_t n_bytes, int64_t nu
     return count_ones(bits.data(), 0, rows);
 }
 
-static void append_parquet_utf8(Table& t, const std::string& name, int32_t max_def_level, int32_t codec, const uint8_t* chunk, int64_t n_bytes,
+static void append_parquet_utf8(AppendTxn& txn, const std::string& name, int32_t max_def_level, int32_t codec, const uint8_t* chunk, int64_t n_bytes,
                                 int64_t num_values);
+static void append_parquet_fixed(AppendTxn& txn, const std::string& name, int32_t dtype, int32_t max_def_level, int32_t codec, const uint8_t* chunk,
+                                 int64_t n_bytes, int64_t num_values);
 
 void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype, int32_t max_def_level, int32_t codec,
                                 const uint8_t* chunk, int64_t n_bytes, int64_t num_values) {
-    Engine& e = *t.eng;
-    std::lock_guard<std::mutex> g(e.mu);
-    TG_CUDA(cudaSetDevice(e.device));
+    AppendTxn txn(t);
     if (!chunk || n_bytes <= 0 || num_values < 0) throw Error(TG_ERR_INVALID_ARG, "empty Parquet column chunk");
     if (!codec_supported(codec))
         throw Error(TG_ERR_UNSUPPORTED, "Parquet: codec " + std::to_string(codec) + " (UNCOMPRESSED, SNAPPY, GZIP, BROTLI, ZSTD and LZ4_RAW chunks are decoded)");
     if (max_def_level < 0 || max_def_level > 1) throw Error(TG_ERR_UNSUPPORTED, "Parquet: nested columns (max definition level > 1)");
     if (num_values >= ((int64_t)1 << 31)) throw Error(TG_ERR_UNSUPPORTED, "Parquet: column chunk with 2^31 or more values");
-    if (dtype == TG_UTF8) {
-        append_parquet_utf8(t, name, max_def_level, codec, chunk, n_bytes, num_values);
-        return;
-    }
+    if (dtype == TG_UTF8) append_parquet_utf8(txn, name, max_def_level, codec, chunk, n_bytes, num_values);
+    else append_parquet_fixed(txn, name, dtype, max_def_level, codec, chunk, n_bytes, num_values);
+    txn.commit();
+}
+
+// INT64 / DOUBLE / INT32 / FLOAT / INT96 / BOOLEAN chunks
+static void append_parquet_fixed(AppendTxn& txn, const std::string& name, int32_t dtype, int32_t max_def_level, int32_t codec, const uint8_t* chunk,
+                                 int64_t n_bytes, int64_t num_values) {
+    Engine& e = txn.e;
     const bool is_bool = dtype == TG_BOOL, int96 = dtype == TG_PQ_INT96;
     if (dtype != TG_INT64 && dtype != TG_FLOAT64 && dtype != TG_INT32 && dtype != TG_FLOAT32 && !is_bool && !int96)
         throw Error(TG_ERR_UNSUPPORTED, "Parquet: only INT64 / DOUBLE / INT32 / FLOAT / INT96 / BOOLEAN / BYTE_ARRAY (Utf8) columns are decoded on the device");
     const int32_t stored = int96 ? TG_INT64 : dtype;
     if (int96) {  // an INT96 column is Timestamp(Nanosecond, None) and nothing else
-        const Column* have_c = t.find(name);
+        const Column* have_c = txn.t.find(name);
         if (have_c && !(have_c->src_type && strcmp(have_c->src_type, "Timestamp") == 0 && have_c->temporal_unit == 'n'))
             throw Error(TG_ERR_TYPE_MISMATCH, "column '" + name + "' was registered with a different type than INT96 (Timestamp(Nanosecond, None))");
     }
-    Column& c = *table_get_or_add(t, name, stored);
-    if (c.adopted) throw Error(TG_ERR_INVALID_ARG, "cannot append to an adopted device column");
+    Column& c = txn.column(name, stored);
     if (int96) {  // what tg_table_set_column_arrow_type(.., "tsn:") declares
         c.src_type = "Timestamp";
         c.src_unsigned = false;
@@ -1132,10 +1136,7 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
 
     PqChunk pc;
     collect_sections(chunk, n_bytes, codec, max_def_level, num_values, dtype, pc);
-    if (num_values == 0) {
-        t.n_rows = std::max(t.n_rows, c.n_rows);
-        return;
-    }
+    if (num_values == 0) return;
 
     // PLAIN pages of required columns go straight into place; everything else is staged and expanded by a kernel
     if (is_bool) e.dev_reserve(c.values, (size_t)(have + num_values + 7) / 8, (size_t)(have + 7) / 8);
@@ -1206,7 +1207,6 @@ void table_append_parquet_chunk(Table& t, const std::string& name, int32_t dtype
         c.value_bytes = (have + num_values) * (int64_t)w;
     }
     c.n_rows = have + num_values;
-    t.n_rows = std::max(t.n_rows, c.n_rows);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
@@ -1314,18 +1314,14 @@ __global__ void __launch_bounds__(PQ_THREADS) pq_str_write_kernel(const uint8_t*
     }
 }
 
-static void append_parquet_utf8(Table& t, const std::string& name, int32_t max_def_level, int32_t codec, const uint8_t* chunk, int64_t n_bytes,
+static void append_parquet_utf8(AppendTxn& txn, const std::string& name, int32_t max_def_level, int32_t codec, const uint8_t* chunk, int64_t n_bytes,
                                 int64_t num_values) {
-    Engine& e = *t.eng;  // (the caller holds the engine's lock)
-    Column& c = *table_get_or_add(t, name, TG_UTF8);
-    if (c.adopted) throw Error(TG_ERR_INVALID_ARG, "cannot append to an adopted device column");
+    Engine& e = txn.e;
+    Column& c = txn.column(name, TG_UTF8);
     const int64_t have = c.n_rows;
     PqChunk pc;
     collect_sections(chunk, n_bytes, codec, max_def_level, num_values, TG_UTF8, pc);
-    if (num_values == 0) {
-        t.n_rows = std::max(t.n_rows, c.n_rows);
-        return;
-    }
+    if (num_values == 0) return;
     const PqStaged st = stage_chunk(e, pc, PQ_KIND_STR, 0, max_def_level, num_values);
     std::vector<uint64_t> dict_ents;
     if (pc.dict_count > 0) {
@@ -1354,10 +1350,10 @@ static void append_parquet_utf8(Table& t, const std::string& name, int32_t max_d
         reinterpret_cast<const uint64_t*>(d[4]), (uint32_t)pc.dict_count, reinterpret_cast<uint64_t*>(d[5]), x.block_bytes);
     TG_CUDA(cudaGetLastError());
     e.launches += 1;
-    append_utf8_from_entries(e, t, c, x, num_values);
+    append_utf8_from_entries(e, c, x, num_values);
 }
 
-uint32_t append_utf8_from_entries(Engine& e, Table& t, Column& c, const Utf8Entries& x, int64_t num_values) {
+uint32_t append_utf8_from_entries(Engine& e, Column& c, const Utf8Entries& x, int64_t num_values) {
     const int64_t have = c.n_rows, nb = x.n_blocks;
     const int grid = pq_str_grid(e, nb);
     pq_block_scan_kernel<<<1, 1024, 0, e.copy_stream>>>(x.block_bytes, nb, x.block_base);
@@ -1380,7 +1376,6 @@ uint32_t append_utf8_from_entries(Engine& e, Table& t, Column& c, const Utf8Entr
     c.value_bytes += (int64_t)total;
     c.last_offset = (int32_t)c.value_bytes;
     c.n_rows = have + num_values;
-    t.n_rows = std::max(t.n_rows, c.n_rows);
     return 0;
 }
 

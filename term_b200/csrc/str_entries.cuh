@@ -51,7 +51,7 @@ struct Utf8Entries {
 // After the locate kernel (queued on e.copy_stream): pq_block_scan_kernel over the block totals, the byte total (and the
 // error flag) read back, the 2 GiB check, the column's value / offset buffers reserved, pq_str_write_kernel, and the
 // column's value_bytes / last_offset / n_rows. Validity is the caller's. Returns the error flag: when it is not 0,
-// nothing was appended. The caller holds the engine's lock.
-uint32_t append_utf8_from_entries(Engine& e, Table& t, Column& c, const Utf8Entries& x, int64_t num_values);
+// nothing was appended. The caller holds the engine's lock (an AppendTxn).
+uint32_t append_utf8_from_entries(Engine& e, Column& c, const Utf8Entries& x, int64_t num_values);
 
 }  // namespace tg

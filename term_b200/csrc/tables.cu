@@ -98,6 +98,57 @@ Column* table_get_or_add(Table& t, const std::string& name, int32_t dtype) {
     return t.cols.back().get();
 }
 
+AppendTxn::AppendTxn(Table& t_) : e(*t_.eng), t(t_), g(e.mu), n_cols(t.cols.size()), n_rows(t.n_rows) {
+    TG_CUDA(cudaSetDevice(e.device));
+}
+
+Column& AppendTxn::column(const std::string& name, int32_t dtype) {
+    Column& c = *table_get_or_add(t, name, dtype);
+    if (c.adopted) throw Error(TG_ERR_INVALID_ARG, "cannot append to an adopted device column");
+    for (const Saved& s : saved)
+        if (s.c == &c) return c;
+    saved.push_back(Saved{&c, c.n_rows, c.value_bytes, c.null_count, c.last_offset, c.tail_byte, c.tail_vbyte, c.pivot_set, c.validity.p != nullptr,
+                          c.pivot, c.ipivot, c.src_type, c.src_unsigned, c.temporal, c.temporal_unit});
+    return c;
+}
+
+void AppendTxn::commit() {
+    for (const Saved& s : saved) t.n_rows = std::max(t.n_rows, s.c->n_rows);
+    committed = true;
+}
+
+AppendTxn::~AppendTxn() {
+    if (committed) return;
+    // copies and kernels of the call may still be writing the buffers freed below
+    cudaStreamSynchronize(e.copy_stream);
+    if (e.side[0]) cudaStreamSynchronize(e.side[0]);
+    for (const Saved& s : saved) {
+        Column& c = *s.c;
+        c.n_rows = s.n_rows;
+        c.value_bytes = s.value_bytes;
+        c.null_count = s.null_count;
+        c.last_offset = s.last_offset;
+        c.tail_byte = s.tail_byte;
+        c.tail_vbyte = s.tail_vbyte;
+        c.pivot_set = s.pivot_set;
+        c.pivot = s.pivot;
+        c.ipivot = s.ipivot;
+        c.src_type = s.src_type;
+        c.src_unsigned = s.src_unsigned;
+        c.temporal = s.temporal;
+        c.temporal_unit = s.temporal_unit;
+        if (!s.had_validity && c.validity.p) {
+            if (c.validity.owned) e.dev_free(c.validity.p, c.validity.cap);
+            c.validity = DevBuf{};
+        }
+    }
+    while (t.cols.size() > n_cols) {
+        column_free(e, *t.cols.back());
+        t.cols.pop_back();
+    }
+    t.n_rows = n_rows;
+}
+
 // appends the validity of `n` rows (bitmap `validity` read from bit `bit_offset`; nullptr = no NULLs) to a column that
 // holds `have` rows; materialises the bitmap lazily the first time a NULL shows up
 void append_validity(Engine& e, Column& c, int64_t have, const uint8_t* validity, int64_t bit_offset, int64_t n) {
@@ -191,19 +242,14 @@ void append_validity_device(Engine& e, Column& c, int64_t have, const uint32_t* 
     }
 }
 
-void table_append_host(Table& t, const std::string& name, int32_t dtype, int64_t n, const void* values,
-                       const int32_t* offsets, const uint8_t* validity, int64_t bit_offset) {
-    Engine& e = *t.eng;
-    std::lock_guard<std::mutex> g(e.mu);
-    TG_CUDA(cudaSetDevice(e.device));
+// table_append_host inside a caller's transaction (table_append_arrow appends every child of a batch in one)
+static void append_host_column(AppendTxn& txn, const std::string& name, int32_t dtype, int64_t n, const void* values,
+                               const int32_t* offsets, const uint8_t* validity, int64_t bit_offset) {
+    Engine& e = txn.e;
     if (n < 0) throw Error(TG_ERR_INVALID_ARG, "negative row count");
-    Column& c = *table_get_or_add(t, name, dtype);
-    if (c.adopted) throw Error(TG_ERR_INVALID_ARG, "cannot append to an adopted device column");
+    Column& c = txn.column(name, dtype);
     const int64_t have = c.n_rows;
-    if (n == 0) {
-        t.n_rows = std::max(t.n_rows, c.n_rows);
-        return;
-    }
+    if (n == 0) return;
     // ---- fixed-width values first: their DMA (the bulk of the bytes) is queued before the host walks the validity
     // bitmap below, so counting NULLs overlaps the copy instead of delaying it ----
     const bool fixed_width = dtype == TG_INT64 || dtype == TG_FLOAT64 || dtype == TG_INT32 || dtype == TG_FLOAT32;
@@ -245,7 +291,13 @@ void table_append_host(Table& t, const std::string& name, int32_t dtype, int64_t
         default: throw Error(TG_ERR_INVALID_ARG, "unknown dtype");
     }
     c.n_rows = have + n;
-    t.n_rows = std::max(t.n_rows, c.n_rows);
+}
+
+void table_append_host(Table& t, const std::string& name, int32_t dtype, int64_t n, const void* values,
+                       const int32_t* offsets, const uint8_t* validity, int64_t bit_offset) {
+    AppendTxn txn(t);
+    append_host_column(txn, name, dtype, n, values, offsets, validity, bit_offset);
+    txn.commit();
 }
 
 void table_adopt_device(Table& t, const std::string& name, int32_t dtype, int64_t n, const void* d_values,
@@ -497,15 +549,9 @@ ArrowStage arrow_stage(Engine& e, size_t payload_b, size_t tables_b, int64_t n, 
     return s;
 }
 
-Column& arrow_utf8_column(Table& t, const char* name) {
-    Column& c = *table_get_or_add(t, name, TG_UTF8);
-    if (c.adopted) throw Error(TG_ERR_INVALID_ARG, "cannot append to an adopted device column");
-    return c;
-}
-
 // the shared tail; a flag raised by the locate kernel becomes the error (and nothing was appended)
-void arrow_utf8_finish(Engine& e, Table& t, Column& c, const ArrowStage& s, int64_t n, const std::string& range_msg, const char* name) {
-    const uint32_t err = append_utf8_from_entries(e, t, c, s.x, n);
+void arrow_utf8_finish(Engine& e, Column& c, const ArrowStage& s, int64_t n, const std::string& range_msg, const char* name) {
+    const uint32_t err = append_utf8_from_entries(e, c, s.x, n);
     if (err & STR_ERR_RANGE) throw Error(TG_ERR_INVALID_ARG, std::string("column '") + name + "': " + range_msg);
     if (err & STR_ERR_LONG) throw Error(TG_ERR_UNSUPPORTED, std::string("column '") + name + "': string value of 16 MiB or more");
 }
@@ -513,16 +559,11 @@ void arrow_utf8_finish(Engine& e, Table& t, Column& c, const ArrowStage& s, int6
 }  // namespace
 
 // dictionary<index fmt, utf8 | large_utf8>: `dict` is the dictionary child (its own offset and validity)
-static void append_arrow_dict_utf8(Table& t, const char* name, char index_fmt, bool large_values, const ArrowArray* ca, const ArrowArray* dict) {
-    Engine& e = *t.eng;
-    std::lock_guard<std::mutex> g(e.mu);
-    TG_CUDA(cudaSetDevice(e.device));
-    Column& c = arrow_utf8_column(t, name);
+static void append_arrow_dict_utf8(AppendTxn& txn, const char* name, char index_fmt, bool large_values, const ArrowArray* ca, const ArrowArray* dict) {
+    Engine& e = txn.e;
+    Column& c = txn.column(name, TG_UTF8);
     const int64_t n = ca->length, off = ca->offset;
-    if (n == 0) {
-        t.n_rows = std::max(t.n_rows, c.n_rows);
-        return;
-    }
+    if (n == 0) return;
     if (n >= ((int64_t)1 << 31)) throw Error(TG_ERR_UNSUPPORTED, std::string("column '") + name + "': a batch of 2^31 rows or more");
     const int iw = index_fmt == 'c' || index_fmt == 'C' ? 1 : index_fmt == 's' || index_fmt == 'S' ? 2 : index_fmt == 'i' || index_fmt == 'I' ? 4 : 8;
     const bool idx_signed = index_fmt == 'c' || index_fmt == 's' || index_fmt == 'i' || index_fmt == 'l';
@@ -603,21 +644,16 @@ static void append_arrow_dict_utf8(Table& t, const char* name, char index_fmt, b
     TG_CUDA(cudaGetLastError());
     e.launches += 1;
     const int64_t have = c.n_rows;
-    arrow_utf8_finish(e, t, c, s, n, "a dictionary index lies outside the dictionary", name);
+    arrow_utf8_finish(e, c, s, n, "a dictionary index lies outside the dictionary", name);
     append_validity(e, c, have, validity, bit_off, n);
 }
 
 // utf8_view: buffers = validity, views, data buffers.., variadic buffer sizes (int64 per data buffer)
-static void append_arrow_view_utf8(Table& t, const char* name, const ArrowArray* ca) {
-    Engine& e = *t.eng;
-    std::lock_guard<std::mutex> g(e.mu);
-    TG_CUDA(cudaSetDevice(e.device));
-    Column& c = arrow_utf8_column(t, name);
+static void append_arrow_view_utf8(AppendTxn& txn, const char* name, const ArrowArray* ca) {
+    Engine& e = txn.e;
+    Column& c = txn.column(name, TG_UTF8);
     const int64_t n = ca->length, off = ca->offset;
-    if (n == 0) {
-        t.n_rows = std::max(t.n_rows, c.n_rows);
-        return;
-    }
+    if (n == 0) return;
     if (n >= ((int64_t)1 << 31)) throw Error(TG_ERR_UNSUPPORTED, std::string("column '") + name + "': a batch of 2^31 rows or more");
     if (ca->n_buffers < 3) throw Error(TG_ERR_INVALID_ARG, std::string("Utf8View column '") + name + "': expected a variadic buffer-sizes buffer");
     const int64_t n_data = ca->n_buffers - 3;
@@ -648,7 +684,7 @@ static void append_arrow_view_utf8(Table& t, const char* name, const ArrowArray*
     TG_CUDA(cudaGetLastError());
     e.launches += 1;
     const int64_t have = c.n_rows;
-    arrow_utf8_finish(e, t, c, s, n, "a Utf8View view lies outside its data buffer", name);
+    arrow_utf8_finish(e, c, s, n, "a Utf8View view lies outside its data buffer", name);
     append_validity(e, c, have, validity, off, n);
 }
 
@@ -670,6 +706,7 @@ void table_append_arrow(Table& t, const void* schema_p, const void* array_p) {
     if (!sc || !ar || !sc->format || strcmp(sc->format, "+s") != 0)
         throw Error(TG_ERR_INVALID_ARG, "expected a struct-typed ArrowArray (a RecordBatch)");
     if (ar->offset != 0) throw Error(TG_ERR_UNSUPPORTED, "sliced struct arrays are not supported");
+    AppendTxn txn(t);  // a child that fails undoes the children before it
     for (int64_t i = 0; i < sc->n_children; ++i) {
         const ArrowSchema* cs = sc->children[i];
         const ArrowArray* ca = ar->children[i];
@@ -683,11 +720,11 @@ void table_append_arrow(Table& t, const void* schema_p, const void* array_p) {
             if (!int_index || !utf8_values || !ca->dictionary)
                 throw Error(TG_ERR_UNSUPPORTED, std::string("column '") + cs->name + "': dictionary of " + arrow_type_name(vf) +
                                                     " values (index type " + arrow_type_name(fmt.c_str()) + ") is not supported; string dictionaries only");
-            append_arrow_dict_utf8(t, cs->name, fmt[0], vf[0] == 'U', ca, ca->dictionary);
+            append_arrow_dict_utf8(txn, cs->name, fmt[0], vf[0] == 'U', ca, ca->dictionary);
             continue;
         }
         if (fmt == "vu") {
-            append_arrow_view_utf8(t, cs->name, ca);
+            append_arrow_view_utf8(txn, cs->name, ca);
             continue;
         }
         if (fmt == "vz") throw Error(TG_ERR_UNSUPPORTED, std::string("column '") + cs->name + "': BinaryView is not supported");
@@ -714,13 +751,13 @@ void table_append_arrow(Table& t, const void* schema_p, const void* array_p) {
                 if (d > 0x7fffffffll) throw Error(TG_ERR_UNSUPPORTED, std::string("LargeUtf8 column '") + cs->name + "': a batch holds 2 GiB or more of string bytes");
                 o32[(size_t)r] = (int32_t)d;
             }
-            table_append_host(t, cs->name, dtype, n, (const uint8_t*)ca->buffers[2] + base, o32.data(), validity, off);
+            append_host_column(txn, cs->name, dtype, n, (const uint8_t*)ca->buffers[2] + base, o32.data(), validity, off);
         } else if (dtype == TG_UTF8) {
             const int32_t* offs = (const int32_t*)ca->buffers[1] + off;
-            table_append_host(t, cs->name, dtype, n, ca->buffers[2], offs, validity, off);
+            append_host_column(txn, cs->name, dtype, n, ca->buffers[2], offs, validity, off);
         } else if (dtype == TG_BOOL) {
             // values bitmap shares the array offset; append_bits takes one bit offset for both
-            table_append_host(t, cs->name, dtype, n, ca->buffers[1], nullptr, validity, off);
+            append_host_column(txn, cs->name, dtype, n, ca->buffers[1], nullptr, validity, off);
         } else if (src_w && src_w != (dtype == TG_INT64 ? 8 : 4)) {
             // Int8 / Int16 / UInt8 / UInt16 -> Int32, UInt32 -> Int64: widened exactly on the host
             const uint8_t* src = (const uint8_t*)ca->buffers[1] + off * src_w;
@@ -741,7 +778,7 @@ void table_append_arrow(Table& t, const void* schema_p, const void* array_p) {
                     memcpy(wide.data() + r * 8, &v, 8);
                 }
             }
-            table_append_host(t, cs->name, dtype, n, wide.data(), nullptr, validity, off);
+            append_host_column(txn, cs->name, dtype, n, wide.data(), nullptr, validity, off);
         } else {
             const int w = dtype == TG_INT64 || dtype == TG_FLOAT64 ? 8 : 4;
             const uint8_t* vals = (const uint8_t*)ca->buffers[1] + off * w;
@@ -751,7 +788,7 @@ void table_append_arrow(Table& t, const void* schema_p, const void* array_p) {
                     if (vals[r * 8 + 7] & 0x80) throw Error(TG_ERR_UNSUPPORTED, std::string("UInt64 column '") + cs->name + "' holds values above the Int64 range");
                 }
             }
-            table_append_host(t, cs->name, dtype, n, vals, nullptr, validity, off);
+            append_host_column(txn, cs->name, dtype, n, vals, nullptr, validity, off);
         }
         if (src_type) {
             Column* c = t.find(cs->name);
@@ -761,6 +798,7 @@ void table_append_arrow(Table& t, const void* schema_p, const void* array_p) {
             c->temporal_unit = F.temporal_unit;
         }
     }
+    txn.commit();
 }
 
 }  // namespace tg
