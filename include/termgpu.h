@@ -385,6 +385,24 @@ TG_API tg_status tg_table_shuffle_fingerprints(tg_engine* eng, const char* table
  * batch's rows. */
 TG_API tg_status tg_table_append_arrow(tg_table* t, const void* arrow_schema, const void* arrow_array);
 
+/* Arrow C Device Data Interface ingestion: `arrow_device_array` is a struct ArrowDeviceArray* (128 bytes: the ArrowArray,
+ * int64 device_id, int32 device_type at byte 88, void* sync_event at byte 96, reserved) of a struct-typed array (a
+ * RecordBatch); `arrow_schema` as for tg_table_append_arrow. The caller keeps ownership; the engine never calls release.
+ * By device_type:
+ *   CPU (1): tg_table_append_arrow.
+ *   CUDA_HOST (3): tg_table_append_arrow, after cudaEventSynchronize(*(cudaEvent_t*)sync_event) when an event is given.
+ *   CUDA (2), CUDA_MANAGED (13): converted in HBM by copies and kernels on the engine's device. device_id must be the
+ *     engine's device (TG_ERR_INVALID_ARG otherwise); a given sync_event (a cudaEvent_t*) is waited for on the device
+ *     before any work. Before any copy or kernel, every buffer is checked with cudaPointerGetAttributes: device or managed
+ *     memory of the engine's device only (a host pointer labelled CUDA, or another GPU's memory: TG_ERR_INVALID_ARG). The
+ *     Utf8View variadic-sizes buffer may be host or device memory. Index, offset and value buffers read by a kernel must be
+ *     aligned to their element size (TG_ERR_INVALID_ARG otherwise).
+ *   Any other device type: TG_ERR_UNSUPPORTED.
+ * Types, results and errors are those of tg_table_append_arrow: the call leaves exactly the state a host append of the same
+ * batch leaves, and a failed call leaves the table as it was. The call returns only after every copy and kernel that reads
+ * the producer's buffers has finished: the producer may free or reuse them as soon as it returns. */
+TG_API tg_status tg_table_append_arrow_device(tg_table* t, const void* arrow_schema, const void* arrow_device_array);
+
 /*
  * CSV -> HBM: replaces the reference's CsvSource::register -> DataFusion CSV scan (arrow-csv) -> Arrow batches -> H2D for
  * the GPU path. `bytes` = the file's bytes, or any run of whole records (the caller maps the file; the engine does no I/O).

@@ -105,6 +105,7 @@ SIGNATURES = {
     "tg_table_append_host": (C.c_int, [P, C.c_char_p, C.c_int32, C.c_int64, P, P, P, C.c_int64]),
     "tg_table_adopt_device": (C.c_int, [P, C.c_char_p, C.c_int32, C.c_int64, P, P, P, C.c_int64]),
     "tg_table_append_arrow": (C.c_int, [P, P, P]),
+    "tg_table_append_arrow_device": (C.c_int, [P, P, P]),
     "tg_table_append_csv": (C.c_int, [P, STRS, STRS, C.c_int32, P, C.c_int64, C.c_int32, C.c_int32, C.POINTER(C.c_int64)]),
     "tg_csv_parse_value": (C.c_int, [C.c_char_p, P, C.c_int64, P, C.POINTER(C.c_int32)]),
     "tg_table_append_csv_format": (C.c_int, [P, STRS, STRS, C.c_int32, P, C.c_int64, C.POINTER(tg_csv_format), C.POINTER(C.c_int64)]),

@@ -499,6 +499,30 @@ class SessionContext:
         self._schemas[name] = schema
         return t
 
+    def register_arrow_device(self, name: str, data):
+        """Register RecordBatches through the Arrow C Device Data Interface: `data` is one object implementing
+        `__arrow_c_device_array__` (a RecordBatch; CUDA, CUDA_MANAGED, CUDA_HOST or CPU memory) or a list of them, each one
+        tg_table_append_arrow_device call. CUDA batches are converted in HBM; the producer may free or reuse its buffers as
+        soon as this returns. A failed append drops the table, as register_table does."""
+        if pa is None:
+            raise TypeError("register_arrow_device needs pyarrow")
+        batches = list(data) if isinstance(data, (list, tuple)) else [data]
+        t = self._create(name)
+        schema = None
+        try:
+            for b in batches:
+                sc, ac = b.__arrow_c_device_array__()
+                F.check(F.lib().tg_table_append_arrow_device(t, _capsule_pointer(sc, b"arrow_schema"), _capsule_pointer(ac, b"arrow_device_array")))
+                if schema is None:
+                    schema = pa.Schema._import_from_c_capsule(sc)
+        except Exception:
+            F.lib().tg_table_drop(self._h, name.encode())
+            raise
+        if not hasattr(self, "_schemas"):
+            self._schemas = {}
+        self._schemas[name] = schema
+        return t
+
     def register_device_table(self, name: str, columns: Dict[str, dict], keepalive=None):
         """Adopt HBM-resident Arrow buffers without copying. columns[name] = dict(dtype=TG_*, n_rows=,
         values=ptr, validity=ptr|None, offsets=ptr|None, n_value_bytes=int). Pointers are device addresses."""
@@ -508,6 +532,12 @@ class SessionContext:
                                                   d.get("offsets"), d.get("validity"), d.get("n_value_bytes", 0)))
         self._keepalive[name] = keepalive
         return t
+
+
+def _capsule_pointer(capsule, name: bytes) -> int:
+    get = C.pythonapi.PyCapsule_GetPointer
+    get.restype, get.argtypes = C.c_void_p, [C.py_object, C.c_char_p]
+    return get(capsule, name)
 
 
 def _to_arrow(v):

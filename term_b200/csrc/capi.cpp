@@ -22,6 +22,7 @@ int64_t parquet_decode_to_plain(int32_t encoding, int32_t elem_width, const uint
 void table_adopt_device(Table& t, const std::string& name, int32_t dtype, int64_t n, const void* d_values,
                         const int32_t* d_offsets, const uint8_t* d_validity, int64_t n_value_bytes);
 void table_append_arrow(Table& t, const void* schema_p, const void* array_p);
+void table_append_arrow_device(Table& t, const void* schema_p, const void* device_array_p);
 void table_append_csv(Table& t, const std::vector<std::string>& names, const std::vector<std::string>& fmts, const uint8_t* bytes, int64_t n_bytes,
                       const tg_csv_format* format, int64_t* rows_out);
 void csv_parse_value(const std::string& fmt, const uint8_t* p, int64_t n, void* out, int32_t* is_null);
@@ -357,6 +358,12 @@ tg_status tg_table_append_arrow(tg_table* t, const void* schema, const void* arr
     return guard([&] {
         if (!t) throw Error(TG_ERR_INVALID_ARG, "NULL argument");
         table_append_arrow(*reinterpret_cast<Table*>(t), schema, array);
+    });
+}
+tg_status tg_table_append_arrow_device(tg_table* t, const void* schema, const void* device_array) {
+    return guard([&] {
+        if (!t) throw Error(TG_ERR_INVALID_ARG, "NULL argument");
+        table_append_arrow_device(*reinterpret_cast<Table*>(t), schema, device_array);
     });
 }
 
