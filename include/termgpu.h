@@ -700,6 +700,11 @@ typedef struct {
     double sketch_ms;
     uint64_t bytes_scanned; /* algorithmic bytes (SURVEY §8d) of the last execute */
     uint64_t launches;
+    /* shape of the fused numeric scan (K1) of the last execute, as the planner chose it */
+    uint64_t scan_passes;        /* scan passes run */
+    uint64_t scan_min_tile_rows; /* smallest tile of any pass, rows (0: no pass ran) */
+    uint64_t scan_max_units;     /* largest number of units (aggregate x row slice) of any pass */
+    uint64_t scan_smem_state;    /* 1: some pass kept its unit states in shared memory (more units than consumer warps) */
 } tg_exec_stats;
 TG_API tg_status tg_plan_exec_stats(const tg_plan* plan, tg_exec_stats* out);
 

@@ -249,6 +249,8 @@ def stat_value(col: Col, stat: str) -> Optional[float]:
         if n < 2:
             return None
         f = [float(x) for x in v]
+        if not all(math.isfinite(x) for x in f):  # NaN, or inf - inf (math.fsum raises on +inf with -inf): NaN, as DataFusion
+            return math.nan
         mean = math.fsum(f) / n
         var = math.fsum((x - mean) ** 2 for x in f) / (n - 1)
         return math.sqrt(var) if stat == "StandardDeviation" else var
@@ -1015,6 +1017,9 @@ def _ev(e, row):
         if e[1] == "%":
             if b == 0:
                 raise DivideByZero()
+            if ints:  # truncated remainder (sign of the dividend), exact beyond 2^53
+                r = abs(a) % abs(b)
+                return r if a >= 0 else -r
             return int(math.fmod(a, b))
     if k == "tscale":  # a date / timestamp value in nanoseconds (Python integers: exact)
         v = _ev(e[1], row)

@@ -73,7 +73,8 @@ class tg_csv_format(C.Structure):
 class tg_exec_stats(C.Structure):
     _fields_ = [("gpu_ms", C.c_double), ("scan_ms", C.c_double), ("string_ms", C.c_double),
                 ("hash_ms", C.c_double), ("sketch_ms", C.c_double), ("bytes_scanned", C.c_uint64),
-                ("launches", C.c_uint64)]
+                ("launches", C.c_uint64), ("scan_passes", C.c_uint64), ("scan_min_tile_rows", C.c_uint64),
+                ("scan_max_units", C.c_uint64), ("scan_smem_state", C.c_uint64)]
 
 
 P = C.c_void_p

@@ -178,6 +178,15 @@ __global__ void scan_states_kernel(const ScanAggOut* __restrict__ out, const Sca
 
 static void run_scan_pass(Engine& e, Table& t, Plan& p, std::vector<ScanOp>& ops) {
     if (ops.empty()) return;
+    // the moment sums need K to be an element of the column (their error bound is ~n·eps only then)
+    for (auto& o : ops)
+        if (o.kind == UNIT_NUM_F64 || o.kind == UNIT_NUM_I64 || o.kind == UNIT_PAIR)
+            for (Column* c : {o.c0, o.c1})
+                if (c && !c->pivot_set) {
+                    const uint64_t before = e.launches;
+                    pivot_search(e, *c);
+                    p.stats.launches += e.launches - before;
+                }
     auto P = std::make_unique<ScanParams>();
     memset(P.get(), 0, sizeof(ScanParams));
     std::vector<TileCol> tcols;
@@ -364,6 +373,10 @@ static void run_scan_pass(Engine& e, Table& t, Plan& p, std::vector<ScanOp>& ops
     P->n_aggs = (int)ops.size();
     P->n_code = code_off;
     P->n_terms = term_off;
+    p.stats.scan_passes += 1;
+    if (p.stats.scan_min_tile_rows == 0 || (uint64_t)tile_rows < p.stats.scan_min_tile_rows) p.stats.scan_min_tile_rows = (uint64_t)tile_rows;
+    p.stats.scan_max_units = std::max<uint64_t>(p.stats.scan_max_units, (uint64_t)P->n_units);
+    if (P->n_state_units > 0) p.stats.scan_smem_state = 1;
     for (size_t i = 0; i < units.size(); ++i) P->tab.units[i] = units[i].d;
 
     const int grid = (int)std::min<int64_t>(std::max<int64_t>(P->n_tiles, 1), e.sm_count);
@@ -560,6 +573,62 @@ __global__ void widen_kernel(const uint32_t* __restrict__ src, uint64_t* __restr
     }
 }
 
+// The first (up to) five finite valid values of each block's contiguous row segment, in row order: block b writes them to
+// out[5b..] and their number to out[5 * gridDim.x + b]. The segments in block order then list the column's first values.
+constexpr int PIVOT_SEARCH_THREADS = 256;
+__global__ void pivot_search_kernel(const uint64_t* __restrict__ vals, const uint8_t* __restrict__ bits, int64_t n, int is_f64, uint64_t* __restrict__ out) {
+    __shared__ uint32_t wmask[PIVOT_SEARCH_THREADS / 32];
+    __shared__ int found;
+    const int64_t seg = ((n + gridDim.x - 1) / gridDim.x + PIVOT_SEARCH_THREADS - 1) / PIVOT_SEARCH_THREADS * PIVOT_SEARCH_THREADS;
+    const int64_t beg = (int64_t)blockIdx.x * seg, end = min(n, beg + seg);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (threadIdx.x == 0) found = 0;
+    __syncthreads();
+    for (int64_t base = beg; base < end; base += PIVOT_SEARCH_THREADS) {
+        const int64_t r = base + threadIdx.x;
+        uint64_t v = 0;
+        bool ok = false;
+        if (r < end) {
+            v = vals[r];
+            ok = (!bits || ((bits[r >> 3] >> (r & 7)) & 1)) && (!is_f64 || isfinite(__longlong_as_double((long long)v)));
+        }
+        const uint32_t m = __ballot_sync(0xffffffffu, ok);
+        if (lane == 0) wmask[warp] = m;
+        __syncthreads();
+        const int have = found;
+        int before = __popc(m & ((1u << lane) - 1u)), total = 0;
+        for (int w = 0; w < PIVOT_SEARCH_THREADS / 32; ++w) {
+            if (w < warp) before += __popc(wmask[w]);
+            total += __popc(wmask[w]);
+        }
+        if (ok && have + before < 5) out[5 * blockIdx.x + have + before] = v;
+        __syncthreads();  // every thread has read `found` and the masks
+        if (threadIdx.x == 0) found = min(5, have + total);
+        __syncthreads();
+        if (found == 5) break;
+    }
+    if (threadIdx.x == 0) out[5 * gridDim.x + blockIdx.x] = (uint64_t)found;
+}
+
+void pivot_search(Engine& e, Column& c) {
+    if (c.pivot_set || (c.dtype != TG_INT64 && c.dtype != TG_FLOAT64) || c.n_rows <= c.null_count || !c.values.p) return;
+    const int grid = (int)std::min<int64_t>((c.n_rows + PIVOT_SEARCH_THREADS - 1) / PIVOT_SEARCH_THREADS, e.sm_count);
+    const size_t bytes = (size_t)grid * 6 * 8;
+    uint64_t* d = reinterpret_cast<uint64_t*>(e.scratch(bytes));
+    pivot_search_kernel<<<grid, PIVOT_SEARCH_THREADS, 0, e.stream>>>(reinterpret_cast<const uint64_t*>(c.values.p), c.validity.p, c.n_rows,
+                                                                     c.dtype == TG_FLOAT64 ? 1 : 0, d);
+    TG_CUDA(cudaGetLastError());
+    e.launches += 1;
+    uint64_t* h = reinterpret_cast<uint64_t*>(e.host_scratch(bytes));
+    TG_CUDA(cudaMemcpyAsync(h, d, bytes, cudaMemcpyDeviceToHost, e.stream));
+    TG_CUDA(cudaStreamSynchronize(e.stream));
+    uint64_t first[5];
+    int m = 0;
+    for (int b = 0; b < grid && m < 5; ++b)
+        for (uint64_t k = 0; k < h[5 * grid + b] && m < 5; ++k) first[m++] = h[5 * b + k];
+    set_pivot_host(c, c.dtype, m, first, nullptr, 0);
+}
+
 Column* numeric_view(Engine& e, Column* c) {
     if (!c) return nullptr;
     if (c->dtype == TG_INT64 || c->dtype == TG_FLOAT64) return c;
@@ -577,17 +646,10 @@ Column* numeric_view(Engine& e, Column* c) {
                                                      c->n_rows, c->dtype == TG_FLOAT32 ? 1 : 0);
             TG_CUDA(cudaGetLastError());
             e.launches += 1;
-            // pivot of the shifted sums: from the first values, like every 8-byte column
-            const int64_t head = std::min<int64_t>(c->n_rows, 65536);
-            std::vector<uint8_t> hv((size_t)head * 8), hb((size_t)(head + 7) / 8);
-            TG_CUDA(cudaMemcpyAsync(hv.data(), w.values.p, hv.size(), cudaMemcpyDeviceToHost, e.stream));
-            if (c->validity.p) TG_CUDA(cudaMemcpyAsync(hb.data(), c->validity.p, hb.size(), cudaMemcpyDeviceToHost, e.stream));
-            TG_CUDA(cudaStreamSynchronize(e.stream));
-            w.pivot_set = false;
-            set_pivot_host(w, w.dtype, head, hv.data(), c->validity.p ? hb.data() : nullptr, 0);
         }
         w.n_rows = c->n_rows;
         w.value_bytes = c->n_rows * 8;
+        w.pivot_set = false;  // the scan finds the pivot (pivot_search) before its first moment sums over this view
     }
     w.validity.p = c->validity.p;  // (may have been reallocated by an append: refreshed on every use)
     w.validity.cap = 0;

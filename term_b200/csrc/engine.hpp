@@ -185,6 +185,9 @@ struct Engine {
 
 // the column itself when it is Int64 / Float64, the widened shadow of an Int32 / Float32 column, nullptr for other types
 Column* numeric_view(Engine& e, Column* c);
+// pivot of an Int64 / Float64 column that has none yet (the append paths look at a head window only, which may hold no
+// finite valid value): set_pivot_host on the first five finite valid values of the whole column, found on the device
+void pivot_search(Engine& e, Column& c);
 void column_free(Engine& e, Column& c);
 
 // One append call (tg_table_append_*): holds the engine's lock and makes the call all or nothing. A call that throws

@@ -1016,6 +1016,18 @@ static std::string join(const std::vector<std::string>& v, const char* sep) {
     return r;
 }
 
+// Σ(x-x̄)² from the shifted sums: m2 = Σd² - (Σd)²/n with d = x - K.
+//  * a rounding-negative m2 is 0;
+//  * a NaN or an infinite value in the column makes Σd and Σd² NaN / infinite and m2 NaN (DataFusion's VARIANCE is NaN);
+//  * finite values whose squared deviations overflow leave Σd finite (an infinite value would make it infinite or NaN)
+//    but Σd² = +inf, and inf - inf would read NaN: the variance is beyond the double range, +inf (as DataFusion's).
+static double central_m2(double n, double sd, double sdd) {
+    const double m2 = sdd - sd * sd / n;
+    if (m2 < 0.0) return 0.0;
+    if (std::isnan(m2) && std::isfinite(sd) && sdd == INFINITY) return INFINITY;
+    return m2;
+}
+
 // value of a SQL aggregate over the A_NUM state, with DataFusion result typing
 // (constraints/statistics.rs:278-308): returns false when the SQL result is NULL
 static bool stat_value(const Agg& a, int kind, double* out) {
@@ -1042,8 +1054,7 @@ static bool stat_value(const Agg& a, int kind, double* out) {
         case TG_STAT_VARIANCE: {
             if (n < 2) return false;
             double nn = (double)n;
-            double m2 = a.f[2] - a.f[1] * a.f[1] / nn;
-            double var = std::max(0.0, m2 / (nn - 1.0));
+            double var = central_m2(nn, a.f[1], a.f[2]) / (nn - 1.0);
             *out = kind == TG_STAT_STDDEV ? std::sqrt(var) : var;
             return true;
         }
@@ -1664,7 +1675,7 @@ static void finalize_analyzer(Plan& p, Slot& s) {
             r.metric_kind = 2;
             // metric map (standard_deviation.rs:239-279) from the shifted moments (better conditioned than
             // the reference's E[x^2]-E[x]^2, equal to it in exact arithmetic)
-            const double m2 = std::max(0.0, a.f[2] - a.f[1] * a.f[1] / n);
+            const double m2 = central_m2(n, a.f[1], a.f[2]);
             const double pop_var = m2 / n;
             s.map.emplace_back("count", n);
             s.map.emplace_back("mean", r.f[2]);
