@@ -574,6 +574,22 @@ TG_API tg_status tg_plan_execute(tg_engine* eng, tg_plan* plan, const char* tabl
  * merges every rank's blob IN RANK ORDER and finalizes — mirrors AnalyzerState::merge
  * (analyzers/traits.rs:154-179). */
 TG_API tg_status tg_plan_execute_partial(tg_engine* eng, tg_plan* plan, const char* table_name);
+
+/* Row-level verdicts (an engine extension beyond the reference's ConstraintResult). A slot whose mask was requested before an
+ * execute (tg_plan_execute or tg_plan_execute_partial; the exchange entry points build none) gets an Arrow Boolean array of the
+ * executed table's rows: values bit i = row i is counted in the slot's metric numerator, validity bit i = row i is in its
+ * denominator (no validity buffer: every row is). popcount(values & validity) / popcount(validity) is the reported metric.
+ * Supported: completeness of one column, custom_sql / satisfies, containment, non_negative, format / pattern, data type,
+ * length, and the completeness and compliance analyzers; other kinds are TG_ERR_UNSUPPORTED, a bad slot TG_ERR_INVALID_ARG.
+ * Plans that request no mask run exactly the kernels they run without this feature. */
+TG_API tg_status tg_plan_request_row_mask(tg_plan* plan, int32_t slot);
+/* Fills a struct ArrowSchema (format "b") and a struct ArrowDeviceArray (CUDA, the engine's device; buffers[0] = validity or
+ * NULL, buffers[1] = values; sync_event NULL: execute synchronised before returning). The array holds a reference to its
+ * buffers: it stays valid after the plan is re-executed or destroyed, until its release is called, which must happen
+ * before the engine is destroyed. Errors: a slot not requested, or not executed since the request: TG_ERR_INVALID_ARG;
+ * a slot whose evaluation failed: that error (division by zero in a predicate: TG_ERR_INVALID_ARG), message in
+ * tg_last_error(). */
+TG_API tg_status tg_plan_export_row_mask(const tg_plan* plan, int32_t slot, void* arrow_schema_out, void* arrow_device_array_out);
 TG_API tg_status tg_plan_partial_size(const tg_plan* plan, size_t* n_bytes);
 TG_API tg_status tg_plan_partial_export(const tg_plan* plan, void* buf, size_t n_bytes);
 /* host-only: build partials for a plan without a GPU from an exported blob (tests, incremental runs) */

@@ -143,6 +143,8 @@ SIGNATURES = {
     "tg_plan_add_value_histogram": (C.c_int32, [P, C.c_char_p]),
     "tg_plan_execute": (C.c_int, [P, P, C.c_char_p]),
     "tg_plan_execute_partial": (C.c_int, [P, P, C.c_char_p]),
+    "tg_plan_request_row_mask": (C.c_int, [P, C.c_int32]),
+    "tg_plan_export_row_mask": (C.c_int, [P, C.c_int32, P, P]),
     "tg_plan_partial_size": (C.c_int, [P, C.POINTER(C.c_size_t)]),
     "tg_plan_partial_export": (C.c_int, [P, P, C.c_size_t]),
     "tg_plan_partial_reset": (C.c_int, [P]),

@@ -551,6 +551,58 @@ def _to_arrow(v):
     return pa.array(v)
 
 
+# Arrow PyCapsule protocol for the row masks a plan exports: the structs live in malloc'ed memory owned by the capsule; its
+# destructor releases a struct the consumer did not move out (release still set) and frees the memory.
+_libc = C.CDLL(None)
+_libc.malloc.restype, _libc.malloc.argtypes = C.c_void_p, [C.c_size_t]
+_libc.free.restype, _libc.free.argtypes = None, [C.c_void_p]
+_CAP_SCHEMA, _CAP_DEVICE_ARRAY = b"arrow_schema", b"arrow_device_array"
+_capsule_new = C.pythonapi.PyCapsule_New
+_capsule_new.restype, _capsule_new.argtypes = C.py_object, [C.c_void_p, C.c_char_p, C.c_void_p]
+_RELEASE = C.CFUNCTYPE(None, C.c_void_p)
+_capsule_structs = {}  # address of a live capsule -> its struct (the destructor touches no C API of the dying object)
+
+
+def _capsule_destructor(release_offset: int):
+    def dtor(capsule):
+        p = _capsule_structs.pop(capsule, None)
+        if p:
+            rel = C.c_void_p.from_address(p + release_offset).value
+            if rel:
+                _RELEASE(rel)(p)
+            _libc.free(p)
+    return C.CFUNCTYPE(None, C.c_void_p)(dtor)
+
+
+_SCHEMA_DTOR = _capsule_destructor(56)        # ArrowSchema.release
+_DEVICE_ARRAY_DTOR = _capsule_destructor(64)  # ArrowDeviceArray.array.release
+
+
+class RowMask:
+    """Row verdicts of one slot: an Arrow Boolean array in the engine's device memory (values bit i = row i is in the
+    metric's numerator, validity bit i = row i is in its denominator). Consumed through `__arrow_c_device_array__`; it owns
+    its buffers until the consumer imports it or this object is collected, which must happen before the engine is closed."""
+
+    def __init__(self, plan_handle, slot: int):
+        sp, ap = _libc.malloc(72), _libc.malloc(128)
+        C.memset(sp, 0, 72)
+        C.memset(ap, 0, 128)
+        # the capsules own the memory from here on, also when the export fails (release stays NULL then)
+        self._schema = _capsule_new(sp, _CAP_SCHEMA, C.cast(_SCHEMA_DTOR, C.c_void_p))
+        self._array = _capsule_new(ap, _CAP_DEVICE_ARRAY, C.cast(_DEVICE_ARRAY_DTOR, C.c_void_p))
+        _capsule_structs[id(self._schema)] = sp
+        _capsule_structs[id(self._array)] = ap
+        F.check(F.lib().tg_plan_export_row_mask(plan_handle, slot, sp, ap))
+        self.length = C.c_int64.from_address(ap).value
+        self.null_count = C.c_int64.from_address(ap + 8).value
+        bufs = C.c_void_p.from_address(ap + 40).value
+        self.validity_ptr = C.c_void_p.from_address(bufs).value or 0
+        self.values_ptr = C.c_void_p.from_address(bufs + 8).value or 0
+
+    def __arrow_c_device_array__(self, requested_schema=None, **kwargs):
+        return self._schema, self._array
+
+
 # ----------------------------------------------------------------------------- plan ----
 class Plan:
     """Thin RAII wrapper of tg_plan."""
@@ -580,6 +632,14 @@ class Plan:
         self._ctx_schema = getattr(ctx, "_schemas", {}).get(table)
         self._ctx = ctx
         F.check(F.lib().tg_plan_execute_partial(ctx.handle, self._h, table.encode()))
+
+    def request_row_mask(self, slot: int):
+        """Ask the next execute to keep slot `slot`'s row verdicts (tg_plan_request_row_mask)."""
+        F.check(F.lib().tg_plan_request_row_mask(self._h, slot))
+
+    def row_mask(self, slot: int) -> RowMask:
+        """The row verdicts of slot `slot` from the last execute (tg_plan_export_row_mask)."""
+        return RowMask(self._h, slot)
 
     def partial_export(self) -> bytes:
         n = C.c_size_t()

@@ -1,6 +1,7 @@
 // extern "C" surface declared in include/termgpu.h
 #include <cstring>
 
+#include "arrow_abi.h"
 #include "engine.hpp"
 #include "hashpart.hpp"
 #include "radix_sort.cuh"
@@ -125,6 +126,12 @@ void tg_engine_destroy(tg_engine* h) {
         }
     }
     e.tables.clear();
+    {
+        std::lock_guard<std::mutex> g(e.mask_returns->mu);
+        for (auto& b : e.mask_returns->blocks) cudaFree(b.first);
+        e.mask_returns->blocks.clear();
+        e.mask_returns->engine_alive = false;
+    }
     for (auto& b : e.deferred_free) cudaFree(b.first);  // the device is idle (synchronised above)
     e.deferred_free.clear();
     e.dev_trim();
@@ -483,6 +490,53 @@ tg_status tg_plan_execute(tg_engine* h, tg_plan* p, const char* table_name) {
         p->p.finalize();
     });
 }
+tg_status tg_plan_request_row_mask(tg_plan* p, int32_t slot) {
+    return guard([&] {
+        if (!p) throw Error(TG_ERR_INVALID_ARG, "NULL argument");
+        plan_request_row_mask(p->p, slot);
+    });
+}
+
+// private data of an exported row mask: the schema owns nothing; the array keeps the mask's buffers alive
+struct RowMaskExport {
+    std::shared_ptr<RowMask> mask;
+    const void* buffers[2];
+};
+static void row_mask_release_schema(ArrowSchema* s) { s->release = nullptr; }
+static void row_mask_release_array(ArrowArray* a) {
+    delete static_cast<RowMaskExport*>(a->private_data);
+    a->release = nullptr;
+}
+
+tg_status tg_plan_export_row_mask(const tg_plan* p, int32_t slot, void* arrow_schema_out, void* arrow_device_array_out) {
+    return guard([&] {
+        if (!p || !arrow_schema_out || !arrow_device_array_out) throw Error(TG_ERR_INVALID_ARG, "NULL argument");
+        if (slot < 0 || slot >= (int32_t)p->p.slots.size()) throw Error(TG_ERR_INVALID_ARG, "slot index out of range");
+        const Slot& s = p->p.slots[slot];
+        if (!s.mask_requested) throw Error(TG_ERR_INVALID_ARG, "row mask of slot " + std::to_string(slot) + " was not requested");
+        if (!s.mask_built) throw Error(TG_ERR_INVALID_ARG, "row mask of slot " + std::to_string(slot) + " was requested but the plan was not executed since");
+        if (s.mask_err != TG_OK) throw Error(s.mask_err, s.mask_err_msg);
+        auto* x = new RowMaskExport{s.mask, {s.mask->validity, s.mask->values}};
+        ArrowSchema* sc = static_cast<ArrowSchema*>(arrow_schema_out);
+        *sc = ArrowSchema{};
+        sc->format = "b";
+        sc->name = "";
+        sc->flags = 2;  // ARROW_FLAG_NULLABLE
+        sc->release = row_mask_release_schema;
+        ArrowDeviceArray* da = static_cast<ArrowDeviceArray*>(arrow_device_array_out);
+        *da = ArrowDeviceArray{};
+        da->array.length = s.mask->n_rows;
+        da->array.null_count = s.mask->null_count;
+        da->array.n_buffers = 2;
+        da->array.buffers = x->buffers;
+        da->array.release = row_mask_release_array;
+        da->array.private_data = x;
+        da->device_id = s.mask->device;
+        da->device_type = ARROW_DEVICE_CUDA;
+        da->sync_event = nullptr;
+    });
+}
+
 tg_status tg_plan_partial_size(const tg_plan* p, size_t* n) {
     return guard([&] {
         if (!p || !n) throw Error(TG_ERR_INVALID_ARG, "NULL argument");

@@ -348,6 +348,7 @@ static void run_scan_pass(Engine& e, Table& t, Plan& p, std::vector<ScanOp>& ops
             u.d.c0_is_i64 = o.c0 && o.c0->dtype == TG_INT64;
             u.d.c1_is_i64 = o.c1 && o.c1->dtype == TG_INT64;
             u.d.flags = o.flags;
+            u.d.bits = o.kind == UNIT_PRED || o.kind == UNIT_TERMS ? p.aggs[o.agg].bits : nullptr;
             u.cost = o.cost * u.d.nrows / tile_rows;
             units.push_back(u);
         }
@@ -1419,6 +1420,124 @@ void exec_scan_jobs(Engine& e, Table& t, Plan& p, const std::vector<int>& agg_id
     }
 }
 
+// ------------------------------------------------------------------ row verdicts ----
+// One Arrow Boolean array per requested slot, from the words the kernels stored for its aggregate and the column's validity:
+//   values   = bits (or the column's validity when bits is null: completeness), OR-ed with ~validity when or_invalid
+//   validity = the column's validity when validity_out is given (the metric's population is its non-null rows), else none
+// Bits past n_rows are zero. valid_count receives the popcount of the written validity.
+constexpr int MASK_THREADS = 256;
+__global__ void __launch_bounds__(MASK_THREADS) row_mask_kernel(const uint32_t* __restrict__ bits, const uint32_t* __restrict__ valid,
+                                                                 int or_invalid, int64_t n_rows, uint32_t* __restrict__ values_out,
+                                                                 uint32_t* __restrict__ validity_out, unsigned long long* valid_count) {
+    const int64_t n_words = (n_rows + 31) >> 5;
+    uint32_t cnt = 0;
+    for (int64_t i = (int64_t)blockIdx.x * MASK_THREADS + threadIdx.x; i < n_words; i += (int64_t)gridDim.x * MASK_THREADS) {
+        const int64_t rem = n_rows - 32 * i;
+        const uint32_t tail = rem >= 32 ? 0xffffffffu : (1u << rem) - 1u;
+        const uint32_t v = valid ? valid[i] : 0xffffffffu;
+        uint32_t b = bits ? bits[i] : v;
+        if (or_invalid) b |= ~v;
+        values_out[i] = b & tail;
+        if (validity_out) {
+            validity_out[i] = v & tail;
+            cnt += __popc(v & tail);
+        }
+    }
+    if (!validity_out) return;
+    for (int m = 16; m > 0; m >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, m);
+    if ((threadIdx.x & 31) == 0 && cnt) atomicAdd(valid_count, (unsigned long long)cnt);
+}
+
+static void give_back_row_masks(Engine& e) {
+    std::vector<std::pair<uint8_t*, size_t>> blocks;
+    {
+        std::lock_guard<std::mutex> g(e.mask_returns->mu);
+        blocks.swap(e.mask_returns->blocks);
+    }
+    for (auto& b : blocks) e.dev_free(b.first, b.second);
+}
+
+static size_t row_words_bytes(int64_t n_rows) { return std::max<size_t>(256, round_up((size_t)((n_rows + 31) / 32) * 4, 256)); }
+
+// aggregates that store row words for a requested slot get a word buffer for this execute
+static void alloc_row_bits(Engine& e, Table* t, Plan& p) {
+    if (!t || t->n_rows == 0) return;
+    for (auto& a : p.aggs)
+        if (a.row_bits && a.err == TG_OK && (a.kind == A_PRED || a.kind == A_REGEX || a.kind == A_LENGTH))
+            a.bits = reinterpret_cast<uint32_t*>(e.dev_alloc(row_words_bytes(t->n_rows)));
+}
+static void free_row_bits(Engine& e, Table* t, Plan& p) {
+    for (auto& a : p.aggs)
+        if (a.bits) {
+            e.dev_free(reinterpret_cast<uint8_t*>(a.bits), row_words_bytes(t->n_rows));
+            a.bits = nullptr;
+        }
+}
+
+static void build_row_masks(Engine& e, Table* t, Plan& p) {
+    const int64_t n = t ? t->n_rows : 0;
+    const size_t bytes = row_words_bytes(n);
+    unsigned long long* d_counts = nullptr;
+    std::vector<std::shared_ptr<RowMask>> counted;
+    bool launched = false;
+    for (auto& s : p.slots) {
+        if (!s.mask_requested) continue;
+        s.mask_built = true;
+        s.mask.reset();
+        s.mask_err = TG_OK;
+        s.mask_err_msg.clear();
+        const Agg& a = p.aggs[s.aggs[0]];
+        const Agg* valid_agg = s.kind == SL_CONTAINMENT || s.kind == SL_NON_NEGATIVE ? &p.aggs[s.aggs[1]] : nullptr;
+        if (a.err != TG_OK || (valid_agg && valid_agg->err != TG_OK)) {
+            const Agg& bad = a.err != TG_OK ? a : *valid_agg;
+            s.mask_err = bad.err;
+            s.mask_err_msg = bad.err_msg;
+            continue;
+        }
+        if (a.kind == A_PRED && a.u[1]) {  // the reference's query fails: there are no verdicts
+            s.mask_err = TG_ERR_INVALID_ARG;
+            s.mask_err_msg = "SQL execution error: Arrow error: Divide by zero error. Expression: '" + a.text + "'";
+            continue;
+        }
+        Column* c = s.columns.empty() || !t ? nullptr : t->find(s.columns[0]);
+        const uint32_t* valid = c ? reinterpret_cast<const uint32_t*>(c->validity.p) : nullptr;
+        const bool or_invalid = s.kind == SL_LENGTH || (s.kind == SL_FORMAT && s.fopt.null_is_valid);
+        const bool emit_validity = valid && (s.kind == SL_CONTAINMENT || s.kind == SL_NON_NEGATIVE || s.kind == SL_DATA_TYPE);
+        auto m = std::make_shared<RowMask>();
+        m->n_rows = n;
+        m->bytes = bytes;
+        m->device = e.device;
+        std::shared_ptr<MaskReturns> box = e.mask_returns;
+        m->give_back = [box](uint8_t* b, size_t sz) {
+            std::lock_guard<std::mutex> g(box->mu);
+            if (box->engine_alive) box->blocks.emplace_back(b, sz);
+            else cudaFree(b);
+        };
+        m->values = e.dev_alloc(bytes);
+        if (emit_validity) m->validity = e.dev_alloc(bytes);
+        if (emit_validity && !d_counts) {
+            d_counts = reinterpret_cast<unsigned long long*>(e.scratch(8 * p.slots.size()));
+            TG_CUDA(cudaMemsetAsync(d_counts, 0, 8 * p.slots.size(), e.stream));
+        }
+        const int grid = (int)std::max<int64_t>(1, std::min<int64_t>(((n + 31) / 32 + MASK_THREADS - 1) / MASK_THREADS, (int64_t)e.sm_count * 4));
+        row_mask_kernel<<<grid, MASK_THREADS, 0, e.stream>>>(a.kind == A_VALID ? nullptr : a.bits, valid, or_invalid ? 1 : 0, n,
+                                                              reinterpret_cast<uint32_t*>(m->values), reinterpret_cast<uint32_t*>(m->validity),
+                                                              emit_validity ? d_counts + counted.size() : nullptr);
+        TG_CUDA(cudaGetLastError());
+        e.launches += 1;
+        p.stats.launches += 1;
+        launched = true;
+        if (emit_validity) counted.push_back(m);
+        s.mask = std::move(m);
+    }
+    if (!launched) return;
+    std::vector<unsigned long long> h(counted.size());
+    if (!counted.empty()) TG_CUDA(cudaMemcpyAsync(h.data(), d_counts, 8 * counted.size(), cudaMemcpyDeviceToHost, e.stream));
+    // the exported arrays carry no sync_event: every mask is complete when execute returns
+    TG_CUDA(cudaStreamSynchronize(e.stream));
+    for (size_t i = 0; i < counted.size(); ++i) counted[i]->null_count = n - (int64_t)h[i];
+}
+
 // ------------------------------------------------------------------ execute ----
 
 void execute_partial(Engine& e, Plan& p, const std::string& table_name) {
@@ -1428,6 +1547,7 @@ void execute_partial(Engine& e, Plan& p, const std::string& table_name) {
     p.stats = tg_exec_stats{};
     p.executed = false;
     e.sync_copies();
+    give_back_row_masks(e);
     auto it = e.tables.find(table_name);
     Table* t = it == e.tables.end() ? nullptr : it->second.get();
     std::vector<int> scan_ids, string_ids, kll_ids, length_ids, grouped_ids;
@@ -1457,6 +1577,14 @@ void execute_partial(Engine& e, Plan& p, const std::string& table_name) {
             default: break;
         }
     }
+    // word buffers of the aggregates behind requested row verdicts live for this execute only
+    struct RowBits {
+        Engine& e;
+        Table* t;
+        Plan& p;
+        ~RowBits() { free_row_bits(e, t, p); }
+    } row_bits{e, t, p};
+    alloc_row_bits(e, t, p);
     if (t && !scan_ids.empty()) exec_scan_jobs(e, *t, p, scan_ids);
     if (t && !string_ids.empty()) exec_string_jobs(e, *t, p, string_ids);
     if (t && !length_ids.empty()) exec_length_jobs(e, *t, p, length_ids);
@@ -1489,6 +1617,7 @@ void execute_partial(Engine& e, Plan& p, const std::string& table_name) {
             a.err_msg = er.msg;
         }
     }
+    build_row_masks(e, t, p);
 }
 
 // ------------------------------------------------------------------ fused multi-GPU step (scan-only plans) ----

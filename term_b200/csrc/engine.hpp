@@ -25,7 +25,12 @@ namespace tg {
     } while (0)
 
 struct Engine;
-struct RankSession;  // ranks.cu: state of a Spearman evaluation between its stages
+struct RankSession;
+struct MaskReturns {
+    std::mutex mu;
+    std::vector<std::pair<uint8_t*, size_t>> blocks;
+    bool engine_alive = true;
+};  // ranks.cu: state of a Spearman evaluation between its stages
 
 struct DevBuf {
     uint8_t* p = nullptr;
@@ -154,6 +159,9 @@ struct Engine {
     uint8_t* dev_alloc(size_t bytes);
     void dev_free(uint8_t* p, size_t bytes);
     void dev_trim();
+    // device blocks of row masks whose last owner (a slot or an exported Arrow array) let go; the next execute hands them to
+    // dev_free. Shared with the masks: one that outlives the engine frees its blocks itself.
+    std::shared_ptr<MaskReturns> mask_returns = std::make_shared<MaskReturns>();
 
     // side streams: independent bucket pipelines of the partitioned hash jobs run concurrently on them
     cudaStream_t side[4] = {nullptr, nullptr, nullptr, nullptr};

@@ -1062,6 +1062,32 @@ static bool stat_value(const Agg& a, int kind, double* out) {
     return false;
 }
 
+bool slot_has_row_mask(const Slot& s) {
+    switch (s.kind) {
+        case SL_COMPLETENESS: return s.columns.size() == 1;
+        case SL_SQL:
+        case SL_CONTAINMENT:
+        case SL_NON_NEGATIVE:
+        case SL_FORMAT:
+        case SL_DATA_TYPE:
+        case SL_LENGTH: return true;
+        case SL_ANALYZER: return s.sub_kind == TG_AN_COMPLETENESS || s.sub_kind == TG_AN_COMPLIANCE;
+        default: return false;
+    }
+}
+
+void plan_request_row_mask(Plan& p, int slot) {
+    if (slot < 0 || slot >= (int)p.slots.size()) throw Error(TG_ERR_INVALID_ARG, "slot index out of range");
+    Slot& s = p.slots[slot];
+    if (!slot_has_row_mask(s))
+        throw Error(TG_ERR_UNSUPPORTED, "row verdicts are not available for the '" + s.name + "' slot (row-level constraints only)");
+    s.mask_requested = true;
+    s.mask_built = false;
+    // the first aggregate holds the per-row decision (predicate, pattern, length range); COUNT(c) needs no bits: the column's
+    // validity bitmap is its verdict
+    p.aggs[s.aggs[0]].row_bits = true;
+}
+
 static void finalize_completeness(Plan& p, Slot& s) {
     // per-column evaluate_column (completeness.rs:137-246)
     struct ColRes {

@@ -4,6 +4,8 @@
 //   aggregates : the de-duplicated device work the slots need; each aggregate has a partial state that
 //                merges across row shards (GPUs) like AnalyzerState::merge (analyzers/traits.rs:154-179)
 #pragma once
+#include <functional>
+#include <memory>
 #include <string>
 #include <utility>
 #include <vector>
@@ -42,6 +44,10 @@ struct Agg {
     // multi-GPU shuffle: read this aggregate's keys from another registered table (the hash-shuffled shard) instead
     // of the plan's table; [0] = the table of a DISTINCT aggregate or the child table of an FK, [1] = the FK parent
     std::string redirect[2];
+    // some slot requested its row verdicts (tg_plan_request_row_mask): the kernels of this aggregate also store one word per 32
+    // rows to `bits` (device, held by execute_partial for the duration of one execute). Not part of the de-duplication key.
+    bool row_bits = false;
+    uint32_t* bits = nullptr;
     // construction-time problem the reference only reports when the constraint is evaluated
     tg_status ctor_err = TG_OK;
     std::string ctor_err_msg;
@@ -90,6 +96,24 @@ enum SlotKind : int32_t {
     SL_VALUE_HIST,
 };
 
+// One slot's row verdicts as an Arrow Boolean array in device memory (engine.cu build_row_masks): values bit i = row i is in
+// the metric's numerator, validity bit i = row i is in its denominator (validity null: every row). Shared between the slot and
+// the arrays exported from it; the last owner hands the buffers back to the engine through `give_back`.
+struct RowMask {
+    int64_t n_rows = 0, null_count = 0;
+    uint8_t* values = nullptr;
+    uint8_t* validity = nullptr;
+    size_t bytes = 0;  // capacity of each buffer
+    int device = 0;
+    std::function<void(uint8_t*, size_t)> give_back;
+    ~RowMask() {
+        if (give_back) {
+            give_back(values, bytes);
+            if (validity) give_back(validity, bytes);
+        }
+    }
+};
+
 struct StatReq {
     int32_t kind;
     double percentile;
@@ -130,7 +154,15 @@ struct Slot {
     tg_analyzer_result ares{};
     std::string metric_key;
     std::vector<std::pair<std::string, double>> map;
+    // row verdicts: requested before execute; the mask (or the reason there is none) of the last execute since the request
+    bool mask_requested = false, mask_built = false;
+    std::shared_ptr<RowMask> mask;
+    tg_status mask_err = TG_OK;
+    std::string mask_err_msg;
 };
+
+// slot kinds whose row verdicts can be exported; false for the others (and for completeness over several columns)
+bool slot_has_row_mask(const Slot& s);
 
 struct Plan {
     std::vector<Agg> aggs;
@@ -175,6 +207,8 @@ int plan_add_quantile(Plan& p, const std::string& col, int mode, const std::vect
                       const std::vector<tg_assertion>& assertions, int strict);
 // HistogramConstraint (constraints/histogram.rs:208-244): value frequencies of one column, as a grouped count of the column by itself
 int plan_add_value_histogram(Plan& p, const std::string& col);
+// marks a slot's row verdicts for the next execute (TG_ERR_UNSUPPORTED for a kind without them, TG_ERR_INVALID_ARG out of range)
+void plan_request_row_mask(Plan& p, int slot);
 int plan_add_grouped_completeness(Plan& p, const std::string& col, const std::vector<std::string>& groups,
                                   int max_groups, int include_overall);
 

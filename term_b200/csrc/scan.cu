@@ -78,6 +78,7 @@ __device__ __forceinline__ void max_if_i64(int64_t& mx, int64_t x, uint32_t m) {
 
 // ---- COUNT: popcount of validity words ----
 struct CountUnit {
+    static constexpr bool MASK = false;
     uint32_t bits_off;
     int w0, nw, row0, lane;
     uint64_t n;
@@ -112,6 +113,7 @@ struct CountUnit {
 template <bool IS_I64, int FLAGS>
 struct NumUnit {
     static constexpr bool MOM = (FLAGS & UF_MOMENTS) != 0, MM = (FLAGS & UF_MINMAX) != 0, ISUM = IS_I64 && (FLAGS & UF_ISUM) != 0;
+    static constexpr bool MASK = false;
     uint32_t val_off, bits_off;  // bits_off == ~0u: no bitmap
     int row0, nrows, lane;
     double K;
@@ -255,6 +257,7 @@ struct NumUnit {
 // ---- PAIR: co-moments over the rows where both columns are valid ----
 template <bool XI, bool YI>
 struct PairUnit {
+    static constexpr bool MASK = false;
     uint32_t vx_off, vy_off, bx_off, by_off;
     int row0, nrows, lane;
     double Kx, Ky, sx[2], sy[2], sxx[2], syy[2], sxy[2];
@@ -419,12 +422,18 @@ __device__ __forceinline__ uint32_t valid_loop(const uint4* b4, int nq, uint32_t
     return pm;
 }
 
+// MASK_: also store the TRUE word of every 32 rows to the aggregate's bit buffer (tile_row0 = the tile's first table row)
+template <bool MASK_>
 struct TermsUnit {
+    static constexpr bool MASK = MASK_;
     const ScanTables* T;
     int t0, nt, row0, nrows, lane;
     bool is_or;
     uint64_t cnt;
+    uint32_t *bits, *tbits;  // the aggregate's words / those of the current tile (null: no verdicts requested)
+    __device__ __forceinline__ void at_tile(int64_t tile_row0) { tbits = bits ? bits + (tile_row0 >> 5) : nullptr; }
     __device__ __forceinline__ void setup(const ScanTables& T_, const ScanUnitDesc& u, int lane_) {
+        if constexpr (MASK) bits = u.bits;
         T = &T_;
         t0 = u.code_off;
         nt = u.code_len;
@@ -469,6 +478,18 @@ struct TermsUnit {
             if (partial) ng = max(0, min(ng, (rows - base - lane + 31) >> 5));
             const uint32_t gmask = ng >= 32 ? 0xffffffffu : ((1u << ng) - 1u);
             cnt += __popc(m & gmask);
+            if (MASK && tbits) {
+                // transpose: lane g collects the word of group g (bit l = row base + 32 g + l); a 32-row word lies in exactly
+                // one unit slice of one tile, so it has exactly one writer
+                const int ngrp = 4 * nq;
+                uint32_t word = 0;
+                for (int g = 0; g < ngrp; ++g) {
+                    const uint32_t b = __ballot_sync(0xffffffffu, (m >> g) & 1u);
+                    if (lane == g) word = b;
+                }
+                if (lane < ngrp && (!partial || base + 32 * lane < rows))
+                    tbits[(base >> 5) + lane] = partial ? word & tail_mask(base + 32 * lane, rows) : word;
+            }
         }
     }
     __device__ __forceinline__ void store(Slots& r) {
@@ -571,8 +592,10 @@ __device__ __noinline__ void pred_select(const ScanTables& P, const uint8_t* sta
         if (k == ins.dst) nt[k] = a;
 }
 
+// MASK: lane 0 also stores the TRUE word of every 32 rows to bits[] (bits[0] = the word of the unit's first row in this tile)
+template <bool MASK>
 __device__ __noinline__ void unit_pred(const ScanTables& P, const ScanUnitDesc& u, const uint8_t* stage, int lane,
-                                       int rows_in_tile, uint64_t* cnt_out, uint64_t* div0_out) {
+                                       int rows_in_tile, uint64_t* cnt_out, uint64_t* div0_out, uint32_t* bits) {
     uint64_t cnt = 0;
     uint32_t div0 = 0;
     const int nw = u.nrows >> 5;
@@ -710,7 +733,12 @@ __device__ __noinline__ void unit_pred(const ScanTables& P, const ScanUnitDesc& 
             }
         }
 #pragma unroll
-        for (int g = 0; g < PG; ++g) cnt += __popc(bt[0].t[g] & tail_mask(u.row0 + 32 * (j + g), rows_in_tile));
+        for (int g = 0; g < PG; ++g) {
+            const uint32_t tw = bt[0].t[g] & tail_mask(u.row0 + 32 * (j + g), rows_in_tile);
+            cnt += __popc(tw);
+            if constexpr (MASK)
+                if (bits && lane == 0 && u.row0 + 32 * (j + g) < rows_in_tile) bits[j + g] = tw;
+        }
     }
     // masks are warp-uniform: lane 0 carries the counts
     if (lane == 0) {
@@ -720,11 +748,15 @@ __device__ __noinline__ void unit_pred(const ScanTables& P, const ScanUnitDesc& 
 }
 
 
+template <bool MASK_>
 struct PredUnit {
+    static constexpr bool MASK = MASK_;
     const ScanTables* T;
     const ScanUnitDesc* u;
     int lane;
     uint64_t cnt, div0;
+    uint32_t* tbits;
+    __device__ __forceinline__ void at_tile(int64_t tile_row0) { tbits = u->bits ? u->bits + ((tile_row0 + u->row0) >> 5) : nullptr; }
     __device__ __forceinline__ void setup(const ScanTables& T_, const ScanUnitDesc& u_, int lane_) {
         T = &T_;
         u = &u_;
@@ -734,7 +766,9 @@ struct PredUnit {
         cnt = r[0];
         div0 = r[1];
     }
-    __device__ __forceinline__ void tile(const uint8_t* stage, int rows, bool) { unit_pred(*T, *u, stage, lane, rows, &cnt, &div0); }
+    __device__ __forceinline__ void tile(const uint8_t* stage, int rows, bool) {
+        unit_pred<MASK>(*T, *u, stage, lane, rows, &cnt, &div0, MASK ? tbits : nullptr);
+    }
     __device__ __forceinline__ void store(Slots& r) {
 #pragma unroll
         for (int k = 0; k < SCAN_STATE_SLOTS; ++k) r[k] = 0;
@@ -825,6 +859,7 @@ __device__ __forceinline__ void run_single(const Pipe& p, const ScanTables& T, c
     for (int64_t t = blockIdx.x; t < p.n_tiles; t += gridDim.x) {
         mbar_wait(&p.full[s], ph);
         const bool partial = t == p.t_partial;
+        if constexpr (U::MASK) unit.at_tile(t * p.tile_rows);
         unit.tile(p.stages + (size_t)s * p.stage_bytes, partial ? p.rows_partial : p.tile_rows, partial);
         __syncwarp();
         if (lane == 0) mbar_arrive(&p.empty[s]);
@@ -840,9 +875,10 @@ __device__ __forceinline__ void run_single(const Pipe& p, const ScanTables& T, c
 // a warp that owns several units: per-lane state lives in shared memory between tiles
 template <class U>
 __device__ __forceinline__ void run_once(const ScanTables& T, const ScanUnitDesc& ud, uint64_t* st, int lane, const uint8_t* stage,
-                                         int rows, bool partial) {
+                                         int rows, bool partial, int64_t tile_row0) {
     U unit;
     unit.setup(T, ud, lane);
+    if constexpr (U::MASK) unit.at_tile(tile_row0);
     Slots r;
 #pragma unroll
     for (int k = 0; k < SCAN_STATE_SLOTS; ++k) r[k] = st[k * 32 + lane];
@@ -856,9 +892,9 @@ __device__ __forceinline__ void run_once(const ScanTables& T, const ScanUnitDesc
 // kind / flag dispatch, shared by both execution modes (SINGLE: whole tile loop inside; else one tile)
 template <bool SINGLE, class U>
 __device__ __forceinline__ void run_unit(const Pipe& p, const ScanTables& T, const ScanUnitDesc& ud, uint64_t* st, int lane,
-                                         const uint8_t* stage, int rows, bool partial) {
+                                         const uint8_t* stage, int rows, bool partial, int64_t tile_row0 = 0) {
     if (SINGLE) run_single<U>(p, T, ud, st, lane);
-    else run_once<U>(T, ud, st, lane, stage, rows, partial);
+    else run_once<U>(T, ud, st, lane, stage, rows, partial, tile_row0);
 }
 template <bool SINGLE, bool IS_I64>
 __device__ __forceinline__ void dispatch_num(const Pipe& p, const ScanTables& T, const ScanUnitDesc& ud, uint64_t* st, int lane,
@@ -875,9 +911,10 @@ __device__ __forceinline__ void dispatch_num(const Pipe& p, const ScanTables& T,
     }
 }
 // st: SINGLE -> global partial record of (CTA, unit); else this unit's per-lane state in shared memory
-template <bool SINGLE>
+// MASKS: some unit of the pass writes row verdicts; its PRED / TERMS units store words where their descriptor has `bits`
+template <bool SINGLE, bool MASKS>
 __device__ __forceinline__ void dispatch_unit(const Pipe& p, const ScanTables& T, const ScanUnitDesc& ud, uint64_t* st, int lane,
-                                              const uint8_t* stage, int rows, bool partial) {
+                                              const uint8_t* stage, int rows, bool partial, int64_t tile_row0) {
     switch (ud.kind) {
         case UNIT_COUNT: run_unit<SINGLE, CountUnit>(p, T, ud, st, lane, stage, rows, partial); break;
         case UNIT_NUM_F64: dispatch_num<SINGLE, false>(p, T, ud, st, lane, stage, rows, partial); break;
@@ -890,11 +927,12 @@ __device__ __forceinline__ void dispatch_unit(const Pipe& p, const ScanTables& T
                 default: run_unit<SINGLE, PairUnit<true, true>>(p, T, ud, st, lane, stage, rows, partial); break;
             }
             break;
-        case UNIT_TERMS: run_unit<SINGLE, TermsUnit>(p, T, ud, st, lane, stage, rows, partial); break;
-        default: run_unit<SINGLE, PredUnit>(p, T, ud, st, lane, stage, rows, partial); break;
+        case UNIT_TERMS: run_unit<SINGLE, TermsUnit<MASKS>>(p, T, ud, st, lane, stage, rows, partial, tile_row0); break;
+        default: run_unit<SINGLE, PredUnit<MASKS>>(p, T, ud, st, lane, stage, rows, partial, tile_row0); break;
     }
 }
 
+template <bool MASKS>
 __global__ void __launch_bounds__(SCAN_THREADS, 1) scan_kernel(const __grid_constant__ ScanParams P) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     uint8_t* stages = scan_smem;
@@ -967,8 +1005,8 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) scan_kernel(const __grid_cons
             // every warp owns at most one unit: registers only
             if (n_mine == 1) {
                 const int u = T->warp_units[cw][1];
-                dispatch_unit<true>(pipe, *T, T->units[u], P.partials + ((size_t)blockIdx.x * P.n_units + u) * SCAN_STATE_SLOTS,
-                                    lane, nullptr, 0, false);
+                dispatch_unit<true, MASKS>(pipe, *T, T->units[u], P.partials + ((size_t)blockIdx.x * P.n_units + u) * SCAN_STATE_SLOTS,
+                                           lane, nullptr, 0, false, 0);
             } else {
                 // idle warp: keep the ring moving
                 int s = 0;
@@ -999,7 +1037,8 @@ __global__ void __launch_bounds__(SCAN_THREADS, 1) scan_kernel(const __grid_cons
                 const uint8_t* stage = stages + (size_t)s * pipe.stage_bytes;
                 for (int k = 0; k < n_mine; ++k) {
                     const int u = T->warp_units[cw][1 + k];
-                    dispatch_unit<false>(pipe, *T, T->units[u], state + (size_t)u * SCAN_STATE_SLOTS * 32, lane, stage, rows, partial);
+                    dispatch_unit<false, MASKS>(pipe, *T, T->units[u], state + (size_t)u * SCAN_STATE_SLOTS * 32, lane, stage, rows, partial,
+                                                t * pipe.tile_rows);
                 }
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&empty[s]);
@@ -1085,10 +1124,14 @@ size_t scan_smem_bytes(const ScanParams& P) {
 
 cudaError_t scan_launch(const ScanParams& P, int grid, ScanAggOut* d_out, cudaStream_t stream) {
     size_t smem = scan_smem_bytes(P);
+    // passes without requested row verdicts run the kernel that has no code for them
+    bool masks = false;
+    for (int u = 0; u < P.n_units; ++u) masks |= P.tab.units[u].bits != nullptr;
+    const auto kernel = masks ? scan_kernel<true> : scan_kernel<false>;
     // the opt-in is per device (and per context): set it before every launch, it is a host-side table write
-    cudaError_t e = cudaFuncSetAttribute(scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
     if (e != cudaSuccess) return e;
-    scan_kernel<<<grid, SCAN_THREADS, smem, stream>>>(P);
+    kernel<<<grid, SCAN_THREADS, smem, stream>>>(P);
     e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     scan_finalize_kernel<<<P.n_aggs, FIN_THREADS, 0, stream>>>(P, grid, d_out);

@@ -70,6 +70,8 @@ struct ScanUnitDesc {
     int32_t warp;          // owning consumer warp (0-based)
     int32_t c0_is_i64, c1_is_i64;  // pair units: convert on load
     int32_t flags;                 // NUM units: UF_MOMENTS | UF_MINMAX | UF_ISUM ; TERMS units: 1 = OR (else AND)
+    uint32_t* bits;                // PRED / TERMS units of an aggregate whose row verdicts were requested: one TRUE word per
+                                   // 32 rows of the table (word i = rows 32 i .. 32 i + 31), else null
 };
 
 // Predicate code (SQL three-valued logic) for the warp-mask evaluator:

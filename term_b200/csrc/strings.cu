@@ -57,6 +57,7 @@ struct StrParams {
     uint32_t stage;           // bytes per warp stage buffer (multiple of 128)
     const uint8_t* g_blob;    // [256 B class map (uint8 class)][table]
     unsigned long long* out;  // [STR_MAX_DFA] match counts, [STR_MAX_DFA] = valid (non-null) rows
+    uint32_t* bits[STR_MAX_DFA];  // MASK kernels: per pattern, one match word per 32 rows of the table (null: not requested)
 };
 
 extern __shared__ __align__(256) uint8_t str_smem[];
@@ -140,7 +141,8 @@ __device__ __forceinline__ uint32_t run_dfa_gmem(const uint8_t* bytes, uint32_t 
 // R = rows per lane per block: a warp's block is 32*R consecutive rows (lane l owns rows base + j*32 + l, j < R).
 // R = 2 halves the per-block bookkeeping (offset prefetch, TMA issue, mbarrier wait) per string and evens out the
 // string-length imbalance between lanes; R = 1 keeps small inputs spread over all SMs.
-template <int NDFA, int R, bool DIRECT>
+// MASK: also store, per requested pattern, the word of every 32 rows whose bit l says "row of lane l matched"
+template <int NDFA, int R, bool DIRECT, bool MASK>
 __global__ void __launch_bounds__(STR_MAX_WARPS * 32) dfa_kernel(const __grid_constant__ StrParams P) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
     // ---- stage class map + transition table ----
@@ -232,6 +234,7 @@ __global__ void __launch_bounds__(STR_MAX_WARPS * 32) dfa_kernel(const __grid_co
 #pragma unroll
         for (int j = 0; j < R; ++j) {
             const bool valid = (c0.vw[j] >> lane) & 1u;
+            uint32_t m = 0;
             if (valid && (blk * R + j) * 32 + lane < n) {
                 ++nvalid;
                 uint32_t E;
@@ -251,9 +254,18 @@ __global__ void __launch_bounds__(STR_MAX_WARPS * 32) dfa_kernel(const __grid_co
                     }
                     E = run_dfa_gmem<DIRECT>(P.bytes, p, e, P.start, cls_base, tab_addr, term_limit);
                 }
-                const uint32_t m = lds_u16(tab_addr + 2u * (2u * E + n_classes));  // END entry = match mask
+                m = lds_u16(tab_addr + 2u * (2u * E + n_classes));  // END entry = match mask
 #pragma unroll
                 for (int i = 0; i < NDFA; ++i) cnt[i] += (m >> i) & 1u;
+            }
+            if constexpr (MASK) {
+                // every lane of the warp is here (the block loop is warp-uniform); NULL rows and rows past the end match nothing
+#pragma unroll
+                for (int i = 0; i < NDFA; ++i)
+                    if (P.bits[i]) {
+                        const uint32_t w = __ballot_sync(0xffffffffu, (m >> i) & 1u);
+                        if (lane == 0 && (blk * R + j) * 32 < n) P.bits[i][blk * R + j] = w;
+                    }
             }
         }
         c0 = c1;
@@ -431,9 +443,24 @@ static const Product& cached_product(const std::vector<std::pair<std::string, bo
     return cache.emplace(key, build_product(ptrs, budget, allow_direct)).first->second;
 }
 
+typedef void (*Kernel)(const StrParams);
+template <bool MASK>
+static Kernel pick_dfa_kernel(int nd, int R, bool direct) {
+    const Kernel k1 = nd <= 1 ? (Kernel)dfa_kernel<1, 1, false, MASK> : nd <= 2 ? (Kernel)dfa_kernel<2, 1, false, MASK> : nd <= 4 ? (Kernel)dfa_kernel<4, 1, false, MASK> : (Kernel)dfa_kernel<8, 1, false, MASK>;
+    const Kernel k2 = nd <= 1 ? (Kernel)dfa_kernel<1, 2, false, MASK> : nd <= 2 ? (Kernel)dfa_kernel<2, 2, false, MASK> : nd <= 4 ? (Kernel)dfa_kernel<4, 2, false, MASK> : (Kernel)dfa_kernel<8, 2, false, MASK>;
+    const Kernel d1 = nd <= 1 ? (Kernel)dfa_kernel<1, 1, true, MASK> : nd <= 2 ? (Kernel)dfa_kernel<2, 1, true, MASK> : nd <= 4 ? (Kernel)dfa_kernel<4, 1, true, MASK> : (Kernel)dfa_kernel<8, 1, true, MASK>;
+    const Kernel d2 = nd <= 1 ? (Kernel)dfa_kernel<1, 2, true, MASK> : nd <= 2 ? (Kernel)dfa_kernel<2, 2, true, MASK> : nd <= 4 ? (Kernel)dfa_kernel<4, 2, true, MASK> : (Kernel)dfa_kernel<8, 2, true, MASK>;
+    return direct ? (R == 2 ? d2 : d1) : (R == 2 ? k2 : k1);
+}
+
 static void run_string_pass(Engine& e, Table& t, Plan& p, Column& c, const std::vector<int>& ids, const Product& pr, bool trim) {
     const int nd = (int)ids.size();
     StrParams P{};
+    bool masks = false;
+    for (int i = 0; i < nd; ++i) {
+        P.bits[i] = p.aggs[ids[i]].bits;
+        masks |= P.bits[i] != nullptr;
+    }
     P.trim = trim ? 1 : 0;
     P.n_classes = pr.n_classes;
     P.term_limit = pr.term_limit;
@@ -471,12 +498,7 @@ static void run_string_pass(Engine& e, Table& t, Plan& p, Column& c, const std::
     P.validity = reinterpret_cast<const uint32_t*>(c.validity.p);
     P.n_rows = t.n_rows;
     P.n_blocks = (t.n_rows + 32 * R - 1) / (32 * R);
-    typedef void (*Kernel)(const StrParams);
-    const Kernel k1 = nd <= 1 ? (Kernel)dfa_kernel<1, 1, false> : nd <= 2 ? (Kernel)dfa_kernel<2, 1, false> : nd <= 4 ? (Kernel)dfa_kernel<4, 1, false> : (Kernel)dfa_kernel<8, 1, false>;
-    const Kernel k2 = nd <= 1 ? (Kernel)dfa_kernel<1, 2, false> : nd <= 2 ? (Kernel)dfa_kernel<2, 2, false> : nd <= 4 ? (Kernel)dfa_kernel<4, 2, false> : (Kernel)dfa_kernel<8, 2, false>;
-    const Kernel d1 = nd <= 1 ? (Kernel)dfa_kernel<1, 1, true> : nd <= 2 ? (Kernel)dfa_kernel<2, 1, true> : nd <= 4 ? (Kernel)dfa_kernel<4, 1, true> : (Kernel)dfa_kernel<8, 1, true>;
-    const Kernel d2 = nd <= 1 ? (Kernel)dfa_kernel<1, 2, true> : nd <= 2 ? (Kernel)dfa_kernel<2, 2, true> : nd <= 4 ? (Kernel)dfa_kernel<4, 2, true> : (Kernel)dfa_kernel<8, 2, true>;
-    const Kernel kernel = pr.direct ? (R == 2 ? d2 : d1) : (R == 2 ? k2 : k1);
+    const Kernel kernel = masks ? pick_dfa_kernel<true>(nd, R, pr.direct) : pick_dfa_kernel<false>(nd, R, pr.direct);
     TG_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)STR_SMEM_MAX));
     const int threads = warps * 32;
     int per_sm = 1;
@@ -575,6 +597,18 @@ void exec_string_jobs(Engine& e, Table& t, Plan& p, const std::vector<int>& agg_
 // bytes minus UTF-8 continuation bytes. A row's byte length (two offsets) already bounds its character count
 // (ceil(bytes/4) <= chars <= bytes), so the value bytes are only read for rows some range cannot decide from that.
 constexpr int LEN_MAX_RANGES = 8;
+
+// SQL LENGTH of one non-null row: bytes minus the UTF-8 continuation bytes (need_bytes false: the byte count, unused then)
+template <class LP>
+__device__ __forceinline__ long long row_chars(const LP& P, int32_t b, int32_t e, bool need_bytes, uint64_t w0, uint64_t w1) {
+    if (!need_bytes) return e - b;
+    int cont = __popcll(w0 & (~w0 << 1) & 0x8080808080808080ull) + __popcll(w1 & (~w1 << 1) & 0x8080808080808080ull);
+    for (int32_t q = b + 16; q < e; q += 8) {
+        const uint64_t w = load_upto8(P.bytes, q, min(8, e - q));
+        cont += __popcll(w & (~w << 1) & 0x8080808080808080ull);
+    }
+    return (long long)(e - b) - cont;
+}
 constexpr int LEN_THREADS = 256;
 constexpr int LEN_ILP = 4;
 struct LenParams {
@@ -586,8 +620,10 @@ struct LenParams {
     int32_t pad;
     long long lo[LEN_MAX_RANGES], hi[LEN_MAX_RANGES];
     unsigned long long* out;  // [LEN_MAX_RANGES] matching non-null rows, [LEN_MAX_RANGES] = non-null rows
+    uint32_t* bits[LEN_MAX_RANGES];  // MASK kernel: per requested range, one word per 32 rows (bit set: non-null and in range)
 };
 
+template <bool MASK>
 __global__ void __launch_bounds__(LEN_THREADS) length_kernel(const __grid_constant__ LenParams P) {
     uint32_t cnt[LEN_MAX_RANGES];
 #pragma unroll
@@ -624,6 +660,30 @@ __global__ void __launch_bounds__(LEN_THREADS) length_kernel(const __grid_consta
         }
 #pragma unroll
         for (int k = 0; k < LEN_ILP; ++k) {
+            if constexpr (MASK) {
+                // the ballot needs every lane: NULL rows and rows past the end are out of every range
+                uint32_t inm = 0;
+                if (live[k]) {
+                    ++nvalid;
+                    const long long chars = row_chars(P, b[k], e[k], need[k], w0[k], w1[k]);
+                    const long long nbytes = e[k] - b[k], min_chars = (nbytes + 3) >> 2;
+#pragma unroll
+                    for (int i = 0; i < LEN_MAX_RANGES; ++i)
+                        if (i < P.n_ranges) {
+                            const bool in = need[k] ? (chars >= P.lo[i] && chars <= P.hi[i]) : (min_chars >= P.lo[i] && nbytes <= P.hi[i]);
+                            cnt[i] += in;
+                            inm |= (uint32_t)in << i;
+                        }
+                }
+                const int64_t row = base + (int64_t)k * LEN_THREADS + threadIdx.x;
+#pragma unroll
+                for (int i = 0; i < LEN_MAX_RANGES; ++i)
+                    if (i < P.n_ranges && P.bits[i]) {
+                        const uint32_t w = __ballot_sync(0xffffffffu, (inm >> i) & 1u);
+                        if ((threadIdx.x & 31) == 0 && row < P.n_rows) P.bits[i][row >> 5] = w;
+                    }
+                continue;
+            }
             if (!live[k]) continue;
             ++nvalid;
             const long long nbytes = e[k] - b[k], min_chars = (nbytes + 3) >> 2;
@@ -703,8 +763,14 @@ void exec_length_jobs(Engine& e, Table& t, Plan& p, const std::vector<int>& agg_
                 TG_CUDA(cudaMemsetAsync(scr, 0, 128, e.stream));
                 const int64_t per_cta = (int64_t)LEN_THREADS * LEN_ILP;
                 const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((t.n_rows + per_cta - 1) / per_cta, (int64_t)e.sm_count * 8));
+                bool masks = false;
+                for (size_t i = 0; i < cnt; ++i) {
+                    P.bits[i] = p.aggs[kv.second[first + i]].bits;
+                    masks |= P.bits[i] != nullptr;
+                }
                 TG_CUDA(cudaEventRecord(e.ev[2], e.stream));
-                length_kernel<<<grid, LEN_THREADS, 0, e.stream>>>(P);
+                if (masks) length_kernel<true><<<grid, LEN_THREADS, 0, e.stream>>>(P);
+                else length_kernel<false><<<grid, LEN_THREADS, 0, e.stream>>>(P);
                 TG_CUDA(cudaGetLastError());
                 TG_CUDA(cudaEventRecord(e.ev[3], e.stream));
                 TG_CUDA(cudaMemcpyAsync(h_out, scr, 128, cudaMemcpyDeviceToHost, e.stream));

@@ -5,6 +5,7 @@
 #include <cstddef>
 #include <cstring>
 
+#include "arrow_abi.h"
 #include "engine.hpp"
 #include "str_entries.cuh"
 
@@ -330,31 +331,6 @@ void table_adopt_device(Table& t, const std::string& name, int32_t dtype, int64_
     }
     t.n_rows = std::max(t.n_rows, n);
 }
-
-// ---- Arrow C Data Interface (https://arrow.apache.org/docs/format/CDataInterface.html) ----
-struct ArrowSchema {
-    const char* format;
-    const char* name;
-    const char* metadata;
-    int64_t flags;
-    int64_t n_children;
-    struct ArrowSchema** children;
-    struct ArrowSchema* dictionary;
-    void (*release)(struct ArrowSchema*);
-    void* private_data;
-};
-struct ArrowArray {
-    int64_t length;
-    int64_t null_count;
-    int64_t offset;
-    int64_t n_buffers;
-    int64_t n_children;
-    const void** buffers;
-    struct ArrowArray** children;
-    struct ArrowArray* dictionary;
-    void (*release)(struct ArrowArray*);
-    void* private_data;
-};
 
 // Arrow C Data Interface format string -> the stored type; width / signedness of the delivered values when they are widened
 // on the host; DataFusion's name of the delivered type (nullptr: it is the stored type)
@@ -817,17 +793,6 @@ void table_append_arrow(Table& t, const void* schema_p, const void* array_p) {
 // A RecordBatch whose buffers are in HBM is appended by copies and kernels on the device: it leaves exactly the state that
 // table_append_arrow leaves for the same batch in host memory (buffers, NULL counts, pivots, tail mirrors, delivered types,
 // errors). Nothing crosses PCIe but the small read-backs named below.
-struct ArrowDeviceArray {
-    ArrowArray array;
-    int64_t device_id;
-    int32_t device_type;
-    void* sync_event;
-    int64_t reserved[3];
-};
-static_assert(sizeof(ArrowDeviceArray) == 128 && offsetof(ArrowDeviceArray, device_type) == 88 && offsetof(ArrowDeviceArray, sync_event) == 96,
-              "ArrowDeviceArray layout");
-constexpr int32_t ARROW_DEVICE_CPU = 1, ARROW_DEVICE_CUDA = 2, ARROW_DEVICE_CUDA_HOST = 3, ARROW_DEVICE_CUDA_MANAGED = 13;
-
 // what the kernels of one column report; read back once per batch
 struct ArrowDevResult {
     unsigned long long zeros;    // clear bits of the column's validity (its NULL rows)
