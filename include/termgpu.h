@@ -590,6 +590,30 @@ TG_API tg_status tg_plan_request_row_mask(tg_plan* plan, int32_t slot);
  * a slot whose evaluation failed: that error (division by zero in a predicate: TG_ERR_INVALID_ARG), message in
  * tg_last_error(). */
 TG_API tg_status tg_plan_export_row_mask(const tg_plan* plan, int32_t slot, void* arrow_schema_out, void* arrow_device_array_out);
+
+/* Key-level row verdicts of uniqueness and foreign-key slots (an engine extension beyond the reference's ConstraintResult),
+ * requested before an execute and exported after it like row masks: same Arrow Boolean layout, lifetime, buffers and
+ * synchronisation (no sync_event; release before the engine is destroyed).
+ *   Uniqueness slots (every tg_uniqueness_kind) take DUPLICATE and FIRST. A row's key is the tuple of the slot's columns,
+ *   equal exactly when the distinct counts treat it so (-0.0 = +0.0, one NaN; Utf8 and composite keys by 128-bit
+ *   fingerprint). DUPLICATE bit i = row i's key occurs in at least two rows; FIRST bit i = row i is the lowest-indexed row
+ *   holding its key, so filtering by FIRST de-duplicates the table. One column: a NULL row has no key and is NULL in the
+ *   array (no validity buffer when the column has no NULLs). Several columns: a tuple with NULL components is a value and
+ *   every row is valid. The verdicts depend on the columns only, not on the uniqueness kind.
+ *     popcount(FIRST & validity)     = the COUNT(DISTINCT ..) behind FULL / DISTINCTNESS / COMPOSITE
+ *     popcount(DUPLICATE & validity) = valid rows - rows whose key occurs once
+ *   Foreign-key slots take ORPHAN, an array over the CHILD table's rows (length = its row count): bit i = child row i has a
+ *   non-NULL key without a parent; NULL child rows are NULL (null_count = the NULL child rows), allow_nulls is the caller's.
+ *     popcount(ORPHAN & validity) = the violations, minus the NULL child rows when allow_nulls is off
+ * Other slot kinds: TG_ERR_UNSUPPORTED; a kind the slot does not take or a bad slot index: TG_ERR_INVALID_ARG; export before a
+ * request or before an execute since: TG_ERR_INVALID_ARG; an aggregate whose keys were shuffled to other ranks
+ * (tg_plan_redirect_aggregate, fingerprint-record shards): TG_ERR_UNSUPPORTED at export, as its rows are not the executed
+ * table's. tg_plan_execute_partial on one shard gives the verdicts of the rows that engine holds (shard-local duplicates).
+ * Plans that request none launch exactly the kernels they launch without this feature. */
+typedef enum { TG_KEY_ROWS_DUPLICATE = 0, TG_KEY_ROWS_FIRST = 1, TG_KEY_ROWS_ORPHAN = 2 } tg_key_rows_kind;
+TG_API tg_status tg_plan_request_key_rows(tg_plan* plan, int32_t slot, int32_t kind);
+TG_API tg_status tg_plan_export_key_rows(const tg_plan* plan, int32_t slot, int32_t kind, void* arrow_schema_out,
+                                         void* arrow_device_array_out);
 TG_API tg_status tg_plan_partial_size(const tg_plan* plan, size_t* n_bytes);
 TG_API tg_status tg_plan_partial_export(const tg_plan* plan, void* buf, size_t n_bytes);
 /* host-only: build partials for a plan without a GPU from an exported blob (tests, incremental runs) */

@@ -31,6 +31,7 @@ TG_INT64, TG_FLOAT64, TG_UTF8, TG_INT32, TG_FLOAT32, TG_BOOL, TG_FP128 = 1, 2, 3
 TG_PQ_INT96 = 8  # tg_table_append_parquet_chunk only: a Parquet INT96 timestamp chunk
 # tg_constraint_status
 TG_SUCCESS, TG_FAILURE, TG_SKIPPED = 0, 1, 2
+TG_KEY_ROWS_DUPLICATE, TG_KEY_ROWS_FIRST, TG_KEY_ROWS_ORPHAN = 0, 1, 2  # tg_key_rows_kind
 
 
 class tg_assertion(C.Structure):
@@ -145,6 +146,8 @@ SIGNATURES = {
     "tg_plan_execute_partial": (C.c_int, [P, P, C.c_char_p]),
     "tg_plan_request_row_mask": (C.c_int, [P, C.c_int32]),
     "tg_plan_export_row_mask": (C.c_int, [P, C.c_int32, P, P]),
+    "tg_plan_request_key_rows": (C.c_int, [P, C.c_int32, C.c_int32]),
+    "tg_plan_export_key_rows": (C.c_int, [P, C.c_int32, C.c_int32, P, P]),
     "tg_plan_partial_size": (C.c_int, [P, C.POINTER(C.c_size_t)]),
     "tg_plan_partial_export": (C.c_int, [P, P, C.c_size_t]),
     "tg_plan_partial_reset": (C.c_int, [P]),

@@ -578,12 +578,15 @@ _SCHEMA_DTOR = _capsule_destructor(56)        # ArrowSchema.release
 _DEVICE_ARRAY_DTOR = _capsule_destructor(64)  # ArrowDeviceArray.array.release
 
 
+KEY_ROWS_DUPLICATE, KEY_ROWS_FIRST, KEY_ROWS_ORPHAN = F.TG_KEY_ROWS_DUPLICATE, F.TG_KEY_ROWS_FIRST, F.TG_KEY_ROWS_ORPHAN
+
+
 class RowMask:
     """Row verdicts of one slot: an Arrow Boolean array in the engine's device memory (values bit i = row i is in the
-    metric's numerator, validity bit i = row i is in its denominator). Consumed through `__arrow_c_device_array__`; it owns
+    metric's numerator, validity bit i = row i is in its denominator; for key-level verdicts, see tg_plan_export_key_rows). Consumed through `__arrow_c_device_array__`; it owns
     its buffers until the consumer imports it or this object is collected, which must happen before the engine is closed."""
 
-    def __init__(self, plan_handle, slot: int):
+    def __init__(self, plan_handle, slot: int, key_rows_kind=None):
         sp, ap = _libc.malloc(72), _libc.malloc(128)
         C.memset(sp, 0, 72)
         C.memset(ap, 0, 128)
@@ -592,7 +595,10 @@ class RowMask:
         self._array = _capsule_new(ap, _CAP_DEVICE_ARRAY, C.cast(_DEVICE_ARRAY_DTOR, C.c_void_p))
         _capsule_structs[id(self._schema)] = sp
         _capsule_structs[id(self._array)] = ap
-        F.check(F.lib().tg_plan_export_row_mask(plan_handle, slot, sp, ap))
+        if key_rows_kind is None:
+            F.check(F.lib().tg_plan_export_row_mask(plan_handle, slot, sp, ap))
+        else:
+            F.check(F.lib().tg_plan_export_key_rows(plan_handle, slot, key_rows_kind, sp, ap))
         self.length = C.c_int64.from_address(ap).value
         self.null_count = C.c_int64.from_address(ap + 8).value
         bufs = C.c_void_p.from_address(ap + 40).value
@@ -640,6 +646,15 @@ class Plan:
     def row_mask(self, slot: int) -> RowMask:
         """The row verdicts of slot `slot` from the last execute (tg_plan_export_row_mask)."""
         return RowMask(self._h, slot)
+
+    def request_key_rows(self, slot: int, kind: int):
+        """Ask the next execute to keep key-level row verdicts of a uniqueness slot (KEY_ROWS_DUPLICATE / KEY_ROWS_FIRST) or a
+        foreign-key slot (KEY_ROWS_ORPHAN, over the child table's rows) (tg_plan_request_key_rows)."""
+        F.check(F.lib().tg_plan_request_key_rows(self._h, slot, kind))
+
+    def key_rows(self, slot: int, kind: int) -> RowMask:
+        """The key-level row verdicts of `kind` of slot `slot` from the last execute (tg_plan_export_key_rows)."""
+        return RowMask(self._h, slot, kind)
 
     def partial_export(self) -> bytes:
         n = C.c_size_t()

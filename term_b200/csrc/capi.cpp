@@ -508,6 +508,29 @@ static void row_mask_release_array(ArrowArray* a) {
     a->release = nullptr;
 }
 
+// fills the Arrow structs of one verdict array; the array shares ownership of the buffers with the slot
+static void export_mask(const std::shared_ptr<RowMask>& mask, void* arrow_schema_out, void* arrow_device_array_out) {
+    const RowMask& m = *mask;
+    auto* x = new RowMaskExport{mask, {m.validity, m.values}};
+    ArrowSchema* sc = static_cast<ArrowSchema*>(arrow_schema_out);
+    *sc = ArrowSchema{};
+    sc->format = "b";
+    sc->name = "";
+    sc->flags = 2;  // ARROW_FLAG_NULLABLE
+    sc->release = row_mask_release_schema;
+    ArrowDeviceArray* da = static_cast<ArrowDeviceArray*>(arrow_device_array_out);
+    *da = ArrowDeviceArray{};
+    da->array.length = m.n_rows;
+    da->array.null_count = m.null_count;
+    da->array.n_buffers = 2;
+    da->array.buffers = x->buffers;
+    da->array.release = row_mask_release_array;
+    da->array.private_data = x;
+    da->device_id = m.device;
+    da->device_type = ARROW_DEVICE_CUDA;
+    da->sync_event = nullptr;
+}
+
 tg_status tg_plan_export_row_mask(const tg_plan* p, int32_t slot, void* arrow_schema_out, void* arrow_device_array_out) {
     return guard([&] {
         if (!p || !arrow_schema_out || !arrow_device_array_out) throw Error(TG_ERR_INVALID_ARG, "NULL argument");
@@ -516,24 +539,26 @@ tg_status tg_plan_export_row_mask(const tg_plan* p, int32_t slot, void* arrow_sc
         if (!s.mask_requested) throw Error(TG_ERR_INVALID_ARG, "row mask of slot " + std::to_string(slot) + " was not requested");
         if (!s.mask_built) throw Error(TG_ERR_INVALID_ARG, "row mask of slot " + std::to_string(slot) + " was requested but the plan was not executed since");
         if (s.mask_err != TG_OK) throw Error(s.mask_err, s.mask_err_msg);
-        auto* x = new RowMaskExport{s.mask, {s.mask->validity, s.mask->values}};
-        ArrowSchema* sc = static_cast<ArrowSchema*>(arrow_schema_out);
-        *sc = ArrowSchema{};
-        sc->format = "b";
-        sc->name = "";
-        sc->flags = 2;  // ARROW_FLAG_NULLABLE
-        sc->release = row_mask_release_schema;
-        ArrowDeviceArray* da = static_cast<ArrowDeviceArray*>(arrow_device_array_out);
-        *da = ArrowDeviceArray{};
-        da->array.length = s.mask->n_rows;
-        da->array.null_count = s.mask->null_count;
-        da->array.n_buffers = 2;
-        da->array.buffers = x->buffers;
-        da->array.release = row_mask_release_array;
-        da->array.private_data = x;
-        da->device_id = s.mask->device;
-        da->device_type = ARROW_DEVICE_CUDA;
-        da->sync_event = nullptr;
+        export_mask(s.mask, arrow_schema_out, arrow_device_array_out);
+    });
+}
+
+tg_status tg_plan_request_key_rows(tg_plan* p, int32_t slot, int32_t kind) {
+    return guard([&] {
+        if (!p) throw Error(TG_ERR_INVALID_ARG, "NULL argument");
+        plan_request_key_rows(p->p, slot, kind);
+    });
+}
+
+tg_status tg_plan_export_key_rows(const tg_plan* p, int32_t slot, int32_t kind, void* arrow_schema_out, void* arrow_device_array_out) {
+    return guard([&] {
+        if (!p || !arrow_schema_out || !arrow_device_array_out) throw Error(TG_ERR_INVALID_ARG, "NULL argument");
+        const Slot& s = key_rows_slot(p->p, slot, kind);
+        const std::string what = "key-level row verdicts (kind " + std::to_string(kind) + ") of slot " + std::to_string(slot);
+        if (!(s.key_rows_requested & (1u << kind))) throw Error(TG_ERR_INVALID_ARG, what + " were not requested");
+        if (!s.mask_built) throw Error(TG_ERR_INVALID_ARG, what + " were requested but the plan was not executed since");
+        if (s.mask_err != TG_OK) throw Error(s.mask_err, s.mask_err_msg);
+        export_mask(s.key_rows[kind], arrow_schema_out, arrow_device_array_out);
     });
 }
 

@@ -1474,18 +1474,58 @@ static void free_row_bits(Engine& e, Table* t, Plan& p) {
         }
 }
 
+std::shared_ptr<RowMask> new_row_mask(Engine& e, int64_t n_rows, bool with_validity) {
+    auto m = std::make_shared<RowMask>();
+    m->n_rows = n_rows;
+    m->bytes = row_words_bytes(n_rows);
+    m->device = e.device;
+    std::shared_ptr<MaskReturns> box = e.mask_returns;
+    m->give_back = [box](uint8_t* b, size_t sz) {
+        std::lock_guard<std::mutex> g(box->mu);
+        if (box->engine_alive) box->blocks.emplace_back(b, sz);
+        else cudaFree(b);
+    };
+    m->values = e.dev_alloc(m->bytes);
+    if (with_validity) m->validity = e.dev_alloc(m->bytes);
+    return m;
+}
+
+// key-level verdicts: the arrays the hash job of the slot's aggregate built (shared by the slots of that aggregate)
+static void take_key_rows(const Plan& p, Slot& s) {
+    const Agg& a = p.aggs[s.aggs[0]];
+    if (a.err != TG_OK) {
+        s.mask_err = a.err;
+        s.mask_err_msg = a.err_msg;
+        return;
+    }
+    for (int k = 0; k < 3; ++k) {
+        if (!(s.key_rows_requested & (1u << k))) continue;
+        if (!a.key_mask[k]) {  // the job read keys shuffled here from other ranks (redirect / fingerprint records)
+            s.mask_err = TG_ERR_UNSUPPORTED;
+            s.mask_err_msg = "key-level row verdicts are not available for the '" + s.name +
+                             "' slot: its keys were shuffled to other ranks, so its rows are not the executed table's";
+            return;
+        }
+        s.key_rows[k] = a.key_mask[k];
+    }
+}
+
 static void build_row_masks(Engine& e, Table* t, Plan& p) {
     const int64_t n = t ? t->n_rows : 0;
-    const size_t bytes = row_words_bytes(n);
     unsigned long long* d_counts = nullptr;
     std::vector<std::shared_ptr<RowMask>> counted;
     bool launched = false;
     for (auto& s : p.slots) {
-        if (!s.mask_requested) continue;
+        if (!s.mask_requested && !s.key_rows_requested) continue;
         s.mask_built = true;
         s.mask.reset();
+        for (auto& m : s.key_rows) m.reset();
         s.mask_err = TG_OK;
         s.mask_err_msg.clear();
+        if (s.key_rows_requested) {
+            take_key_rows(p, s);
+            continue;
+        }
         const Agg& a = p.aggs[s.aggs[0]];
         const Agg* valid_agg = s.kind == SL_CONTAINMENT || s.kind == SL_NON_NEGATIVE ? &p.aggs[s.aggs[1]] : nullptr;
         if (a.err != TG_OK || (valid_agg && valid_agg->err != TG_OK)) {
@@ -1503,18 +1543,7 @@ static void build_row_masks(Engine& e, Table* t, Plan& p) {
         const uint32_t* valid = c ? reinterpret_cast<const uint32_t*>(c->validity.p) : nullptr;
         const bool or_invalid = s.kind == SL_LENGTH || (s.kind == SL_FORMAT && s.fopt.null_is_valid);
         const bool emit_validity = valid && (s.kind == SL_CONTAINMENT || s.kind == SL_NON_NEGATIVE || s.kind == SL_DATA_TYPE);
-        auto m = std::make_shared<RowMask>();
-        m->n_rows = n;
-        m->bytes = bytes;
-        m->device = e.device;
-        std::shared_ptr<MaskReturns> box = e.mask_returns;
-        m->give_back = [box](uint8_t* b, size_t sz) {
-            std::lock_guard<std::mutex> g(box->mu);
-            if (box->engine_alive) box->blocks.emplace_back(b, sz);
-            else cudaFree(b);
-        };
-        m->values = e.dev_alloc(bytes);
-        if (emit_validity) m->validity = e.dev_alloc(bytes);
+        auto m = new_row_mask(e, n, emit_validity);
         if (emit_validity && !d_counts) {
             d_counts = reinterpret_cast<unsigned long long*>(e.scratch(8 * p.slots.size()));
             TG_CUDA(cudaMemsetAsync(d_counts, 0, 8 * p.slots.size(), e.stream));

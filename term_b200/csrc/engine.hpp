@@ -248,6 +248,8 @@ void declare_arrow_type(Column& c, const std::string& fmt);
 void exec_scan_jobs(Engine& e, Table& t, Plan& p, const std::vector<int>& agg_ids);   // engine.cu + scan.cu
 void exec_string_jobs(Engine& e, Table& t, Plan& p, const std::vector<int>& agg_ids); // strings.cu
 void exec_length_jobs(Engine& e, Table& t, Plan& p, const std::vector<int>& agg_ids); // strings.cu
+// an n_rows-row Arrow Boolean array (values, and validity when asked) in blocks of the engine's recycler (engine.cu)
+std::shared_ptr<RowMask> new_row_mask(Engine& e, int64_t n_rows, bool with_validity);
 void exec_distinct_job(Engine& e, Table& t, Plan& p, int agg_id);                     // hashing.cu
 void exec_fk_job(Engine& e, Plan& p, int agg_id);                                     // hashing.cu
 void exec_kll_jobs(Engine& e, Table& t, Plan& p, const std::vector<int>& agg_ids);  // sketch.cu

@@ -120,5 +120,101 @@ __device__ __forceinline__ uint64_t upsert128(const Table128& t, Fp f, bool& cre
     }
 }
 
+// ---- key-level row verdicts (tg_plan_request_key_rows) ----
+// fmix64 is a bijection; its inverse turns the hashes the sorted-bucket path de-duplicates back into keys
+__host__ __device__ __forceinline__ uint64_t fmix64_inv(uint64_t h) {
+    h ^= h >> 33;
+    h *= 0x9cb4b2f8129337dbull;  // inverse of 0xc4ceb9fe1a85ec53 mod 2^64
+    h ^= h >> 33;
+    h *= 0x4f74430c22a54005ull;  // inverse of 0xff51afd7ed558ccd mod 2^64
+    h ^= h >> 33;
+    return h;
+}
+
+// Repeated-key table R: every key that occurs in at least two rows, inserted by the counting kernels at the moment a key's
+// count goes from 1 to 2 (so each key once), then the lowest row holding it (atomicMin by the row pass). 64-bit keys are
+// the canonical values; Utf8 / composite keys the two fingerprint words (h2 != nullptr). The 64-bit key equal to the EMPTY
+// word (the Int64 value -1) has its own cell: empty_key[0] = 1 when it is repeated, empty_key[1] = its lowest row.
+// R never holds more than half its slots: an insert first claims one of those places (`fill`), and past them the counting
+// pass inserts nothing more. The host, which knows the repeated-key count, then repeats the job once with R sized from it.
+// So no insert probes a full or crowded table, whatever the number of repeated keys.
+struct RepTab {
+    unsigned long long* h1 = nullptr;  // nullptr: no key is repeated (every row is the first of its key)
+    unsigned long long* h2 = nullptr;
+    unsigned long long* minrow = nullptr;
+    unsigned long long* empty_key = nullptr;
+    unsigned long long* fill = nullptr;  // places claimed so far
+    uint64_t mask = 0;
+};
+__device__ __forceinline__ uint64_t rep_home(uint64_t a, uint64_t b) { return fmix64(a ^ 0x9e3779b97f4a7c15ull ^ (b << 1)); }
+// (the plain load first: once R is at half, the remaining repeated keys of the pass read one L2-resident word, no atomic)
+__device__ __forceinline__ bool rep_claim(const RepTab& R) {
+    const unsigned long long half = (R.mask + 1) / 2;
+    return *reinterpret_cast<volatile unsigned long long*>(R.fill) < half && atomicAdd(R.fill, 1ull) < half;
+}
+
+__device__ __forceinline__ void rep_insert64(const RepTab& R, uint64_t key) {
+    if (key == EMPTY64) {
+        R.empty_key[0] = 1ull;
+        return;
+    }
+    if (!rep_claim(R)) return;
+    uint64_t slot = rep_home(key, 0) & R.mask;
+    for (uint64_t probes = 0; probes <= R.mask; ++probes) {
+        if (atomicCAS(&R.h1[slot], EMPTY64, (unsigned long long)key) == EMPTY64) return;
+        slot = (slot + 1) & R.mask;
+    }
+}
+__device__ __forceinline__ void rep_insert128(const RepTab& R, Fp f) {
+    const uint64_t a = f.h1 == EMPTY64 ? 0 : f.h1, b = f.h2;  // (a free slot is h1 == EMPTY, as in upsert128)
+    if (!rep_claim(R)) return;
+    uint64_t slot = rep_home(a, b) & R.mask;
+    for (uint64_t probes = 0; probes <= R.mask; ++probes) {
+        if (atomicCAS(&R.h1[slot], EMPTY64, (unsigned long long)a) == EMPTY64) {
+            R.h2[slot] = b;  // read only by the row passes, which are later launches
+            return;
+        }
+        slot = (slot + 1) & R.mask;
+    }
+}
+// the min-row cell of a key, nullptr when it is not repeated
+__device__ __forceinline__ unsigned long long* rep_cell64(const RepTab& R, uint64_t key) {
+    if (!R.h1) return nullptr;
+    if (key == EMPTY64) return R.empty_key[0] ? &R.empty_key[1] : nullptr;
+    uint64_t slot = rep_home(key, 0) & R.mask;
+    for (uint64_t probes = 0; probes <= R.mask; ++probes) {
+        const unsigned long long v = R.h1[slot];
+        if (v == key) return &R.minrow[slot];
+        if (v == EMPTY64) return nullptr;
+        slot = (slot + 1) & R.mask;
+    }
+    return nullptr;
+}
+__device__ __forceinline__ unsigned long long* rep_cell128(const RepTab& R, Fp f) {
+    if (!R.h1) return nullptr;
+    const uint64_t a = f.h1 == EMPTY64 ? 0 : f.h1, b = f.h2;
+    uint64_t slot = rep_home(a, b) & R.mask;
+    for (uint64_t probes = 0; probes <= R.mask; ++probes) {
+        const unsigned long long v = R.h1[slot];
+        if (v == EMPTY64) return nullptr;
+        if (v == a && R.h2[slot] == b) return &R.minrow[slot];
+        slot = (slot + 1) & R.mask;
+    }
+    return nullptr;
+}
+
+// Output words of one key-level verdict array (Arrow Boolean: values, and validity or nullptr)
+struct VerdictOut {
+    uint32_t* values = nullptr;
+    uint32_t* validity = nullptr;
+};
+// One warp stores the 32-row word w: lane l holds row 32 w + l (bits past the last row are false)
+__device__ __forceinline__ void store_verdict_word(int64_t w, bool bit, bool valid, const VerdictOut& o) {
+    const uint32_t vb = __ballot_sync(0xffffffffu, bit && valid), vv = __ballot_sync(0xffffffffu, valid);
+    if ((threadIdx.x & 31) == 0) {
+        if (o.values) o.values[w] = vb;
+        if (o.validity) o.validity[w] = vv;
+    }
+}
 
 }  // namespace tg

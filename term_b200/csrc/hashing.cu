@@ -23,9 +23,11 @@
 namespace tg {
 
 // ---------------------------------------------------------------- path A: exact 64-bit keys ----
+// MASK: also inserts each key that reaches a count of two into the repeated-key table R (key-level row verdicts)
+template <bool MASK>
 __global__ void __launch_bounds__(HASH_THREADS) insert64_kernel(const uint64_t* values, const uint32_t* validity,
                                                                 int64_t n, int is_f64, unsigned long long* keys,
-                                                                uint32_t* counts, uint64_t mask, HashCounters* ctr) {
+                                                                uint32_t* counts, uint64_t mask, HashCounters* ctr, RepTab R) {
     unsigned long long d = 0, sp = 0, sm = 0, nulls = 0, special = 0;
     for (int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; row < n; row += (int64_t)gridDim.x * blockDim.x) {
         if (!row_valid(validity, row)) {
@@ -48,6 +50,7 @@ __global__ void __launch_bounds__(HASH_THREADS) insert64_kernel(const uint64_t* 
                     ++sp;
                 } else if (old == 1) {
                     ++sm;
+                    if (MASK) rep_insert64(R, key);
                 }
                 break;
             }
@@ -118,8 +121,9 @@ __global__ void fp_utf8_kernel(const int32_t* offsets, const uint8_t* bytes, con
     }
 }
 
+template <bool MASK>
 __global__ void __launch_bounds__(HASH_THREADS) insert128_kernel(const Fp* fp, const uint8_t* nullflag, int64_t n,
-                                                                 Table128 t, HashCounters* ctr) {
+                                                                 Table128 t, HashCounters* ctr, RepTab R) {
     unsigned long long da = 0, dn = 0, sp = 0, sm = 0, nulls = 0;
     for (int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; row < n; row += (int64_t)gridDim.x * blockDim.x) {
         const bool has_null = nullflag[row] != 0;
@@ -133,6 +137,7 @@ __global__ void __launch_bounds__(HASH_THREADS) insert128_kernel(const Fp* fp, c
             ++sp;
         } else if (old == 1) {
             ++sm;
+            if (MASK) rep_insert128(R, fp[row]);
         }
     }
     flush_counter(da, &ctr->distinct_all);
@@ -266,6 +271,101 @@ __global__ void __launch_bounds__(HASH_THREADS) fk_probe128_kernel(const Fp* fp,
     flush_counter(viol, &ctr->violations);
     flush_counter(nullc, &ctr->null_children);
     if (collect) flush_counter(dist, &ctr->distinct_all);
+}
+
+// ---------------------------------------------------------------- key-level row verdicts ----
+// The key of a row: the canonical 64-bit value or the fingerprint (FP; nullflag given for a single-column key, whose NULL
+// rows have no key; a composite key is a value in every row). validity: the single key column's (nullptr: every row valid).
+struct RowKeys {
+    const uint64_t* values;
+    const uint32_t* validity;
+    int is_f64;
+    const Fp* fp;
+    const uint8_t* nullflag;
+};
+template <bool FP>
+__device__ __forceinline__ bool row_key_valid(const RowKeys& k, int64_t row) {
+    return FP ? !(k.nullflag && k.nullflag[row]) : row_valid(k.validity, row);
+}
+template <bool FP>
+__device__ __forceinline__ unsigned long long* row_rep_cell(const RepTab& R, const RowKeys& k, int64_t row) {
+    if (!R.h1) return nullptr;  // no repeated key: the key is not read
+    if (FP) return rep_cell128(R, k.fp[row]);
+    const uint64_t v = k.values[row];
+    return rep_cell64(R, k.is_f64 ? canon_f64(v) : v);
+}
+
+__global__ void rep_mark_kernel(RepTab R, uint64_t key) { rep_insert64(R, key); }
+
+// row pass 1: the lowest row of every repeated key
+template <bool FP>
+__global__ void __launch_bounds__(HASH_THREADS) rep_min_rows_kernel(RowKeys k, int64_t n, RepTab R) {
+    for (int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; row < n; row += (int64_t)gridDim.x * blockDim.x) {
+        if (!row_key_valid<FP>(k, row)) continue;
+        unsigned long long* cell = row_rep_cell<FP>(R, k, row);
+        if (cell) atomicMin(cell, (unsigned long long)row);
+    }
+}
+// row pass 2: one warp per 32-row word; DUPLICATE = the key is in R, FIRST = it is not, or this row is its lowest
+template <bool FP>
+__global__ void __launch_bounds__(HASH_THREADS) rep_verdict_kernel(RowKeys k, int64_t n, RepTab R, VerdictOut dup, VerdictOut first) {
+    const int64_t n_words = (n + 31) >> 5, warps = (int64_t)gridDim.x * (HASH_THREADS / 32);
+    if (!R.h1) {  // no repeated key: DUPLICATE = 0 and FIRST = validity, one thread per word, no key read
+        for (int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; w < n_words; w += (int64_t)gridDim.x * blockDim.x) {
+            const int64_t rem = n - 32 * w;
+            const uint32_t v = (k.validity ? k.validity[w] : 0xffffffffu) & (rem >= 32 ? 0xffffffffu : (1u << rem) - 1u);
+            if (dup.values) dup.values[w] = 0u;
+            if (dup.validity) dup.validity[w] = v;
+            if (first.values) first.values[w] = v;
+            if (first.validity) first.validity[w] = v;
+        }
+        return;
+    }
+    for (int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n_words; w += warps) {
+        const int64_t row = 32 * w + (threadIdx.x & 31);
+        const bool valid = row < n && row_key_valid<FP>(k, row);
+        const unsigned long long* cell = valid ? row_rep_cell<FP>(R, k, row) : nullptr;
+        store_verdict_word(w, cell != nullptr, valid, dup);
+        store_verdict_word(w, !cell || *cell == (unsigned long long)row, valid, first);
+    }
+}
+
+// FK: bit = the child row's key is in the exact table of distinct orphan keys that the probe path built
+struct Key64 {
+    const uint64_t* values;
+    int is_f64;
+    const unsigned long long* vkeys;  // nullptr: no key violates
+    uint64_t vmask;
+    int shift;           // slot = (fmix64(key) >> shift) & vmask, as the path's probe kernel placed it
+    int special_orphan;  // the EMPTY-sentinel key (Int64 -1), kept out of the table, has no parent
+    __device__ __forceinline__ bool orphan(int64_t row) const {
+        uint64_t key = values[row];
+        if (is_f64) key = canon_f64(key);
+        if (key == EMPTY64) return special_orphan != 0;
+        if (!vkeys) return false;
+        uint64_t slot = (fmix64(key) >> shift) & vmask;
+        for (uint64_t probes = 0; probes <= vmask; ++probes) {
+            const unsigned long long v = vkeys[slot];
+            if (v == key) return true;
+            if (v == EMPTY64) return false;
+            slot = (slot + 1) & vmask;
+        }
+        return false;
+    }
+};
+struct Fp128 {
+    const Fp* fp;
+    Table128 vtab;  // h1 == nullptr: no key violates
+    __device__ __forceinline__ bool orphan(int64_t row) const { return vtab.h1 && set128_contains(vtab, fp[row]); }
+};
+template <class K>
+__global__ void __launch_bounds__(HASH_THREADS) fk_orphan_rows_kernel(K k, const uint32_t* validity, int64_t n, VerdictOut out) {
+    const int64_t n_words = (n + 31) >> 5, warps = (int64_t)gridDim.x * (HASH_THREADS / 32);
+    for (int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n_words; w += warps) {
+        const int64_t row = 32 * w + (threadIdx.x & 31);
+        const bool valid = row < n && row_valid(validity, row);
+        store_verdict_word(w, valid && k.orphan(row), valid, out);
+    }
 }
 
 // ================================================================== host side ==================
@@ -436,19 +536,63 @@ void partition_fingerprints_by_rank(Engine& e, Table& t, const std::vector<std::
     *d_records = e.d_shuffle;
 }
 
-void exec_distinct_job(Engine& e, Table& t, Plan& p, int agg_id) {
-    Agg& a = p.aggs[agg_id];
-    std::vector<Column*> cols;
-    // a hash-shuffled shard of a Utf8 / composite key arrives as ONE column of fingerprint records
-    Column* shard = t.find("tg_fp");
-    const bool from_records = shard && shard->dtype == TG_FP128;
-    if (from_records) cols.push_back(shard);
-    else
-        for (auto& name : a.cols) cols.push_back(need_col(t, name));
+// ---------------------------------------------------------------- key-level row verdicts (host) ----
+static int word_grid(Engine& e, int64_t n) {
+    const int64_t blocks = ((n + 31) / 32 + HASH_THREADS / 32 - 1) / (HASH_THREADS / 32);
+    return (int)std::max<int64_t>(1, std::min<int64_t>(blocks, (int64_t)e.sm_count * 8));
+}
+
+// R in one recycled device block: h1 [cap], h2 [cap] (fingerprints only), minrow [cap], empty_key [2], fill [1]
+static size_t rep_bytes(uint64_t cap, bool fp) { return (size_t)cap * 8 * (fp ? 3 : 2) + 24; }
+void rep_reset(Engine& e, const RepTab& R) {
+    TG_CUDA(cudaMemsetAsync(R.h1, 0xFF, rep_bytes(R.mask + 1, R.h2 != nullptr), e.stream));
+    TG_CUDA(cudaMemsetAsync(R.empty_key, 0, 8, e.stream));
+    TG_CUDA(cudaMemsetAsync(R.fill, 0, 8, e.stream));
+}
+void rep_mark(Engine& e, const RepTab& R, uint64_t key) {
+    rep_mark_kernel<<<1, 1, 0, e.stream>>>(R, key);
+    TG_CUDA(cudaGetLastError());
+}
+struct RepBuf {
+    Engine& e;
+    RepTab R;
+    uint8_t* block = nullptr;
+    size_t bytes = 0;
+    explicit RepBuf(Engine& e_) : e(e_) {}
+    ~RepBuf() { release(); }
+    void release() {
+        if (block) e.dev_free(block, bytes);
+        block = nullptr;
+    }
+    void alloc(uint64_t cap, bool fp) {
+        release();
+        bytes = rep_bytes(cap, fp);
+        block = e.dev_alloc(bytes);
+        unsigned long long* q = reinterpret_cast<unsigned long long*>(block);
+        R.h1 = q;
+        R.h2 = fp ? q + cap : nullptr;
+        R.minrow = q + cap * (fp ? 2 : 1);
+        R.empty_key = q + cap * (fp ? 3 : 2);
+        R.fill = R.empty_key + 2;
+        R.mask = cap - 1;
+    }
+};
+constexpr uint64_t REP_CAP0 = 1u << 20;
+
+static VerdictOut verdict_out(const std::shared_ptr<RowMask>& m) {
+    VerdictOut o;
+    if (m) {
+        o.values = reinterpret_cast<uint32_t*>(m->values);
+        o.validity = reinterpret_cast<uint32_t*>(m->validity);
+    }
+    return o;
+}
+
+// the job's repeated-key count after the counting pass: the keys R has to hold
+static uint64_t count_distinct(Engine& e, Table& t, Plan& p, Agg& a, const std::vector<Column*>& cols, Column* shard, const RepTab* R,
+                               Fp*& d_fp, uint8_t*& d_null) {
     const int64_t n = t.n_rows;
-    a.u[0] = (uint64_t)n;
-    for (auto* c : cols) p.stats.bytes_scanned += from_records ? (uint64_t)n * sizeof(FpRecord) : col_bytes(*c, n);
-    if (n == 0) return;
+    const bool from_records = shard != nullptr;
     const bool exact64 = cols.size() == 1 && (cols[0]->dtype == TG_INT64 || cols[0]->dtype == TG_FLOAT64);
     if (exact64 && n > (1 << 20)) {
         // large key column: dense Int64 ranges are counted in bitmaps (hashpart.cu); anything else is hashed, radix-sorted by
@@ -457,9 +601,9 @@ void exec_distinct_job(Engine& e, Table& t, Plan& p, int agg_id) {
         Distinct64Result r;
         Timer tm(e, p);
         int launches = 0;
-        bool ok = distinct64_dense(e, *cols[0], n, (a.flags & 1) != 0, r, launches);
-        if (!ok && (size_t)n > distinct64_min_rows()) ok = distinct64_sorted(e, *cols[0], n, r, launches);
-        if (!ok && (size_t)n > distinct64_min_rows()) ok = distinct64_partitioned(e, *cols[0], n, r, launches);
+        bool ok = distinct64_dense(e, *cols[0], n, (a.flags & 1) != 0, r, launches, R);
+        if (!ok && (size_t)n > distinct64_min_rows()) ok = distinct64_sorted(e, *cols[0], n, r, launches, R);
+        if (!ok && (size_t)n > distinct64_min_rows()) ok = distinct64_partitioned(e, *cols[0], n, r, launches, R);
         tm.stop(launches);
         if (ok) {
             const uint64_t singles = r.distinct - r.dup_keys;
@@ -468,7 +612,7 @@ void exec_distinct_job(Engine& e, Table& t, Plan& p, int agg_id) {
             a.u[3] = r.nulls;
             a.u[4] = r.nulls;
             a.u[5] = r.distinct + (r.nulls > 0 ? 1 : 0);
-            return;
+            return r.dup_keys;
         }
         // a bucket table overflowed (adversarial hash skew): fall through to the single-table path
     }
@@ -476,6 +620,7 @@ void exec_distinct_job(Engine& e, Table& t, Plan& p, int agg_id) {
     HashCounters h{};
     Timer tm(e, p);
     int launches = 0;
+    if (R) rep_reset(e, *R);
     if (exact64) {
         const size_t keys_b = cap * 8, cnt_b = cap * 4;
         uint8_t* scr = e.scratch(keys_b + cnt_b + 256);
@@ -484,9 +629,13 @@ void exec_distinct_job(Engine& e, Table& t, Plan& p, int agg_id) {
         HashCounters* d_ctr = (HashCounters*)(scr + keys_b + cnt_b);
         TG_CUDA(cudaMemsetAsync(keys, 0xFF, keys_b, e.stream));
         TG_CUDA(cudaMemsetAsync(counts, 0, cnt_b + 256, e.stream));
-        insert64_kernel<<<grid_for(e, n), HASH_THREADS, 0, e.stream>>>((const uint64_t*)cols[0]->values.p,
-                                                                       (const uint32_t*)cols[0]->validity.p, n,
-                                                                       cols[0]->dtype == TG_FLOAT64, keys, counts, cap - 1, d_ctr);
+        const uint64_t* vals = (const uint64_t*)cols[0]->values.p;
+        const uint32_t* valid = (const uint32_t*)cols[0]->validity.p;
+        const int is_f64 = cols[0]->dtype == TG_FLOAT64;
+        if (R)
+            insert64_kernel<true><<<grid_for(e, n), HASH_THREADS, 0, e.stream>>>(vals, valid, n, is_f64, keys, counts, cap - 1, d_ctr, *R);
+        else
+            insert64_kernel<false><<<grid_for(e, n), HASH_THREADS, 0, e.stream>>>(vals, valid, n, is_f64, keys, counts, cap - 1, d_ctr, RepTab{});
         TG_CUDA(cudaGetLastError());
         launches = 1;
         TG_CUDA(cudaMemcpyAsync(&h, d_ctr, sizeof(h), cudaMemcpyDeviceToHost, e.stream));
@@ -496,19 +645,21 @@ void exec_distinct_job(Engine& e, Table& t, Plan& p, int agg_id) {
             distinct_nonnull += 1;
             singles += h.special == 1;
         }
+        // the Int64 value -1 is the table's EMPTY word: counted apart, and marked repeated by hand
+        if (R && h.special > 1) rep_mark(e, *R, EMPTY64);
         const uint64_t nulls = h.any_null_rows;
         a.u[1] = distinct_nonnull;
         a.u[2] = singles + (nulls == 1 ? 1 : 0);  // the NULL group of GROUP BY
         a.u[3] = nulls;
         a.u[4] = nulls;
         a.u[5] = distinct_nonnull + (nulls > 0 ? 1 : 0);
-        return;
+        return h.singles_minus + (h.special > 1 ? 1 : 0);
     }
     const size_t fp_b = round_up((size_t)n * 16, 256), nf_b = round_up((size_t)n, 256);
     const size_t h_b = cap * 8, cnt_b = cap * 4;
     uint8_t* scr = e.scratch(fp_b + nf_b + 2 * h_b + cnt_b + 256);
-    Fp* d_fp = (Fp*)scr;
-    uint8_t* d_null = scr + fp_b;
+    d_fp = (Fp*)scr;
+    d_null = scr + fp_b;
     Table128 tb{(unsigned long long*)(scr + fp_b + nf_b), (unsigned long long*)(scr + fp_b + nf_b + h_b),
                 (uint32_t*)(scr + fp_b + nf_b + 2 * h_b), cap - 1};
     HashCounters* d_ctr = (HashCounters*)(scr + fp_b + nf_b + 2 * h_b + cnt_b);
@@ -520,7 +671,8 @@ void exec_distinct_job(Engine& e, Table& t, Plan& p, int agg_id) {
     } else {
         launches += compute_fingerprints(e, t, cols, d_fp, d_null);
     }
-    insert128_kernel<<<grid_for(e, n), HASH_THREADS, 0, e.stream>>>(d_fp, d_null, n, tb, d_ctr);
+    if (R) insert128_kernel<true><<<grid_for(e, n), HASH_THREADS, 0, e.stream>>>(d_fp, d_null, n, tb, d_ctr, *R);
+    else insert128_kernel<false><<<grid_for(e, n), HASH_THREADS, 0, e.stream>>>(d_fp, d_null, n, tb, d_ctr, RepTab{});
     TG_CUDA(cudaGetLastError());
     ++launches;
     TG_CUDA(cudaMemcpyAsync(&h, d_ctr, sizeof(h), cudaMemcpyDeviceToHost, e.stream));
@@ -530,6 +682,72 @@ void exec_distinct_job(Engine& e, Table& t, Plan& p, int agg_id) {
     a.u[3] = h.any_null_rows;
     a.u[4] = h.any_null_rows;
     a.u[5] = h.distinct_all;
+    return h.singles_minus;
+}
+
+void exec_distinct_job(Engine& e, Table& t, Plan& p, int agg_id) {
+    Agg& a = p.aggs[agg_id];
+    std::vector<Column*> cols;
+    // a hash-shuffled shard of a Utf8 / composite key arrives as ONE column of fingerprint records
+    Column* shard = t.find("tg_fp");
+    const bool from_records = shard && shard->dtype == TG_FP128;
+    if (from_records) cols.push_back(shard);
+    else
+        for (auto& name : a.cols) cols.push_back(need_col(t, name));
+    if (!from_records) shard = nullptr;
+    const int64_t n = t.n_rows;
+    a.u[0] = (uint64_t)n;
+    for (auto* c : cols) p.stats.bytes_scanned += from_records ? (uint64_t)n * sizeof(FpRecord) : col_bytes(*c, n);
+    // key-level row verdicts of the rows of this table (a shard of keys shuffled here from other ranks has none: the
+    // export reports it); a NULL single-column key has none either, a composite key is a value in every row
+    const bool verdicts = (a.key_rows & ((1 << TG_KEY_ROWS_DUPLICATE) | (1 << TG_KEY_ROWS_FIRST))) && a.redirect[0].empty() && !from_records;
+    const bool single = cols.size() == 1;
+    const bool emit_validity = single && cols[0]->validity.p && cols[0]->null_count > 0;
+    if (verdicts)
+        for (int k : {TG_KEY_ROWS_DUPLICATE, TG_KEY_ROWS_FIRST})
+            if (a.key_rows & (1 << k)) a.key_mask[k] = new_row_mask(e, n, emit_validity);
+    if (n == 0) return;
+    const bool fp = !(single && (cols[0]->dtype == TG_INT64 || cols[0]->dtype == TG_FLOAT64));
+    RepBuf rb(e);
+    if (verdicts) rb.alloc(REP_CAP0, fp);
+    Fp* d_fp = nullptr;
+    uint8_t* d_null = nullptr;
+    uint64_t reps = count_distinct(e, t, p, a, cols, shard, verdicts ? &rb.R : nullptr, d_fp, d_null);
+    if (!verdicts) return;
+    if (reps > REP_CAP0 / 2) {
+        // more repeated keys than R holds at load 1/2: repeat the job once with R sized from the now-known count
+        rb.alloc(pow2_at_least(reps * 2), fp);
+        reps = count_distinct(e, t, p, a, cols, shard, &rb.R, d_fp, d_null);
+    }
+    // no repeated key (a passing is_unique): no row pass against R, every valid row is the first of its key
+    const RepTab R = reps ? rb.R : RepTab{};
+    const RowKeys k{fp ? nullptr : (const uint64_t*)cols[0]->values.p, single ? (const uint32_t*)cols[0]->validity.p : nullptr,
+                    !fp && cols[0]->dtype == TG_FLOAT64, d_fp, fp && single ? d_null : nullptr};
+    const VerdictOut dup = verdict_out(a.key_mask[TG_KEY_ROWS_DUPLICATE]), first = verdict_out(a.key_mask[TG_KEY_ROWS_FIRST]);
+    Timer tm(e, p);
+    int launches = 1;
+    if (reps) {
+        if (fp) rep_min_rows_kernel<true><<<grid_for(e, n), HASH_THREADS, 0, e.stream>>>(k, n, R);
+        else rep_min_rows_kernel<false><<<grid_for(e, n), HASH_THREADS, 0, e.stream>>>(k, n, R);
+        ++launches;
+    }
+    if (fp) rep_verdict_kernel<true><<<word_grid(e, n), HASH_THREADS, 0, e.stream>>>(k, n, R, dup, first);
+    else rep_verdict_kernel<false><<<word_grid(e, n), HASH_THREADS, 0, e.stream>>>(k, n, R, dup, first);
+    TG_CUDA(cudaGetLastError());
+    tm.stop(launches);
+    const int64_t nulls = emit_validity ? (int64_t)a.u[3] : 0;
+    for (auto& m : a.key_mask)
+        if (m) m->null_count = nulls;
+}
+
+// FK orphan rows of a 64-bit child key column (the paths of hashpart.cu call this with their orphan table)
+void fk_orphan_rows64(Engine& e, const Column& child, int64_t nc, const unsigned long long* vkeys, uint64_t vmask, int shift,
+                      bool special_orphan, const VerdictOut& out, int& launches) {
+    if (nc == 0) return;
+    const Key64 k{(const uint64_t*)child.values.p, child.dtype == TG_FLOAT64, vkeys, vmask, shift, special_orphan ? 1 : 0};
+    fk_orphan_rows_kernel<Key64><<<word_grid(e, nc), HASH_THREADS, 0, e.stream>>>(k, (const uint32_t*)child.validity.p, nc, out);
+    TG_CUDA(cudaGetLastError());
+    ++launches;
 }
 
 // value of a row as the reference prints violation examples (foreign_key.rs:250-290)
@@ -581,6 +799,17 @@ void exec_fk_job(Engine& e, Plan& p, int agg_id) {
     const int64_t nc = ct.n_rows, np = pt.n_rows;
     p.stats.bytes_scanned += from_records ? (uint64_t)(nc + np) * sizeof(FpRecord) : col_bytes(*cc, nc) + col_bytes(*pc, np);
     const int allow_nulls = a.flags, max_examples = std::max(0, a.iparam);
+    // orphan row verdicts cover the child table's rows; keys shuffled here from other ranks are not that table's rows
+    VerdictOut orphan;
+    const VerdictOut* orphan_rows = nullptr;
+    if ((a.key_rows & (1 << TG_KEY_ROWS_ORPHAN)) && a.redirect[0].empty() && a.redirect[1].empty()) {
+        const bool emit_validity = cc->validity.p && cc->null_count > 0;
+        auto& m = a.key_mask[TG_KEY_ROWS_ORPHAN];
+        m = new_row_mask(e, nc, emit_validity);
+        m->null_count = emit_validity ? cc->null_count : 0;
+        orphan = verdict_out(m);
+        orphan_rows = &orphan;
+    }
     if (nc == 0) return;
     const bool exact64 = cc->dtype == TG_INT64 || cc->dtype == TG_FLOAT64;
     const uint64_t pcap = pow2_at_least((uint64_t)std::max<int64_t>(np, 1) * 2);
@@ -592,8 +821,9 @@ void exec_fk_job(Engine& e, Plan& p, int agg_id) {
         // hashpart.cu: a dense Int64 parent range becomes a bitmap; a parent key set too large for an L2-resident
         // table is radix-partitioned together with the child keys by the same hash bits
         Fk64Result r;
-        bool ok = fk64_dense(e, *cc, nc, *pc, np, allow_nulls, max_examples, r, launches);
-        if (!ok && (size_t)np > distinct64_min_rows()) ok = fk64_partitioned(e, *cc, nc, *pc, np, allow_nulls, max_examples, r, launches);
+        bool ok = fk64_dense(e, *cc, nc, *pc, np, allow_nulls, max_examples, r, launches, orphan_rows);
+        if (!ok && (size_t)np > distinct64_min_rows())
+            ok = fk64_partitioned(e, *cc, nc, *pc, np, allow_nulls, max_examples, r, launches, orphan_rows);
         if (ok) {
             tm.stop(launches);
             a.u[0] = r.violations;
@@ -679,9 +909,12 @@ void exec_fk_job(Engine& e, Plan& p, int agg_id) {
             ++launches;
             TG_CUDA(cudaMemcpyAsync(&h, d_ctr, sizeof(h), cudaMemcpyDeviceToHost, e.stream));
             TG_CUDA(cudaStreamSynchronize(e.stream));
+            if (orphan_rows) fk_orphan_rows64(e, *cc, nc, vkeys, vcap - 1, 0, h.special > 0, orphan, launches);
             const size_t ne = (size_t)std::min<uint64_t>(h.n_examples, (uint64_t)max_examples);
             ex_rows.resize(ne);
             if (ne) TG_CUDA(cudaMemcpy(ex_rows.data(), d_ex, ne * 8, cudaMemcpyDeviceToHost));
+        } else if (orphan_rows) {
+            fk_orphan_rows64(e, *cc, nc, nullptr, 0, 0, false, orphan, launches);  // no key violates
         }
     } else if (cc->dtype == TG_UTF8 || from_records) {
         const size_t cfp_b = round_up((size_t)nc * 16, 256), cnf_b = round_up((size_t)nc, 256);
@@ -723,6 +956,13 @@ void exec_fk_job(Engine& e, Plan& p, int agg_id) {
         ++launches;
         TG_CUDA(cudaMemcpyAsync(&h, d_ctr, sizeof(h), cudaMemcpyDeviceToHost, e.stream));
         TG_CUDA(cudaStreamSynchronize(e.stream));
+        if (orphan_rows) {
+            const bool key_viol = h.violations > (allow_nulls ? 0 : h.null_children);
+            const Fp128 k{cfp, key_viol ? vtab : Table128{}};
+            fk_orphan_rows_kernel<Fp128><<<word_grid(e, nc), HASH_THREADS, 0, e.stream>>>(k, (const uint32_t*)cc->validity.p, nc, orphan);
+            TG_CUDA(cudaGetLastError());
+            ++launches;
+        }
         // (a shard of fingerprint records has no strings to show: counts only, the examples stay empty)
         const size_t ne = from_records ? 0 : (size_t)std::min<uint64_t>(h.n_examples, (uint64_t)max_examples);
         ex_rows.resize(ne);

@@ -304,9 +304,11 @@ static int hash_lanes() {
 
 constexpr int BUCKET_ILP = 4;  // independent probe chains per thread (the loop is bound by L2 atomic latency)
 
+// MASK: a key seen twice also goes into the repeated-key table R (key-level row verdicts)
+template <bool MASK>
 __global__ void __launch_bounds__(HASH_THREADS) insert_bucket_kernel(const uint64_t* __restrict__ keys, const unsigned long long* offsets,
                                                                      int bucket, unsigned long long* table, uint32_t mask, uint32_t* bits,
-                                                                     HashCounters* ctr) {
+                                                                     HashCounters* ctr, RepTab R) {
     const int64_t begin = (int64_t)offsets[bucket], end = (int64_t)offsets[bucket + 1];
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     unsigned long long d = 0, dup = 0, ovf = 0;
@@ -336,7 +338,10 @@ __global__ void __launch_bounds__(HASH_THREADS) insert_bucket_kernel(const uint6
                 }
                 if (prev[u] == key[u]) {
                     const uint32_t bit = 1u << (slot[u] & 31);
-                    if (!(atomicOr(&bits[slot[u] >> 5], bit) & bit)) ++dup;
+                    if (!(atomicOr(&bits[slot[u] >> 5], bit) & bit)) {
+                        ++dup;
+                        if (MASK) rep_insert64(R, key[u]);
+                    }
                     break;
                 }
                 if (probes >= mask) {
@@ -522,12 +527,13 @@ __global__ void __launch_bounds__(PART_THREADS) sample_minmax_i64_kernel(const l
 }
 
 // mode 0: distinct / seen-twice counting; mode 1: build the parent set (non-returning OR); mode 2: probe
-template <int MODE>
+// MASK (mode 0): a key seen twice also goes into the repeated-key table R (key-level row verdicts)
+template <int MODE, bool MASK = false>
 __global__ void __launch_bounds__(PART_THREADS) dense_kernel(const long long* __restrict__ values, const uint32_t* __restrict__ validity,
                                                              int64_t n, long long lo, unsigned long long range, uint32_t* seen,
                                                              uint32_t* dup, unsigned long long* vkeys, uint64_t vmask,
                                                              unsigned long long* examples, int max_examples, HashCounters* ctr,
-                                                             unsigned long long* nulls_out = nullptr) {
+                                                             unsigned long long* nulls_out = nullptr, RepTab R = RepTab{}) {
     unsigned long long d = 0, dupk = 0, viol = 0, dist = 0, nulls = 0, special = 0, nulls_count = 0, oob = 0;
     const int64_t n_tiles = (n + PART_TILE - 1) / PART_TILE;
     for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
@@ -572,7 +578,10 @@ __global__ void __launch_bounds__(PART_THREADS) dense_kernel(const long long* __
                 } else {
                     const unsigned long long idx = ((unsigned long long)v[k] - (unsigned long long)lo);
                     const uint32_t bit = 1u << (idx & 31);
-                    if (!(atomicOr(&dup[idx >> 5], bit) & bit)) ++dupk;
+                    if (!(atomicOr(&dup[idx >> 5], bit) & bit)) {
+                        ++dupk;
+                        if (MASK) rep_insert64(R, (uint64_t)v[k]);
+                    }
                 }
             } else if (MODE == 2 && !old[k]) {
                 ++viol;
@@ -787,7 +796,7 @@ bool column_minmax_i64(Engine& e, const Column& c, int64_t n, long long* mn, lon
     return any;
 }
 
-bool distinct64_partitioned(Engine& e, const Column& c, int64_t n, Distinct64Result& r, int& launches) {
+bool distinct64_partitioned(Engine& e, const Column& c, int64_t n, Distinct64Result& r, int& launches, const RepTab* R) {
     const int lanes = hash_lanes();
     const uint32_t parts = parts_for(n, lanes);
     const uint64_t cap = pow2_at_least(((uint64_t)n + parts - 1) / parts * slots_factor(), 1024);
@@ -799,6 +808,7 @@ bool distinct64_partitioned(Engine& e, const Column& c, int64_t n, Distinct64Res
     m.bind(tables + (size_t)lanes * (tab_b + bits_b));
     HashCounters* d_ctr = (HashCounters*)(tables + (size_t)lanes * (tab_b + bits_b) + PartMeta::bytes());
     TG_CUDA(cudaMemsetAsync(d_ctr, 0, sizeof(HashCounters), e.stream));
+    if (R) rep_reset(e, *R);
     launches += partition_column<PM_BUCKET>(e, c, n, parts, m, part_keys);
     const int grid = bucket_grid(e, n / parts / BUCKET_ILP + 1);
     // fan out: lane l handles buckets l, l + lanes, .. on its own stream and table; fan back in before the read-back
@@ -812,7 +822,8 @@ bool distinct64_partitioned(Engine& e, const Column& c, int64_t n, Distinct64Res
         for (uint32_t b = (uint32_t)l; b < parts; b += (uint32_t)lanes) {
             fill_async(e, table, tab_b, 0xFFFFFFFFu, st);
             fill_async(e, bits, bits_b, 0u, st);
-            insert_bucket_kernel<<<grid, HASH_THREADS, 0, st>>>(part_keys, m.offsets, (int)b, table, (uint32_t)(cap - 1), bits, d_ctr);
+            if (R) insert_bucket_kernel<true><<<grid, HASH_THREADS, 0, st>>>(part_keys, m.offsets, (int)b, table, (uint32_t)(cap - 1), bits, d_ctr, *R);
+            else insert_bucket_kernel<false><<<grid, HASH_THREADS, 0, st>>>(part_keys, m.offsets, (int)b, table, (uint32_t)(cap - 1), bits, d_ctr, RepTab{});
             ++launches;
         }
         if (lanes > 1) {
@@ -827,6 +838,7 @@ bool distinct64_partitioned(Engine& e, const Column& c, int64_t n, Distinct64Res
     TG_CUDA(cudaMemcpyAsync(&pc, m.ctr, sizeof(pc), cudaMemcpyDeviceToHost, e.stream));
     TG_CUDA(cudaStreamSynchronize(e.stream));
     if (h.overflow) return false;
+    if (R && pc.special > 1) rep_mark(e, *R, EMPTY64);  // the Int64 value -1 never enters the bucket tables
     r.distinct = h.distinct_nonnull + (pc.special ? 1 : 0);
     r.dup_keys = h.singles_minus + (pc.special > 1 ? 1 : 0);
     r.nulls = pc.nulls;
@@ -834,7 +846,7 @@ bool distinct64_partitioned(Engine& e, const Column& c, int64_t n, Distinct64Res
 }
 
 bool fk64_partitioned(Engine& e, const Column& child, int64_t nc, const Column& parent, int64_t np, int allow_nulls, int max_examples,
-                      Fk64Result& r, int& launches) {
+                      Fk64Result& r, int& launches, const VerdictOut* orphan_rows) {
     const uint32_t parts = parts_for(np);
     const uint64_t cap = pow2_at_least(((uint64_t)np + parts - 1) / parts * slots_factor(), 1024);
     const size_t ck_b = round_up((size_t)nc * 8, 256), pk_b = round_up((size_t)std::max<int64_t>(np, 1) * 8, 256), tab_b = cap * 8;
@@ -903,13 +915,18 @@ bool fk64_partitioned(Engine& e, const Column& child, int64_t nc, const Column& 
             TG_CUDA(cudaStreamSynchronize(e.stream));
             r.distinct_violations = h.distinct_all;
             fetch_examples(d_ex0, h.n_examples);
+            if (orphan_rows) {
+                fk_orphan_rows64(e, child, nc, vkeys, vcap - 1, 20, special_orphan, *orphan_rows, launches);
+                TG_CUDA(cudaStreamSynchronize(e.stream));  // the pass reads `extra`, freed below
+            }
         } catch (...) {
             cudaFree(extra);
             throw;
         }
         cudaFree(extra);
-    } else if (h.violations > 0) {
-        fetch_examples(d_ex0, h.n_examples);
+    } else {
+        if (h.violations > 0) fetch_examples(d_ex0, h.n_examples);
+        if (orphan_rows) fk_orphan_rows64(e, child, nc, h.violations > 0 ? vkeys0 : nullptr, FK_VCAP - 1, 20, special_orphan, *orphan_rows, launches);
     }
     if (special_orphan) {
         r.distinct_violations += 1;
@@ -969,7 +986,7 @@ static bool dense_enough(const MinMaxOut& h) {
 
 // one bitmap pass over [lo, lo + range]; returns the counters (overflow = keys outside the range)
 static HashCounters dense_distinct_pass(Engine& e, const Column& c, int64_t n, bool need_singles, long long lo, unsigned long long range,
-                                        int& launches) {
+                                        int& launches, const RepTab* R) {
     const size_t bm_b = round_up((size_t)(range / 32 + 1) * 4, 256);
     uint8_t* scr = e.scratch(2 * bm_b + 256);
     uint32_t* seen = (uint32_t*)scr;
@@ -978,8 +995,14 @@ static HashCounters dense_distinct_pass(Engine& e, const Column& c, int64_t n, b
     if (need_singles) {
         // one RETURNING atomicOr per key: the old bit tells first from repeated occurrence
         fill_async(e, scr, 2 * bm_b + 256, 0u);
-        dense_kernel<0><<<part_grid(e, n), PART_THREADS, 0, e.stream>>>((const long long*)c.values.p, (const uint32_t*)c.validity.p, n, lo, range,
-                                                                       seen, dup, nullptr, 0, nullptr, 0, d_ctr);
+        if (R) {
+            rep_reset(e, *R);
+            dense_kernel<0, true><<<part_grid(e, n), PART_THREADS, 0, e.stream>>>((const long long*)c.values.p, (const uint32_t*)c.validity.p, n, lo,
+                                                                                  range, seen, dup, nullptr, 0, nullptr, 0, d_ctr, nullptr, *R);
+        } else {
+            dense_kernel<0><<<part_grid(e, n), PART_THREADS, 0, e.stream>>>((const long long*)c.values.p, (const uint32_t*)c.validity.p, n, lo, range,
+                                                                           seen, dup, nullptr, 0, nullptr, 0, d_ctr);
+        }
         launches += 2;
     } else {
         // only COUNT(DISTINCT) is wanted: non-returning ORs (190 vs 126 G/s in L2), then count the set bits
@@ -999,8 +1022,9 @@ static HashCounters dense_distinct_pass(Engine& e, const Column& c, int64_t n, b
     return h;
 }
 
-bool distinct64_dense(Engine& e, const Column& c, int64_t n, bool need_singles, Distinct64Result& r, int& launches) {
+bool distinct64_dense(Engine& e, const Column& c, int64_t n, bool need_singles, Distinct64Result& r, int& launches, const RepTab* R) {
     if (c.dtype != TG_INT64 || getenv("TG_HASH_NO_DENSE")) return false;
+    need_singles = need_singles || R;  // the row verdicts need the 1 -> 2 transitions of the seen-twice map
     auto fill_result = [&](const HashCounters& h) {
         r.distinct = h.distinct_nonnull;
         r.dup_keys = need_singles ? h.singles_minus : 0;  // unused by the slots of this plan when !need_singles
@@ -1035,7 +1059,7 @@ bool distinct64_dense(Engine& e, const Column& c, int64_t n, bool need_singles, 
             const long long hi = g.mx > INT64_MAX - (long long)pad ? INT64_MAX : g.mx + (long long)pad;
             const unsigned long long range = (unsigned long long)hi - (unsigned long long)lo;
             if (range < DENSE_MAX_RANGE && range <= 32ull * (unsigned long long)n + 4096ull) {
-                const HashCounters h = dense_distinct_pass(e, c, n, need_singles, lo, range, launches);
+                const HashCounters h = dense_distinct_pass(e, c, n, need_singles, lo, range, launches, R);
                 if (h.overflow == 0) {
                     fill_result(h);
                     return true;
@@ -1051,12 +1075,12 @@ bool distinct64_dense(Engine& e, const Column& c, int64_t n, bool need_singles, 
     }
     if (!dense_enough(mm)) return false;
     const unsigned long long range = (unsigned long long)mm.mx - (unsigned long long)mm.mn;
-    fill_result(dense_distinct_pass(e, c, n, need_singles, mm.mn, range, launches));
+    fill_result(dense_distinct_pass(e, c, n, need_singles, mm.mn, range, launches, R));
     return true;
 }
 
 bool fk64_dense(Engine& e, const Column& child, int64_t nc, const Column& parent, int64_t np, int allow_nulls, int max_examples,
-                Fk64Result& r, int& launches) {
+                Fk64Result& r, int& launches, const VerdictOut* orphan_rows) {
     if (child.dtype != TG_INT64 || parent.dtype != TG_INT64 || getenv("TG_HASH_NO_DENSE")) return false;
     MinMaxOut mm{};
     const bool have_parent = minmax_i64(e, parent, np, mm, launches);
@@ -1101,11 +1125,17 @@ bool fk64_dense(Engine& e, const Column& child, int64_t nc, const Column& parent
             probe((unsigned long long*)extra, vcap - 1);
             TG_CUDA(cudaMemcpyAsync(&h, d_ctr, sizeof(h), cudaMemcpyDeviceToHost, e.stream));
             TG_CUDA(cudaStreamSynchronize(e.stream));
+            if (orphan_rows) {
+                fk_orphan_rows64(e, child, nc, (const unsigned long long*)extra, vcap - 1, 20, h.special > 0, *orphan_rows, launches);
+                TG_CUDA(cudaStreamSynchronize(e.stream));  // the pass reads `extra`, freed below
+            }
         } catch (...) {
             cudaFree(extra);
             throw;
         }
         cudaFree(extra);
+    } else if (orphan_rows) {
+        fk_orphan_rows64(e, child, nc, h.violations > h.special ? vkeys0 : nullptr, FK_VCAP - 1, 20, h.special > 0, *orphan_rows, launches);
     }
     r.null_children = h.any_null_rows;
     r.violations = h.violations + (allow_nulls ? 0 : h.any_null_rows);

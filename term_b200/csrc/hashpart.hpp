@@ -7,6 +7,15 @@
 
 namespace tg {
 
+// key-level row verdicts (hash_common.cuh): a counting path given R (not nullptr) also inserts every key it sees a second
+// time into R; a foreign-key path given `orphan_rows` also writes the child rows whose key it found without a parent
+struct RepTab;
+struct VerdictOut;
+void rep_reset(Engine& e, const RepTab& R);              // empties R before a counting attempt
+void rep_mark(Engine& e, const RepTab& R, uint64_t key);  // a key the path counted apart occurs twice or more
+void fk_orphan_rows64(Engine& e, const Column& child, int64_t nc, const unsigned long long* vkeys, uint64_t vmask, int shift,
+                      bool special_orphan, const VerdictOut& out, int& launches);
+
 struct Distinct64Result {
     uint64_t distinct = 0;   // distinct non-null keys
     uint64_t dup_keys = 0;   // keys that occur at least twice
@@ -14,15 +23,16 @@ struct Distinct64Result {
 };
 // COUNT(DISTINCT c) / GROUP BY c HAVING COUNT(*) = 1 over a single 64-bit key column. Returns false when a bucket
 // table overflowed (pathologically skewed hash): the caller falls back to the single-table path.
-bool distinct64_partitioned(Engine& e, const Column& c, int64_t n, Distinct64Result& r, int& launches);
+bool distinct64_partitioned(Engine& e, const Column& c, int64_t n, Distinct64Result& r, int& launches, const RepTab* R = nullptr);
 size_t distinct64_min_rows();
 // The same counts for sparse keys without a global atomic (hashsort.cu): hashes of the valid keys, two or three radix passes
 // over their low bits, shared-memory de-duplication of the contiguous hash buckets. Returns false (nothing counted) on a
 // hot key / skewed bucket or for n >= 2^30: the caller takes the partitioned path.
-bool distinct64_sorted(Engine& e, const Column& c, int64_t n, Distinct64Result& r, int& launches);
+bool distinct64_sorted(Engine& e, const Column& c, int64_t n, Distinct64Result& r, int& launches, const RepTab* R = nullptr);
 // Dense Int64 key range (max - min < 2^28 and < 32 n): exact bitmap counting, no partitioning. Returns false when
 // the column does not qualify (nothing is counted then).
-bool distinct64_dense(Engine& e, const Column& c, int64_t n, bool need_singles, Distinct64Result& r, int& launches);
+bool distinct64_dense(Engine& e, const Column& c, int64_t n, bool need_singles, Distinct64Result& r, int& launches,
+                      const RepTab* R = nullptr);
 
 struct Fk64Result {
     uint64_t violations = 0;           // child rows without a parent (NULL children included when not allowed)
@@ -31,10 +41,10 @@ struct Fk64Result {
     std::vector<uint64_t> example_keys;  // up to max_examples distinct orphan keys (raw 64-bit values)
 };
 bool fk64_partitioned(Engine& e, const Column& child, int64_t nc, const Column& parent, int64_t np, int allow_nulls,
-                      int max_examples, Fk64Result& r, int& launches);
+                      int max_examples, Fk64Result& r, int& launches, const VerdictOut* orphan_rows = nullptr);
 
 bool fk64_dense(Engine& e, const Column& child, int64_t nc, const Column& parent, int64_t np, int allow_nulls, int max_examples,
-                Fk64Result& r, int& launches);
+                Fk64Result& r, int& launches, const VerdictOut* orphan_rows = nullptr);
 
 // Multi-GPU shuffle, step 1 (SURVEY §8e): the valid keys of a column grouped by destination rank
 // (hash_rank of the canonical key). d_keys stays valid until the next partition call on this engine.

@@ -137,7 +137,9 @@ __global__ void __launch_bounds__(HS_THREADS) hs_prep_kernel(const uint64_t* __r
 struct HsLocal {
     uint32_t distinct, dups, overflow;
 };
-__device__ __forceinline__ void hs_insert(unsigned long long* tab, uint32_t* twice, uint64_t k, int slot_shift, HsLocal& L) {
+// MASK: a key seen twice also goes into the repeated-key table R, as the key its hash came from
+template <bool MASK>
+__device__ __forceinline__ void hs_insert(unsigned long long* tab, uint32_t* twice, uint64_t k, int slot_shift, HsLocal& L, const RepTab& R) {
     uint32_t slot = (uint32_t)(k >> slot_shift) & (HS_SLOTS - 1);
     for (int probes = 0; probes < HS_SLOTS; ++probes) {
         unsigned long long cur = *reinterpret_cast<volatile unsigned long long*>(&tab[slot]);
@@ -152,7 +154,10 @@ __device__ __forceinline__ void hs_insert(unsigned long long* tab, uint32_t* twi
             const uint32_t bit = 1u << (slot & 31);
             if (!(*reinterpret_cast<volatile uint32_t*>(&twice[slot >> 5]) & bit)) {
                 const uint32_t prev = atomicOr(&twice[slot >> 5], bit);
-                if (!(prev & bit)) ++L.dups;
+                if (!(prev & bit)) {
+                    ++L.dups;
+                    if (MASK) rep_insert64(R, fmix64_inv(k));
+                }
             }
             return;
         }
@@ -162,8 +167,9 @@ __device__ __forceinline__ void hs_insert(unsigned long long* tab, uint32_t* twi
 }
 
 // H (buffer ctl->result of k0 / k1): n hashes sorted by their low bits (h & mask). slot_shift: first hash bit above the mask.
+template <bool MASK>
 __global__ void __launch_bounds__(HS_THREADS) hs_dedup_kernel(const uint64_t* __restrict__ k0, const uint64_t* __restrict__ k1, const RsControl* ctl,
-                                                              int64_t n, uint64_t mask, int slot_shift, HsCounters* ctr) {
+                                                              int64_t n, uint64_t mask, int slot_shift, HsCounters* ctr, RepTab R) {
     extern __shared__ __align__(16) uint8_t hs_smem[];
     unsigned long long* tab = reinterpret_cast<unsigned long long*>(hs_smem);
     uint32_t* twice = reinterpret_cast<uint32_t*>(hs_smem + (size_t)HS_SLOTS * 8);
@@ -190,7 +196,7 @@ __global__ void __launch_bounds__(HS_THREADS) hs_dedup_kernel(const uint64_t* __
 #pragma unroll
             for (int i = 0; i < HS_CHUNK / HS_THREADS; ++i) {
                 const int64_t j = s + i * HS_THREADS + tid;
-                if (j < e && (!has_prev || (kb[i] & mask) != b_prev)) hs_insert(tab, twice, kb[i], slot_shift, L);
+                if (j < e && (!has_prev || (kb[i] & mask) != b_prev)) hs_insert<MASK>(tab, twice, kb[i], slot_shift, L, R);
             }
         }
         // the chunk's last bucket, if it began inside the chunk, is ours to its end. The first HS_SPEC rounds past the chunk
@@ -204,7 +210,7 @@ __global__ void __launch_bounds__(HS_THREADS) hs_dedup_kernel(const uint64_t* __
             }
 #pragma unroll
             for (int r = 0; r < HS_SPEC; ++r)
-                if ((kk[r] & mask) == b_last) hs_insert(tab, twice, kk[r], slot_shift, L);
+                if ((kk[r] & mask) == b_last) hs_insert<MASK>(tab, twice, kk[r], slot_shift, L, R);
             for (int r = HS_SPEC;; ++r) {
                 const int64_t jl = e + (int64_t)r * HS_THREADS - 1;  // (sorted: the last key of the round before decides for all)
                 if (jl >= n || (__ldg(H + jl) & mask) != b_last) break;
@@ -215,7 +221,7 @@ __global__ void __launch_bounds__(HS_THREADS) hs_dedup_kernel(const uint64_t* __
                 const int64_t j = e + (int64_t)r * HS_THREADS + tid;
                 if (j < n) {
                     const uint64_t k = __ldg(H + j);
-                    if ((k & mask) == b_last) hs_insert(tab, twice, k, slot_shift, L);
+                    if ((k & mask) == b_last) hs_insert<MASK>(tab, twice, k, slot_shift, L, R);
                 }
             }
         }
@@ -227,8 +233,9 @@ __global__ void __launch_bounds__(HS_THREADS) hs_dedup_kernel(const uint64_t* __
     flush_counter_block((unsigned long long)skew, &ctr->skew);
 }
 
-bool distinct64_sorted(Engine& e, const Column& c, int64_t n, Distinct64Result& r, int& launches) {
+bool distinct64_sorted(Engine& e, const Column& c, int64_t n, Distinct64Result& r, int& launches, const RepTab* R) {
     if (n <= 0 || n >= ((int64_t)1 << 30) || getenv("TG_HASH_NO_SORTED")) return false;
+    if (R) rep_reset(e, *R);
     int n_passes = n > ((int64_t)1 << 27) ? 3 : 2;
     if (const char* f = getenv("TG_HS_PASSES")) n_passes = atoi(f) == 3 ? 3 : n_passes;  // (tests reach the 24-bit bucket mode without 2^27 rows)
     const size_t keys_b = hs_round_up((size_t)n * 8, 256), tmp_b = hs_round_up(rs_temp_bytes(n, n_passes), 256);
@@ -254,18 +261,22 @@ bool distinct64_sorted(Engine& e, const Column& c, int64_t n, Distinct64Result& 
         uint32_t* no_vals[2] = {nullptr, nullptr};
         launches += rs_sort_pairs<uint32_t>(e.stream, bufs, no_vals, nv, 0, n_passes, false, T, e.sm_count, nullptr, true);
         const size_t smem = (size_t)HS_SLOTS * 8 + HS_SLOTS / 8;
-        TG_CUDA(cudaFuncSetAttribute(hs_dedup_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        auto* dedup = R ? hs_dedup_kernel<true> : hs_dedup_kernel<false>;
+        TG_CUDA(cudaFuncSetAttribute(dedup, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         const int64_t n_chunks = (nv + HS_CHUNK - 1) / HS_CHUNK;
         int per_sm = 1;
-        TG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, hs_dedup_kernel, HS_THREADS, smem));
+        TG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, dedup, HS_THREADS, smem));
         const int dgrid = (int)std::max<int64_t>(1, std::min<int64_t>(n_chunks, (int64_t)e.sm_count * std::max(per_sm, 1)));
-        hs_dedup_kernel<<<dgrid, HS_THREADS, smem, e.stream>>>(bufs[0], bufs[1], T.ctl, nv, ((uint64_t)1 << (8 * n_passes)) - 1, 8 * n_passes, d_ctr);
+        dedup<<<dgrid, HS_THREADS, smem, e.stream>>>(bufs[0], bufs[1], T.ctl, nv, ((uint64_t)1 << (8 * n_passes)) - 1, 8 * n_passes, d_ctr,
+                                                     R ? *R : RepTab{});
         TG_CUDA(cudaGetLastError());
         ++launches;
         TG_CUDA(cudaMemcpyAsync(&h, d_ctr, sizeof(h), cudaMemcpyDeviceToHost, e.stream));
         TG_CUDA(cudaStreamSynchronize(e.stream));
         if (h.overflow || h.skew) return false;
     }
+    // the key whose hash is the EMPTY word is counted apart (R holds keys: its key is an ordinary one there)
+    if (R && h.special > 1) rep_mark(e, *R, fmix64_inv(EMPTY64));
     r.distinct = h.distinct + (h.special ? 1 : 0);
     r.dup_keys = h.dup_keys + (h.special > 1 ? 1 : 0);
     r.nulls = h.nulls;

@@ -1088,6 +1088,26 @@ void plan_request_row_mask(Plan& p, int slot) {
     p.aggs[s.aggs[0]].row_bits = true;
 }
 
+const Slot& key_rows_slot(const Plan& p, int slot, int kind) {
+    if (slot < 0 || slot >= (int)p.slots.size()) throw Error(TG_ERR_INVALID_ARG, "slot index out of range");
+    const Slot& s = p.slots[slot];
+    if (s.kind != SL_UNIQ && s.kind != SL_FK)
+        throw Error(TG_ERR_UNSUPPORTED, "key-level row verdicts are not available for the '" + s.name + "' slot (uniqueness and foreign-key constraints only)");
+    const bool fits = s.kind == SL_UNIQ ? kind == TG_KEY_ROWS_DUPLICATE || kind == TG_KEY_ROWS_FIRST : kind == TG_KEY_ROWS_ORPHAN;
+    if (!fits)
+        throw Error(TG_ERR_INVALID_ARG, "key-level row verdict kind " + std::to_string(kind) + " does not apply to the '" + s.name +
+                                            "' slot (uniqueness: DUPLICATE or FIRST; foreign key: ORPHAN)");
+    return s;
+}
+
+void plan_request_key_rows(Plan& p, int slot, int kind) {
+    key_rows_slot(p, slot, kind);
+    Slot& s = p.slots[slot];
+    s.key_rows_requested |= (uint8_t)(1u << kind);
+    s.mask_built = false;
+    p.aggs[s.aggs[0]].key_rows |= (uint8_t)(1u << kind);
+}
+
 static void finalize_completeness(Plan& p, Slot& s) {
     // per-column evaluate_column (completeness.rs:137-246)
     struct ColRes {

@@ -31,6 +31,8 @@ enum AggKind : int32_t {
     A_HIST = 12,     // equal-width histogram over [min, max] of the column's NUM aggregate: f0 min f1 max u0 is_i64 u7 pending (shards disagreed on the range) ; blob = bucket counts
 };
 
+struct RowMask;
+
 struct Agg {
     AggKind kind;
     std::string key;                 // de-duplication key
@@ -48,6 +50,10 @@ struct Agg {
     // rows to `bits` (device, held by execute_partial for the duration of one execute). Not part of the de-duplication key.
     bool row_bits = false;
     uint32_t* bits = nullptr;
+    // key-level row verdicts some slot requested (tg_plan_request_key_rows): bit k = tg_key_rows_kind k. The hash job of this
+    // aggregate builds key_mask[k] for the execute's rows; the slots take them over. Not part of the de-duplication key.
+    uint8_t key_rows = 0;
+    std::shared_ptr<RowMask> key_mask[3];
     // construction-time problem the reference only reports when the constraint is evaluated
     tg_status ctor_err = TG_OK;
     std::string ctor_err_msg;
@@ -69,6 +75,7 @@ struct Agg {
         err = ctor_err;
         err_msg = ctor_err_msg;
         narrow = 0;
+        for (auto& m : key_mask) m.reset();
     }
 };
 
@@ -155,8 +162,12 @@ struct Slot {
     std::string metric_key;
     std::vector<std::pair<std::string, double>> map;
     // row verdicts: requested before execute; the mask (or the reason there is none) of the last execute since the request
+    // key-level row verdicts (uniqueness and foreign-key slots): bit k of key_rows_requested = tg_key_rows_kind k; they share
+    // mask_built / mask_err with the row mask, which these slots never have
     bool mask_requested = false, mask_built = false;
     std::shared_ptr<RowMask> mask;
+    uint8_t key_rows_requested = 0;
+    std::shared_ptr<RowMask> key_rows[3];
     tg_status mask_err = TG_OK;
     std::string mask_err_msg;
 };
@@ -209,6 +220,11 @@ int plan_add_quantile(Plan& p, const std::string& col, int mode, const std::vect
 int plan_add_value_histogram(Plan& p, const std::string& col);
 // marks a slot's row verdicts for the next execute (TG_ERR_UNSUPPORTED for a kind without them, TG_ERR_INVALID_ARG out of range)
 void plan_request_row_mask(Plan& p, int slot);
+// marks one kind of a uniqueness / foreign-key slot's key-level row verdicts for the next execute (TG_ERR_UNSUPPORTED for other
+// slot kinds, TG_ERR_INVALID_ARG for a kind the slot has not or an index out of range)
+void plan_request_key_rows(Plan& p, int slot, int kind);
+// the slot a key-level verdict of `kind` can be exported from (the same errors as plan_request_key_rows)
+const Slot& key_rows_slot(const Plan& p, int slot, int kind);
 int plan_add_grouped_completeness(Plan& p, const std::string& col, const std::vector<std::string>& groups,
                                   int max_groups, int include_overall);
 
